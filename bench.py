@@ -7,6 +7,7 @@ vehicles, reference-derived default candidate set, 25-cycle scripted episodes.  
 Decision+Planning cycle for every scene of the batch (the Decision and the Planning launch of dp_cycle_kernel, overlapped).
 
   python bench.py [--gpus N] [--steps K] [--warmup W]          our CUDA path (one rank per GPU)
+  python bench.py [...] --dump-outputs DIR                     ... and the plan records of its last timed step, as .npy files
   python bench.py --impl reference [...]                       the reference's own CPU code (oracle/_ref)
 
 Prints ONE JSON line (rank 0).  See DESIGN.md section 6 for how each number is obtained.
@@ -124,7 +125,7 @@ def run_reference(args, rank, world):
     for _ in range(max(1, min(args.warmup, 2))):
         arm.step()
     traj = 0; secs = 0.0; cyc = 0
-    steps = max(1, min(args.steps, 20))
+    steps = args.steps
     for _ in range(steps):
         t, dt, c = arm.step()
         traj += t; secs += dt; cyc += c
@@ -341,6 +342,13 @@ def run_ours(args, rank, world, local_rank):
         for r in range(world):
             assert float(g[r].sum(dtype=torch.int64).item()) == float(allchk[r].item()), "gathered slice of rank %d differs" % r
         planner.set_record_mirrors([])
+    dump = None
+    if args.dump_outputs:                                    # copied now: the loops below write into d_recs again
+        mine = d_recs[(W + K - 1) % 3]
+        parts = [torch.empty_like(mine) for _ in range(world)] if world > 1 else [mine]
+        if world > 1:
+            dist.all_gather(parts, mine)
+        dump = np.concatenate([t.cpu().numpy() for t in parts]).view(abi.plan_record).reshape(-1)
     launches = planner.launch_count() - l0 - sum(1 for i in range(W, W + K) if i % EPISODE == 0)
     kern_ms = np.array([ev[i][0].elapsed_time(ev[i][1]) for i in range(W, W + K)])
     step_ms = np.array([ev[i][0].elapsed_time(ev[i][2]) for i in range(W, W + K)])
@@ -610,9 +618,27 @@ def run_ours(args, rank, world, local_rank):
         except Exception as e:  # noqa: BLE001
             line["cpu_baseline"] = {"value": None, "unit": UNIT, "cores": 0, "kind": "port", "sample": "failed: %r" % (e,)}
     emit(line)
+    if dump is not None:
+        dump_records(args.dump_outputs, dump)
     planner.close()
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_MAX_BYTES = 64 * 10 ** 6
+
+
+def dump_records(path, rec):
+    """one float64 array per plan-record field, plus `scene`: the global scene index (= seed) of each row.  When all
+    scenes would pass DUMP_MAX_BYTES, a fixed seeded sample of them, the same for every build of the project."""
+    os.makedirs(path, exist_ok=True)
+    names = ("scene",) + rec.dtype.names
+    cap = DUMP_MAX_BYTES // (8 * len(names)) - 16             # (16 x 8 bytes: the .npy header of each file)
+    idx = np.arange(rec.size) if rec.size <= cap else np.sort(np.random.default_rng(0).choice(rec.size, cap, replace=False))
+    for f in names:
+        a = idx if f == "scene" else rec[f][idx]
+        np.save(os.path.join(path, f + ".npy"), a.astype(np.float64))
+    print("plan records of the last timed step: %d of %d scenes written to %s" % (idx.size, rec.size, path), file=sys.stderr)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -1081,7 +1107,13 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the latency histogram and the config 3 / 4 / 5 keys")
     ap.add_argument("--scenes", type=int, default=SCENES,
                     help="scenes per GPU (default = BASELINE config 2; 131072 x 8 GPUs = config 4, the 1M-scene sweep)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the plan records of the last one (every rank's) as DIR/<field>.npy, float64")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the CUDA path computed: use it with --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -12,7 +12,7 @@ from conftest import ROOT
 pytestmark = pytest.mark.gpu
 
 
-def test_cpp_facade_matches_oracle(oracle, the_map):
+def test_cpp_facade_matches_oracle(oracle, the_map, tmp_path):
     from dmpp_b200 import scenes
     n, cycles, n_obs = 96, 25, 10
     ep = scenes.Episodes(the_map, np.arange(60_000, 60_000 + n), cycles=cycles, n_obs=n_obs)
@@ -22,7 +22,7 @@ def test_cpp_facade_matches_oracle(oracle, the_map):
     v, wl, wg = scenes.v2x_events(the_map, H[0], seed=5)
     f0, f1 = oracle.v2x_event(H[0], v, wl, wg, 0), oracle.v2x_event(H[0], v, wl, wg, 1)
     m = the_map
-    exe = os.path.join(tempfile.gettempdir(), "dmpp_facade_main")
+    exe = str(tmp_path / "dmpp_facade_main")                 # (per-test directory: never a file another user left behind)
     pkg = os.path.join(ROOT, "decision-making-and-path-planning_b200")
     subprocess.check_call(["g++", "-std=c++17", "-O1", "-o", exe, os.path.join(ROOT, "tests", "cpp", "facade_main.cpp"),
                            "-L" + pkg, "-ldmpp_b200", "-Wl,-rpath," + pkg])

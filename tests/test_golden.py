@@ -9,6 +9,7 @@ import numpy as np
 import pytest
 
 from conftest import ROOT, assert_records_equal, same
+from test_oracle_vs_ref import CARRY
 
 sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
 from make_golden import episodes, sig  # noqa: E402
@@ -43,6 +44,7 @@ def test_oracle_matches_golden(path, oracle, the_map):
     assert (same(sig(a["path_ll"], 2), g["path_ll_sig"]) | ~clean).all()
     assert np.array_equal(a["n_calls"], g["n_calls"])
     assert np.array_equal(sig(a["calls"], 2), g["calls_sig"])
+    assert_records_equal(a["carry"], g["carry"], CARRY, what="final state")
     assert np.array_equal(sig(a["last_path"], 1), g["last_path_sig"])
 
 
@@ -60,4 +62,5 @@ def test_cuda_matches_golden(path, the_map):
     assert (np.abs(a["rec"]["path_dir_err"] - g["rec"]["path_dir_err"]) <= 1e-9)[clean].all()
     assert (same(sig(a["path_xy"], 2), g["path_sig"]) | ~clean).all()
     assert (same(sig(a["path_ll"], 2), g["path_ll_sig"]) | ~clean).all()
+    assert_records_equal(a["carry"], g["carry"], CARRY, what="final state")
     assert np.array_equal(sig(a["last_path"], 1), g["last_path_sig"])
