@@ -128,7 +128,7 @@ class Params(C.Structure):
 
 class WorldParams(C.Structure):
     _fields_ = [("a_max", C.c_double), ("loc_back", C.c_int32), ("loc_fwd", C.c_int32), ("end_margin", C.c_int32),
-                ("reserved", C.c_int32)]
+                ("pre_junction_pts", C.c_int32)]
 
 
 class MapDesc(C.Structure):

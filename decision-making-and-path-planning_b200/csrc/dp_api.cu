@@ -387,7 +387,8 @@ int dp_map_upload(dp_ctx* c, const dp_map_desc* m) {
     // every map table lives in ONE arena (256-byte aligned pieces), so that a single L2 access-policy window covers the map
     const size_t np = (size_t)m->n_points;
     const size_t arena_bytes = 16 * 256 + np * (8 * 3 + 16 * 2 + 8 * 2 + 8 + 4 * 2 + 2 * 2) + (size_t)m->n_lanes * (4 * 3 + 8 + 4) +
-                               (size_t)(m->n_roads + m->n_lanes + 2) * 4 + (size_t)m->n_conn * sizeof(dp_connector) + 32 * 256;
+                               (size_t)(m->n_roads + m->n_lanes + 2) * 4 + (size_t)m->n_conn * sizeof(dp_connector) + (size_t)m->n_lanes * 4 +
+                               33 * 256;
     char* arena = nullptr;
     {
         cudaError_t e = cudaMalloc((void**)&arena, arena_bytes);
@@ -410,6 +411,23 @@ int dp_map_upload(dp_ctx* c, const dp_map_desc* m) {
             return fail(DP_ERR_ARG, "dp_map_upload: lane too wide for DP_MAX_SWEEP avoid candidates per side");
     for (int i = 0; i < m->n_lanes; ++i)
         if (m->lane_pt_off[i + 1] - m->lane_pt_off[i] > 65535) return fail(DP_ERR_ARG, "dp_map_upload: lane longer than 65535 points");
+    // successor of every lane (the world step's agents follow it through junctions): a road lane -> the lane of the lowest
+    // connector leaving it, a connector's pseudo-lane -> lane_index(next_road, next_lane); -1 none
+    const int n_road_lanes = m->road_lane_base[m->n_roads];
+    auto lanes_of = [&](int r) { return m->road_lane_base[r] - m->road_lane_base[r - 1]; };
+    for (int k = 0; k < m->n_conn; ++k) {
+        const dp_connector& q = m->conn[k];
+        if (q.lane < n_road_lanes || q.lane >= m->n_lanes || q.last_road < 1 || q.last_road > m->n_roads || q.next_road < 1 ||
+            q.next_road > m->n_roads || q.last_lane < 1 || q.last_lane > lanes_of(q.last_road) || q.next_lane < 1 ||
+            q.next_lane > lanes_of(q.next_road))
+            return fail(DP_ERR_ARG, "dp_map_upload: connector names no road lane / pseudo-lane of the map");
+    }
+    std::vector<int32_t> lane_next(m->n_lanes, -1);
+    for (int r = 1; r <= m->n_roads; ++r)
+        for (int gl = m->road_lane_base[r - 1]; gl < m->road_lane_base[r]; ++gl)
+            for (int k = 0; k < m->n_conn; ++k)
+                if (m->conn[k].last_road == r && m->conn[k].last_lane == gl - m->road_lane_base[r - 1] + 1) { lane_next[gl] = m->conn[k].lane; break; }
+    for (int k = 0; k < m->n_conn; ++k) lane_next[m->conn[k].lane] = m->road_lane_base[m->conn[k].next_road - 1] + m->conn[k].next_lane - 1;
     DgMap d;
     int r;
     double* d_lenf = nullptr; float* d_hmax = nullptr; float* d_dnmax = nullptr; float* d_hmin = nullptr;
@@ -433,6 +451,7 @@ int dp_map_upload(dp_ctx* c, const dp_map_desc* m) {
     if ((r = up(m->road_lane_base, (size_t)(m->n_roads + 1) * 4, (void**)&d.road_lane_base))) return r;
     if ((r = up(m->lane_pt_off, (size_t)(m->n_lanes + 1) * 4, (void**)&d.lane_pt_off))) return r;
     if ((r = up(m->conn, (size_t)m->n_conn * sizeof(dp_connector), (void**)&d.conn))) return r;
+    if ((r = up(lane_next.data(), (size_t)m->n_lanes * 4, (void**)&d.lane_next))) return r;
     d.n_roads = m->n_roads; d.n_lanes = m->n_lanes; d.n_conn = m->n_conn;
     CK(dp_launch_map_prep(d.x, d.y, d.attr, d.lane_pt_off, d.n_lanes, (double2*)d.xy, (double2*)d.nrm, (double*)d.lenp, d_lenf, d_hmax, d_hmin,
                           d_dnmax, d_cump, d_cerr, d_re0, d_re1, c->st[0]));

@@ -79,6 +79,8 @@ struct DgMap {
     const uint16_t* width; const uint16_t* attr;
     const int32_t* road_lane_base; const int32_t* lane_pt_off;
     const dp_connector* conn;
+    const int32_t* lane_next;                      // per lane: successor lane (road lane -> lowest connector leaving it, connector ->
+                                                   // its next lane), -1 none; read by the world step with junctions on
     const float* lane_hmax;                        // per lane: upper bound of its segment lengths
     const float* lane_hmin;                        // per lane: lower bound of its segment lengths (0: duplicate points)
     const float* lane_dnmax;                       // per lane: upper bound of |nrm[i+1]-nrm[i]| over the segments of the lane

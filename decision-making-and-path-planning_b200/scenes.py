@@ -409,19 +409,35 @@ class Episodes:
 
 class World:
     """Initial worlds for the closed-loop episode runner (include/dmpp_b200.h section 9): the scene drawn by
-    `Episodes(kind='highway')` at cycle 0 -- ego pose, speed, navigation slice -- plus one `dp_agent` per obstacle (lane, map
+    `Episodes(kind=kind)` at cycle 0 -- ego pose, speed, navigation slice -- plus one `dp_agent` per obstacle (lane, map
     index, offset into the segment, speed, lateral offset).  From there on nothing is scripted: the library advances ego,
-    agents and localisation itself.  The cycle period is a whole number of milliseconds per scene, fixed over the episode."""
+    agents and localisation itself.  The cycle period is a whole number of milliseconds per scene, fixed over the episode.
+    kind 'junction' / 'urban': the agents sit on the approach lane, the connector or the departure lane by arclength, as
+    `Episodes.obstacles` spreads them; the ego crosses the junction only with dp_world_params.pre_junction_pts > 0
+    (`PRE_JUNCTION_PTS[kind]` matches the scripted episodes)."""
+    PRE_JUNCTION_PTS = {"highway": 0, "junction": 60, "urban": 400}
 
-    def __init__(self, m: Map, seeds, n_obs=10, roads=None):
-        ep = Episodes(m, seeds, n_obs=n_obs, kind="highway", cycles=1, roads=roads)
-        self.m, self.n, self.n_obs = m, ep.n, int(n_obs)
+    def __init__(self, m: Map, seeds, n_obs=10, roads=None, kind="highway"):
+        ep = Episodes(m, seeds, n_obs=n_obs, kind=kind, cycles=1, roads=roads)
+        self.m, self.n, self.n_obs, self.kind = m, ep.n, int(n_obs), kind
         self.hdr = ep.hdr(0)
         self.hdr["period_ms"] = ep.period_ticks(0).astype(np.float64)
         a = np.zeros((self.n, self.n_obs), abi.agent)
-        gl = m.road_lane_base[ep.road - 1].astype(np.int64)[:, None] + ep.ob_lane - 1
+        s = ep.ob_s0
+        if kind == "highway":
+            gl = m.road_lane_base[ep.road - 1].astype(np.int64)[:, None] + ep.ob_lane - 1
+        else:
+            app_len = 399 * SPACING
+            gl6 = m.road_lane_base[5].astype(np.int64) + ep.ob_lane - 1
+            gl7 = m.road_lane_base[6].astype(np.int64) + ep.ob_lane - 1
+            gc = m.conn["lane"][ep.ob_lane - 1].astype(np.int64)
+            clen = (m.lane_pt_off[gc + 1] - m.lane_pt_off[gc] - 1) * SPACING
+            in_app = s < app_len
+            in_con = (~in_app) & (s < app_len + clen)
+            gl = np.where(in_app, gl6, np.where(in_con, gc, gl7))
+            s = np.where(in_app, s, np.where(in_con, s - app_len, s - app_len - clen))
         cnt = (m.lane_pt_off[gl + 1] - m.lane_pt_off[gl]).astype(np.int64)
-        f = np.clip(ep.ob_s0 / SPACING, 0.0, cnt - 2.0)
+        f = np.clip(s / SPACING, 0.0, cnt - 2.0)
         i = np.floor(f).astype(np.int64)
         a["lane"] = gl
         a["i"] = i

@@ -161,7 +161,8 @@ int dp_create(dp_ctx** out, int device, const dp_params* params, int max_scenes,
 int dp_destroy(dp_ctx* ctx);
 
 /* (2) map upload: replaces the app-owned tables read at Decision.cpp:562-666, Planning.cpp:331-374.
- * Precomputes per-point segment length and unit normal on the device. */
+ * Precomputes per-point segment length and unit normal on the device, and the successor of every lane (section 9).  A connector
+ * whose roads / lanes are not in the map, or whose `lane` is not a pseudo-lane (index >= road_lane_base[n_roads]), is DP_ERR_ARG. */
 int dp_map_upload(dp_ctx* ctx, const dp_map_desc* map);
 
 /* reset the carry of scenes [first, first+count) to the constructor state
@@ -392,18 +393,39 @@ int dp_pack_frames(dp_ctx* ctx, int first_scene, int n_scenes, const dp_plan_rec
  * counters Decision.cpp:915-917, carried path Planning.cpp:6, his_behavior / count Planning.cpp:216-223) never leaves HBM, and
  * a whole episode is ONE CUDA graph launch.  The reference has no vehicle or traffic model (localisation, perception and
  * control are other modules of its application); the world step below is this library's, its arithmetic is frozen in
- * oracle/world_spec.h and the parity of this part is oracle-only by construction.  Segment driving (pos 0) only.
+ * oracle/world_spec.h (junction transitions: tools/junction_oracle/world_junction.h) and the parity of this part is oracle-only by
+ * construction.  Segment driving (pos 0) always; junctions
+ * (pos 0 -> 1 -> 2 -> 0 through a connector) when dp_world_params.pre_junction_pts > 0.
  *
  * world step of one scene, given the record of the cycle that just ran (rec == NULL: place the agents and localise only):
  *   ego    target speed = rec.brakespeed [m/s, the unit of the planner's constants 3 / 10, Planning.cpp:888-990] * 3.6 km/h,
  *          approached with |dv| <= a_max * dt; distance = mean speed * dt, walked along the carried local path from
  *          rec.path_near_id (perfect tracking); heading = CalcGlobalDir of the segment it lands on; an ego whose lane index
- *          is within end_margin points of the lane end stops;
+ *          is within end_margin points of the lane end stops (with junctions on: only in pos 0 with no connector ahead);
  *   agents agent k moves v[k] * dt along its lane (index i, offset u into segment i -> i+1), keeps its lateral offset `lat`
- *          (LEFT positive) and stops at the lane end; its obstacle point is written to obs_x / obs_y;
+ *          (LEFT positive) and stops at the lane end (with junctions on: continues on the lane's successor, see below); its
+ *          obstacle point is written to obs_x / obs_y;
  *   localisation  hdr.id[l] = nearest point of lane l of the ego's road within [id[l] - loc_back, id[l] + loc_fwd]
  *          (squared distance, strict '<'), hdr.lane_num = the lane with the smallest such distance (lowest lane on ties),
- *          hdr.x / y / dir / velocity = the new ego state; everything else in the header is left as it is. */
+ *          hdr.x / y / dir / velocity = the new ego state; everything else in the header is left as it is.
+ *
+ * junction transitions (pre_junction_pts = J > 0; J = 0 is the step above, bit for bit).  The ego's connector is the lowest c
+ * with conn[c].(last_road, next_road, last_lane) = (road_num, next_roadnum, lane_num) and next_roadnum != road_num.  Nearest
+ * points are searched as in the localisation (squared distance, strict '<', lowest index on ties); a pos other than 1 / 2 is 0.
+ *   pos 0  localisation as above; then, when the ego has a connector c and id[lane_num-1] >= (points of its lane) - 1 - J:
+ *          pos = 1, conn = c, last_roadnum = road_num, last_lanenum = lane_num, next_lanenum = conn[c].next_lane
+ *          (also in the placement step);
+ *   pos 1  localisation as above, then conn / last_roadnum / last_lanenum / next_lanenum re-picked from lane_num (no connector
+ *          for that lane: back to pos 0, conn = -1); the connector is searched in [0, loc_fwd]; when its nearest point is
+ *          strictly nearer than the nearest approach point: pos = 2, road_num = next_roadnum, lane_num = next_lanenum and
+ *          id[l] = that connector index for every lane l of the approach road (Decision reads id[last_lanenum-1]);
+ *   pos 2  the connector is searched in [id[last_lanenum-1] - loc_back, id[last_lanenum-1] + loc_fwd], every lane of the
+ *          departure road (road_num) in [0, loc_fwd]; when the departure road's nearest point is strictly nearer than the
+ *          connector's: pos = 0, conn = -1, path_num + 1, stub_attribute = 0, id[] / lane_num from the departure road; otherwise
+ *          id[l] = the connector index as in pos 1.  An invalid conn or last_lanenum counts as a connector infinitely far away.
+ *   agents an agent that walks past the end of a lane with a successor (lane_next, built by dp_map_upload: road lane -> the
+ *          lowest connector leaving it, connector -> its next lane) continues on the successor from i = 0 with the leftover u
+ *          (the gap between a lane end and its successor's start is jumped, not walked); at most 8 lanes per step. */
 typedef struct dp_agent {
     double u;                        /* metres into segment i -> i+1 */
     double v;                        /* m/s along the lane */
@@ -415,7 +437,8 @@ typedef struct dp_world_params {
     double a_max;                    /* m/s^2, default 3.0 (the planner's own braking command, Planning.cpp des_acc = -3) */
     int32_t loc_back, loc_fwd;       /* localisation window in map points, default 8 / 56 */
     int32_t end_margin;              /* default 160: the front region (120 points + ID_MORE) stays inside the lane */
-    int32_t reserved;
+    int32_t pre_junction_pts;        /* default 0 = junction transitions off; > 0: length of the pre-junction zone in map points
+                                        (60 = the 30 m of Episodes(kind="junction"), >= 400 = kind="urban") */
 } dp_world_params;
 void dp_world_default_params(dp_world_params* p);
 int dp_world_set_params(dp_ctx* ctx, const dp_world_params* p);

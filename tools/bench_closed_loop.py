@@ -1,8 +1,11 @@
 """closed-loop episodes (dp_run_closed_loop_dev: ONE graph launch per episode) against the same launches enqueued one by one,
-for a full batch and for a single scene (where the launch latency is the cycle), and the output-frame kernel against the HBM
-copy peak.  CUDA events on the launching stream; prints one JSON line."""
+for a full batch and for a single scene (where the launch latency is the cycle), 4096 junction worlds x 120 cycles through the
+connector (dp_world_params.pre_junction_pts = 60), the world step alone (highway against junction worlds), and the output-frame
+kernel against the HBM copy peak.  CUDA events on the launching stream; prints one JSON line with the card's name and power
+limit read in the same run."""
 import json
 import os
+import subprocess
 import sys
 import time
 
@@ -30,10 +33,16 @@ def u8(a):
     return torch.from_numpy(np.ascontiguousarray(a).view(np.uint8).reshape(-1)).to(dev)
 
 
-def episode(n, graph):
-    os.environ["DP_EPISODE_GRAPH"] = "1" if graph else "0"
+def planner(n, kind):
     p = Planner(n, 10); p.upload_map(m)
-    w = scenes.World(m, np.arange(n), 10)
+    wp = p.world_params(); wp.pre_junction_pts = scenes.World.PRE_JUNCTION_PTS[kind]
+    p.set_world_params(wp)
+    return p, scenes.World(m, np.arange(n), 10, kind=kind)
+
+
+def episode(n, graph, kind="highway", cycles=cycles):
+    os.environ["DP_EPISODE_GRAPH"] = "1" if graph else "0"
+    p, w = planner(n, kind)
     h0, a0 = u8(w.hdr), u8(w.agents)
     d_h, d_a = torch.empty_like(h0), torch.empty_like(a0)
     d_x = torch.zeros((n, 10), dtype=torch.float64, device=dev); d_y = torch.zeros_like(d_x)
@@ -56,8 +65,45 @@ def episode(n, graph):
     out = {"ms_per_episode": best, "us_per_cycle": best / cycles * 1e3, "wall_us_per_cycle": bw / cycles * 1e3,
            "plan_cycles_per_s": n * cycles / (best * 1e-3), "trajectories_per_s": float(rec["n_traj"].sum()) / (best * 1e-3),
            "launches_per_episode": 3 * cycles + 1}
+    if kind != "highway":
+        hdr = np.frombuffer(d_h.cpu().numpy().tobytes(), abi.scene_hdr)
+        out["share_through_junction"] = float((hdr["path_num"] == 1).mean())
     p.close()
     return out, rec
+
+
+def world_step(n, kind, launches=50):
+    """dp_world_step_dev alone on the world and records left by a 20-cycle episode; the world is restored before every timed
+    window of `launches` back-to-back steps (the steps move it in place)"""
+    os.environ["DP_EPISODE_GRAPH"] = "1"
+    p, w = planner(n, kind)
+    d_h, d_a = u8(w.hdr), u8(w.agents)
+    d_x = torch.zeros((n, 10), dtype=torch.float64, device=dev); d_y = torch.zeros_like(d_x)
+    d_r = torch.zeros((20, n, 128), dtype=torch.uint8, device=dev)
+    st = torch.cuda.current_stream()
+    p.reset_dev(0, n, stream=st.cuda_stream)
+    p.run_closed_loop_dev(n, 20, d_h.data_ptr(), d_a.data_ptr(), d_x.data_ptr(), d_y.data_ptr(), d_r.data_ptr(), stream=st.cuda_stream)
+    torch.cuda.synchronize()
+    h0, a0 = d_h.clone(), d_a.clone()
+    rec = d_r[-1].contiguous()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    us = []
+    for r in range(reps):
+        d_h.copy_(h0); d_a.copy_(a0)
+        e0.record(st)
+        for _ in range(launches):
+            p.world_step_dev(n, d_h.data_ptr(), d_a.data_ptr(), d_x.data_ptr(), d_y.data_ptr(), rec.data_ptr(), stream=st.cuda_stream)
+        e1.record(st); torch.cuda.synchronize()
+        us.append(e0.elapsed_time(e1) * 1e3 / launches)
+    p.close()
+    return {"scenes": n, "kind": kind, "us_per_step": float(np.median(us[3:])), "us_min": float(np.min(us[3:])),
+            "us_max": float(np.max(us[3:])), "launches_per_window": launches, "windows": reps - 3}
+
+
+def card():
+    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader", "-i", "0"],
+                       capture_output=True, text=True)
+    return {"torch_name": torch.cuda.get_device_name(0), "nvidia_smi": q.stdout.strip()}
 
 
 def frames(n):
@@ -86,11 +132,16 @@ def frames(n):
             "hbm_peak_gb_per_s": hbm_peak, "l2": "256 MiB written before every launch"}
 
 
-out = {"cycles": cycles}
+out = {"cycles": cycles, "card": card()}
 for n in (4096, 1):
     g, rg = episode(n, True)
     d, rd = episode(n, False)
     assert rg.tobytes() == rd.tobytes(), "graph and direct launches disagree"
     out["scenes_%d" % n] = {"graph": g, "direct": d}
+jg, rjg = episode(4096, True, "junction", 120)
+jd, rjd = episode(4096, False, "junction", 120)
+assert rjg.tobytes() == rjd.tobytes(), "junction: graph and direct launches disagree"
+out["junction_4096x120"] = {"graph": jg, "direct": jd}
+out["world_step_4096"] = [world_step(4096, k) for k in ("highway", "junction", "highway", "junction")]   # alternated
 out["frames"] = [frames(4096), frames(131072)]
 print(json.dumps(out))

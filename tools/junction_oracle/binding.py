@@ -1,0 +1,68 @@
+"""tools/junction_oracle/binding.py -- TEST INFRASTRUCTURE: ctypes loaders of the junction world-step oracle
+(libjunction_oracle.so) and of the unmodified reference's closed loop with that step (libref_junction.so, where the reference
+was built).  Same dictionaries as oracle.binding's run_closed_loop.  Imported by tests/ only."""
+import ctypes as C
+import os
+import subprocess
+import sys
+
+import numpy as np
+
+_here = os.path.dirname(os.path.abspath(__file__))
+_root = os.path.dirname(os.path.dirname(_here))
+if _root not in sys.path:
+    sys.path.insert(0, _root)
+import dmpp_b200  # noqa: E402,F401
+from dmpp_b200 import abi  # noqa: E402
+from oracle import binding as ob  # noqa: E402
+
+
+def build():
+    subprocess.check_call(["make", "-s", "-C", _here, "all"])
+
+
+class JunctionOracle:
+    def __init__(self):
+        build()
+        self.lib = C.CDLL(os.path.join(_here, "libjunction_oracle.so"), mode=os.RTLD_NOW)
+        self._base = ob.Oracle()
+        self.params = self._base.params
+
+    def set_map(self, m):
+        self._keep = m
+        self._desc = m.desc()
+        assert self.lib.jo_set_map(C.byref(self._desc)) == 0
+        self._n_lanes = m.n_lanes
+
+    def world_params(self):
+        return self._base.world_params()
+
+    def lane_next(self):
+        out = np.zeros(self._n_lanes, np.int32)
+        assert self.lib.jo_lane_next(abi.ptr(out)) == 0
+        return out
+
+    def world_step(self, hdr, agents, ox, oy, rec=None, last_path=None, wp=None):
+        """in place; rec None: place the agents and localise only"""
+        wp = wp or self.world_params()
+        n, max_obs = ox.shape
+        assert self.lib.jo_world_step(C.byref(self.params), C.byref(wp), C.c_int(n), C.c_int(max_obs), abi.ptr(hdr), abi.ptr(agents),
+                                      abi.ptr(ox), abi.ptr(oy), abi.ptr(rec), abi.ptr(last_path)) == 0
+
+    def run_closed_loop(self, hdr, agents, cycles, wp=None, paths=False, threads=1):
+        """hdr[n], agents[n][max_obs] (copied; the final world is returned)"""
+        return ob._closed_loop(self.lib, "jo_run_closed_loop", self.params, wp or self.world_params(), hdr, agents, cycles, paths, threads)
+
+
+class JunctionReference:
+    """needs an oracle.binding.Reference whose map is set (the loop reads the reference's own map tables)"""
+
+    @staticmethod
+    def available():
+        return os.path.exists(os.path.join(_here, "libref_junction.so"))
+
+    def __init__(self):
+        self.lib = C.CDLL(os.path.join(_here, "libref_junction.so"), mode=os.RTLD_NOW)
+
+    def run_closed_loop(self, params, wp, hdr, agents, cycles, paths=False):
+        return ob._closed_loop(self.lib, "ref_run_closed_loop_junction", params, wp, hdr, agents, cycles, paths, None)
