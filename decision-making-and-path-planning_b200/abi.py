@@ -131,6 +131,26 @@ class WorldParams(C.Structure):
                 ("pre_junction_pts", C.c_int32)]
 
 
+episode_metrics = np.dtype(
+    [
+        ("distance", "<f8"), ("min_clearance", "<f8"), ("min_lead_gap", "<f8"), ("min_ttc", "<f8"),
+        ("max_accel", "<f8"), ("min_accel", "<f8"), ("max_abs_jerk", "<f8"), ("last_accel", "<f8"),
+        ("max_abs_lat_err", "<f8"), ("max_abs_dir_err", "<f8"),
+        ("steps", "<i4"), ("first_collision_step", "<i4"), ("first_collision_agent", "<i4"),
+        ("collision_steps", "<i4"), ("collision_steps_front", "<i4"), ("collision_steps_rear", "<i4"), ("ttc_warn_steps", "<i4"),
+        ("stopped_steps", "<i4"), ("end_stop_steps", "<i4"), ("replans", "<i4"), ("aeb_steps", "<i4"),
+        ("accel_steps", "<i4"), ("last_behavior", "<i4"), ("behavior_switches", "<i4"),
+        ("behavior_steps", "<u4", (8,)), ("pad", "<u4", (6,)),
+    ]
+)
+assert episode_metrics.itemsize == 192
+
+
+class MetricsParams(C.Structure):
+    _fields_ = [("front", C.c_double), ("rear", C.c_double), ("half_width", C.c_double), ("corridor_half", C.c_double),
+                ("ttc_warn", C.c_double)]
+
+
 class MapDesc(C.Structure):
     _fields_ = [
         ("n_roads", C.c_int32), ("road_lane_base", C.c_void_p),

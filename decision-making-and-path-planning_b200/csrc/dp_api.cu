@@ -4,6 +4,7 @@
 // that chunks of a large batch overlap H2D / kernel / D2H.  No CPU compute path exists here:
 // every entry point either launches the CUDA kernels or returns an error.
 #include <cuda_runtime.h>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -62,6 +63,8 @@ struct dp_ctx {
     long long launches = 0;
     // closed-loop episodes (dp_run_closed_loop_dev): world-step parameters, the capture stream, the cached episode graph and its key
     dp_world_params wp;
+    dp_metrics_params mp;                                   // episode metrics (dp_world_set_metrics): d_met == nullptr disarmed
+    dp_episode_metrics* d_met = nullptr;
     cudaStream_t ep_stream = nullptr;
     cudaGraphExec_t ep_exec = nullptr;
     const void* ep_key[8] = {}; int ep_dims[3] = {-1, -1, -1};
@@ -304,6 +307,7 @@ int dp_create(dp_ctx** out, int device, const dp_params* params, int max_scenes,
     if (const char* e = getenv("DP_ZERO_COPY")) c->zero_copy = atoi(e) != 0;
     if (const char* e = getenv("DP_EPISODE_GRAPH")) c->ep_graph = atoi(e) != 0;
     dp_world_default_params(&c->wp);
+    dp_metrics_default_params(&c->mp);
     // Kernel choice, from the measurements in profiles/README.md (round 2): the warp-per-scene kernel wins while a scene's
     // obstacles fit one warp pass (N < 32: 71 vs 96 us per 4096-scene cycle at N = 10); the group kernel, whose scans are flat
     // (trajectory, obstacle) lists with exact pruning, wins for crowded scenes (N = 200: 135 vs 212 us per 1024 junction scenes).
@@ -1404,6 +1408,24 @@ int dp_world_set_params(dp_ctx* c, const dp_world_params* p) {
     if (c->ep_exec) { cudaGraphExecDestroy(c->ep_exec); c->ep_exec = nullptr; }   // (the parameters are baked into the graph's launches)
     return DP_OK;
 }
+void dp_metrics_default_params(dp_metrics_params* p) {
+    if (!p) return;
+    memset(p, 0, sizeof(*p));
+    p->front = 4.0; p->rear = 1.0; p->half_width = 0.9; p->corridor_half = 1.1; p->ttc_warn = 2.0;
+}
+int dp_world_set_metrics(dp_ctx* c, const dp_metrics_params* p, dp_episode_metrics* m) {
+    if (!c || (m && !p)) return fail(DP_ERR_ARG, "dp_world_set_metrics: bad argument");
+    if (p) {
+        const double v[5] = {p->front, p->rear, p->half_width, p->corridor_half, p->ttc_warn};
+        for (double x : v) if (!std::isfinite(x)) return fail(DP_ERR_ARG, "dp_world_set_metrics: parameters must be finite");
+        if (!(p->front >= 0) || !(p->rear >= 0) || !(p->half_width > 0) || !(p->corridor_half >= 0) || !(p->ttc_warn >= 0))
+            return fail(DP_ERR_ARG, "dp_world_set_metrics: front, rear, corridor_half, ttc_warn >= 0 and half_width > 0");
+        if (m) c->mp = *p;
+    }
+    c->d_met = m;
+    if (c->ep_exec) { cudaGraphExecDestroy(c->ep_exec); c->ep_exec = nullptr; }   // (the row pointer and parameters are baked into the graph)
+    return DP_OK;
+}
 int dp_world_step_dev(dp_ctx* c, int first, int n, dp_scene_hdr* hdr, dp_agent* agents, double* ox, double* oy, const dp_plan_record* rec,
                       void* stream) {
     if (!c || !hdr || !agents || !ox || !oy || n < 0 || first < 0 || first + n > c->max_scenes)
@@ -1412,7 +1434,7 @@ int dp_world_step_dev(dp_ctx* c, int first, int n, dp_scene_hdr* hdr, dp_agent* 
     CK(cudaSetDevice(c->device));
     c->launches += n > 0 ? 1 : 0;
     CK(dp_launch_world(c->gmap, c->p, c->wp, n, c->max_obs, hdr, agents, ox, oy, rec, c->d_last + (size_t)first * DP_PATH_POINTS,
-                       (cudaStream_t)stream));
+                       c->mp, c->d_met, (cudaStream_t)stream));
     return DP_OK;
 }
 namespace {
@@ -1425,7 +1447,7 @@ cudaError_t enqueue_closed_loop(dp_ctx* c, int first, int n, int cycles, dp_scen
     // a replayed graph re-uses its hand-off epochs: the per-scene Decision -> Planning flags start every replay from 0
     if (rearm && (e = cudaMemsetAsync(c->d_done + first, 0, (size_t)n * sizeof(unsigned), st)) != cudaSuccess) return e;
     c->launches += 1;
-    if ((e = dp_launch_world(c->gmap, c->p, c->wp, n, c->max_obs, hdr, agents, ox, oy, nullptr, last, st)) != cudaSuccess) return e;
+    if ((e = dp_launch_world(c->gmap, c->p, c->wp, n, c->max_obs, hdr, agents, ox, oy, nullptr, last, c->mp, c->d_met, st)) != cudaSuccess) return e;
     for (int k = 0; k < cycles; ++k) {
         if (hdr_log && (e = cudaMemcpyAsync(hdr_log + (size_t)k * n, hdr, (size_t)n * sizeof(dp_scene_hdr), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
         if (olx && (e = cudaMemcpyAsync(olx + (size_t)k * n * mo, ox, (size_t)n * mo * sizeof(double), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
@@ -1433,7 +1455,8 @@ cudaError_t enqueue_closed_loop(dp_ctx* c, int first, int n, int cycles, dp_scen
         const DpIo io = make_io(c, first, nullptr);
         if ((e = run_cycle(c, first, n, hdr, ox, oy, rec + (size_t)k * n, nullptr, nullptr, nullptr, st, io)) != cudaSuccess) return e;
         c->launches += 1;
-        if ((e = dp_launch_world(c->gmap, c->p, c->wp, n, c->max_obs, hdr, agents, ox, oy, rec + (size_t)k * n, last, st)) != cudaSuccess) return e;
+        if ((e = dp_launch_world(c->gmap, c->p, c->wp, n, c->max_obs, hdr, agents, ox, oy, rec + (size_t)k * n, last, c->mp, c->d_met, st)) != cudaSuccess)
+            return e;
     }
     return cudaSuccess;
 }

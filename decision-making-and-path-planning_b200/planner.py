@@ -26,6 +26,7 @@ SYMBOLS = [
     "dp_set_tracks", "dp_set_tracks_dev", "dp_clear_tracks",
     "dp_pack_frames_dev", "dp_pack_frames", "dp_world_default_params", "dp_world_set_params", "dp_world_step_dev",
     "dp_run_closed_loop_dev", "dp_closed_loop_is_graph", "dp_v2x_event_batch", "dp_v2x_event_batch_dev", "dp_v2x_apply", "dp_v2x_apply_dev",
+    "dp_metrics_default_params", "dp_world_set_metrics",
     "dp_gather_create", "dp_gather_attach", "dp_gather_arm", "dp_gather_chain", "dp_gather_arm_deferred", "dp_gather_set_lag", "dp_gather_flush", "dp_gather_disarm", "dp_gather_wait", "dp_gather_buffer", "dp_gather_destroy",
 ]
 
@@ -52,6 +53,13 @@ class DpError(RuntimeError):
 def _ck(rc, what):
     if rc != 0:
         raise DpError("%s failed (%d): %s" % (what, rc, load().dp_last_error().decode()))
+
+
+def metrics_params():
+    """dp_metrics_default_params (no GPU needed)"""
+    p = abi.MetricsParams()
+    load().dp_metrics_default_params(C.byref(p))
+    return p
 
 
 def default_params():
@@ -208,6 +216,15 @@ class Planner:
     def set_world_params(self, wp):
         _ck(self.lib.dp_world_set_params(self.ctx, C.byref(wp)), "dp_world_set_params")
 
+    def metrics_params(self):
+        return metrics_params()
+
+    def set_metrics(self, params, d_metrics):
+        """arm the episode metrics (include/dmpp_b200.h section 11): d_metrics = device address of rows [n] indexed like hdr;
+        d_metrics None / 0 disarms"""
+        _ck(self.lib.dp_world_set_metrics(self.ctx, C.byref(params) if params is not None else None, C.c_void_p(d_metrics or 0)),
+            "dp_world_set_metrics")
+
     def world_step_dev(self, n, d_hdr, d_agents, d_ox, d_oy, d_rec=None, first=0, stream=0):
         _ck(self.lib.dp_world_step_dev(self.ctx, C.c_int(first), C.c_int(n), C.c_void_p(d_hdr), C.c_void_p(d_agents), C.c_void_p(d_ox),
                                        C.c_void_p(d_oy), C.c_void_p(d_rec or 0), C.c_void_p(stream)), "dp_world_step_dev")
@@ -222,13 +239,17 @@ class Planner:
     def closed_loop_is_graph(self):
         return bool(self.lib.dp_closed_loop_is_graph(self.ctx))
 
-    def run_closed_loop(self, hdr, agents, cycles, log=True, repeat=1):
+    def run_closed_loop(self, hdr, agents, cycles, log=True, repeat=1, metrics=None):
         """host arrays in, host arrays out (the same dictionary as oracle.binding's run_closed_loop); `repeat` > 1 replays the
-        episode from the same initial world (same device buffers, i.e. the cached graph) and returns the last run"""
+        episode from the same initial world (same device buffers, i.e. the cached graph) and returns the last run.
+        metrics: None, or MetricsParams: the episode metrics are armed for this call (and disarmed after it) and the rows are
+        returned under the key "metrics"."""
         n, mo = agents.shape
         assert mo == self.max_obs and hdr.shape == (n,)
         sizes = {"hdr": n * 128, "agents": n * mo * 32, "ox": n * mo * 8, "oy": n * mo * 8, "rec": cycles * n * 128,
                  "hdr_log": cycles * n * 128, "obs_log_x": cycles * n * mo * 8, "obs_log_y": cycles * n * mo * 8}
+        if metrics is not None:
+            sizes["metrics"] = n * abi.episode_metrics.itemsize
         d = {}
         try:
             for k, b in sizes.items():
@@ -236,6 +257,8 @@ class Planner:
                     p = C.c_void_p()
                     _ck(self.lib.dp_dev_alloc(self.ctx, C.byref(p), C.c_size_t(b)), "dp_dev_alloc")
                     d[k] = p.value
+            if metrics is not None:
+                self.set_metrics(metrics, d["metrics"])
             h0, a0 = np.ascontiguousarray(hdr), np.ascontiguousarray(agents)
             for _ in range(repeat):
                 self.reset(0, n)
@@ -249,6 +272,8 @@ class Planner:
                  "rec": np.zeros((cycles, n), abi.plan_record)}
             if log:
                 o.update(hdr_log=np.zeros((cycles, n), abi.scene_hdr), obs_log_x=np.zeros((cycles, n, mo)), obs_log_y=np.zeros((cycles, n, mo)))
+            if metrics is not None:
+                o["metrics"] = np.zeros(n, abi.episode_metrics)
             for k in o:
                 _ck(self.lib.dp_memcpy_d2h(self.ctx, abi.ptr(o[k]), C.c_void_p(d[k]), C.c_size_t(sizes[k]), None), "d2h")
             _ck(self.lib.dp_stream_sync(self.ctx, None), "sync")
@@ -256,6 +281,8 @@ class Planner:
             o["graph"] = self.closed_loop_is_graph()
             return o
         finally:
+            if metrics is not None:
+                self.set_metrics(None, None)
             for p in d.values():
                 self.lib.dp_dev_free(self.ctx, C.c_void_p(p))
 

@@ -495,6 +495,68 @@ int dp_v2x_event_batch_dev(dp_ctx* ctx, int n_scenes, const dp_scene_hdr* hdr, c
 int dp_v2x_apply(dp_ctx* ctx, int n_scenes, const dp_v2x_flags* flags, dp_plan_record* rec);
 int dp_v2x_apply_dev(dp_ctx* ctx, int n_scenes, const dp_v2x_flags* flags, dp_plan_record* rec, void* stream);
 
+/* (11) Closed-loop episode metrics: one row per world, accumulated by the world step of section 9 in the warp that has just
+ * moved the ego and the agents.  They only observe: no decision, record, world state or log changes with them, and with
+ * metrics disarmed (the default) nothing is written.  The arithmetic is frozen in tools/junction_oracle/episode_metrics.h.
+ *
+ * When a row is written:
+ *   placement step (rec == NULL, the first node of every episode): the row is initialised, also for a header that names no lane,
+ *          so a replayed episode graph starts every episode from a clean row;
+ *   every later step (rec != NULL) on a header that names a lane: the row is updated after the ego and the agents have moved (a
+ *          header that names no lane leaves its row alone, as it leaves its world alone).
+ * IEEE binary64, operations in the order written, no contraction; min / max updates are `if (x < m) m = x` / `if (x > m) m = x`.
+ * Per step: v, vn = ego speed before / after the step (km/h); dt = period_ms / 1000; (c, s) = spec_sincos_deg(new dir);
+ * ds = the step's distance (0 when the end_margin stop fired).  For every agent k < min(n_obs, max_obs), at its new obstacle
+ * point (ox, oy), on map segment (ddx, ddy) of length L:
+ *   dx = ox - x, dy = oy - y, lon = dx*c + dy*s, lat = dy*c - dx*s                      (ego frame, LEFT positive)
+ *   inside    -rear <= lon <= front  &&  -half_width <= lat <= half_width
+ *   clearance ex = lon > front ? lon - front : (lon < -rear ? -rear - lon : 0); ey = |lat| > half_width ? |lat| - half_width : 0;
+ *             d = sqrt(ex*ex + ey*ey)
+ *   lead      lon > front && |lat| <= corridor_half:  gap = lon - front,
+ *             va = L == 0 ? 0 : v_agent * (ddx/L*c + ddy/L*s),  closing = vn/3.6 - va,  ttc = closing > 0 ? gap/closing : +inf
+ * Fields (initial value):
+ *   distance                 sum of ds in step order (0)
+ *   min_clearance            min of d over steps and agents (+inf)
+ *   min_lead_gap, min_ttc    min of gap / ttc over steps and lead agents (+inf)
+ *   max_accel, min_accel     a = (vn - v) / 3.6 / dt, on steps with dt > 0 (-inf / +inf)
+ *   max_abs_jerk             |a - last_accel| / dt on every step with an a after the first one (0)
+ *   last_accel, accel_steps  the previous a (0) and the number of steps with an a (0)
+ *   max_abs_lat_err / _dir_err  max of |rec.path_lat_dis| / |rec.path_dir_err| (0)
+ *   steps                    steps accumulated (0)
+ *   first_collision_step     1-based step of the first step with an agent inside, and the lowest such agent (-1 / -1)
+ *   first_collision_agent
+ *   collision_steps          steps with an agent inside; _front: with one inside at lon >= 0; _rear: with one inside at lon < 0
+ *   collision_steps_front/_rear  (a step can count as both; agents do not react, so rear strikes are theirs)
+ *   ttc_warn_steps           steps whose smallest ttc is < ttc_warn
+ *   stopped_steps            steps with vn == 0;  end_stop_steps: steps on which the end_margin stop fired
+ *   replans, aeb_steps       sum of rec.afresh_planning / rec.acc_flag
+ *   behavior_steps[b]        steps with rec.behavior == b (b < 8)
+ *   last_behavior            rec.behavior of the previous step (-1)
+ *   behavior_switches        steps whose rec.behavior differs from the previous step's (the first step never counts) */
+typedef struct dp_metrics_params {
+    double front, rear;              /* ego box along its heading from the header's (x, y): default 4.0 (antenna to bumper,
+                                        Planning.cpp:896) and 1.0 (this library's choice) */
+    double half_width;               /* default 0.9 = Vehicle_Width / 2 */
+    double corridor_half;            /* lead corridor, default 1.1 (the local-path corridor, Planning.cpp:168) */
+    double ttc_warn;                 /* seconds, default 2.0 */
+} dp_metrics_params;
+typedef struct dp_episode_metrics {
+    double distance, min_clearance, min_lead_gap, min_ttc;
+    double max_accel, min_accel, max_abs_jerk, last_accel;
+    double max_abs_lat_err, max_abs_dir_err;
+    int32_t steps, first_collision_step, first_collision_agent;
+    int32_t collision_steps, collision_steps_front, collision_steps_rear, ttc_warn_steps;
+    int32_t stopped_steps, end_stop_steps, replans, aeb_steps;
+    int32_t accel_steps, last_behavior, behavior_switches;
+    uint32_t behavior_steps[8];
+    uint32_t pad[6];                 /* zero */
+} dp_episode_metrics;                /* 192 bytes */
+void dp_metrics_default_params(dp_metrics_params* p);
+/* m: device array indexed like hdr (the s-th scene of every later dp_world_step_dev / dp_run_closed_loop_dev call);
+ * m == NULL disarms (p may then be NULL).  p must be finite with front, rear, corridor_half, ttc_warn >= 0 and half_width > 0,
+ * else DP_ERR_ARG.  Context state like dp_world_set_params: the cached episode graph is rebuilt on its next call. */
+int dp_world_set_metrics(dp_ctx* ctx, const dp_metrics_params* p, dp_episode_metrics* m);
+
 /* diagnostic: phase time stamps (globaltimer, ns) of the most recent cycle launch, one row of 32 per CTA (row b = scenes
  * [b*g, (b+1)*g) of the batch; stamp 0 = CTA start, stamp i = end of phase i of csrc/dp_group.cuh).  Only contexts created
  * with DP_TIMELINE=1 in the environment record them; used by tools/group_timeline.py, never by the product path. */

@@ -49,9 +49,39 @@ class JunctionOracle:
         assert self.lib.jo_world_step(C.byref(self.params), C.byref(wp), C.c_int(n), C.c_int(max_obs), abi.ptr(hdr), abi.ptr(agents),
                                       abi.ptr(ox), abi.ptr(oy), abi.ptr(rec), abi.ptr(last_path)) == 0
 
-    def run_closed_loop(self, hdr, agents, cycles, wp=None, paths=False, threads=1):
-        """hdr[n], agents[n][max_obs] (copied; the final world is returned)"""
-        return ob._closed_loop(self.lib, "jo_run_closed_loop", self.params, wp or self.world_params(), hdr, agents, cycles, paths, threads)
+    def run_closed_loop(self, hdr, agents, cycles, wp=None, paths=False, threads=1, metrics=None):
+        """hdr[n], agents[n][max_obs] (copied; the final world is returned); metrics = MetricsParams: the episode metrics of every
+        world under "metrics" (jo_run_closed_loop_metrics)"""
+        wp = wp or self.world_params()
+        if metrics is None:
+            return ob._closed_loop(self.lib, "jo_run_closed_loop", self.params, wp, hdr, agents, cycles, paths, threads)
+        n = hdr.shape[0]
+        met = np.frombuffer(np.full(n * abi.episode_metrics.itemsize, 0xAB, np.uint8).tobytes(), abi.episode_metrics).copy()
+        f = self.lib.jo_run_closed_loop_metrics
+        f.restype = C.c_longlong
+        tail = (C.byref(metrics), abi.ptr(met))
+
+        class _Lib:                                         # ob._closed_loop's call, with the params and the rows appended
+            jo_run_closed_loop_metrics = staticmethod(lambda *a: f(*a, *tail))
+        o = ob._closed_loop(_Lib, "jo_run_closed_loop_metrics", self.params, wp, hdr, agents, cycles, paths, threads)
+        o["metrics"] = met
+        return o
+
+    def metrics_step(self, hdr, agents, ox, oy, met, mp, rec=None, last_path=None, wp=None):
+        """one world step plus its metric update, in place (jo_metrics_step)"""
+        wp = wp or self.world_params()
+        n, max_obs = ox.shape
+        assert met.dtype == abi.episode_metrics and met.shape == (n,)
+        assert self.lib.jo_metrics_step(C.byref(self.params), C.byref(wp), C.byref(mp), C.c_int(n), C.c_int(max_obs), abi.ptr(hdr),
+                                        abi.ptr(agents), abi.ptr(ox), abi.ptr(oy), abi.ptr(rec), abi.ptr(last_path), abi.ptr(met)) == 0
+
+    def metrics_sizeof(self):
+        return int(self.lib.jo_metrics_sizeof())
+
+    def sincos_deg(self, a):
+        c, s = C.c_double(0), C.c_double(0)
+        self.lib.jo_sincos_deg(C.c_double(a), C.byref(c), C.byref(s))
+        return c.value, s.value
 
 
 class JunctionReference:

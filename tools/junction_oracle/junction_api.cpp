@@ -1,11 +1,15 @@
 // tools/junction_oracle/junction_api.cpp -- TEST INFRASTRUCTURE. C API of libjunction_oracle.so: the restated cycle of oracle/
 // (planner_oracle.cpp, compiled in unchanged) with the junction world step of world_junction.cpp between its cycles; the
-// same arrays as oracle_world_step / oracle_run_closed_loop of oracle/oracle_api.cpp.
+// same arrays as oracle_world_step / oracle_run_closed_loop of oracle/oracle_api.cpp; and the episode metrics of
+// episode_metrics.cpp after every world step (jo_run_closed_loop_metrics, jo_metrics_step).
+#include <algorithm>
 #include <atomic>
 #include <cstring>
 #include <thread>
 #include <vector>
+#include "episode_metrics.h"
 #include "world_junction.h"
+#include "../../oracle/cshare_spec.h"
 
 namespace { junction::JMap g_map; bool g_have_map = false; }
 
@@ -30,10 +34,14 @@ int jo_world_step(const dp_params* p, const dp_world_params* wp, int n, int max_
     return 0;
 }
 
-long long jo_run_closed_loop(const dp_params* p, const dp_world_params* wp, int n, int cycles, int max_obs, dp_scene_hdr* hdr,
-                             dp_agent* agents, double* ox, double* oy, dp_plan_record* rec, dp_scene_hdr* hdr_log, double* obs_log_x,
-                             double* obs_log_y, double* path_xy, dp_carry* carry_out, double* last_path_out, int threads,
-                             int32_t* ub_scene) {
+}  // extern "C"
+
+namespace {
+// the closed loop of jo_run_closed_loop; mp / met non-null: the episode metrics accumulated after every world step
+long long closed_loop(const dp_params* p, const dp_world_params* wp, int n, int cycles, int max_obs, dp_scene_hdr* hdr, dp_agent* agents,
+                      double* ox, double* oy, dp_plan_record* rec, dp_scene_hdr* hdr_log, double* obs_log_x, double* obs_log_y,
+                      double* path_xy, dp_carry* carry_out, double* last_path_out, int threads, int32_t* ub_scene,
+                      const dp_metrics_params* mp, dp_episode_metrics* met) {
     if (!g_have_map) return -1;
     if (threads < 1) threads = 1;
     std::atomic<long long> ub(0);
@@ -46,6 +54,7 @@ long long jo_run_closed_loop(const dp_params* p, const dp_world_params* wp, int 
             dp_agent* ag = agents + (size_t)s * max_obs;
             double* sx = ox + (size_t)s * max_obs; double* sy = oy + (size_t)s * max_obs;
             junction::world_step(g_map, *p, *wp, hdr[s], ag, sx, sy, nullptr, nullptr, nullptr);
+            if (met) metrics::init(met[s]);
             for (int c = 0; c < cycles; ++c) {
                 const size_t e = (size_t)c * n + s;
                 if (hdr_log) hdr_log[e] = hdr[s];
@@ -56,7 +65,9 @@ long long jo_run_closed_loop(const dp_params* p, const dp_world_params* wp, int 
                 o.path_xy = path_xy ? path_xy + e * 400 : nullptr;
                 oracle::cycle(g_map.m, *p, hdr[s], sx, sy, st, o, false);
                 lub += o.ub_hits;
+                const dp_scene_hdr h0 = hdr[s];
                 junction::world_step(g_map, *p, *wp, hdr[s], ag, sx, sy, rec + e, st.last_x, st.last_y);
+                if (met) metrics::update(g_map, *wp, *mp, met[s], h0, hdr[s], ag, sx, sy, std::min((int)h0.n_obs, max_obs), rec[e]);
             }
             if (ub_scene) ub_scene[s] = (int32_t)(lub - lub0);
             if (carry_out) carry_out[s] = st.c;
@@ -75,5 +86,48 @@ long long jo_run_closed_loop(const dp_params* p, const dp_world_params* wp, int 
     }
     return ub.load();
 }
+}  // namespace
+
+extern "C" {
+
+long long jo_run_closed_loop(const dp_params* p, const dp_world_params* wp, int n, int cycles, int max_obs, dp_scene_hdr* hdr,
+                             dp_agent* agents, double* ox, double* oy, dp_plan_record* rec, dp_scene_hdr* hdr_log, double* obs_log_x,
+                             double* obs_log_y, double* path_xy, dp_carry* carry_out, double* last_path_out, int threads,
+                             int32_t* ub_scene) {
+    return closed_loop(p, wp, n, cycles, max_obs, hdr, agents, ox, oy, rec, hdr_log, obs_log_x, obs_log_y, path_xy, carry_out, last_path_out,
+                       threads, ub_scene, nullptr, nullptr);
+}
+
+// jo_run_closed_loop with the episode metrics of every world in met[n] (include/dmpp_b200.h section 11)
+long long jo_run_closed_loop_metrics(const dp_params* p, const dp_world_params* wp, int n, int cycles, int max_obs, dp_scene_hdr* hdr,
+                                     dp_agent* agents, double* ox, double* oy, dp_plan_record* rec, dp_scene_hdr* hdr_log, double* obs_log_x,
+                                     double* obs_log_y, double* path_xy, dp_carry* carry_out, double* last_path_out, int threads,
+                                     int32_t* ub_scene, const dp_metrics_params* mp, dp_episode_metrics* met) {
+    if (!mp || !met) return -1;
+    return closed_loop(p, wp, n, cycles, max_obs, hdr, agents, ox, oy, rec, hdr_log, obs_log_x, obs_log_y, path_xy, carry_out, last_path_out,
+                       threads, ub_scene, mp, met);
+}
+
+// one world step plus its metric update for every scene, as the armed kernel does it: rec == NULL initialises the rows (also for a
+// header that names no lane); a header that names no lane leaves its world and its row alone
+int jo_metrics_step(const dp_params* p, const dp_world_params* wp, const dp_metrics_params* mp, int n, int max_obs, dp_scene_hdr* hdr,
+                    dp_agent* agents, double* ox, double* oy, const dp_plan_record* rec, const double* last_path, dp_episode_metrics* met) {
+    if (!g_have_map) return -1;
+    for (int s = 0; s < n; ++s) {
+        if (!rec) metrics::init(met[s]);
+        if (!metrics::header_valid(g_map.m, hdr[s])) continue;
+        const dp_scene_hdr h0 = hdr[s];
+        dp_agent* ag = agents + (size_t)s * max_obs;
+        double* sx = ox + (size_t)s * max_obs; double* sy = oy + (size_t)s * max_obs;
+        junction::world_step(g_map, *p, *wp, hdr[s], ag, sx, sy, rec ? rec + s : nullptr, last_path ? last_path + (size_t)s * 400 : nullptr,
+                             last_path ? last_path + (size_t)s * 400 + 200 : nullptr);
+        if (rec) metrics::update(g_map, *wp, *mp, met[s], h0, hdr[s], ag, sx, sy, std::min((int)h0.n_obs, max_obs), rec[s]);
+    }
+    return 0;
+}
+
+int jo_metrics_sizeof(void) { return (int)sizeof(dp_episode_metrics); }
+
+void jo_sincos_deg(double a, double* c, double* s) { spec::spec_sincos_deg(a, c, s); }
 
 }  // extern "C"

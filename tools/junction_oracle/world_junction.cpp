@@ -30,8 +30,9 @@ inline double nearest(const oracle::MapView& m, int gl, int lo, int hi, double x
     }
     return be;
 }
-// the ego's connector (include/dmpp_b200.h section 9): lowest c leaving (road, lane) towards hdr.next_roadnum, -1 none
-inline int ego_connector(const oracle::MapView& m, const dp_scene_hdr& h, int road, int lane) {
+}  // namespace
+
+int ego_connector(const oracle::MapView& m, const dp_scene_hdr& h, int road, int lane) {
     if (h.next_roadnum == road) return -1;
     for (int c = 0; c < m.d.n_conn; ++c) {
         const dp_connector& k = m.d.conn[c];
@@ -39,7 +40,6 @@ inline int ego_connector(const oracle::MapView& m, const dp_scene_hdr& h, int ro
     }
     return -1;
 }
-}  // namespace
 
 void JMap::set(const dp_map_desc& m) {
     this->m.d = m;

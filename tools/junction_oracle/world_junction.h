@@ -27,6 +27,9 @@ struct JMap {
     void set(const dp_map_desc& d);
 };
 
+// the ego's connector (include/dmpp_b200.h section 9): lowest c leaving (road, lane) towards h.next_roadnum, -1 none
+int ego_connector(const oracle::MapView& m, const dp_scene_hdr& h, int road, int lane);
+
 // one world step of one scene; rec == nullptr: place the agents and localise only (and the 0 -> 1 / 1 -> 2 / 2 -> 0 rules).
 // last_x / last_y: the carried local path (road_points of the cycle that produced rec).
 void world_step(const JMap& m, const dp_params& p, const dp_world_params& wp, dp_scene_hdr& h, dp_agent* agents, double* ox,
