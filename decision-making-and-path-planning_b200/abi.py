@@ -151,6 +151,11 @@ class MetricsParams(C.Structure):
                 ("ttc_warn", C.c_double)]
 
 
+class AgentModelParams(C.Structure):
+    _fields_ = [("a_max", C.c_double), ("b", C.c_double), ("b_max", C.c_double), ("T", C.c_double), ("s0", C.c_double),
+                ("length", C.c_double), ("ego_rear", C.c_double), ("look", C.c_double)]
+
+
 class MapDesc(C.Structure):
     _fields_ = [
         ("n_roads", C.c_int32), ("road_lane_base", C.c_void_p),

@@ -65,6 +65,8 @@ struct dp_ctx {
     dp_world_params wp;
     dp_metrics_params mp;                                   // episode metrics (dp_world_set_metrics): d_met == nullptr disarmed
     dp_episode_metrics* d_met = nullptr;
+    dp_agent_model_params amp;                              // reactive agents (dp_world_set_agent_model): d_v0 == nullptr disarmed
+    const double* d_v0 = nullptr;
     cudaStream_t ep_stream = nullptr;
     cudaGraphExec_t ep_exec = nullptr;
     const void* ep_key[8] = {}; int ep_dims[3] = {-1, -1, -1};
@@ -308,6 +310,7 @@ int dp_create(dp_ctx** out, int device, const dp_params* params, int max_scenes,
     if (const char* e = getenv("DP_EPISODE_GRAPH")) c->ep_graph = atoi(e) != 0;
     dp_world_default_params(&c->wp);
     dp_metrics_default_params(&c->mp);
+    dp_agent_model_default_params(&c->amp);
     // Kernel choice, from the measurements in profiles/README.md (round 2): the warp-per-scene kernel wins while a scene's
     // obstacles fit one warp pass (N < 32: 71 vs 96 us per 4096-scene cycle at N = 10); the group kernel, whose scans are flat
     // (trajectory, obstacle) lists with exact pruning, wins for crowded scenes (N = 200: 135 vs 212 us per 1024 junction scenes).
@@ -1426,6 +1429,31 @@ int dp_world_set_metrics(dp_ctx* c, const dp_metrics_params* p, dp_episode_metri
     if (c->ep_exec) { cudaGraphExecDestroy(c->ep_exec); c->ep_exec = nullptr; }   // (the row pointer and parameters are baked into the graph)
     return DP_OK;
 }
+void dp_agent_model_default_params(dp_agent_model_params* p) {
+    if (!p) return;
+    memset(p, 0, sizeof(*p));
+    p->a_max = 1.0; p->b = 1.5; p->b_max = 8.0; p->T = 1.5; p->s0 = 2.0; p->length = 4.5; p->ego_rear = 1.0; p->look = 100.0;
+}
+int dp_world_set_agent_model(dp_ctx* c, const dp_agent_model_params* p, const double* v0) {
+    if (!c || (v0 && !p)) return fail(DP_ERR_ARG, "dp_world_set_agent_model: bad argument");
+    if (p) {
+        const double v[8] = {p->a_max, p->b, p->b_max, p->T, p->s0, p->length, p->ego_rear, p->look};
+        for (double x : v) if (!std::isfinite(x)) return fail(DP_ERR_ARG, "dp_world_set_agent_model: parameters must be finite");
+        if (!(p->a_max > 0) || !(p->b > 0) || !(p->b_max > 0) || !(p->T > 0) || !(p->length > 0) || !(p->look > 0) || !(p->s0 >= 0) ||
+            !(p->ego_rear >= 0))
+            return fail(DP_ERR_ARG, "dp_world_set_agent_model: a_max, b, b_max, T, length, look > 0 and s0, ego_rear >= 0");
+    }
+    if (v0) {
+        if (c->max_obs > DP_AGENT_MODEL_MAX_OBS)
+            return fail(DP_ERR_ARG, "dp_world_set_agent_model: the context's max_obs exceeds DP_AGENT_MODEL_MAX_OBS");
+        CK(cudaSetDevice(c->device));
+        CK(dp_world_agents_prepare());                      // function attributes are set before any launch or capture of the armed step
+        c->amp = *p;
+    }
+    c->d_v0 = v0;
+    if (c->ep_exec) { cudaGraphExecDestroy(c->ep_exec); c->ep_exec = nullptr; }   // (the speeds pointer and parameters are baked into the graph)
+    return DP_OK;
+}
 int dp_world_step_dev(dp_ctx* c, int first, int n, dp_scene_hdr* hdr, dp_agent* agents, double* ox, double* oy, const dp_plan_record* rec,
                       void* stream) {
     if (!c || !hdr || !agents || !ox || !oy || n < 0 || first < 0 || first + n > c->max_scenes)
@@ -1434,7 +1462,7 @@ int dp_world_step_dev(dp_ctx* c, int first, int n, dp_scene_hdr* hdr, dp_agent* 
     CK(cudaSetDevice(c->device));
     c->launches += n > 0 ? 1 : 0;
     CK(dp_launch_world(c->gmap, c->p, c->wp, n, c->max_obs, hdr, agents, ox, oy, rec, c->d_last + (size_t)first * DP_PATH_POINTS,
-                       c->mp, c->d_met, (cudaStream_t)stream));
+                       c->mp, c->d_met, c->amp, c->d_v0, (cudaStream_t)stream));
     return DP_OK;
 }
 namespace {
@@ -1447,7 +1475,8 @@ cudaError_t enqueue_closed_loop(dp_ctx* c, int first, int n, int cycles, dp_scen
     // a replayed graph re-uses its hand-off epochs: the per-scene Decision -> Planning flags start every replay from 0
     if (rearm && (e = cudaMemsetAsync(c->d_done + first, 0, (size_t)n * sizeof(unsigned), st)) != cudaSuccess) return e;
     c->launches += 1;
-    if ((e = dp_launch_world(c->gmap, c->p, c->wp, n, c->max_obs, hdr, agents, ox, oy, nullptr, last, c->mp, c->d_met, st)) != cudaSuccess) return e;
+    if ((e = dp_launch_world(c->gmap, c->p, c->wp, n, c->max_obs, hdr, agents, ox, oy, nullptr, last, c->mp, c->d_met, c->amp, c->d_v0, st)) != cudaSuccess)
+        return e;
     for (int k = 0; k < cycles; ++k) {
         if (hdr_log && (e = cudaMemcpyAsync(hdr_log + (size_t)k * n, hdr, (size_t)n * sizeof(dp_scene_hdr), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
         if (olx && (e = cudaMemcpyAsync(olx + (size_t)k * n * mo, ox, (size_t)n * mo * sizeof(double), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
@@ -1455,7 +1484,8 @@ cudaError_t enqueue_closed_loop(dp_ctx* c, int first, int n, int cycles, dp_scen
         const DpIo io = make_io(c, first, nullptr);
         if ((e = run_cycle(c, first, n, hdr, ox, oy, rec + (size_t)k * n, nullptr, nullptr, nullptr, st, io)) != cudaSuccess) return e;
         c->launches += 1;
-        if ((e = dp_launch_world(c->gmap, c->p, c->wp, n, c->max_obs, hdr, agents, ox, oy, rec + (size_t)k * n, last, c->mp, c->d_met, st)) != cudaSuccess)
+        if ((e = dp_launch_world(c->gmap, c->p, c->wp, n, c->max_obs, hdr, agents, ox, oy, rec + (size_t)k * n, last, c->mp, c->d_met, c->amp, c->d_v0,
+                                   st)) != cudaSuccess)
             return e;
     }
     return cudaSuccess;

@@ -8,7 +8,8 @@ cudaError_t dp_launch_world_metrics(const DevMap& m, const dp_params& p, const d
                                     const dp_metrics_params& mp, dp_episode_metrics* met, cudaStream_t st) {
     if (n <= 0) return cudaSuccess;
     const int g = (n + WPB - 1) / WPB;
-    if (wp.pre_junction_pts > 0) dp_world_kernel<true, true><<<g, WPB * 32, 0, st>>>(m, p, wp, n, max_obs, hdr, agents, obs_x, obs_y, rec, last_path, mp, met);
-    else dp_world_kernel<false, true><<<g, WPB * 32, 0, st>>>(m, p, wp, n, max_obs, hdr, agents, obs_x, obs_y, rec, last_path, mp, met);
+    const AgentModel am = {};
+    if (wp.pre_junction_pts > 0) dp_world_kernel<true, true, false><<<g, WPB * 32, 0, st>>>(m, p, wp, n, max_obs, hdr, agents, obs_x, obs_y, rec, last_path, mp, met, am);
+    else dp_world_kernel<false, true, false><<<g, WPB * 32, 0, st>>>(m, p, wp, n, max_obs, hdr, agents, obs_x, obs_y, rec, last_path, mp, met, am);
     return cudaGetLastError();
 }

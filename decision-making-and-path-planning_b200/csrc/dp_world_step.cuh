@@ -1,7 +1,8 @@
 // csrc/dp_world_step.cuh -- the world step of the closed-loop episode runner (dp_world_kernel, see dp_world.cu), with the
-// episode metrics of include/dmpp_b200.h section 11 as a compile-time option.  dp_world.cu instantiates the disarmed kernels
-// (METRICS = false) and dp_world_metrics.cu the armed ones: kept in separate translation units, the disarmed instances compile
-// to exactly what they compiled to before the metrics existed.
+// episode metrics of include/dmpp_b200.h section 11 and the reactive agents of section 12 as compile-time options.  dp_world.cu
+// instantiates the disarmed kernels (METRICS = REACT = false), dp_world_metrics.cu the metrics instances and dp_world_agents.cu
+// the reactive ones: kept in separate translation units, the disarmed instances compile to exactly what they compiled to before
+// the options existed.
 #pragma once
 #include <type_traits>
 
@@ -143,15 +144,109 @@ __device__ __forceinline__ void metrics_step(MetricLane& ml, double* row, dp_epi
     if (lane < MET_WORDS) reinterpret_cast<double*>(out)[lane] = row[lane];
 }
 
+// ---- reactive agents (include/dmpp_b200.h section 12): the intelligent driver model on the lane chain ----
+constexpr int REACT_SLOT_BYTES = 24;   // staged per agent slot and world: (station, speed) as a double2 and the lane (int, padded)
+// bytes of dynamic shared memory per warp (16-byte aligned: the double2 array comes first)
+__host__ __device__ constexpr size_t react_stage_bytes(int max_obs) { return ((size_t)max_obs * REACT_SLOT_BYTES + 15) & ~(size_t)15; }
+static_assert(WPB * (react_stage_bytes(DP_AGENT_MODEL_MAX_OBS) + (32 + 2 * MET_WORDS) * 4) <= 227 * 1024,
+              "the staging of DP_AGENT_MODEL_MAX_OBS agent slots fits the shared memory of a CTA");
+struct AgentModel {
+    dp_agent_model_params p;
+    const double* v0;                  // [n][max_obs] desired speeds
+};
+
+// length of map lane gl: the last entry of its sequential prefix of segment lengths
+__device__ __forceinline__ double lane_len(const DevMap& m, int gl) { return m.cump[m.lane_pt_off[gl + 1] - 1]; }
+
+// rewrite agents[].v of one scene from the state at the start of the step (Jacobi): stage (lane, s, v) of every agent in the
+// warp's slice of dynamic shared memory, then each lane scans the staged candidates for each of its agents (broadcast reads)
+__device__ __forceinline__ void react_step(const DevMap& m, const AgentModel& am, const dp_scene_hdr& h, int pos, int n_obs, double dt,
+                                           dp_agent* ag, const double* v0, unsigned char* stage, int max_obs, int lane) {
+    double2* SV = reinterpret_cast<double2*>(stage);
+    int* L = reinterpret_cast<int*>(SV + max_obs);
+    for (int k = lane; k < n_obs; k += 32) {
+        const dp_agent a = ag[k];
+        SV[k] = make_double2(m.cump[m.lane_pt_off[a.lane] + a.i] + a.u, a.v);
+        L[k] = a.lane;
+    }
+    // the ego candidate (warp-uniform): its lane, station and speed from the start-of-step header
+    int le = -1, idx = 0;
+    if (pos != 2) { le = m.road_lane_base[h.road_num - 1] + h.lane_num - 1; idx = h.id[h.lane_num - 1]; }
+    else if (h.conn >= 0 && h.conn < m.n_conn && h.last_lanenum >= 1 && h.last_lanenum <= DP_LANESUM) {
+        le = m.conn[h.conn].lane; idx = h.id[h.last_lanenum - 1];
+    }
+    double se = 0;
+    if (le >= 0) {
+        const int off = m.lane_pt_off[le], cnt = m.lane_pt_off[le + 1] - off;
+        if (idx > cnt - 1) idx = cnt - 1;
+        if (idx < 0) idx = 0;
+        se = m.cump[off + idx];
+    }
+    const double ve = h.velocity / 3.6;
+    const dp_agent_model_params& p = am.p;
+    const double inf = __longlong_as_double(0x7ff0000000000000LL);
+    const double sab = 2.0 * sqrt(p.a_max * p.b);
+    __syncwarp();
+    for (int k = lane; k < n_obs; k += 32) {
+        const double vd = v0[k];
+        if (!(vd > 0)) continue;
+        const double2 own = SV[k];
+        const double sk = own.x, v = own.y;
+        const int l0 = L[k], l1 = m.lane_next[l0], l2 = l1 >= 0 ? m.lane_next[l1] : -1;
+        const double D1 = lane_len(m, l0) - sk, D2 = l1 >= 0 ? D1 + lane_len(m, l1) : 0.0;
+        double best = inf, vl = 0;
+        bool lead = false;
+        if (le >= 0) {
+            double ds = inf;
+            if (le == l0 && se >= sk) ds = se - sk;
+            if (le == l1) { const double c = D1 + se; if (c < ds) ds = c; }
+            if (l2 >= 0 && le == l2) { const double c = D2 + se; if (c < ds) ds = c; }
+            if (ds <= p.look) { best = ds - p.ego_rear; vl = ve; lead = true; }
+        }
+#pragma unroll 4
+        for (int j = 0; j < n_obs; ++j) {                   // warp-uniform j: broadcast reads
+            const int lj = L[j];
+            const double2 c2 = SV[j];
+            const double sj = c2.x;
+            double ds = inf;
+            if (lj == l0 && (sj > sk || (sj == sk && j > k))) ds = sj - sk;
+            if (lj == l1) { const double c = D1 + sj; if (c < ds) ds = c; }
+            if (l2 >= 0 && lj == l2) { const double c = D2 + sj; if (c < ds) ds = c; }
+            if (ds <= p.look) {
+                const double g = ds - p.length;
+                if (!lead || g < best) { best = g; vl = c2.y; lead = true; }
+            }
+        }
+        const double r = v / vd;
+        double fr = r * r;
+        fr = fr * fr;
+        double acc;
+        if (lead) {
+            const double dv = v - vl;
+            double z = v * p.T + v * dv / sab;
+            if (z < 0) z = 0;
+            const double ss = p.s0 + z;
+            if (best > 0) { const double q = ss / best; acc = p.a_max * (1.0 - fr - q * q); }
+            else acc = -p.b_max;
+        } else acc = p.a_max * (1.0 - fr);
+        if (acc < -p.b_max) acc = -p.b_max;
+        double vn = v + acc * dt;
+        if (vn < 0) vn = 0;
+        ag[k].v = vn;
+    }
+}
+
 // JUNC = (pre_junction_pts > 0): the segment-only step (false) carries none of the junction code.
 // METRICS = episode metrics armed (met != nullptr): the disarmed instances carry none of the metric code; the armed ones read the
 // scene's row at entry and write it at the end as one coalesced 192-byte access each, staged behind the header in shared memory.
-template <bool JUNC, bool METRICS>
-__global__ void __launch_bounds__(WPB * 32, METRICS ? 8 : 0) dp_world_kernel(DevMap m, dp_params p, dp_world_params wp, int n, int max_obs,
+// REACT = reactive agents armed (am.v0 != nullptr): before the agent loop the armed instances rewrite agents[].v (react_step),
+// staging max_obs * REACT_SLOT_BYTES of dynamic shared memory per warp.
+template <bool JUNC, bool METRICS, bool REACT>
+__global__ void __launch_bounds__(WPB * 32, (METRICS || REACT) ? 8 : 0) dp_world_kernel(DevMap m, dp_params p, dp_world_params wp, int n, int max_obs,
                                                             dp_scene_hdr* __restrict__ hdr, dp_agent* __restrict__ agents,
                                                             double* __restrict__ obs_x, double* __restrict__ obs_y,
                                                             const dp_plan_record* __restrict__ rec, const double2* __restrict__ last_path,
-                                                            dp_metrics_params mp, dp_episode_metrics* __restrict__ met) {
+                                                            dp_metrics_params mp, dp_episode_metrics* __restrict__ met, AgentModel am) {
     __shared__ __align__(16) uint32_t sh[WPB][METRICS ? 32 + 2 * MET_WORDS : 32];
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     const int scene = blockIdx.x * WPB + wib;
@@ -236,6 +331,13 @@ __global__ void __launch_bounds__(WPB * 32, METRICS ? 8 : 0) dp_world_kernel(Dev
             double c, sn;
             dp_sincos_deg(dir, &c, &sn);
             ml.c = c; ml.s = sn;
+        }
+    }
+    if constexpr (REACT) {
+        if (step) {
+            extern __shared__ __align__(16) unsigned char react_stage[];
+            react_step(m, am, h, pos, n_obs, dt, agents + (size_t)scene * max_obs, am.v0 + (size_t)scene * max_obs,
+                       react_stage + wib * react_stage_bytes(max_obs), max_obs, lane);
         }
     }
     // ---- agents: constant speed along their lanes (junctions on: and on into the lane's successor), then their obstacle points ----

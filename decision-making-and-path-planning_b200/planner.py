@@ -26,7 +26,7 @@ SYMBOLS = [
     "dp_set_tracks", "dp_set_tracks_dev", "dp_clear_tracks",
     "dp_pack_frames_dev", "dp_pack_frames", "dp_world_default_params", "dp_world_set_params", "dp_world_step_dev",
     "dp_run_closed_loop_dev", "dp_closed_loop_is_graph", "dp_v2x_event_batch", "dp_v2x_event_batch_dev", "dp_v2x_apply", "dp_v2x_apply_dev",
-    "dp_metrics_default_params", "dp_world_set_metrics",
+    "dp_metrics_default_params", "dp_world_set_metrics", "dp_agent_model_default_params", "dp_world_set_agent_model",
     "dp_gather_create", "dp_gather_attach", "dp_gather_arm", "dp_gather_chain", "dp_gather_arm_deferred", "dp_gather_set_lag", "dp_gather_flush", "dp_gather_disarm", "dp_gather_wait", "dp_gather_buffer", "dp_gather_destroy",
 ]
 
@@ -59,6 +59,13 @@ def metrics_params():
     """dp_metrics_default_params (no GPU needed)"""
     p = abi.MetricsParams()
     load().dp_metrics_default_params(C.byref(p))
+    return p
+
+
+def agent_model_params():
+    """dp_agent_model_default_params (no GPU needed)"""
+    p = abi.AgentModelParams()
+    load().dp_agent_model_default_params(C.byref(p))
     return p
 
 
@@ -225,6 +232,15 @@ class Planner:
         _ck(self.lib.dp_world_set_metrics(self.ctx, C.byref(params) if params is not None else None, C.c_void_p(d_metrics or 0)),
             "dp_world_set_metrics")
 
+    def agent_model_params(self):
+        return agent_model_params()
+
+    def set_agent_model(self, params, d_v0):
+        """arm the reactive agents (include/dmpp_b200.h section 12): d_v0 = device address of desired speeds [n][max_obs] (m/s)
+        indexed like hdr; d_v0 None / 0 disarms"""
+        _ck(self.lib.dp_world_set_agent_model(self.ctx, C.byref(params) if params is not None else None, C.c_void_p(d_v0 or 0)),
+            "dp_world_set_agent_model")
+
     def world_step_dev(self, n, d_hdr, d_agents, d_ox, d_oy, d_rec=None, first=0, stream=0):
         _ck(self.lib.dp_world_step_dev(self.ctx, C.c_int(first), C.c_int(n), C.c_void_p(d_hdr), C.c_void_p(d_agents), C.c_void_p(d_ox),
                                        C.c_void_p(d_oy), C.c_void_p(d_rec or 0), C.c_void_p(stream)), "dp_world_step_dev")
@@ -239,17 +255,23 @@ class Planner:
     def closed_loop_is_graph(self):
         return bool(self.lib.dp_closed_loop_is_graph(self.ctx))
 
-    def run_closed_loop(self, hdr, agents, cycles, log=True, repeat=1, metrics=None):
+    def run_closed_loop(self, hdr, agents, cycles, log=True, repeat=1, metrics=None, agent_model=None):
         """host arrays in, host arrays out (the same dictionary as oracle.binding's run_closed_loop); `repeat` > 1 replays the
         episode from the same initial world (same device buffers, i.e. the cached graph) and returns the last run.
         metrics: None, or MetricsParams: the episode metrics are armed for this call (and disarmed after it) and the rows are
-        returned under the key "metrics"."""
+        returned under the key "metrics".  agent_model: None, or (AgentModelParams, v0[n][max_obs] desired speeds in m/s): the
+        reactive agents are armed for this call (and disarmed after it)."""
         n, mo = agents.shape
         assert mo == self.max_obs and hdr.shape == (n,)
         sizes = {"hdr": n * 128, "agents": n * mo * 32, "ox": n * mo * 8, "oy": n * mo * 8, "rec": cycles * n * 128,
                  "hdr_log": cycles * n * 128, "obs_log_x": cycles * n * mo * 8, "obs_log_y": cycles * n * mo * 8}
         if metrics is not None:
             sizes["metrics"] = n * abi.episode_metrics.itemsize
+        if agent_model is not None:
+            am, v0 = agent_model
+            v0 = np.ascontiguousarray(v0, np.float64)
+            assert v0.shape == (n, mo)
+            sizes["v0"] = n * mo * 8
         d = {}
         try:
             for k, b in sizes.items():
@@ -259,6 +281,9 @@ class Planner:
                     d[k] = p.value
             if metrics is not None:
                 self.set_metrics(metrics, d["metrics"])
+            if agent_model is not None:
+                _ck(self.lib.dp_memcpy_h2d(self.ctx, C.c_void_p(d["v0"]), abi.ptr(v0), C.c_size_t(sizes["v0"]), None), "h2d")
+                self.set_agent_model(am, d["v0"])
             h0, a0 = np.ascontiguousarray(hdr), np.ascontiguousarray(agents)
             for _ in range(repeat):
                 self.reset(0, n)
@@ -283,6 +308,8 @@ class Planner:
         finally:
             if metrics is not None:
                 self.set_metrics(None, None)
+            if agent_model is not None:
+                self.set_agent_model(None, None)
             for p in d.values():
                 self.lib.dp_dev_free(self.ctx, C.c_void_p(p))
 

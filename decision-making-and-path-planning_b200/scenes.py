@@ -414,7 +414,8 @@ class World:
     agents and localisation itself.  The cycle period is a whole number of milliseconds per scene, fixed over the episode.
     kind 'junction' / 'urban': the agents sit on the approach lane, the connector or the departure lane by arclength, as
     `Episodes.obstacles` spreads them; the ego crosses the junction only with dp_world_params.pre_junction_pts > 0
-    (`PRE_JUNCTION_PTS[kind]` matches the scripted episodes)."""
+    (`PRE_JUNCTION_PTS[kind]` matches the scripted episodes).  `v0`: the agents' desired speeds for the reactive agents of
+    include/dmpp_b200.h section 12, by default their initial speeds."""
     PRE_JUNCTION_PTS = {"highway": 0, "junction": 60, "urban": 400}
 
     def __init__(self, m: Map, seeds, n_obs=10, roads=None, kind="highway"):
@@ -445,6 +446,7 @@ class World:
         a["v"] = ep.ob_v
         a["lat"] = ep.ob_lat
         self.agents = np.ascontiguousarray(a)
+        self.v0 = np.ascontiguousarray(a["v"])
 
 
 def v2x_events(m: Map, hdr, seed=0, p_far=0.12):

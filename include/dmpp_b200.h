@@ -526,7 +526,7 @@ int dp_v2x_apply_dev(dp_ctx* ctx, int n_scenes, const dp_v2x_flags* flags, dp_pl
  *   first_collision_step     1-based step of the first step with an agent inside, and the lowest such agent (-1 / -1)
  *   first_collision_agent
  *   collision_steps          steps with an agent inside; _front: with one inside at lon >= 0; _rear: with one inside at lon < 0
- *   collision_steps_front/_rear  (a step can count as both; agents do not react, so rear strikes are theirs)
+ *   collision_steps_front/_rear  (a step can count as both; unless the agents react (section 12), rear strikes are theirs)
  *   ttc_warn_steps           steps whose smallest ttc is < ttc_warn
  *   stopped_steps            steps with vn == 0;  end_stop_steps: steps on which the end_margin stop fired
  *   replans, aeb_steps       sum of rec.afresh_planning / rec.acc_flag
@@ -556,6 +556,57 @@ void dp_metrics_default_params(dp_metrics_params* p);
  * m == NULL disarms (p may then be NULL).  p must be finite with front, rear, corridor_half, ttc_warn >= 0 and half_width > 0,
  * else DP_ERR_ARG.  Context state like dp_world_set_params: the cached episode graph is rebuilt on its next call. */
 int dp_world_set_metrics(dp_ctx* ctx, const dp_metrics_params* p, dp_episode_metrics* m);
+
+/* (12) Reactive agents (opt-in): longitudinal car-following with the intelligent driver model.  Each agent adapts its speed to
+ * the nearest vehicle ahead of it on its lane chain, the ego included.  The model only REWRITES EACH AGENT'S SPEED at the start
+ * of a world step of section 9, from the state at the start of that step (Jacobi: every agent reads the old state of every
+ * other agent and of the ego); the agent motion of section 9 then runs unchanged with the new v.  It runs on steps with
+ * rec != NULL on headers that name a lane (the same early return as the step), for agents k < min(n_obs, max_obs).  With the
+ * model disarmed (the default) nothing changes.  The arithmetic is frozen in tools/junction_oracle/agent_model.h.
+ * Out of scope: lateral behaviour (agent lane changes and merges); yielding to a vehicle on a DIFFERENT connector that merges
+ * into the same lane (it is seen only once it is on the chain); any change to how the ego moves.
+ *
+ * IEEE binary64, operations in the order written, no contraction; min updates are `if (x < m) m = x`.
+ *   opt-out   !(v0[k] > 0) (0, negative, NaN): agent k keeps its speed (it moves exactly as in the disarmed step) but is still a
+ *             leader for the others
+ *   station   s = cump[off + i] + u, cump[off + i] = the sequential prefix (index order) of the lane's segment lengths
+ *             sqrt(dx*dx + dy*dy) that dp_map_upload builds; len(l) = cump[off(l) + cnt(l) - 1]
+ *   ego       pos as the step of section 9 reads it (0 when pre_junction_pts is 0), from the start-of-step header:
+ *             pos 0 / 1: lane road_lane_base[road_num-1] + lane_num - 1, index id[lane_num-1];
+ *             pos 2: lane conn[conn].lane, index id[last_lanenum-1] (an invalid conn or last_lanenum: no ego leader);
+ *             the index clamped to [0, cnt-1], s_e = cump[off + index]; its speed is velocity / 3.6
+ *   chain     l0 = the agent's lane, l1 = lane_next[l0], l2 = lane_next[l1] (stopping at -1; at most 2 hops);
+ *             D1 = len(l0) - s_k, D2 = D1 + len(l1)
+ *   candidate on l0: ds = s_j - s_k when s_j > s_k, or s_j == s_k && j > k (the ego: when s_e >= s_k);
+ *             on l1: ds = D1 + s_j; on l2: ds = D2 + s_j; a lane that appears twice in the chain takes the smaller ds;
+ *             only candidates with ds <= look count
+ *   leader    g = ds - length (an agent) or ds - ego_rear (the ego); the candidate with the smallest g, the ego first on a tie,
+ *             then the lowest agent index
+ *   IDM       (delta = 4) with v = the agent's v, dt = period_ms / 1000:
+ *               r = v / v0; fr = r * r; fr = fr * fr;
+ *               leader:    dv = v - vl; z = v * T + v * dv / (2.0 * sqrt(a_max * b)); if (z < 0) z = 0; ss = s0 + z;
+ *                          if (g > 0) { q = ss / g; acc = a_max * (1.0 - fr - q * q); } else acc = -b_max;
+ *               no leader: acc = a_max * (1.0 - fr);
+ *               if (acc < -b_max) acc = -b_max;
+ *               vn = v + acc * dt; if (vn < 0) vn = 0;   v = vn */
+typedef struct dp_agent_model_params {
+    double a_max;                    /* IDM acceleration, m/s^2, default 1.0 */
+    double b;                        /* comfortable deceleration, m/s^2, default 1.5 */
+    double b_max;                    /* hardest deceleration, m/s^2, default 8.0 (the clamp, and the answer for an overlapping leader) */
+    double T;                        /* time headway, s, default 1.5 */
+    double s0;                       /* jam distance, m, default 2.0 */
+    double length;                   /* point-to-point spacing subtracted for an agent leader, m, default 4.5 */
+    double ego_rear;                 /* subtracted for the ego as leader, m, default 1.0 (= dp_metrics_params.rear) */
+    double look;                     /* leader search horizon along the lane chain, m, default 100 */
+} dp_agent_model_params;             /* 64 bytes */
+/* the largest max_obs of a context that can arm the model: the world step stages 24 bytes per agent slot and world in shared memory */
+#define DP_AGENT_MODEL_MAX_OBS 2048
+void dp_agent_model_default_params(dp_agent_model_params* p);
+/* v0: device array [n][max_obs] of desired speeds (m/s), indexed like hdr (the s-th scene of every later dp_world_step_dev /
+ * dp_run_closed_loop_dev call); v0 == NULL disarms (p may then be NULL).  Context state like dp_world_set_metrics: the cached
+ * episode graph is rebuilt on its next call.  DP_ERR_ARG for non-finite parameters, a_max, b, b_max, T, length, look <= 0,
+ * s0, ego_rear < 0, or a context max_obs above DP_AGENT_MODEL_MAX_OBS. */
+int dp_world_set_agent_model(dp_ctx* ctx, const dp_agent_model_params* p, const double* v0);
 
 /* diagnostic: phase time stamps (globaltimer, ns) of the most recent cycle launch, one row of 32 per CTA (row b = scenes
  * [b*g, (b+1)*g) of the batch; stamp 0 = CTA start, stamp i = end of phase i of csrc/dp_group.cuh).  Only contexts created

@@ -49,23 +49,47 @@ class JunctionOracle:
         assert self.lib.jo_world_step(C.byref(self.params), C.byref(wp), C.c_int(n), C.c_int(max_obs), abi.ptr(hdr), abi.ptr(agents),
                                       abi.ptr(ox), abi.ptr(oy), abi.ptr(rec), abi.ptr(last_path)) == 0
 
-    def run_closed_loop(self, hdr, agents, cycles, wp=None, paths=False, threads=1, metrics=None):
+    def run_closed_loop(self, hdr, agents, cycles, wp=None, paths=False, threads=1, metrics=None, agent_model=None):
         """hdr[n], agents[n][max_obs] (copied; the final world is returned); metrics = MetricsParams: the episode metrics of every
-        world under "metrics" (jo_run_closed_loop_metrics)"""
+        world under "metrics" (jo_run_closed_loop_metrics); agent_model = (AgentModelParams, v0[n][max_obs]): the reactive agents
+        (jo_run_closed_loop_agents)"""
         wp = wp or self.world_params()
-        if metrics is None:
+        if metrics is None and agent_model is None:
             return ob._closed_loop(self.lib, "jo_run_closed_loop", self.params, wp, hdr, agents, cycles, paths, threads)
         n = hdr.shape[0]
-        met = np.frombuffer(np.full(n * abi.episode_metrics.itemsize, 0xAB, np.uint8).tobytes(), abi.episode_metrics).copy()
-        f = self.lib.jo_run_closed_loop_metrics
+        met = None
+        if metrics is not None:
+            met = np.frombuffer(np.full(n * abi.episode_metrics.itemsize, 0xAB, np.uint8).tobytes(), abi.episode_metrics).copy()
+        if agent_model is None:
+            name, tail = "jo_run_closed_loop_metrics", (C.byref(metrics), abi.ptr(met))
+        else:
+            am, v0 = agent_model
+            v0 = np.ascontiguousarray(v0, np.float64)
+            assert v0.shape == agents.shape
+            name = "jo_run_closed_loop_agents"
+            tail = (C.byref(metrics) if metrics is not None else None, abi.ptr(met), C.byref(am), abi.ptr(v0))
+        f = getattr(self.lib, name)
         f.restype = C.c_longlong
-        tail = (C.byref(metrics), abi.ptr(met))
 
         class _Lib:                                         # ob._closed_loop's call, with the params and the rows appended
-            jo_run_closed_loop_metrics = staticmethod(lambda *a: f(*a, *tail))
-        o = ob._closed_loop(_Lib, "jo_run_closed_loop_metrics", self.params, wp, hdr, agents, cycles, paths, threads)
-        o["metrics"] = met
+            pass
+        setattr(_Lib, name, staticmethod(lambda *a: f(*a, *tail)))
+        o = ob._closed_loop(_Lib, name, self.params, wp, hdr, agents, cycles, paths, threads)
+        if met is not None:
+            o["metrics"] = met
         return o
+
+    def react_step(self, hdr, agents, v0, am, wp=None):
+        """the react phase alone, agents[n][max_obs] in place (jo_react_step)"""
+        wp = wp or self.world_params()
+        n, max_obs = agents.shape
+        v0 = np.ascontiguousarray(v0, np.float64)
+        assert v0.shape == agents.shape and hdr.shape == (n,) and agents.flags["C_CONTIGUOUS"]
+        assert self.lib.jo_react_step(C.byref(wp), C.byref(am), C.c_int(n), C.c_int(max_obs), abi.ptr(np.ascontiguousarray(hdr)),
+                                      abi.ptr(agents), abi.ptr(v0)) == 0
+
+    def agent_model_sizeof(self):
+        return int(self.lib.jo_agent_model_sizeof())
 
     def metrics_step(self, hdr, agents, ox, oy, met, mp, rec=None, last_path=None, wp=None):
         """one world step plus its metric update, in place (jo_metrics_step)"""

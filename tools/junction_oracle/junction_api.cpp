@@ -1,12 +1,14 @@
 // tools/junction_oracle/junction_api.cpp -- TEST INFRASTRUCTURE. C API of libjunction_oracle.so: the restated cycle of oracle/
 // (planner_oracle.cpp, compiled in unchanged) with the junction world step of world_junction.cpp between its cycles; the
-// same arrays as oracle_world_step / oracle_run_closed_loop of oracle/oracle_api.cpp; and the episode metrics of
-// episode_metrics.cpp after every world step (jo_run_closed_loop_metrics, jo_metrics_step).
+// same arrays as oracle_world_step / oracle_run_closed_loop of oracle/oracle_api.cpp; the episode metrics of
+// episode_metrics.cpp after every world step (jo_run_closed_loop_metrics, jo_metrics_step); and the reactive agents of
+// agent_model.cpp before every world step (jo_run_closed_loop_agents, jo_react_step).
 #include <algorithm>
 #include <atomic>
 #include <cstring>
 #include <thread>
 #include <vector>
+#include "agent_model.h"
 #include "episode_metrics.h"
 #include "world_junction.h"
 #include "../../oracle/cshare_spec.h"
@@ -37,11 +39,12 @@ int jo_world_step(const dp_params* p, const dp_world_params* wp, int n, int max_
 }  // extern "C"
 
 namespace {
-// the closed loop of jo_run_closed_loop; mp / met non-null: the episode metrics accumulated after every world step
+// the closed loop of jo_run_closed_loop; mp / met non-null: the episode metrics accumulated after every world step; am / v0
+// non-null: the agents react (v0[n][max_obs]) before every world step
 long long closed_loop(const dp_params* p, const dp_world_params* wp, int n, int cycles, int max_obs, dp_scene_hdr* hdr, dp_agent* agents,
                       double* ox, double* oy, dp_plan_record* rec, dp_scene_hdr* hdr_log, double* obs_log_x, double* obs_log_y,
                       double* path_xy, dp_carry* carry_out, double* last_path_out, int threads, int32_t* ub_scene,
-                      const dp_metrics_params* mp, dp_episode_metrics* met) {
+                      const dp_metrics_params* mp, dp_episode_metrics* met, const dp_agent_model_params* am, const double* v0) {
     if (!g_have_map) return -1;
     if (threads < 1) threads = 1;
     std::atomic<long long> ub(0);
@@ -66,6 +69,7 @@ long long closed_loop(const dp_params* p, const dp_world_params* wp, int n, int 
                 oracle::cycle(g_map.m, *p, hdr[s], sx, sy, st, o, false);
                 lub += o.ub_hits;
                 const dp_scene_hdr h0 = hdr[s];
+                if (am) agents::react(g_map, *wp, *am, h0, ag, std::min((int)h0.n_obs, max_obs), v0 + (size_t)s * max_obs);
                 junction::world_step(g_map, *p, *wp, hdr[s], ag, sx, sy, rec + e, st.last_x, st.last_y);
                 if (met) metrics::update(g_map, *wp, *mp, met[s], h0, hdr[s], ag, sx, sy, std::min((int)h0.n_obs, max_obs), rec[e]);
             }
@@ -95,7 +99,7 @@ long long jo_run_closed_loop(const dp_params* p, const dp_world_params* wp, int 
                              double* obs_log_y, double* path_xy, dp_carry* carry_out, double* last_path_out, int threads,
                              int32_t* ub_scene) {
     return closed_loop(p, wp, n, cycles, max_obs, hdr, agents, ox, oy, rec, hdr_log, obs_log_x, obs_log_y, path_xy, carry_out, last_path_out,
-                       threads, ub_scene, nullptr, nullptr);
+                       threads, ub_scene, nullptr, nullptr, nullptr, nullptr);
 }
 
 // jo_run_closed_loop with the episode metrics of every world in met[n] (include/dmpp_b200.h section 11)
@@ -105,8 +109,32 @@ long long jo_run_closed_loop_metrics(const dp_params* p, const dp_world_params* 
                                      int32_t* ub_scene, const dp_metrics_params* mp, dp_episode_metrics* met) {
     if (!mp || !met) return -1;
     return closed_loop(p, wp, n, cycles, max_obs, hdr, agents, ox, oy, rec, hdr_log, obs_log_x, obs_log_y, path_xy, carry_out, last_path_out,
-                       threads, ub_scene, mp, met);
+                       threads, ub_scene, mp, met, nullptr, nullptr);
 }
+
+// jo_run_closed_loop with the reactive agents of include/dmpp_b200.h section 12 (am, v0[n][max_obs]); mp / met: the episode
+// metrics as in jo_run_closed_loop_metrics, or both NULL
+long long jo_run_closed_loop_agents(const dp_params* p, const dp_world_params* wp, int n, int cycles, int max_obs, dp_scene_hdr* hdr,
+                                    dp_agent* agents, double* ox, double* oy, dp_plan_record* rec, dp_scene_hdr* hdr_log, double* obs_log_x,
+                                    double* obs_log_y, double* path_xy, dp_carry* carry_out, double* last_path_out, int threads,
+                                    int32_t* ub_scene, const dp_metrics_params* mp, dp_episode_metrics* met, const dp_agent_model_params* am,
+                                    const double* v0) {
+    if (!am || !v0 || (!mp) != (!met)) return -1;
+    return closed_loop(p, wp, n, cycles, max_obs, hdr, agents, ox, oy, rec, hdr_log, obs_log_x, obs_log_y, path_xy, carry_out, last_path_out,
+                       threads, ub_scene, mp, met, am, v0);
+}
+
+// the react phase alone, for every scene (agents[n][max_obs], v0[n][max_obs], k < min(n_obs, max_obs)), as the armed kernel runs
+// it at the start of a step with a record; a header that names no lane leaves its agents alone
+int jo_react_step(const dp_world_params* wp, const dp_agent_model_params* am, int n, int max_obs, const dp_scene_hdr* hdr, dp_agent* agents,
+                  const double* v0) {
+    if (!g_have_map) return -1;
+    for (int s = 0; s < n; ++s)
+        agents::react(g_map, *wp, *am, hdr[s], agents + (size_t)s * max_obs, std::min((int)hdr[s].n_obs, max_obs), v0 + (size_t)s * max_obs);
+    return 0;
+}
+
+int jo_agent_model_sizeof(void) { return (int)sizeof(dp_agent_model_params); }
 
 // one world step plus its metric update for every scene, as the armed kernel does it: rec == NULL initialises the rows (also for a
 // header that names no lane); a header that names no lane leaves its world and its row alone

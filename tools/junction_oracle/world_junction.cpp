@@ -55,6 +55,19 @@ void JMap::set(const dp_map_desc& m) {
         if (k.next_lane < 1 || k.next_lane > m.road_lane_base[k.next_road] - m.road_lane_base[k.next_road - 1]) continue;
         next[k.lane] = m.road_lane_base[k.next_road - 1] + k.next_lane - 1;
     }
+    cump.assign(m.n_lanes > 0 ? m.lane_pt_off[m.n_lanes] : 0, 0.0);
+    for (int gl = 0; gl < m.n_lanes; ++gl) {
+        const int off = m.lane_pt_off[gl], cnt = m.lane_pt_off[gl + 1] - off;
+        double acc = 0.0;
+        for (int i = 0; i < cnt; ++i) {
+            double l = 0.0;
+            if (i + 1 < cnt) {
+                const double dx = m.x[off + i + 1] - m.x[off + i], dy = m.y[off + i + 1] - m.y[off + i];
+                l = std::sqrt(dx * dx + dy * dy);
+            }
+            cump[off + i] = acc; acc += l;
+        }
+    }
 }
 
 void world_step(const JMap& jm, const dp_params& p, const dp_world_params& wp, dp_scene_hdr& h, dp_agent* ag, double* ox, double* oy,

@@ -20,10 +20,12 @@
 
 namespace junction {
 
-// the map view of oracle/ plus lane_next of dp_map_upload: the successor of every lane, -1 none
+// the map view of oracle/ plus lane_next of dp_map_upload: the successor of every lane, -1 none; and its cump: per point i of a
+// lane, the segment lengths sqrt(dx*dx + dy*dy) of points 0 .. i-1 added in index order (dp_map_prep_kernel)
 struct JMap {
     oracle::MapView m;
     std::vector<int> next;
+    std::vector<double> cump;
     void set(const dp_map_desc& d);
 };
 
