@@ -156,6 +156,15 @@ class AgentModelParams(C.Structure):
                 ("length", C.c_double), ("ego_rear", C.c_double), ("look", C.c_double)]
 
 
+class LaneChangeParams(C.Structure):
+    _fields_ = [("politeness", C.c_double), ("a_thr", C.c_double), ("b_safe", C.c_double), ("ego_b_safe", C.c_double),
+                ("ego_front", C.c_double), ("lat_speed", C.c_double), ("cooldown", C.c_double), ("end_guard", C.c_double)]
+
+
+lane_change_state = np.dtype([("lat_goal", "<f8"), ("hold", "<f8"), ("changes_left", "<i4"), ("changes_right", "<i4")])
+assert lane_change_state.itemsize == 24
+
+
 class MapDesc(C.Structure):
     _fields_ = [
         ("n_roads", C.c_int32), ("road_lane_base", C.c_void_p),

@@ -67,6 +67,8 @@ struct dp_ctx {
     dp_episode_metrics* d_met = nullptr;
     dp_agent_model_params amp;                              // reactive agents (dp_world_set_agent_model): d_v0 == nullptr disarmed
     const double* d_v0 = nullptr;
+    dp_lane_change_params lcp;                              // lane changes (dp_world_set_lane_change): d_lcs == nullptr disarmed
+    dp_lane_change_state* d_lcs = nullptr;
     cudaStream_t ep_stream = nullptr;
     cudaGraphExec_t ep_exec = nullptr;
     const void* ep_key[8] = {}; int ep_dims[3] = {-1, -1, -1};
@@ -311,6 +313,7 @@ int dp_create(dp_ctx** out, int device, const dp_params* params, int max_scenes,
     dp_world_default_params(&c->wp);
     dp_metrics_default_params(&c->mp);
     dp_agent_model_default_params(&c->amp);
+    dp_lane_change_default_params(&c->lcp);
     // Kernel choice, from the measurements in profiles/README.md (round 2): the warp-per-scene kernel wins while a scene's
     // obstacles fit one warp pass (N < 32: 71 vs 96 us per 4096-scene cycle at N = 10); the group kernel, whose scans are flat
     // (trajectory, obstacle) lists with exact pruning, wins for crowded scenes (N = 200: 135 vs 212 us per 1024 junction scenes).
@@ -1451,7 +1454,33 @@ int dp_world_set_agent_model(dp_ctx* c, const dp_agent_model_params* p, const do
         c->amp = *p;
     }
     c->d_v0 = v0;
+    if (!v0) c->d_lcs = nullptr;                            // lane changes run on the react phase
     if (c->ep_exec) { cudaGraphExecDestroy(c->ep_exec); c->ep_exec = nullptr; }   // (the speeds pointer and parameters are baked into the graph)
+    return DP_OK;
+}
+void dp_lane_change_default_params(dp_lane_change_params* p) {
+    if (!p) return;
+    memset(p, 0, sizeof(*p));
+    p->politeness = 0.2; p->a_thr = 0.2; p->b_safe = 4.0; p->ego_b_safe = 4.0; p->ego_front = 4.0; p->lat_speed = 1.0;
+    p->cooldown = 5.0; p->end_guard = 30.0;
+}
+int dp_world_set_lane_change(dp_ctx* c, const dp_lane_change_params* p, dp_lane_change_state* st) {
+    if (!c || (st && !p)) return fail(DP_ERR_ARG, "dp_world_set_lane_change: bad argument");
+    if (p) {
+        const double v[8] = {p->politeness, p->a_thr, p->b_safe, p->ego_b_safe, p->ego_front, p->lat_speed, p->cooldown, p->end_guard};
+        for (double x : v) if (!std::isfinite(x)) return fail(DP_ERR_ARG, "dp_world_set_lane_change: parameters must be finite");
+        if (!(p->lat_speed > 0) || !(p->b_safe > 0) || !(p->ego_b_safe > 0) || !(p->politeness >= 0) || !(p->cooldown >= 0) ||
+            !(p->end_guard >= 0) || !(p->ego_front >= 0))
+            return fail(DP_ERR_ARG, "dp_world_set_lane_change: lat_speed, b_safe, ego_b_safe > 0 and politeness, cooldown, end_guard, ego_front >= 0");
+    }
+    if (st) {
+        if (!c->d_v0) return fail(DP_ERR_ARG, "dp_world_set_lane_change: the agent model is not armed (dp_world_set_agent_model)");
+        CK(cudaSetDevice(c->device));
+        CK(dp_world_lanechange_prepare());                  // function attributes are set before any launch or capture of the armed step
+        c->lcp = *p;
+    }
+    c->d_lcs = st;
+    if (c->ep_exec) { cudaGraphExecDestroy(c->ep_exec); c->ep_exec = nullptr; }   // (the state pointer and parameters are baked into the graph)
     return DP_OK;
 }
 int dp_world_step_dev(dp_ctx* c, int first, int n, dp_scene_hdr* hdr, dp_agent* agents, double* ox, double* oy, const dp_plan_record* rec,
@@ -1462,7 +1491,7 @@ int dp_world_step_dev(dp_ctx* c, int first, int n, dp_scene_hdr* hdr, dp_agent* 
     CK(cudaSetDevice(c->device));
     c->launches += n > 0 ? 1 : 0;
     CK(dp_launch_world(c->gmap, c->p, c->wp, n, c->max_obs, hdr, agents, ox, oy, rec, c->d_last + (size_t)first * DP_PATH_POINTS,
-                       c->mp, c->d_met, c->amp, c->d_v0, (cudaStream_t)stream));
+                       c->mp, c->d_met, c->amp, c->d_v0, c->lcp, c->d_lcs, (cudaStream_t)stream));
     return DP_OK;
 }
 namespace {
@@ -1475,7 +1504,7 @@ cudaError_t enqueue_closed_loop(dp_ctx* c, int first, int n, int cycles, dp_scen
     // a replayed graph re-uses its hand-off epochs: the per-scene Decision -> Planning flags start every replay from 0
     if (rearm && (e = cudaMemsetAsync(c->d_done + first, 0, (size_t)n * sizeof(unsigned), st)) != cudaSuccess) return e;
     c->launches += 1;
-    if ((e = dp_launch_world(c->gmap, c->p, c->wp, n, c->max_obs, hdr, agents, ox, oy, nullptr, last, c->mp, c->d_met, c->amp, c->d_v0, st)) != cudaSuccess)
+    if ((e = dp_launch_world(c->gmap, c->p, c->wp, n, c->max_obs, hdr, agents, ox, oy, nullptr, last, c->mp, c->d_met, c->amp, c->d_v0, c->lcp, c->d_lcs, st)) != cudaSuccess)
         return e;
     for (int k = 0; k < cycles; ++k) {
         if (hdr_log && (e = cudaMemcpyAsync(hdr_log + (size_t)k * n, hdr, (size_t)n * sizeof(dp_scene_hdr), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
@@ -1485,7 +1514,7 @@ cudaError_t enqueue_closed_loop(dp_ctx* c, int first, int n, int cycles, dp_scen
         if ((e = run_cycle(c, first, n, hdr, ox, oy, rec + (size_t)k * n, nullptr, nullptr, nullptr, st, io)) != cudaSuccess) return e;
         c->launches += 1;
         if ((e = dp_launch_world(c->gmap, c->p, c->wp, n, c->max_obs, hdr, agents, ox, oy, rec + (size_t)k * n, last, c->mp, c->d_met, c->amp, c->d_v0,
-                                   st)) != cudaSuccess)
+                                   c->lcp, c->d_lcs, st)) != cudaSuccess)
             return e;
     }
     return cudaSuccess;

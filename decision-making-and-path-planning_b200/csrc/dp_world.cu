@@ -3,7 +3,8 @@
 //                     lanes, windowed re-localisation; one warp per scene, everything in place in HBM
 //                     (arithmetic frozen in oracle/world_spec.cpp, junction transitions in tools/junction_oracle/world_junction.cpp;
 //                     IEEE binary64, -fmad=false, operations in that order); the kernel is in dp_world_step.cuh, its
-//                     episode-metrics instances in dp_world_metrics.cu, its reactive-agent instances in dp_world_agents.cu;
+//                     episode-metrics instances in dp_world_metrics.cu, its reactive-agent instances in dp_world_agents.cu,
+//                     its lane-changing instances in dp_world_lanechange.cu;
 //   dp_v2x_kernel     the V2X event handlers (Decision.cpp:1824-2434) as a batch operator next to the cycle;
 //   dp_frames_kernel  the output stage: PlanningOut / PlanningStatus (Planning.cpp:173-214) packed into fixed-layout frames
 //                     from the plan record and the carried local path -- byte work bound by HBM: a warp streams one scene
@@ -212,10 +213,12 @@ cudaError_t dp_launch_v2x(const DevMap& m, const dp_params& p, int n, const dp_s
 cudaError_t dp_launch_world(const DevMap& m, const dp_params& p, const dp_world_params& wp, int n, int max_obs, dp_scene_hdr* hdr,
                             dp_agent* agents, double* obs_x, double* obs_y, const dp_plan_record* rec, const double2* last_path,
                             const dp_metrics_params& mp, dp_episode_metrics* met, const dp_agent_model_params& amp, const double* v0,
-                            cudaStream_t st) {
+                            const dp_lane_change_params& lcp, dp_lane_change_state* lcs, cudaStream_t st) {
     if (n <= 0) return cudaSuccess;
     const int g = (n + WPB - 1) / WPB;
     const bool junc = wp.pre_junction_pts > 0;
+    if (v0 && lcs)
+        return dp_launch_world_lanechange(m, p, wp, n, max_obs, hdr, agents, obs_x, obs_y, rec, last_path, mp, met, amp, v0, lcp, lcs, st);
     if (v0) return dp_launch_world_agents(m, p, wp, n, max_obs, hdr, agents, obs_x, obs_y, rec, last_path, mp, met, amp, v0, st);
     if (met) return dp_launch_world_metrics(m, p, wp, n, max_obs, hdr, agents, obs_x, obs_y, rec, last_path, mp, met, st);
     const AgentModel am = {amp, nullptr};

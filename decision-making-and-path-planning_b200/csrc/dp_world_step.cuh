@@ -1,8 +1,8 @@
 // csrc/dp_world_step.cuh -- the world step of the closed-loop episode runner (dp_world_kernel, see dp_world.cu), with the
-// episode metrics of include/dmpp_b200.h section 11 and the reactive agents of section 12 as compile-time options.  dp_world.cu
-// instantiates the disarmed kernels (METRICS = REACT = false), dp_world_metrics.cu the metrics instances and dp_world_agents.cu
-// the reactive ones: kept in separate translation units, the disarmed instances compile to exactly what they compiled to before
-// the options existed.
+// episode metrics of include/dmpp_b200.h section 11, the reactive agents of section 12 and their lane changes (section 13) as
+// compile-time options.  dp_world.cu instantiates the disarmed kernels (METRICS = REACT = false), dp_world_metrics.cu the
+// metrics instances, dp_world_agents.cu the reactive ones and dp_world_lanechange.cu the lane-changing ones: kept in separate
+// translation units, the disarmed instances compile to exactly what they compiled to before the options existed.
 #pragma once
 #include <type_traits>
 
@@ -154,13 +154,177 @@ struct AgentModel {
     dp_agent_model_params p;
     const double* v0;                  // [n][max_obs] desired speeds
 };
+// the model of the LANECHG instances (section 13): the agent model plus the lane-change parameters and states.  A type of its own,
+// so that the kernel parameters of the other instances stay what they were
+struct LaneChangeModel : AgentModel {
+    dp_lane_change_params lc;
+    dp_lane_change_state* lcs;         // [n][max_obs]
+};
 
 // length of map lane gl: the last entry of its sequential prefix of segment lengths
 __device__ __forceinline__ double lane_len(const DevMap& m, int gl) { return m.cump[m.lane_pt_off[gl + 1] - 1]; }
 
+// ---- lane-changing agents (include/dmpp_b200.h section 13): MOBIL on the react phase's staging ----
+static_assert(sizeof(dp_lane_change_state) == 24, "dp_lane_change_state is 24 bytes");
+
+// section 12's IDM acceleration with its clamp (lead false: free road); sab = 2.0 * sqrt(a_max * b)
+__device__ __forceinline__ double lc_idm(const dp_agent_model_params& p, double sab, double v, double vd, bool lead, double g, double vl) {
+    const double r = v / vd;
+    double fr = r * r;
+    fr = fr * fr;
+    double acc;
+    if (lead) {
+        const double dv = v - vl;
+        double z = v * p.T + v * dv / sab;
+        if (z < 0) z = 0;
+        const double ss = p.s0 + z;
+        if (g > 0) { const double q = ss / g; acc = p.a_max * (1.0 - fr - q * q); }
+        else acc = -p.b_max;
+    } else acc = p.a_max * (1.0 - fr);
+    if (acc < -p.b_max) acc = -p.b_max;
+    return acc;
+}
+
+// the ego as a follower: the interaction term alone (its v0 is unknown), 0 without a leader
+__device__ __forceinline__ double lc_ego_idm(const dp_agent_model_params& p, double sab, double v, bool lead, double g, double vl) {
+    if (!lead) return 0.0;
+    const double dv = v - vl;
+    double z = v * p.T + v * dv / sab;
+    if (z < 0) z = 0;
+    const double ss = p.s0 + z;
+    double acc;
+    if (g > 0) { const double q = ss / g; acc = -p.a_max * (q * q); }
+    else acc = -p.b_max;
+    if (acc < -p.b_max) acc = -p.b_max;
+    return acc;
+}
+
+// an agent that does not change lanes this step: its hold runs down and its lat moves back towards lat_goal
+__device__ __forceinline__ void lc_relax(const dp_lane_change_params& c, double dt, double& lat, dp_lane_change_state& s) {
+    s.hold = s.hold - dt;
+    if (lat != s.lat_goal) {
+        const double e = s.lat_goal - lat, w = c.lat_speed * dt;
+        lat = fabs(e) <= w ? s.lat_goal : (e > 0 ? lat + w : lat - w);
+    }
+}
+
+struct LcSide { bool ok; double delta, atc; int im; };
+
+// one side of agent k: target lane ml, abeam station, leader and follower on ml alone, safety and incentive.  (i, u): the agent's
+// point and offset; (v, vd, ac): its start-of-step speed, desired speed and react-phase acceleration; (le, se, ve): the ego candidate
+__device__ __forceinline__ LcSide lc_side(const DevMap& m, const LaneChangeModel& am, double sab, const double2* SV, const int* L, int n_obs,
+                                          const double* v0, int le, double se, double ve, int ml, int i, double u, double v, double vd,
+                                          double ac) {
+    const dp_agent_model_params& p = am.p;
+    const dp_lane_change_params& c = am.lc;
+    LcSide r;
+    r.ok = false;
+    const int off = m.lane_pt_off[ml], cnt = m.lane_pt_off[ml + 1] - off;
+    r.im = min(i, cnt - 2);
+    const double sm = m.cump[off + r.im] + u;
+    if (!(m.cump[off + cnt - 1] - sm >= c.end_guard)) return r;
+    bool overlap = false, lead = false, foll = false, lego = false, fego = false;
+    double gl = 0, vl = 0, sl = 0, gf = 0, vf = 0, sf = 0;
+    int fj = -1;
+    if (le == ml) {
+        if (se == sm) overlap = true;
+        else if (se > sm) { const double ds = se - sm; if (ds <= p.look) { lead = lego = true; gl = ds - p.ego_rear; vl = ve; sl = se; } }
+        else { const double ds = sm - se; if (ds <= p.look) { foll = fego = true; gf = ds - c.ego_front; vf = ve; sf = se; } }
+    }
+    for (int j = 0; j < n_obs; ++j) {                       // warp-uniform j: broadcast reads
+        if (L[j] != ml) continue;
+        const double2 c2 = SV[j];
+        const double sj = c2.x;
+        if (sj == sm) overlap = true;
+        else if (sj > sm) {
+            const double ds = sj - sm;
+            if (ds <= p.look) {
+                const double g = ds - p.length;
+                if (!lead || g < gl) { gl = g; vl = c2.y; sl = sj; lead = true; lego = false; }
+            }
+        } else {
+            const double ds = sm - sj;
+            if (ds <= p.look) {
+                const double g = ds - p.length;
+                if (!foll || g < gf) { gf = g; vf = c2.y; sf = sj; fj = j; foll = true; fego = false; }
+            }
+        }
+    }
+    if (overlap || (lead && !(gl > 0)) || (foll && !(gf > 0))) return r;
+    r.atc = lc_idm(p, sab, v, vd, lead, gl, vl);
+    double af = 0, atf = 0;
+    if (fego) {
+        af = lc_ego_idm(p, sab, vf, lead, (sl - sf) - c.ego_front, vl);
+        atf = lc_ego_idm(p, sab, vf, true, gf, v);
+        if (!(atf >= -c.ego_b_safe)) return r;
+    } else if (foll) {
+        const double vdf = v0[fj];
+        if (vdf > 0) {
+            af = lc_idm(p, sab, vf, vdf, lead, (sl - sf) - (lego ? p.ego_rear : p.length), vl);
+            atf = lc_idm(p, sab, vf, vdf, true, gf, v);
+        }
+        if (!(atf >= -c.b_safe)) return r;
+    }
+    r.delta = (r.atc - ac) + c.politeness * (atf - af);
+    r.ok = r.delta > c.a_thr;
+    return r;
+}
+
+// agent k after its react phase (acc = a_c, vn = section 12's new speed): MOBIL, then the change or the relaxation; writes the
+// agent and its lane-change state once
+__device__ __forceinline__ void lane_change_agent(const DevMap& m, const LaneChangeModel& am, double sab, const double2* SV, const int* L,
+                                                  int n_obs, const double* v0, int le, double se, double ve, double dt, int k, double v,
+                                                  double vd, double acc, double vn, dp_agent* ag, dp_lane_change_state* lcs) {
+    const dp_lane_change_params& c = am.lc;
+    dp_agent a = ag[k];
+    dp_lane_change_state s = lcs[k];
+    const int l0 = a.lane;
+    if (l0 < m.road_lane_base[m.n_roads] && a.lat == s.lat_goal && s.hold <= 0 && lane_len(m, l0) - SV[k].x >= c.end_guard) {
+        int lo = 1, hi = m.n_roads;                         // the road r: road_lane_base[r-1] <= l0 < road_lane_base[r]
+        while (lo < hi) {
+            const int mid = (lo + hi) >> 1;
+            if (m.road_lane_base[mid] <= l0) lo = mid + 1;
+            else hi = mid;
+        }
+        const int b0 = m.road_lane_base[lo - 1], q = l0 - b0, nl = m.road_lane_base[lo] - b0;
+        const int attr = m.attr[m.lane_pt_off[l0] + a.i];
+        LcSide best;
+        best.ok = false;
+        int side = 0;
+        if (q >= 1 && (attr == 1 || attr == 3)) {
+            best = lc_side(m, am, sab, SV, L, n_obs, v0, le, se, ve, l0 - 1, a.i, a.u, v, vd, acc);
+            side = -1;
+        }
+        if (q + 1 < nl && (attr == 2 || attr == 3)) {
+            const LcSide rs = lc_side(m, am, sab, SV, L, n_obs, v0, le, se, ve, l0 + 1, a.i, a.u, v, vd, acc);
+            if (rs.ok && (!best.ok || rs.delta > best.delta)) { best = rs; side = 1; }
+        }
+        if (best.ok) {
+            const int ml = l0 + side, om = m.lane_pt_off[ml];
+            const double2 P = m.xy[m.lane_pt_off[l0] + a.i], Q = m.xy[om + best.im], R = m.xy[om + best.im + 1];
+            const double dx = R.x - Q.x, dy = R.y - Q.y, Ls = sqrt(dx * dx + dy * dy);
+            const double d = Ls > 0 ? (P.x - Q.x) * (-(dy / Ls)) + (P.y - Q.y) * (dx / Ls) : 0.0;
+            a.lat = a.lat + d; a.lane = ml; a.i = best.im;
+            double vc = v + best.atc * dt;
+            if (vc < 0) vc = 0;
+            a.v = vc;
+            s.hold = c.cooldown;
+            if (side < 0) s.changes_left += 1;
+            else s.changes_right += 1;
+            ag[k] = a; lcs[k] = s;
+            return;
+        }
+    }
+    a.v = vn;
+    lc_relax(c, dt, a.lat, s);
+    ag[k] = a; lcs[k] = s;
+}
+
 // rewrite agents[].v of one scene from the state at the start of the step (Jacobi): stage (lane, s, v) of every agent in the
-// warp's slice of dynamic shared memory, then each lane scans the staged candidates for each of its agents (broadcast reads)
-__device__ __forceinline__ void react_step(const DevMap& m, const AgentModel& am, const dp_scene_hdr& h, int pos, int n_obs, double dt,
+// warp's slice of dynamic shared memory, then each lane scans the staged candidates for each of its agents (broadcast reads).
+// LANECHG: each agent's lane change (section 13) follows its IDM step on the same staging.
+template <bool LANECHG, class Model>
+__device__ __forceinline__ void react_step(const DevMap& m, const Model& am, const dp_scene_hdr& h, int pos, int n_obs, double dt,
                                            dp_agent* ag, const double* v0, unsigned char* stage, int max_obs, int lane) {
     double2* SV = reinterpret_cast<double2*>(stage);
     int* L = reinterpret_cast<int*>(SV + max_obs);
@@ -189,7 +353,16 @@ __device__ __forceinline__ void react_step(const DevMap& m, const AgentModel& am
     __syncwarp();
     for (int k = lane; k < n_obs; k += 32) {
         const double vd = v0[k];
-        if (!(vd > 0)) continue;
+        if (!(vd > 0)) {
+            if constexpr (LANECHG) {
+                dp_lane_change_state* lcs = am.lcs + (v0 - am.v0);   // the scene's states: indexed like v0
+                dp_lane_change_state s = lcs[k];
+                double lat = ag[k].lat;
+                lc_relax(am.lc, dt, lat, s);
+                ag[k].lat = lat; lcs[k] = s;
+            }
+            continue;
+        }
         const double2 own = SV[k];
         const double sk = own.x, v = own.y;
         const int l0 = L[k], l1 = m.lane_next[l0], l2 = l1 >= 0 ? m.lane_next[l1] : -1;
@@ -232,7 +405,8 @@ __device__ __forceinline__ void react_step(const DevMap& m, const AgentModel& am
         if (acc < -p.b_max) acc = -p.b_max;
         double vn = v + acc * dt;
         if (vn < 0) vn = 0;
-        ag[k].v = vn;
+        if constexpr (LANECHG) lane_change_agent(m, am, sab, SV, L, n_obs, v0, le, se, ve, dt, k, v, vd, acc, vn, ag, am.lcs + (v0 - am.v0));
+        else ag[k].v = vn;
     }
 }
 
@@ -241,12 +415,15 @@ __device__ __forceinline__ void react_step(const DevMap& m, const AgentModel& am
 // scene's row at entry and write it at the end as one coalesced 192-byte access each, staged behind the header in shared memory.
 // REACT = reactive agents armed (am.v0 != nullptr): before the agent loop the armed instances rewrite agents[].v (react_step),
 // staging max_obs * REACT_SLOT_BYTES of dynamic shared memory per warp.
-template <bool JUNC, bool METRICS, bool REACT>
+// LANECHG = lane changes armed (am.lcs != nullptr, REACT instances only): the react phase is followed per agent by the lane
+// change of section 13 on the same staging; the placement step initialises the states.
+template <bool JUNC, bool METRICS, bool REACT, bool LANECHG = false>
 __global__ void __launch_bounds__(WPB * 32, (METRICS || REACT) ? 8 : 0) dp_world_kernel(DevMap m, dp_params p, dp_world_params wp, int n, int max_obs,
                                                             dp_scene_hdr* __restrict__ hdr, dp_agent* __restrict__ agents,
                                                             double* __restrict__ obs_x, double* __restrict__ obs_y,
                                                             const dp_plan_record* __restrict__ rec, const double2* __restrict__ last_path,
-                                                            dp_metrics_params mp, dp_episode_metrics* __restrict__ met, AgentModel am) {
+                                                            dp_metrics_params mp, dp_episode_metrics* __restrict__ met,
+                                                            std::conditional_t<LANECHG, LaneChangeModel, AgentModel> am) {
     __shared__ __align__(16) uint32_t sh[WPB][METRICS ? 32 + 2 * MET_WORDS : 32];
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     const int scene = blockIdx.x * WPB + wib;
@@ -260,6 +437,18 @@ __global__ void __launch_bounds__(WPB * 32, (METRICS || REACT) ? 8 : 0) dp_world
             if (lane == 0) metrics_init(*reinterpret_cast<dp_episode_metrics*>(row));
             __syncwarp();
             if (lane < MET_WORDS) reinterpret_cast<double*>(met + scene)[lane] = row[lane];
+        }
+    }
+    if constexpr (LANECHG) {
+        static_assert(REACT, "lane changes run on the react phase");
+        if (rec == nullptr) {                               // placement step: clean states, whatever the header names
+            const int no = min((int)h.n_obs, max_obs);
+            for (int k = lane; k < no; k += 32) {
+                const size_t e = (size_t)scene * max_obs + k;
+                dp_lane_change_state s;
+                s.lat_goal = agents[e].lat; s.hold = 0; s.changes_left = 0; s.changes_right = 0;
+                am.lcs[e] = s;
+            }
         }
     }
     // a header that does not name a lane of the map (device-pointer callers are not validated on the host) leaves its world untouched
@@ -336,8 +525,8 @@ __global__ void __launch_bounds__(WPB * 32, (METRICS || REACT) ? 8 : 0) dp_world
     if constexpr (REACT) {
         if (step) {
             extern __shared__ __align__(16) unsigned char react_stage[];
-            react_step(m, am, h, pos, n_obs, dt, agents + (size_t)scene * max_obs, am.v0 + (size_t)scene * max_obs,
-                       react_stage + wib * react_stage_bytes(max_obs), max_obs, lane);
+            react_step<LANECHG>(m, am, h, pos, n_obs, dt, agents + (size_t)scene * max_obs, am.v0 + (size_t)scene * max_obs,
+                                react_stage + wib * react_stage_bytes(max_obs), max_obs, lane);
         }
     }
     // ---- agents: constant speed along their lanes (junctions on: and on into the lane's successor), then their obstacle points ----

@@ -27,6 +27,7 @@ SYMBOLS = [
     "dp_pack_frames_dev", "dp_pack_frames", "dp_world_default_params", "dp_world_set_params", "dp_world_step_dev",
     "dp_run_closed_loop_dev", "dp_closed_loop_is_graph", "dp_v2x_event_batch", "dp_v2x_event_batch_dev", "dp_v2x_apply", "dp_v2x_apply_dev",
     "dp_metrics_default_params", "dp_world_set_metrics", "dp_agent_model_default_params", "dp_world_set_agent_model",
+    "dp_lane_change_default_params", "dp_world_set_lane_change",
     "dp_gather_create", "dp_gather_attach", "dp_gather_arm", "dp_gather_chain", "dp_gather_arm_deferred", "dp_gather_set_lag", "dp_gather_flush", "dp_gather_disarm", "dp_gather_wait", "dp_gather_buffer", "dp_gather_destroy",
 ]
 
@@ -66,6 +67,13 @@ def agent_model_params():
     """dp_agent_model_default_params (no GPU needed)"""
     p = abi.AgentModelParams()
     load().dp_agent_model_default_params(C.byref(p))
+    return p
+
+
+def lane_change_params():
+    """dp_lane_change_default_params (no GPU needed)"""
+    p = abi.LaneChangeParams()
+    load().dp_lane_change_default_params(C.byref(p))
     return p
 
 
@@ -241,6 +249,15 @@ class Planner:
         _ck(self.lib.dp_world_set_agent_model(self.ctx, C.byref(params) if params is not None else None, C.c_void_p(d_v0 or 0)),
             "dp_world_set_agent_model")
 
+    def lane_change_params(self):
+        return lane_change_params()
+
+    def set_lane_change(self, params, d_state):
+        """arm the lane-changing agents (include/dmpp_b200.h section 13; the agent model must be armed): d_state = device address of
+        dp_lane_change_state [n][max_obs] indexed like hdr, initialised by the placement step; d_state None / 0 disarms"""
+        _ck(self.lib.dp_world_set_lane_change(self.ctx, C.byref(params) if params is not None else None, C.c_void_p(d_state or 0)),
+            "dp_world_set_lane_change")
+
     def world_step_dev(self, n, d_hdr, d_agents, d_ox, d_oy, d_rec=None, first=0, stream=0):
         _ck(self.lib.dp_world_step_dev(self.ctx, C.c_int(first), C.c_int(n), C.c_void_p(d_hdr), C.c_void_p(d_agents), C.c_void_p(d_ox),
                                        C.c_void_p(d_oy), C.c_void_p(d_rec or 0), C.c_void_p(stream)), "dp_world_step_dev")
@@ -255,13 +272,15 @@ class Planner:
     def closed_loop_is_graph(self):
         return bool(self.lib.dp_closed_loop_is_graph(self.ctx))
 
-    def run_closed_loop(self, hdr, agents, cycles, log=True, repeat=1, metrics=None, agent_model=None):
+    def run_closed_loop(self, hdr, agents, cycles, log=True, repeat=1, metrics=None, agent_model=None, lane_change=None):
         """host arrays in, host arrays out (the same dictionary as oracle.binding's run_closed_loop); `repeat` > 1 replays the
         episode from the same initial world (same device buffers, i.e. the cached graph) and returns the last run.
         metrics: None, or MetricsParams: the episode metrics are armed for this call (and disarmed after it) and the rows are
         returned under the key "metrics".  agent_model: None, or (AgentModelParams, v0[n][max_obs] desired speeds in m/s): the
-        reactive agents are armed for this call (and disarmed after it)."""
+        reactive agents are armed for this call (and disarmed after it).  lane_change: None, or LaneChangeParams (needs
+        agent_model): the agents also change lanes for this call, and their final states are returned under "lane_change_state"."""
         n, mo = agents.shape
+        assert lane_change is None or agent_model is not None, "lane changes run on the reactive agents"
         assert mo == self.max_obs and hdr.shape == (n,)
         sizes = {"hdr": n * 128, "agents": n * mo * 32, "ox": n * mo * 8, "oy": n * mo * 8, "rec": cycles * n * 128,
                  "hdr_log": cycles * n * 128, "obs_log_x": cycles * n * mo * 8, "obs_log_y": cycles * n * mo * 8}
@@ -272,6 +291,8 @@ class Planner:
             v0 = np.ascontiguousarray(v0, np.float64)
             assert v0.shape == (n, mo)
             sizes["v0"] = n * mo * 8
+        if lane_change is not None:
+            sizes["lane_change_state"] = n * mo * abi.lane_change_state.itemsize
         d = {}
         try:
             for k, b in sizes.items():
@@ -284,6 +305,8 @@ class Planner:
             if agent_model is not None:
                 _ck(self.lib.dp_memcpy_h2d(self.ctx, C.c_void_p(d["v0"]), abi.ptr(v0), C.c_size_t(sizes["v0"]), None), "h2d")
                 self.set_agent_model(am, d["v0"])
+            if lane_change is not None:
+                self.set_lane_change(lane_change, d["lane_change_state"])
             h0, a0 = np.ascontiguousarray(hdr), np.ascontiguousarray(agents)
             for _ in range(repeat):
                 self.reset(0, n)
@@ -299,6 +322,8 @@ class Planner:
                 o.update(hdr_log=np.zeros((cycles, n), abi.scene_hdr), obs_log_x=np.zeros((cycles, n, mo)), obs_log_y=np.zeros((cycles, n, mo)))
             if metrics is not None:
                 o["metrics"] = np.zeros(n, abi.episode_metrics)
+            if lane_change is not None:
+                o["lane_change_state"] = np.zeros((n, mo), abi.lane_change_state)
             for k in o:
                 _ck(self.lib.dp_memcpy_d2h(self.ctx, abi.ptr(o[k]), C.c_void_p(d[k]), C.c_size_t(sizes[k]), None), "d2h")
             _ck(self.lib.dp_stream_sync(self.ctx, None), "sync")
@@ -308,6 +333,8 @@ class Planner:
         finally:
             if metrics is not None:
                 self.set_metrics(None, None)
+            if lane_change is not None:
+                self.set_lane_change(None, None)
             if agent_model is not None:
                 self.set_agent_model(None, None)
             for p in d.values():

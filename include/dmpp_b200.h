@@ -563,7 +563,7 @@ int dp_world_set_metrics(dp_ctx* ctx, const dp_metrics_params* p, dp_episode_met
  * other agent and of the ego); the agent motion of section 9 then runs unchanged with the new v.  It runs on steps with
  * rec != NULL on headers that name a lane (the same early return as the step), for agents k < min(n_obs, max_obs).  With the
  * model disarmed (the default) nothing changes.  The arithmetic is frozen in tools/junction_oracle/agent_model.h.
- * Out of scope: lateral behaviour (agent lane changes and merges); yielding to a vehicle on a DIFFERENT connector that merges
+ * Lane changes are section 13, on top of this model.  Out of scope: merges; yielding to a vehicle on a DIFFERENT connector that merges
  * into the same lane (it is seen only once it is on the chain); any change to how the ego moves.
  *
  * IEEE binary64, operations in the order written, no contraction; min updates are `if (x < m) m = x`.
@@ -607,6 +607,74 @@ void dp_agent_model_default_params(dp_agent_model_params* p);
  * episode graph is rebuilt on its next call.  DP_ERR_ARG for non-finite parameters, a_max, b, b_max, T, length, look <= 0,
  * s0, ego_rear < 0, or a context max_obs above DP_AGENT_MODEL_MAX_OBS. */
 int dp_world_set_agent_model(dp_ctx* ctx, const dp_agent_model_params* p, const double* v0);
+
+/* (13) Lane-changing agents (opt-in, on top of the reactive agents of section 12): MOBIL ("minimising overall braking induced
+ * by lane changes", Kesting / Treiber / Helbing) with the IDM accelerations of section 12.  The model runs on the steps of
+ * section 12 (rec != NULL, a header that names a lane), for agents k < min(n_obs, max_obs), from the same start-of-step state
+ * (Jacobi): stations s, speeds v and lanes of every agent and the ego as section 12 reads them.  It may move an agent to a
+ * neighbouring lane of its road where the map allows it (lanechg_attr), rewriting its lane / i / lat / v; the agent motion of
+ * section 9 then runs unchanged.  Disarmed (the default) nothing changes.  The arithmetic is frozen in
+ * tools/junction_oracle/lane_change.h.  Uses the agent model's parameters (a_max, b, b_max, T, s0, length, ego_rear, look) and
+ * v0.  Two agents may pick the same gap in the same step (Jacobi): they are not arbitrated; the metrics see the outcome.
+ * Out of scope: changes on connectors, merges between connectors, any change to how the ego moves.
+ *
+ * IEEE binary64, operations in the order written, no contraction.  Per agent k, with a_c = its clamped IDM acceleration of
+ * section 12 (the value before vn = v + acc * dt), v = its start-of-step speed, st = its dp_lane_change_state:
+ *   placement (rec == NULL, every scene, also a header that names no lane): st = {lat_goal = agents[k].lat, hold = 0, 0, 0}
+ *   eligible  v0[k] > 0, l0 = its lane < road_lane_base[n_roads] (a road lane), lat == lat_goal, hold <= 0,
+ *             len(l0) - s_k >= end_guard
+ *   sides     road r with road_lane_base[r-1] <= l0 < road_lane_base[r] (binary search), lane number q = l0 - road_lane_base[r-1];
+ *             attr = lanechg_attr[off(l0) + i]; left: m = l0 - 1 when q >= 1 and attr is 1 or 3; right: m = l0 + 1 when
+ *             q + 1 < lanes of r and attr is 2 or 3.  Left is evaluated first.
+ *   abeam     i_m = min(i, cnt(m) - 2), s_m = cump[off(m) + i_m] + u (exact for lanes sampled abeam, as scenes.Map builds
+ *             them; an approximation for maps that are not); the side needs len(m) - s_m >= end_guard
+ *   candidates on m alone (no chain): the ego (section 12's lane and s_e, when that lane is m) and every agent j with lane m;
+ *             S == s_m for any of them: overlap, the side is unsafe; ahead (S > s_m) with ds = S - s_m <= look, behind (S < s_m)
+ *             with ds = s_m - S <= look.  leader: the ahead candidate with the smallest g, g = ds - length (an agent) or
+ *             ds - ego_rear (the ego); follower: the behind candidate with the smallest g, g = ds - length (an agent) or
+ *             ds - ego_front (the ego); the ego first on a tie, then the lowest agent index (`if (g < best)` in index order)
+ *   IDM       idm(v, v0, lead, g, vl) is section 12's acceleration, clamp at -b_max included (free road without a leader):
+ *               r = v / v0; fr = r * r; fr = fr * fr; leader: dv = v - vl; z = v * T + v * dv / (2.0 * sqrt(a_max * b));
+ *               if (z < 0) z = 0; ss = s0 + z; g > 0 ? a_max * (1.0 - fr - (ss / g) * (ss / g)) : -b_max;
+ *               free: a_max * (1.0 - fr); then if (acc < -b_max) acc = -b_max
+ *             the ego as follower knows no v0 and may stand: only the interaction term, with q = ss / g:
+ *               g > 0 ? -a_max * (q * q) : -b_max, clamped at -b_max; 0 without a leader
+ *   MOBIL     at_c = idm(v, v0[k], leader?, g_leader, v_leader)                                 (agent k on m)
+ *             a_f  = the follower f behind the leader: gap S_l - S_f (stations subtracted directly) minus length (agent leader),
+ *                    ego_rear (ego leader) or ego_front (ego follower); no leader: free road (ego: 0)
+ *             at_f = the follower behind agent k: its own g above, leader speed v
+ *             an agent follower with !(v0[f] > 0): a_f = at_f = 0; no follower: a_f = at_f = 0
+ *             safe:      no overlap, (no leader or g_leader > 0), (no follower or g_follower > 0),
+ *                        at_f >= -b_safe (agent follower) / >= -ego_b_safe (ego follower)
+ *             incentive: delta = (at_c - a_c) + politeness * (at_f - a_f) > a_thr  (the old follower is deliberately left out)
+ *             both sides safe and above threshold: the larger delta, left on a tie
+ *   change    lane = m, i = i_m, u unchanged; P = point i of l0, Q / R = points i_m / i_m + 1 of m, (dx, dy) = R - Q,
+ *             L = sqrt(dx*dx + dy*dy), d = L > 0 ? (P.x - Q.x) * (-(dy / L)) + (P.y - Q.y) * (dx / L) : 0; lat = lat + d
+ *             (the obstacle point stays where it was); v = v + at_c * dt, if (v < 0) v = 0 (replaces section 12's speed);
+ *             hold = cooldown; changes_left or changes_right += 1
+ *   others    every agent k < min(n_obs, max_obs) that does not change this step (opted out, ineligible or not changing):
+ *             hold = hold - dt; if (lat != lat_goal) { e = lat_goal - lat; w = lat_speed * dt;
+ *             lat = fabs(e) <= w ? lat_goal : (e > 0 ? lat + w : lat - w); } */
+typedef struct dp_lane_change_params {
+    double politeness;               /* p, default 0.2 */
+    double a_thr;                    /* incentive threshold, m/s^2, default 0.2 */
+    double b_safe;                   /* an agent as the new follower must not need to brake harder than this, m/s^2, default 4.0 */
+    double ego_b_safe;               /* the same test when the new follower is the ego, default 4.0: the lever for cut-ins */
+    double ego_front;                /* ego box ahead of (x, y) when the ego is the follower, m, default 4.0 (= dp_metrics_params.front) */
+    double lat_speed;                /* lateral speed back to lat_goal, m/s, default 1.0 */
+    double cooldown;                 /* s between two changes of one agent, default 5.0 */
+    double end_guard;                /* no change within this many metres of the end of the agent's lane or the target lane, default 30 */
+} dp_lane_change_params;             /* 64 bytes */
+typedef struct dp_lane_change_state {
+    double lat_goal;                 /* the in-lane offset the agent returns to (its lat at placement) */
+    double hold;                     /* seconds until the agent may start another change */
+    int32_t changes_left, changes_right;
+} dp_lane_change_state;              /* 24 bytes, [n][max_obs] indexed like hdr (the s-th scene of every later call) */
+void dp_lane_change_default_params(dp_lane_change_params* p);
+/* st == NULL disarms (p may then be NULL).  Context state like dp_world_set_agent_model: the cached episode graph is rebuilt on
+ * its next call; disarming the agent model disarms lane changes too.  DP_ERR_ARG for non-finite parameters, lat_speed, b_safe,
+ * ego_b_safe <= 0, politeness, cooldown, end_guard, ego_front < 0, or arming while the agent model is disarmed. */
+int dp_world_set_lane_change(dp_ctx* ctx, const dp_lane_change_params* p, dp_lane_change_state* st);
 
 /* diagnostic: phase time stamps (globaltimer, ns) of the most recent cycle launch, one row of 32 per CTA (row b = scenes
  * [b*g, (b+1)*g) of the batch; stamp 0 = CTA start, stamp i = end of phase i of csrc/dp_group.cuh).  Only contexts created

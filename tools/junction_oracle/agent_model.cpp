@@ -9,12 +9,28 @@
 
 namespace agents {
 
-namespace {
 double lane_len(const junction::JMap& jm, int gl) { return jm.cump[jm.m.d.lane_pt_off[gl + 1] - 1]; }
-}  // namespace
+
+int ego_lane(const junction::JMap& jm, const dp_world_params& wp, const dp_scene_hdr& h0, double* se) {
+    const oracle::MapView& m = jm.m;
+    const int pos = (wp.pre_junction_pts > 0 && (h0.pos == 1 || h0.pos == 2)) ? h0.pos : 0;
+    int le = -1, idx = 0;
+    if (pos != 2) { le = m.lane_index(h0.road_num, h0.lane_num); idx = h0.id[h0.lane_num - 1]; }
+    else if (h0.conn >= 0 && h0.conn < m.d.n_conn && h0.last_lanenum >= 1 && h0.last_lanenum <= DP_LANESUM) {
+        le = m.d.conn[h0.conn].lane; idx = h0.id[h0.last_lanenum - 1];
+    }
+    *se = 0;
+    if (le >= 0) {
+        const int cnt = m.lane_size(le);
+        if (idx > cnt - 1) idx = cnt - 1;
+        if (idx < 0) idx = 0;
+        *se = jm.cump[m.d.lane_pt_off[le] + idx];
+    }
+    return le;
+}
 
 void react(const junction::JMap& jm, const dp_world_params& wp, const dp_agent_model_params& mp, const dp_scene_hdr& h0, dp_agent* ag,
-           int n, const double* v0) {
+           int n, const double* v0, double* acc_out) {
     const oracle::MapView& m = jm.m;
     if (!metrics::header_valid(m, h0)) return;
     const double inf = std::numeric_limits<double>::infinity();
@@ -27,19 +43,8 @@ void react(const junction::JMap& jm, const dp_world_params& wp, const dp_agent_m
         V[k] = ag[k].v; L[k] = ag[k].lane;
     }
     // the ego: lane, station, speed
-    const int pos = (wp.pre_junction_pts > 0 && (h0.pos == 1 || h0.pos == 2)) ? h0.pos : 0;
-    int le = -1, idx = 0;
-    if (pos != 2) { le = m.lane_index(h0.road_num, h0.lane_num); idx = h0.id[h0.lane_num - 1]; }
-    else if (h0.conn >= 0 && h0.conn < m.d.n_conn && h0.last_lanenum >= 1 && h0.last_lanenum <= DP_LANESUM) {
-        le = m.d.conn[h0.conn].lane; idx = h0.id[h0.last_lanenum - 1];
-    }
     double se = 0;
-    if (le >= 0) {
-        const int cnt = m.lane_size(le);
-        if (idx > cnt - 1) idx = cnt - 1;
-        if (idx < 0) idx = 0;
-        se = jm.cump[m.d.lane_pt_off[le] + idx];
-    }
+    const int le = ego_lane(jm, wp, h0, &se);
     const double ve = h0.velocity / 3.6;
     for (int k = 0; k < n; ++k) {
         const double vd = v0[k];
@@ -82,6 +87,7 @@ void react(const junction::JMap& jm, const dp_world_params& wp, const dp_agent_m
             else acc = -mp.b_max;
         } else acc = mp.a_max * (1.0 - fr);
         if (acc < -mp.b_max) acc = -mp.b_max;
+        if (acc_out) acc_out[k] = acc;
         double vn = v + acc * dt;
         if (vn < 0) vn = 0;
         ag[k].v = vn;

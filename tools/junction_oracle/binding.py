@@ -49,15 +49,17 @@ class JunctionOracle:
         assert self.lib.jo_world_step(C.byref(self.params), C.byref(wp), C.c_int(n), C.c_int(max_obs), abi.ptr(hdr), abi.ptr(agents),
                                       abi.ptr(ox), abi.ptr(oy), abi.ptr(rec), abi.ptr(last_path)) == 0
 
-    def run_closed_loop(self, hdr, agents, cycles, wp=None, paths=False, threads=1, metrics=None, agent_model=None):
+    def run_closed_loop(self, hdr, agents, cycles, wp=None, paths=False, threads=1, metrics=None, agent_model=None, lane_change=None):
         """hdr[n], agents[n][max_obs] (copied; the final world is returned); metrics = MetricsParams: the episode metrics of every
         world under "metrics" (jo_run_closed_loop_metrics); agent_model = (AgentModelParams, v0[n][max_obs]): the reactive agents
-        (jo_run_closed_loop_agents)"""
+        (jo_run_closed_loop_agents); lane_change = LaneChangeParams (with agent_model): their lane changes, the final states under
+        "lane_change_state" (jo_run_closed_loop_lanechg)"""
+        assert lane_change is None or agent_model is not None
         wp = wp or self.world_params()
         if metrics is None and agent_model is None:
             return ob._closed_loop(self.lib, "jo_run_closed_loop", self.params, wp, hdr, agents, cycles, paths, threads)
         n = hdr.shape[0]
-        met = None
+        met = lcs = None
         if metrics is not None:
             met = np.frombuffer(np.full(n * abi.episode_metrics.itemsize, 0xAB, np.uint8).tobytes(), abi.episode_metrics).copy()
         if agent_model is None:
@@ -68,6 +70,11 @@ class JunctionOracle:
             assert v0.shape == agents.shape
             name = "jo_run_closed_loop_agents"
             tail = (C.byref(metrics) if metrics is not None else None, abi.ptr(met), C.byref(am), abi.ptr(v0))
+            if lane_change is not None:
+                lcs = np.frombuffer(np.full(agents.size * abi.lane_change_state.itemsize, 0xAB, np.uint8).tobytes(),
+                                    abi.lane_change_state).reshape(agents.shape).copy()
+                name = "jo_run_closed_loop_lanechg"
+                tail = tail + (C.byref(lane_change), abi.ptr(lcs))
         f = getattr(self.lib, name)
         f.restype = C.c_longlong
 
@@ -77,6 +84,8 @@ class JunctionOracle:
         o = ob._closed_loop(_Lib, name, self.params, wp, hdr, agents, cycles, paths, threads)
         if met is not None:
             o["metrics"] = met
+        if lcs is not None:
+            o["lane_change_state"] = lcs
         return o
 
     def react_step(self, hdr, agents, v0, am, wp=None):
@@ -87,6 +96,20 @@ class JunctionOracle:
         assert v0.shape == agents.shape and hdr.shape == (n,) and agents.flags["C_CONTIGUOUS"]
         assert self.lib.jo_react_step(C.byref(wp), C.byref(am), C.c_int(n), C.c_int(max_obs), abi.ptr(np.ascontiguousarray(hdr)),
                                       abi.ptr(agents), abi.ptr(v0)) == 0
+
+    def lane_change_step(self, hdr, agents, v0, am, lp, lcs, wp=None):
+        """the react and lane-change phases alone, agents and lcs [n][max_obs] in place (jo_lane_change_step)"""
+        wp = wp or self.world_params()
+        n, max_obs = agents.shape
+        v0 = np.ascontiguousarray(v0, np.float64)
+        assert v0.shape == agents.shape == lcs.shape and hdr.shape == (n,) and agents.flags["C_CONTIGUOUS"] and lcs.flags["C_CONTIGUOUS"]
+        assert lcs.dtype == abi.lane_change_state
+        assert self.lib.jo_lane_change_step(C.byref(wp), C.byref(am), C.byref(lp), C.c_int(n), C.c_int(max_obs),
+                                            abi.ptr(np.ascontiguousarray(hdr)), abi.ptr(agents), abi.ptr(v0), abi.ptr(lcs)) == 0
+
+    def lane_change_sizeof(self):
+        """sizeof(dp_lane_change_params), sizeof(dp_lane_change_state)"""
+        return int(self.lib.jo_lane_change_sizeof(0)), int(self.lib.jo_lane_change_sizeof(1))
 
     def agent_model_sizeof(self):
         return int(self.lib.jo_agent_model_sizeof())

@@ -1,8 +1,9 @@
 // tools/junction_oracle/junction_api.cpp -- TEST INFRASTRUCTURE. C API of libjunction_oracle.so: the restated cycle of oracle/
 // (planner_oracle.cpp, compiled in unchanged) with the junction world step of world_junction.cpp between its cycles; the
 // same arrays as oracle_world_step / oracle_run_closed_loop of oracle/oracle_api.cpp; the episode metrics of
-// episode_metrics.cpp after every world step (jo_run_closed_loop_metrics, jo_metrics_step); and the reactive agents of
-// agent_model.cpp before every world step (jo_run_closed_loop_agents, jo_react_step).
+// episode_metrics.cpp after every world step (jo_run_closed_loop_metrics, jo_metrics_step); the reactive agents of
+// agent_model.cpp before every world step (jo_run_closed_loop_agents, jo_react_step); and their lane changes of lane_change.cpp
+// (jo_run_closed_loop_lanechg, jo_lane_change_step).
 #include <algorithm>
 #include <atomic>
 #include <cstring>
@@ -10,6 +11,7 @@
 #include <vector>
 #include "agent_model.h"
 #include "episode_metrics.h"
+#include "lane_change.h"
 #include "world_junction.h"
 #include "../../oracle/cshare_spec.h"
 
@@ -40,11 +42,13 @@ int jo_world_step(const dp_params* p, const dp_world_params* wp, int n, int max_
 
 namespace {
 // the closed loop of jo_run_closed_loop; mp / met non-null: the episode metrics accumulated after every world step; am / v0
-// non-null: the agents react (v0[n][max_obs]) before every world step
+// non-null: the agents react (v0[n][max_obs]) before every world step; lp / lcs non-null (with am): and change lanes, states
+// lcs[n][max_obs]
 long long closed_loop(const dp_params* p, const dp_world_params* wp, int n, int cycles, int max_obs, dp_scene_hdr* hdr, dp_agent* agents,
                       double* ox, double* oy, dp_plan_record* rec, dp_scene_hdr* hdr_log, double* obs_log_x, double* obs_log_y,
                       double* path_xy, dp_carry* carry_out, double* last_path_out, int threads, int32_t* ub_scene,
-                      const dp_metrics_params* mp, dp_episode_metrics* met, const dp_agent_model_params* am, const double* v0) {
+                      const dp_metrics_params* mp, dp_episode_metrics* met, const dp_agent_model_params* am, const double* v0,
+                      const dp_lane_change_params* lp, dp_lane_change_state* lcs) {
     if (!g_have_map) return -1;
     if (threads < 1) threads = 1;
     std::atomic<long long> ub(0);
@@ -58,6 +62,7 @@ long long closed_loop(const dp_params* p, const dp_world_params* wp, int n, int 
             double* sx = ox + (size_t)s * max_obs; double* sy = oy + (size_t)s * max_obs;
             junction::world_step(g_map, *p, *wp, hdr[s], ag, sx, sy, nullptr, nullptr, nullptr);
             if (met) metrics::init(met[s]);
+            if (lcs) lanechg::init(ag, std::min((int)hdr[s].n_obs, max_obs), lcs + (size_t)s * max_obs);
             for (int c = 0; c < cycles; ++c) {
                 const size_t e = (size_t)c * n + s;
                 if (hdr_log) hdr_log[e] = hdr[s];
@@ -69,7 +74,9 @@ long long closed_loop(const dp_params* p, const dp_world_params* wp, int n, int 
                 oracle::cycle(g_map.m, *p, hdr[s], sx, sy, st, o, false);
                 lub += o.ub_hits;
                 const dp_scene_hdr h0 = hdr[s];
-                if (am) agents::react(g_map, *wp, *am, h0, ag, std::min((int)h0.n_obs, max_obs), v0 + (size_t)s * max_obs);
+                if (lcs) lanechg::step(g_map, *wp, *am, *lp, h0, ag, std::min((int)h0.n_obs, max_obs), v0 + (size_t)s * max_obs,
+                                       lcs + (size_t)s * max_obs);
+                else if (am) agents::react(g_map, *wp, *am, h0, ag, std::min((int)h0.n_obs, max_obs), v0 + (size_t)s * max_obs);
                 junction::world_step(g_map, *p, *wp, hdr[s], ag, sx, sy, rec + e, st.last_x, st.last_y);
                 if (met) metrics::update(g_map, *wp, *mp, met[s], h0, hdr[s], ag, sx, sy, std::min((int)h0.n_obs, max_obs), rec[e]);
             }
@@ -99,7 +106,7 @@ long long jo_run_closed_loop(const dp_params* p, const dp_world_params* wp, int 
                              double* obs_log_y, double* path_xy, dp_carry* carry_out, double* last_path_out, int threads,
                              int32_t* ub_scene) {
     return closed_loop(p, wp, n, cycles, max_obs, hdr, agents, ox, oy, rec, hdr_log, obs_log_x, obs_log_y, path_xy, carry_out, last_path_out,
-                       threads, ub_scene, nullptr, nullptr, nullptr, nullptr);
+                       threads, ub_scene, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr);
 }
 
 // jo_run_closed_loop with the episode metrics of every world in met[n] (include/dmpp_b200.h section 11)
@@ -109,7 +116,7 @@ long long jo_run_closed_loop_metrics(const dp_params* p, const dp_world_params* 
                                      int32_t* ub_scene, const dp_metrics_params* mp, dp_episode_metrics* met) {
     if (!mp || !met) return -1;
     return closed_loop(p, wp, n, cycles, max_obs, hdr, agents, ox, oy, rec, hdr_log, obs_log_x, obs_log_y, path_xy, carry_out, last_path_out,
-                       threads, ub_scene, mp, met, nullptr, nullptr);
+                       threads, ub_scene, mp, met, nullptr, nullptr, nullptr, nullptr);
 }
 
 // jo_run_closed_loop with the reactive agents of include/dmpp_b200.h section 12 (am, v0[n][max_obs]); mp / met: the episode
@@ -121,7 +128,7 @@ long long jo_run_closed_loop_agents(const dp_params* p, const dp_world_params* w
                                     const double* v0) {
     if (!am || !v0 || (!mp) != (!met)) return -1;
     return closed_loop(p, wp, n, cycles, max_obs, hdr, agents, ox, oy, rec, hdr_log, obs_log_x, obs_log_y, path_xy, carry_out, last_path_out,
-                       threads, ub_scene, mp, met, am, v0);
+                       threads, ub_scene, mp, met, am, v0, nullptr, nullptr);
 }
 
 // the react phase alone, for every scene (agents[n][max_obs], v0[n][max_obs], k < min(n_obs, max_obs)), as the armed kernel runs
@@ -135,6 +142,31 @@ int jo_react_step(const dp_world_params* wp, const dp_agent_model_params* am, in
 }
 
 int jo_agent_model_sizeof(void) { return (int)sizeof(dp_agent_model_params); }
+
+// jo_run_closed_loop_agents with the lane changes of include/dmpp_b200.h section 13 (lp, states lcs[n][max_obs], initialised by
+// the placement step and holding the final states)
+long long jo_run_closed_loop_lanechg(const dp_params* p, const dp_world_params* wp, int n, int cycles, int max_obs, dp_scene_hdr* hdr,
+                                     dp_agent* agents, double* ox, double* oy, dp_plan_record* rec, dp_scene_hdr* hdr_log, double* obs_log_x,
+                                     double* obs_log_y, double* path_xy, dp_carry* carry_out, double* last_path_out, int threads,
+                                     int32_t* ub_scene, const dp_metrics_params* mp, dp_episode_metrics* met, const dp_agent_model_params* am,
+                                     const double* v0, const dp_lane_change_params* lp, dp_lane_change_state* lcs) {
+    if (!am || !v0 || !lp || !lcs || (!mp) != (!met)) return -1;
+    return closed_loop(p, wp, n, cycles, max_obs, hdr, agents, ox, oy, rec, hdr_log, obs_log_x, obs_log_y, path_xy, carry_out, last_path_out,
+                       threads, ub_scene, mp, met, am, v0, lp, lcs);
+}
+
+// the react and lane-change phases alone, for every scene, in place (agents and lcs [n][max_obs], k < min(n_obs, max_obs)), as the
+// armed kernel runs them at the start of a step with a record; a header that names no lane leaves its agents and states alone
+int jo_lane_change_step(const dp_world_params* wp, const dp_agent_model_params* am, const dp_lane_change_params* lp, int n, int max_obs,
+                        const dp_scene_hdr* hdr, dp_agent* agents, const double* v0, dp_lane_change_state* lcs) {
+    if (!g_have_map) return -1;
+    for (int s = 0; s < n; ++s)
+        lanechg::step(g_map, *wp, *am, *lp, hdr[s], agents + (size_t)s * max_obs, std::min((int)hdr[s].n_obs, max_obs),
+                      v0 + (size_t)s * max_obs, lcs + (size_t)s * max_obs);
+    return 0;
+}
+
+int jo_lane_change_sizeof(int which) { return which ? (int)sizeof(dp_lane_change_state) : (int)sizeof(dp_lane_change_params); }
 
 // one world step plus its metric update for every scene, as the armed kernel does it: rec == NULL initialises the rows (also for a
 // header that names no lane); a header that names no lane leaves its world and its row alone
