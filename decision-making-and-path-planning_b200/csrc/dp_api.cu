@@ -8,6 +8,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <initializer_list>
 #include <string>
 #include <algorithm>
 #include <atomic>
@@ -62,13 +63,8 @@ struct dp_ctx {
     double* d_pll[2] = {nullptr, nullptr};
     long long launches = 0;
     // closed-loop episodes (dp_run_closed_loop_dev): world-step parameters, the capture stream, the cached episode graph and its key
-    dp_world_params wp;
-    dp_metrics_params mp;                                   // episode metrics (dp_world_set_metrics): d_met == nullptr disarmed
-    dp_episode_metrics* d_met = nullptr;
-    dp_agent_model_params amp;                              // reactive agents (dp_world_set_agent_model): d_v0 == nullptr disarmed
-    const double* d_v0 = nullptr;
-    dp_lane_change_params lcp;                              // lane changes (dp_world_set_lane_change): d_lcs == nullptr disarmed
-    dp_lane_change_state* d_lcs = nullptr;
+    DpWorldOpts world;                                      // dp_world_set_params and the armed models (dp_world_set_metrics,
+                                                            // dp_world_set_agent_model, dp_world_set_lane_change)
     cudaStream_t ep_stream = nullptr;
     cudaGraphExec_t ep_exec = nullptr;
     const void* ep_key[8] = {}; int ep_dims[3] = {-1, -1, -1};
@@ -310,10 +306,10 @@ int dp_create(dp_ctx** out, int device, const dp_params* params, int max_scenes,
     if (const char* e = getenv("DP_SPLIT")) c->split = atoi(e);   // 0: one fused launch, 1: two launches back to back, 2: overlapped
     if (const char* e = getenv("DP_ZERO_COPY")) c->zero_copy = atoi(e) != 0;
     if (const char* e = getenv("DP_EPISODE_GRAPH")) c->ep_graph = atoi(e) != 0;
-    dp_world_default_params(&c->wp);
-    dp_metrics_default_params(&c->mp);
-    dp_agent_model_default_params(&c->amp);
-    dp_lane_change_default_params(&c->lcp);
+    dp_world_default_params(&c->world.wp);
+    dp_metrics_default_params(&c->world.mp);
+    dp_agent_model_default_params(&c->world.amp);
+    dp_lane_change_default_params(&c->world.lcp);
     // Kernel choice, from the measurements in profiles/README.md (round 2): the warp-per-scene kernel wins while a scene's
     // obstacles fit one warp pass (N < 32: 71 vs 96 us per 4096-scene cycle at N = 10); the group kernel, whose scans are flat
     // (trajectory, obstacle) lists with exact pruning, wins for crowded scenes (N = 200: 135 vs 212 us per 1024 junction scenes).
@@ -1408,11 +1404,21 @@ void dp_world_default_params(dp_world_params* p) {
     memset(p, 0, sizeof(*p));
     p->a_max = 3.0; p->loc_back = 8; p->loc_fwd = 56; p->end_margin = 160;
 }
+namespace {
+// the world options are baked into the launches of a cached episode graph: a change drops it
+int drop_episode_graph(dp_ctx* c) {
+    if (c->ep_exec) { cudaGraphExecDestroy(c->ep_exec); c->ep_exec = nullptr; }
+    return DP_OK;
+}
+bool all_finite(std::initializer_list<double> v) {
+    for (double x : v) if (!std::isfinite(x)) return false;
+    return true;
+}
+}  // namespace
 int dp_world_set_params(dp_ctx* c, const dp_world_params* p) {
     if (!c || !p || !(p->a_max >= 0) || p->loc_back < 0 || p->loc_fwd < 0) return fail(DP_ERR_ARG, "dp_world_set_params: bad argument");
-    c->wp = *p;
-    if (c->ep_exec) { cudaGraphExecDestroy(c->ep_exec); c->ep_exec = nullptr; }   // (the parameters are baked into the graph's launches)
-    return DP_OK;
+    c->world.wp = *p;
+    return drop_episode_graph(c);
 }
 void dp_metrics_default_params(dp_metrics_params* p) {
     if (!p) return;
@@ -1422,15 +1428,14 @@ void dp_metrics_default_params(dp_metrics_params* p) {
 int dp_world_set_metrics(dp_ctx* c, const dp_metrics_params* p, dp_episode_metrics* m) {
     if (!c || (m && !p)) return fail(DP_ERR_ARG, "dp_world_set_metrics: bad argument");
     if (p) {
-        const double v[5] = {p->front, p->rear, p->half_width, p->corridor_half, p->ttc_warn};
-        for (double x : v) if (!std::isfinite(x)) return fail(DP_ERR_ARG, "dp_world_set_metrics: parameters must be finite");
+        if (!all_finite({p->front, p->rear, p->half_width, p->corridor_half, p->ttc_warn}))
+            return fail(DP_ERR_ARG, "dp_world_set_metrics: parameters must be finite");
         if (!(p->front >= 0) || !(p->rear >= 0) || !(p->half_width > 0) || !(p->corridor_half >= 0) || !(p->ttc_warn >= 0))
             return fail(DP_ERR_ARG, "dp_world_set_metrics: front, rear, corridor_half, ttc_warn >= 0 and half_width > 0");
-        if (m) c->mp = *p;
+        if (m) c->world.mp = *p;
     }
-    c->d_met = m;
-    if (c->ep_exec) { cudaGraphExecDestroy(c->ep_exec); c->ep_exec = nullptr; }   // (the row pointer and parameters are baked into the graph)
-    return DP_OK;
+    c->world.met = m;
+    return drop_episode_graph(c);
 }
 void dp_agent_model_default_params(dp_agent_model_params* p) {
     if (!p) return;
@@ -1440,8 +1445,8 @@ void dp_agent_model_default_params(dp_agent_model_params* p) {
 int dp_world_set_agent_model(dp_ctx* c, const dp_agent_model_params* p, const double* v0) {
     if (!c || (v0 && !p)) return fail(DP_ERR_ARG, "dp_world_set_agent_model: bad argument");
     if (p) {
-        const double v[8] = {p->a_max, p->b, p->b_max, p->T, p->s0, p->length, p->ego_rear, p->look};
-        for (double x : v) if (!std::isfinite(x)) return fail(DP_ERR_ARG, "dp_world_set_agent_model: parameters must be finite");
+        if (!all_finite({p->a_max, p->b, p->b_max, p->T, p->s0, p->length, p->ego_rear, p->look}))
+            return fail(DP_ERR_ARG, "dp_world_set_agent_model: parameters must be finite");
         if (!(p->a_max > 0) || !(p->b > 0) || !(p->b_max > 0) || !(p->T > 0) || !(p->length > 0) || !(p->look > 0) || !(p->s0 >= 0) ||
             !(p->ego_rear >= 0))
             return fail(DP_ERR_ARG, "dp_world_set_agent_model: a_max, b, b_max, T, length, look > 0 and s0, ego_rear >= 0");
@@ -1450,13 +1455,12 @@ int dp_world_set_agent_model(dp_ctx* c, const dp_agent_model_params* p, const do
         if (c->max_obs > DP_AGENT_MODEL_MAX_OBS)
             return fail(DP_ERR_ARG, "dp_world_set_agent_model: the context's max_obs exceeds DP_AGENT_MODEL_MAX_OBS");
         CK(cudaSetDevice(c->device));
-        CK(dp_world_agents_prepare());                      // function attributes are set before any launch or capture of the armed step
-        c->amp = *p;
+        CK(dp_world_prepare());                             // function attributes are set before any launch or capture of the armed step
+        c->world.amp = *p;
     }
-    c->d_v0 = v0;
-    if (!v0) c->d_lcs = nullptr;                            // lane changes run on the react phase
-    if (c->ep_exec) { cudaGraphExecDestroy(c->ep_exec); c->ep_exec = nullptr; }   // (the speeds pointer and parameters are baked into the graph)
-    return DP_OK;
+    c->world.v0 = v0;
+    if (!v0) c->world.lcs = nullptr;                        // lane changes run on the react phase
+    return drop_episode_graph(c);
 }
 void dp_lane_change_default_params(dp_lane_change_params* p) {
     if (!p) return;
@@ -1467,21 +1471,20 @@ void dp_lane_change_default_params(dp_lane_change_params* p) {
 int dp_world_set_lane_change(dp_ctx* c, const dp_lane_change_params* p, dp_lane_change_state* st) {
     if (!c || (st && !p)) return fail(DP_ERR_ARG, "dp_world_set_lane_change: bad argument");
     if (p) {
-        const double v[8] = {p->politeness, p->a_thr, p->b_safe, p->ego_b_safe, p->ego_front, p->lat_speed, p->cooldown, p->end_guard};
-        for (double x : v) if (!std::isfinite(x)) return fail(DP_ERR_ARG, "dp_world_set_lane_change: parameters must be finite");
+        if (!all_finite({p->politeness, p->a_thr, p->b_safe, p->ego_b_safe, p->ego_front, p->lat_speed, p->cooldown, p->end_guard}))
+            return fail(DP_ERR_ARG, "dp_world_set_lane_change: parameters must be finite");
         if (!(p->lat_speed > 0) || !(p->b_safe > 0) || !(p->ego_b_safe > 0) || !(p->politeness >= 0) || !(p->cooldown >= 0) ||
             !(p->end_guard >= 0) || !(p->ego_front >= 0))
             return fail(DP_ERR_ARG, "dp_world_set_lane_change: lat_speed, b_safe, ego_b_safe > 0 and politeness, cooldown, end_guard, ego_front >= 0");
     }
     if (st) {
-        if (!c->d_v0) return fail(DP_ERR_ARG, "dp_world_set_lane_change: the agent model is not armed (dp_world_set_agent_model)");
+        if (!c->world.v0) return fail(DP_ERR_ARG, "dp_world_set_lane_change: the agent model is not armed (dp_world_set_agent_model)");
         CK(cudaSetDevice(c->device));
-        CK(dp_world_lanechange_prepare());                  // function attributes are set before any launch or capture of the armed step
-        c->lcp = *p;
+        CK(dp_world_prepare());                             // function attributes are set before any launch or capture of the armed step
+        c->world.lcp = *p;
     }
-    c->d_lcs = st;
-    if (c->ep_exec) { cudaGraphExecDestroy(c->ep_exec); c->ep_exec = nullptr; }   // (the state pointer and parameters are baked into the graph)
-    return DP_OK;
+    c->world.lcs = st;
+    return drop_episode_graph(c);
 }
 int dp_world_step_dev(dp_ctx* c, int first, int n, dp_scene_hdr* hdr, dp_agent* agents, double* ox, double* oy, const dp_plan_record* rec,
                       void* stream) {
@@ -1490,8 +1493,8 @@ int dp_world_step_dev(dp_ctx* c, int first, int n, dp_scene_hdr* hdr, dp_agent* 
     if (!c->have_map) return fail(DP_ERR_STATE, "dp_world_step_dev: map not uploaded");
     CK(cudaSetDevice(c->device));
     c->launches += n > 0 ? 1 : 0;
-    CK(dp_launch_world(c->gmap, c->p, c->wp, n, c->max_obs, hdr, agents, ox, oy, rec, c->d_last + (size_t)first * DP_PATH_POINTS,
-                       c->mp, c->d_met, c->amp, c->d_v0, c->lcp, c->d_lcs, (cudaStream_t)stream));
+    const DpWorldBufs b = {n, c->max_obs, hdr, agents, ox, oy, rec, c->d_last + (size_t)first * DP_PATH_POINTS};
+    CK(dp_launch_world(c->gmap, c->p, c->world, b, (cudaStream_t)stream));
     return DP_OK;
 }
 namespace {
@@ -1499,13 +1502,12 @@ namespace {
 cudaError_t enqueue_closed_loop(dp_ctx* c, int first, int n, int cycles, dp_scene_hdr* hdr, dp_agent* agents, double* ox, double* oy,
                                 dp_plan_record* rec, dp_scene_hdr* hdr_log, double* olx, double* oly, cudaStream_t st, bool rearm) {
     const size_t mo = (size_t)c->max_obs;
-    const double2* last = c->d_last + (size_t)first * DP_PATH_POINTS;
+    DpWorldBufs b = {n, c->max_obs, hdr, agents, ox, oy, nullptr, c->d_last + (size_t)first * DP_PATH_POINTS};
     cudaError_t e;
     // a replayed graph re-uses its hand-off epochs: the per-scene Decision -> Planning flags start every replay from 0
     if (rearm && (e = cudaMemsetAsync(c->d_done + first, 0, (size_t)n * sizeof(unsigned), st)) != cudaSuccess) return e;
     c->launches += 1;
-    if ((e = dp_launch_world(c->gmap, c->p, c->wp, n, c->max_obs, hdr, agents, ox, oy, nullptr, last, c->mp, c->d_met, c->amp, c->d_v0, c->lcp, c->d_lcs, st)) != cudaSuccess)
-        return e;
+    if ((e = dp_launch_world(c->gmap, c->p, c->world, b, st)) != cudaSuccess) return e;
     for (int k = 0; k < cycles; ++k) {
         if (hdr_log && (e = cudaMemcpyAsync(hdr_log + (size_t)k * n, hdr, (size_t)n * sizeof(dp_scene_hdr), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
         if (olx && (e = cudaMemcpyAsync(olx + (size_t)k * n * mo, ox, (size_t)n * mo * sizeof(double), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
@@ -1513,9 +1515,8 @@ cudaError_t enqueue_closed_loop(dp_ctx* c, int first, int n, int cycles, dp_scen
         const DpIo io = make_io(c, first, nullptr);
         if ((e = run_cycle(c, first, n, hdr, ox, oy, rec + (size_t)k * n, nullptr, nullptr, nullptr, st, io)) != cudaSuccess) return e;
         c->launches += 1;
-        if ((e = dp_launch_world(c->gmap, c->p, c->wp, n, c->max_obs, hdr, agents, ox, oy, rec + (size_t)k * n, last, c->mp, c->d_met, c->amp, c->d_v0,
-                                   c->lcp, c->d_lcs, st)) != cudaSuccess)
-            return e;
+        b.rec = rec + (size_t)k * n;
+        if ((e = dp_launch_world(c->gmap, c->p, c->world, b, st)) != cudaSuccess) return e;
     }
     return cudaSuccess;
 }

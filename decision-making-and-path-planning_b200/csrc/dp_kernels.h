@@ -49,30 +49,24 @@ cudaError_t dp_launch_cycle(const DevMap& m, const dp_params& p, int n, const dp
 // (io.prev_epoch != 0 additionally launches the Decision half as a programmatic dependent of the previous cycle's Planning half)
 // set the shared-memory attributes of the warp kernels (done lazily by dp_launch_cycle; called up front before a stream capture)
 void dp_launch_prepare(DpLaunchCfg& lc);
-// closed-loop world step and output frames (dp_world.cu); met != nullptr: episode metrics armed (include/dmpp_b200.h section 11);
-// v0 != nullptr: reactive agents armed (section 12); lcs != nullptr (with v0): lane changes armed (section 13)
-cudaError_t dp_launch_world(const DevMap& m, const dp_params& p, const dp_world_params& wp, int n, int max_obs, dp_scene_hdr* hdr,
-                            dp_agent* agents, double* obs_x, double* obs_y, const dp_plan_record* rec, const double2* last_path,
-                            const dp_metrics_params& mp, dp_episode_metrics* met, const dp_agent_model_params& amp, const double* v0,
-                            const dp_lane_change_params& lcp, dp_lane_change_state* lcs, cudaStream_t st);
-// ... its armed instances (dp_world_metrics.cu, met != nullptr); dp_launch_world forwards to it
-cudaError_t dp_launch_world_metrics(const DevMap& m, const dp_params& p, const dp_world_params& wp, int n, int max_obs, dp_scene_hdr* hdr,
-                                    dp_agent* agents, double* obs_x, double* obs_y, const dp_plan_record* rec, const double2* last_path,
-                                    const dp_metrics_params& mp, dp_episode_metrics* met, cudaStream_t st);
-// ... its reactive-agent instances (dp_world_agents.cu, v0 != nullptr, metrics armed or not); dp_launch_world forwards to it
-cudaError_t dp_launch_world_agents(const DevMap& m, const dp_params& p, const dp_world_params& wp, int n, int max_obs, dp_scene_hdr* hdr,
-                                   dp_agent* agents, double* obs_x, double* obs_y, const dp_plan_record* rec, const double2* last_path,
-                                   const dp_metrics_params& mp, dp_episode_metrics* met, const dp_agent_model_params& amp, const double* v0,
-                                   cudaStream_t st);
+// the closed-loop world step (dp_world_step.cuh): the buffers of one launch, and the option set a context arms.  A model is armed
+// by its pointer: met != nullptr episode metrics (include/dmpp_b200.h section 11), v0 != nullptr reactive agents (section 12),
+// lcs != nullptr with v0 lane changes (section 13); its parameters are read only while it is armed
+struct DpWorldBufs {
+    int n, max_obs;
+    dp_scene_hdr* hdr; dp_agent* agents; double* ox; double* oy;
+    const dp_plan_record* rec;                 // nullptr: the placement step
+    const double2* last_path;
+};
+struct DpWorldOpts {
+    dp_world_params wp;
+    dp_metrics_params mp; dp_episode_metrics* met = nullptr;
+    dp_agent_model_params amp; const double* v0 = nullptr;
+    dp_lane_change_params lcp; dp_lane_change_state* lcs = nullptr;
+};
+cudaError_t dp_launch_world(const DevMap& m, const dp_params& p, const DpWorldOpts& o, const DpWorldBufs& b, cudaStream_t st);
 // allow the reactive instances the dynamic shared memory of DP_AGENT_MODEL_MAX_OBS agent slots (current device; set before a capture)
-cudaError_t dp_world_agents_prepare();
-// ... its lane-changing instances (dp_world_lanechange.cu, lcs != nullptr, metrics armed or not); dp_launch_world forwards to it
-cudaError_t dp_launch_world_lanechange(const DevMap& m, const dp_params& p, const dp_world_params& wp, int n, int max_obs, dp_scene_hdr* hdr,
-                                       dp_agent* agents, double* obs_x, double* obs_y, const dp_plan_record* rec, const double2* last_path,
-                                       const dp_metrics_params& mp, dp_episode_metrics* met, const dp_agent_model_params& amp, const double* v0,
-                                       const dp_lane_change_params& lcp, dp_lane_change_state* lcs, cudaStream_t st);
-// the same shared-memory attribute for the lane-changing instances
-cudaError_t dp_world_lanechange_prepare();
+cudaError_t dp_world_prepare();
 cudaError_t dp_launch_v2x(const DevMap& m, const dp_params& p, int n, const dp_scene_hdr* hdr, const dp_v2x_data* v2x, const double* wp_lat,
                           const double* wp_lng, int mode, dp_v2x_flags* out, cudaStream_t st);
 cudaError_t dp_launch_v2x_apply(int n, const dp_v2x_flags* flags, dp_plan_record* rec, cudaStream_t st);

@@ -2,9 +2,10 @@
 //   dp_world_kernel   the world step of the closed-loop episode runner: ego walked along its own plan, agents along their
 //                     lanes, windowed re-localisation; one warp per scene, everything in place in HBM
 //                     (arithmetic frozen in oracle/world_spec.cpp, junction transitions in tools/junction_oracle/world_junction.cpp;
-//                     IEEE binary64, -fmad=false, operations in that order); the kernel is in dp_world_step.cuh, its
-//                     episode-metrics instances in dp_world_metrics.cu, its reactive-agent instances in dp_world_agents.cu,
-//                     its lane-changing instances in dp_world_lanechange.cu;
+//                     IEEE binary64, -fmad=false, operations in that order); the kernel and its launcher are in
+//                     dp_world_step.cuh, its disarmed instances here, its episode-metrics instances in dp_world_metrics.cu,
+//                     its reactive-agent instances in dp_world_agents.cu, its lane-changing instances in dp_world_lanechange.cu;
+//                     dp_launch_world picks the instance set from the armed options;
 //   dp_v2x_kernel     the V2X event handlers (Decision.cpp:1824-2434) as a batch operator next to the cycle;
 //   dp_frames_kernel  the output stage: PlanningOut / PlanningStatus (Planning.cpp:173-214) packed into fixed-layout frames
 //                     from the plan record and the carried local path -- byte work bound by HBM: a warp streams one scene
@@ -210,21 +211,19 @@ cudaError_t dp_launch_v2x(const DevMap& m, const dp_params& p, int n, const dp_s
     return cudaGetLastError();
 }
 
-cudaError_t dp_launch_world(const DevMap& m, const dp_params& p, const dp_world_params& wp, int n, int max_obs, dp_scene_hdr* hdr,
-                            dp_agent* agents, double* obs_x, double* obs_y, const dp_plan_record* rec, const double2* last_path,
-                            const dp_metrics_params& mp, dp_episode_metrics* met, const dp_agent_model_params& amp, const double* v0,
-                            const dp_lane_change_params& lcp, dp_lane_change_state* lcs, cudaStream_t st) {
-    if (n <= 0) return cudaSuccess;
-    const int g = (n + WPB - 1) / WPB;
-    const bool junc = wp.pre_junction_pts > 0;
-    if (v0 && lcs)
-        return dp_launch_world_lanechange(m, p, wp, n, max_obs, hdr, agents, obs_x, obs_y, rec, last_path, mp, met, amp, v0, lcp, lcs, st);
-    if (v0) return dp_launch_world_agents(m, p, wp, n, max_obs, hdr, agents, obs_x, obs_y, rec, last_path, mp, met, amp, v0, st);
-    if (met) return dp_launch_world_metrics(m, p, wp, n, max_obs, hdr, agents, obs_x, obs_y, rec, last_path, mp, met, st);
-    const AgentModel am = {amp, nullptr};
-    if (junc) dp_world_kernel<true, false, false><<<g, WPB * 32, 0, st>>>(m, p, wp, n, max_obs, hdr, agents, obs_x, obs_y, rec, last_path, mp, met, am);
-    else dp_world_kernel<false, false, false><<<g, WPB * 32, 0, st>>>(m, p, wp, n, max_obs, hdr, agents, obs_x, obs_y, rec, last_path, mp, met, am);
-    return cudaGetLastError();
+template struct WorldStep<false, false, false>;
+
+cudaError_t dp_launch_world(const DevMap& m, const dp_params& p, const DpWorldOpts& o, const DpWorldBufs& b, cudaStream_t st) {
+    if (b.n <= 0) return cudaSuccess;
+    if (o.v0 && o.lcs) return o.met ? WorldStep<true, true, true>::launch(m, p, o, b, st) : WorldStep<false, true, true>::launch(m, p, o, b, st);
+    if (o.v0) return o.met ? WorldStep<true, true, false>::launch(m, p, o, b, st) : WorldStep<false, true, false>::launch(m, p, o, b, st);
+    return o.met ? WorldStep<true, false, false>::launch(m, p, o, b, st) : WorldStep<false, false, false>::launch(m, p, o, b, st);
+}
+cudaError_t dp_world_prepare() {
+    for (auto prepare : {WorldStep<false, true, false>::prepare, WorldStep<true, true, false>::prepare, WorldStep<false, true, true>::prepare,
+                         WorldStep<true, true, true>::prepare})
+        if (const cudaError_t e = prepare(); e != cudaSuccess) return e;
+    return cudaSuccess;
 }
 cudaError_t dp_launch_frames(const dp_params& p, int n, const dp_plan_record* rec, const double2* last_path, dp_ctrl_frame* ctrl,
                              dp_status_frame* status, cudaStream_t st) {

@@ -1,8 +1,9 @@
 // csrc/dp_world_step.cuh -- the world step of the closed-loop episode runner (dp_world_kernel, see dp_world.cu), with the
 // episode metrics of include/dmpp_b200.h section 11, the reactive agents of section 12 and their lane changes (section 13) as
-// compile-time options.  dp_world.cu instantiates the disarmed kernels (METRICS = REACT = false), dp_world_metrics.cu the
-// metrics instances, dp_world_agents.cu the reactive ones and dp_world_lanechange.cu the lane-changing ones: kept in separate
-// translation units, the disarmed instances compile to exactly what they compiled to before the options existed.
+// compile-time options, and its launcher WorldStep<METRICS, REACT, LANECHG>.  dp_world.cu instantiates the disarmed kernels
+// (METRICS = REACT = false), dp_world_metrics.cu the metrics instances, dp_world_agents.cu the reactive ones and
+// dp_world_lanechange.cu the lane-changing ones: kept in separate translation units, the disarmed instances compile to exactly
+// what they compiled to before the options existed.
 #pragma once
 #include <type_traits>
 
@@ -164,11 +165,8 @@ struct LaneChangeModel : AgentModel {
 // length of map lane gl: the last entry of its sequential prefix of segment lengths
 __device__ __forceinline__ double lane_len(const DevMap& m, int gl) { return m.cump[m.lane_pt_off[gl + 1] - 1]; }
 
-// ---- lane-changing agents (include/dmpp_b200.h section 13): MOBIL on the react phase's staging ----
-static_assert(sizeof(dp_lane_change_state) == 24, "dp_lane_change_state is 24 bytes");
-
 // section 12's IDM acceleration with its clamp (lead false: free road); sab = 2.0 * sqrt(a_max * b)
-__device__ __forceinline__ double lc_idm(const dp_agent_model_params& p, double sab, double v, double vd, bool lead, double g, double vl) {
+__device__ __forceinline__ double idm_accel(const dp_agent_model_params& p, double sab, double v, double vd, bool lead, double g, double vl) {
     const double r = v / vd;
     double fr = r * r;
     fr = fr * fr;
@@ -184,6 +182,9 @@ __device__ __forceinline__ double lc_idm(const dp_agent_model_params& p, double 
     if (acc < -p.b_max) acc = -p.b_max;
     return acc;
 }
+
+// ---- lane-changing agents (include/dmpp_b200.h section 13): MOBIL on the react phase's staging ----
+static_assert(sizeof(dp_lane_change_state) == 24, "dp_lane_change_state is 24 bytes");
 
 // the ego as a follower: the interaction term alone (its v0 is unknown), 0 without a leader
 __device__ __forceinline__ double lc_ego_idm(const dp_agent_model_params& p, double sab, double v, bool lead, double g, double vl) {
@@ -251,7 +252,7 @@ __device__ __forceinline__ LcSide lc_side(const DevMap& m, const LaneChangeModel
         }
     }
     if (overlap || (lead && !(gl > 0)) || (foll && !(gf > 0))) return r;
-    r.atc = lc_idm(p, sab, v, vd, lead, gl, vl);
+    r.atc = idm_accel(p, sab, v, vd, lead, gl, vl);
     double af = 0, atf = 0;
     if (fego) {
         af = lc_ego_idm(p, sab, vf, lead, (sl - sf) - c.ego_front, vl);
@@ -260,8 +261,8 @@ __device__ __forceinline__ LcSide lc_side(const DevMap& m, const LaneChangeModel
     } else if (foll) {
         const double vdf = v0[fj];
         if (vdf > 0) {
-            af = lc_idm(p, sab, vf, vdf, lead, (sl - sf) - (lego ? p.ego_rear : p.length), vl);
-            atf = lc_idm(p, sab, vf, vdf, true, gf, v);
+            af = idm_accel(p, sab, vf, vdf, lead, (sl - sf) - (lego ? p.ego_rear : p.length), vl);
+            atf = idm_accel(p, sab, vf, vdf, true, gf, v);
         }
         if (!(atf >= -c.b_safe)) return r;
     }
@@ -390,19 +391,7 @@ __device__ __forceinline__ void react_step(const DevMap& m, const Model& am, con
                 if (!lead || g < best) { best = g; vl = c2.y; lead = true; }
             }
         }
-        const double r = v / vd;
-        double fr = r * r;
-        fr = fr * fr;
-        double acc;
-        if (lead) {
-            const double dv = v - vl;
-            double z = v * p.T + v * dv / sab;
-            if (z < 0) z = 0;
-            const double ss = p.s0 + z;
-            if (best > 0) { const double q = ss / best; acc = p.a_max * (1.0 - fr - q * q); }
-            else acc = -p.b_max;
-        } else acc = p.a_max * (1.0 - fr);
-        if (acc < -p.b_max) acc = -p.b_max;
+        const double acc = idm_accel(p, sab, v, vd, lead, best, vl);
         double vn = v + acc * dt;
         if (vn < 0) vn = 0;
         if constexpr (LANECHG) lane_change_agent(m, am, sab, SV, L, n_obs, v0, le, se, ve, dt, k, v, vd, acc, vn, ag, am.lcs + (v0 - am.v0));
@@ -662,3 +651,39 @@ __global__ void __launch_bounds__(WPB * 32, (METRICS || REACT) ? 8 : 0) dp_world
     }
 }
 }  // namespace
+
+// the launches of one instance set, both JUNC instances: each set is instantiated in its own translation unit (the extern
+// declarations below name it), and dp_launch_world (dp_world.cu) picks the set from the armed options
+template <bool METRICS, bool REACT, bool LANECHG>
+struct WorldStep {
+    static cudaError_t launch(const DevMap& m, const dp_params& p, const DpWorldOpts& o, const DpWorldBufs& b, cudaStream_t st);
+    static cudaError_t prepare();              // REACT: allow the dynamic shared memory of DP_AGENT_MODEL_MAX_OBS agent slots
+    static auto kernel(bool junc) { return junc ? dp_world_kernel<true, METRICS, REACT, LANECHG> : dp_world_kernel<false, METRICS, REACT, LANECHG>; }
+};
+// (defined outside the class: not inline, so the extern declarations below keep the other translation units from instantiating them)
+template <bool METRICS, bool REACT, bool LANECHG>
+cudaError_t WorldStep<METRICS, REACT, LANECHG>::launch(const DevMap& m, const dp_params& p, const DpWorldOpts& o, const DpWorldBufs& b,
+                                                       cudaStream_t st) {
+    std::conditional_t<LANECHG, LaneChangeModel, AgentModel> am;
+    am.p = o.amp; am.v0 = o.v0;
+    if constexpr (LANECHG) { am.lc = o.lcp; am.lcs = o.lcs; }
+    const size_t smem = REACT ? WPB * react_stage_bytes(b.max_obs) : 0;
+    kernel(o.wp.pre_junction_pts > 0)<<<(b.n + WPB - 1) / WPB, WPB * 32, smem, st>>>(
+        m, p, o.wp, b.n, b.max_obs, b.hdr, b.agents, b.ox, b.oy, b.rec, b.last_path, o.mp, o.met, am);
+    return cudaGetLastError();
+}
+template <bool METRICS, bool REACT, bool LANECHG>
+cudaError_t WorldStep<METRICS, REACT, LANECHG>::prepare() {
+    const int bytes = (int)(WPB * react_stage_bytes(DP_AGENT_MODEL_MAX_OBS));
+    for (const bool junc : {false, true}) {
+        const cudaError_t e = cudaFuncSetAttribute(kernel(junc), cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
+}
+extern template struct WorldStep<false, false, false>;   // dp_world.cu
+extern template struct WorldStep<true, false, false>;    // dp_world_metrics.cu
+extern template struct WorldStep<false, true, false>;    // dp_world_agents.cu
+extern template struct WorldStep<true, true, false>;
+extern template struct WorldStep<false, true, true>;     // dp_world_lanechange.cu
+extern template struct WorldStep<true, true, true>;

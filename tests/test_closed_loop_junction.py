@@ -5,36 +5,12 @@ The specification is the junction oracle of tools/junction_oracle (the cycle res
 between its cycles; with the option off its step IS oracle/world_spec.cpp's).  CPU side: known answers on the synthetic map, the
 option switched off is the segment-only step, the loop is alive, and the junction oracle against the UNMODIFIED reference driven
 the same way.  GPU side: dp_run_closed_loop_dev against the junction oracle, bit for bit."""
-import os
-
 import numpy as np
 import pytest
 
 from conftest import assert_records_equal, same
-from test_closed_loop import HDR as HDR0, check_closed_loop as check_segment_loop
 from test_oracle_vs_ref import CARRY, REC
-
-HDR = HDR0 + ["last_roadnum", "next_roadnum", "last_lanenum", "next_lanenum", "stub_attribute", "conn"]
-
-
-@pytest.fixture(scope="module")
-def joracle(the_map):
-    from tools.junction_oracle.binding import JunctionOracle
-    j = JunctionOracle()
-    j.set_map(the_map)
-    return j
-
-
-def jworld(the_map, seed0, n, kind="junction", n_obs=10):
-    from dmpp_b200 import scenes
-    return scenes.World(the_map, np.arange(seed0, seed0 + n), n_obs=n_obs, kind=kind)
-
-
-def jparams(src, kind="junction"):
-    from dmpp_b200 import scenes
-    wp = src.world_params()
-    wp.pre_junction_pts = scenes.World.PRE_JUNCTION_PTS[kind]
-    return wp
+from worlds import HDR, check_closed_loop, joracle, jparams, jworld, planner_with  # noqa: F401  (joracle: the module fixture)
 
 
 def compressed(seq):
@@ -244,26 +220,6 @@ def test_junction_closed_loop_oracle_equals_unmodified_reference(joracle, refere
 
 
 # ---------------------------------------------------------------- GPU
-def check_closed_loop(got, want, what):
-    check_segment_loop(got, want, what)                     # records, logs, final world (every header byte), carry, last path
-    assert_records_equal(got["hdr_log"], want["hdr_log"], HDR, what=what + " logged header")
-
-
-def planner_with(the_map, n, max_obs, J, env=None):
-    from dmpp_b200.planner import Planner
-    env = env or {}
-    os.environ.update(env)
-    try:
-        p = Planner(max_scenes=n, max_obs=max_obs)
-    finally:
-        for k in env:
-            del os.environ[k]
-    p.upload_map(the_map)
-    wp = p.world_params(); wp.pre_junction_pts = J
-    p.set_world_params(wp)
-    return p
-
-
 @pytest.fixture(scope="module")
 def jplanner(the_map):
     p = planner_with(the_map, 4096, 10, 60)

@@ -9,22 +9,7 @@ import ctypes as C
 import numpy as np
 import pytest
 
-from test_closed_loop_junction import check_closed_loop, jparams, jworld, planner_with
-
-WORLD = ("rec", "hdr_log", "hdr", "agents", "ox", "oy", "obs_log_x", "obs_log_y", "carry", "last_path")
-
-
-@pytest.fixture(scope="module")
-def joracle(the_map):
-    from tools.junction_oracle.binding import JunctionOracle
-    j = JunctionOracle()
-    j.set_map(the_map)
-    return j
-
-
-def mparams():
-    from dmpp_b200 import planner
-    return planner.metrics_params()
+from worlds import WORLD, StraightRoad, check_closed_loop, check_rows, joracle, jparams, jworld, mparams, planner_with  # noqa: F401
 
 
 # ---------------------------------------------------------------- CPU: layout and defaults
@@ -38,33 +23,9 @@ def test_layout_and_defaults(joracle):
 
 
 # ---------------------------------------------------------------- CPU: known answers on a straight road
-class StraightMap:
-    """one road, one lane, 1000 points 0.5 m apart along +x"""
-
-    def __init__(self):
-        from dmpp_b200 import abi
-        n = 1000
-        self.road_lane_base = np.array([0, 1], np.int32)
-        self.lane_pt_off = np.array([0, n], np.int32)
-        self.conn = np.zeros(0, abi.connector)
-        self.x, self.y, self.dir = 0.5 * np.arange(n), np.zeros(n), np.zeros(n)
-        self.lane_width = np.full(n, 375, np.uint16)
-        self.lanechg_attr = np.zeros(n, np.uint16)
-        self.n_roads, self.n_lanes = 1, 1
-
-    def desc(self):
-        from dmpp_b200 import abi
-        d = abi.MapDesc()
-        d.n_roads, d.road_lane_base, d.n_lanes, d.lane_pt_off = 1, self.road_lane_base.ctypes.data, 1, self.lane_pt_off.ctypes.data
-        d.n_conn, d.conn, d.n_points = 0, self.conn.ctypes.data, self.x.size
-        d.x, d.y, d.dir = self.x.ctypes.data, self.y.ctypes.data, self.dir.ctypes.data
-        d.lane_width, d.lanechg_attr = self.lane_width.ctypes.data, self.lanechg_attr.ctypes.data
-        return d
-
-
 @pytest.fixture
 def straight(joracle, the_map):
-    joracle.set_map(StraightMap())
+    joracle.set_map(StraightRoad(1000))
     yield joracle
     joracle.set_map(the_map)
 
@@ -300,22 +261,6 @@ def test_metrics_find_things(runs_512):
 
 
 # ---------------------------------------------------------------- GPU
-def check_rows(got, want, what, rec=None):
-    """byte for byte; with rec (the GPU's own records [cycles][n]): max_abs_dir_err is max |rec.path_dir_err| of those records, bit for
-    bit, and within 1e-9 of the checker's -- the one record field the CUDA path reproduces to 1e-9 only (tests/test_closed_loop.py)"""
-    from dmpp_b200 import abi
-    assert got.dtype == want.dtype == abi.episode_metrics
-    for f in abi.episode_metrics.names:
-        if rec is not None and f == "max_abs_dir_err":
-            assert (got[f] == np.abs(rec["path_dir_err"]).max(axis=0)).all(), what
-            assert (np.abs(got[f] - want[f]) <= 1e-9).all(), what
-            continue
-        g, w = got[f].reshape(len(got), -1), want[f].reshape(len(want), -1)
-        bad = (g.view(np.uint8).reshape(len(got), -1) != w.view(np.uint8).reshape(len(want), -1)).any(axis=1)
-        assert not bad.any(), "%s: field %s differs in %d worlds, first %d: got %r want %r" % (
-            what, f, bad.sum(), np.argmax(bad), got[f][np.argmax(bad)], want[f][np.argmax(bad)])
-
-
 @pytest.mark.gpu
 @pytest.mark.parametrize("kind,n,cycles,env", [("highway", 4096, 60, None), ("junction", 4096, 120, None),
                                                ("junction", 4096, 120, {"DP_EPISODE_GRAPH": "0"}),

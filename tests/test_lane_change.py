@@ -10,20 +10,8 @@ import ctypes as C
 import numpy as np
 import pytest
 
-from test_closed_loop_junction import check_closed_loop, jparams, jworld, planner_with
-from test_episode_metrics import WORLD, check_rows, mparams
-from test_reactive_agents import amparams, cump_of, first_strikes, idm, joracle  # noqa: F401  (joracle: the module fixture)
-
-DT = 0.1
-W = 3.75
-
-
-def lcparams(**kw):
-    from dmpp_b200 import planner
-    p = planner.lane_change_params()
-    for k, v in kw.items():
-        setattr(p, k, v)
-    return p
+from worlds import (DT, WORLD, W, StraightRoad, amparams, cump_of, first_strikes, gpu_vs_checker, idm, joracle,  # noqa: F401
+                    jparams, jworld, lcparams, mparams, planner_with)
 
 
 # ---------------------------------------------------------------- CPU: layout and defaults
@@ -37,38 +25,10 @@ def test_layout_and_defaults(joracle):
 
 
 # ---------------------------------------------------------------- CPU: known answers on a straight two-lane road
-class TwoLane:
-    """one road of two lanes 3.75 m apart along +x (lane 1 on the left, at y = +1.875), n points 0.5 m apart, lane-change attribute
-    `attr` on both lanes; with connector=True a third, parallel pseudo-lane (y = -5.625, attribute 3) is a connector leaving lane 2"""
-
-    def __init__(self, n=6000, attr=3, connector=False):
-        from dmpp_b200 import abi
-        ys = [W / 2, -W / 2] + ([-1.5 * W] if connector else [])
-        self.n_roads, self.n_lanes = 1, len(ys)
-        self.road_lane_base = np.array([0, 2], np.int32)
-        self.lane_pt_off = (n * np.arange(len(ys) + 1)).astype(np.int32)
-        self.conn = np.array([(1, 1, 2, 2, 2)] if connector else [], abi.connector)
-        self.x = np.tile(0.5 * np.arange(n), len(ys))
-        self.y = np.repeat(ys, n).astype(np.float64)
-        self.dir = np.zeros(self.x.size)
-        self.lane_width = np.full(self.x.size, 375, np.uint16)
-        self.lanechg_attr = np.full(self.x.size, attr, np.uint16)
-        self.lanechg_attr[2 * n:] = 3
-
-    def desc(self):
-        from dmpp_b200 import abi
-        d = abi.MapDesc()
-        d.n_roads, d.road_lane_base, d.n_lanes, d.lane_pt_off = self.n_roads, self.road_lane_base.ctypes.data, self.n_lanes, self.lane_pt_off.ctypes.data
-        d.n_conn, d.conn, d.n_points = len(self.conn), self.conn.ctypes.data, self.x.size
-        d.x, d.y, d.dir = self.x.ctypes.data, self.y.ctypes.data, self.dir.ctypes.data
-        d.lane_width, d.lanechg_attr = self.lane_width.ctypes.data, self.lanechg_attr.ctypes.data
-        return d
-
-
 @pytest.fixture
 def two_lane(joracle, the_map):
-    def use(**kw):
-        joracle.set_map(TwoLane(**kw))
+    def use(attr=3, connector=False):
+        joracle.set_map(StraightRoad(6000, lanes=2, attr=attr, connector=connector))
         return joracle
     yield use
     joracle.set_map(the_map)
@@ -464,43 +424,21 @@ def test_lane_change_log_replays_open_loop(oracle, highway_steps, kind):
 
 
 # ---------------------------------------------------------------- GPU
-def gpu_vs_checker(joracle, the_map, kind, n, cycles, env=None, n_obs=10, repeat=1, metrics=True):
-    from dmpp_b200 import scenes
-    w = scenes.World(the_map, np.arange(n), n_obs=n_obs, kind=kind)
-    mp = mparams() if metrics else None
-    am, lp = (amparams(), w.v0), lcparams()
-    want = joracle.run_closed_loop(w.hdr, w.agents, cycles, wp=jparams(joracle, kind), threads=16, metrics=mp, agent_model=am, lane_change=lp)
-    p = planner_with(the_map, n, n_obs, scenes.World.PRE_JUNCTION_PTS[kind], env)
-    try:
-        got = p.run_closed_loop(w.hdr, w.agents, cycles, repeat=repeat, metrics=mp, agent_model=am, lane_change=lp)
-    finally:
-        p.close()
-    what = "%s %r" % (kind, env)
-    assert got["graph"] == (env is None and n_obs < 32), what
-    if metrics:
-        check_rows(got["metrics"], want["metrics"], what, rec=got["rec"])
-    check_closed_loop(got, want, what)
-    assert got["lane_change_state"].tobytes() == want["lane_change_state"].tobytes(), what
-    st = got["lane_change_state"]
-    assert (st["changes_left"] + st["changes_right"]).sum() > 0
-    return got
-
-
 @pytest.mark.gpu
 def test_gpu_graph_equals_checker(joracle, the_map):
     """4096 highway worlds as ONE graph launch, replayed three times from the same initial world; metrics armed too"""
-    gpu_vs_checker(joracle, the_map, "highway", 4096, 25, repeat=3)
+    gpu_vs_checker(joracle, the_map, "highway", 4096, 25, repeat=3, lane_change=lcparams())
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("env,metrics", [({"DP_EPISODE_GRAPH": "0"}, False), ({"DP_KERNEL": "group"}, True)])
 def test_gpu_direct_launches_and_group_kernel(joracle, the_map, env, metrics):
-    gpu_vs_checker(joracle, the_map, "highway", 4096, 25, env=env, metrics=metrics)
+    gpu_vs_checker(joracle, the_map, "highway", 4096, 25, env=env, metrics=metrics, lane_change=lcparams())
 
 
 @pytest.mark.gpu
 def test_gpu_highway_200_agents(joracle, the_map):
-    gpu_vs_checker(joracle, the_map, "highway", 1024, 25, n_obs=200)
+    gpu_vs_checker(joracle, the_map, "highway", 1024, 25, n_obs=200, lane_change=lcparams())
 
 
 @pytest.mark.gpu

@@ -10,54 +10,8 @@ import ctypes as C
 import numpy as np
 import pytest
 
-from test_closed_loop_junction import check_closed_loop, jparams, jworld, planner_with
-from test_episode_metrics import WORLD, check_rows, mparams
-
-DT = 0.1
-
-
-@pytest.fixture(scope="module")
-def joracle(the_map):
-    from tools.junction_oracle.binding import JunctionOracle
-    j = JunctionOracle()
-    j.set_map(the_map)
-    return j
-
-
-def amparams(**kw):
-    from dmpp_b200 import planner
-    p = planner.agent_model_params()
-    for k, v in kw.items():
-        setattr(p, k, v)
-    return p
-
-
-def idm(v, v0, p, g=None, vl=None, dt=DT):
-    """the IDM step of section 12 in numpy float64, the operations in the order the header writes them"""
-    v, v0 = np.float64(v), np.float64(v0)
-    r = v / v0
-    fr = r * r
-    fr = fr * fr
-    if g is None:
-        acc = p.a_max * (1.0 - fr)
-    else:
-        dv = v - vl
-        z = v * p.T + v * dv / (2.0 * np.sqrt(p.a_max * p.b))
-        z = max(z, 0.0)
-        ss = p.s0 + z
-        acc = p.a_max * (1.0 - fr - (ss / g) * (ss / g)) if g > 0 else -p.b_max
-    acc = max(acc, -p.b_max)
-    return max(v + acc * np.float64(dt), 0.0)
-
-
-def cump_of(m):
-    """the sequential prefix of every lane's segment lengths (dp_map_prep_kernel), independently in numpy"""
-    c = np.zeros(m.x.size)
-    for gl in range(m.n_lanes):
-        o, e = int(m.lane_pt_off[gl]), int(m.lane_pt_off[gl + 1])
-        dx, dy = np.diff(m.x[o:e]), np.diff(m.y[o:e])
-        c[o + 1:e] = np.add.accumulate(np.sqrt(dx * dx + dy * dy))
-    return c
+from worlds import (DT, WORLD, StraightRoad, amparams, cump_of, first_strikes, gpu_vs_checker, idm, joracle, jparams,  # noqa: F401
+                    jworld, mparams, planner_with)
 
 
 # ---------------------------------------------------------------- CPU: layout and defaults
@@ -69,32 +23,9 @@ def test_layout_and_defaults(joracle):
 
 
 # ---------------------------------------------------------------- CPU: known answers on a straight lane
-class LongStraight:
-    """one road, one lane, n points 0.5 m apart along +x (the StraightMap of test_episode_metrics.py, longer)"""
-
-    def __init__(self, n=6000):
-        from dmpp_b200 import abi
-        self.road_lane_base = np.array([0, 1], np.int32)
-        self.lane_pt_off = np.array([0, n], np.int32)
-        self.conn = np.zeros(0, abi.connector)
-        self.x, self.y, self.dir = 0.5 * np.arange(n), np.zeros(n), np.zeros(n)
-        self.lane_width = np.full(n, 375, np.uint16)
-        self.lanechg_attr = np.zeros(n, np.uint16)
-        self.n_roads, self.n_lanes = 1, 1
-
-    def desc(self):
-        from dmpp_b200 import abi
-        d = abi.MapDesc()
-        d.n_roads, d.road_lane_base, d.n_lanes, d.lane_pt_off = 1, self.road_lane_base.ctypes.data, 1, self.lane_pt_off.ctypes.data
-        d.n_conn, d.conn, d.n_points = 0, self.conn.ctypes.data, self.x.size
-        d.x, d.y, d.dir = self.x.ctypes.data, self.y.ctypes.data, self.dir.ctypes.data
-        d.lane_width, d.lanechg_attr = self.lane_width.ctypes.data, self.lanechg_attr.ctypes.data
-        return d
-
-
 @pytest.fixture
 def straight(joracle, the_map):
-    joracle.set_map(LongStraight())
+    joracle.set_map(StraightRoad(6000))
     yield joracle
     joracle.set_map(the_map)
 
@@ -373,23 +304,6 @@ def test_numpy_restatement_equals_checker(joracle, the_map):
 
 
 # ---------------------------------------------------------------- CPU: what the model is for
-def first_strikes(the_map, w, met):
-    """worlds with a collision, and where their first colliding agent started: on the ego's lane behind it (and of those, how many
-    faster than the ego), ahead of it, or on another lane"""
-    m = the_map
-    cump = cump_of(m)
-    h, a = w.hdr, w.agents
-    s = np.nonzero(met["first_collision_step"] > 0)[0]
-    gl = m.road_lane_base[h["road_num"][s].astype(int) - 1] + h["lane_num"][s].astype(int) - 1
-    se = cump[m.lane_pt_off[gl] + h["id"][s, h["lane_num"][s].astype(int) - 1]]
-    ag = a[s, met["first_collision_agent"][s]]
-    sk = cump[m.lane_pt_off[ag["lane"]] + ag["i"]] + ag["u"]
-    same_lane = ag["lane"] == gl
-    behind = same_lane & (sk < se)
-    return {"worlds": int(s.size), "behind": int(behind.sum()), "behind_faster": int((behind & (ag["v"] > h["velocity"][s] / 3.6)).sum()),
-            "ahead": int((same_lane & ~behind).sum()), "other_lane": int((~same_lane).sum())}
-
-
 @pytest.fixture(scope="module")
 def runs_512(joracle, the_map):
     out = {}
@@ -419,26 +333,6 @@ def test_reactive_log_replays_open_loop(oracle, runs_512, kind):
 
 
 # ---------------------------------------------------------------- GPU
-def gpu_vs_checker(joracle, the_map, kind, n, cycles, env=None, n_obs=10, repeat=1, metrics=True):
-    from dmpp_b200 import scenes
-    w = scenes.World(the_map, np.arange(n), n_obs=n_obs, kind=kind)
-    mp = mparams() if metrics else None
-    am = (amparams(), w.v0)
-    want = joracle.run_closed_loop(w.hdr, w.agents, cycles, wp=jparams(joracle, kind), threads=16, metrics=mp, agent_model=am)
-    p = planner_with(the_map, n, n_obs, scenes.World.PRE_JUNCTION_PTS[kind], env)
-    try:
-        got = p.run_closed_loop(w.hdr, w.agents, cycles, repeat=repeat, metrics=mp, agent_model=am)
-    finally:
-        p.close()
-    what = "%s %r" % (kind, env)
-    assert got["graph"] == (env is None and n_obs < 32), what   # (from 32 agents up the cycle runs on the group kernel)
-    if metrics:
-        check_rows(got["metrics"], want["metrics"], what, rec=got["rec"])
-    check_closed_loop(got, want, what)
-    assert (got["agents"]["v"] != w.agents["v"]).any()
-    return got
-
-
 @pytest.mark.gpu
 @pytest.mark.parametrize("kind,cycles", [("highway", 25), ("junction", 120)])
 def test_gpu_graph_equals_checker(joracle, the_map, kind, cycles):

@@ -5,6 +5,7 @@ import ctypes as C
 import os
 import subprocess
 import sys
+import types
 
 import numpy as np
 
@@ -50,38 +51,28 @@ class JunctionOracle:
                                       abi.ptr(ox), abi.ptr(oy), abi.ptr(rec), abi.ptr(last_path)) == 0
 
     def run_closed_loop(self, hdr, agents, cycles, wp=None, paths=False, threads=1, metrics=None, agent_model=None, lane_change=None):
-        """hdr[n], agents[n][max_obs] (copied; the final world is returned); metrics = MetricsParams: the episode metrics of every
-        world under "metrics" (jo_run_closed_loop_metrics); agent_model = (AgentModelParams, v0[n][max_obs]): the reactive agents
-        (jo_run_closed_loop_agents); lane_change = LaneChangeParams (with agent_model): their lane changes, the final states under
-        "lane_change_state" (jo_run_closed_loop_lanechg)"""
+        """hdr[n], agents[n][max_obs] (copied; the final world is returned), through jo_run_closed_loop; metrics = MetricsParams: the
+        episode metrics of every world under "metrics"; agent_model = (AgentModelParams, v0[n][max_obs]): the reactive agents;
+        lane_change = LaneChangeParams (with agent_model): their lane changes, the final states under "lane_change_state"
+        """
         assert lane_change is None or agent_model is not None
-        wp = wp or self.world_params()
-        if metrics is None and agent_model is None:
-            return ob._closed_loop(self.lib, "jo_run_closed_loop", self.params, wp, hdr, agents, cycles, paths, threads)
-        n = hdr.shape[0]
+        am, v0 = agent_model if agent_model is not None else (None, None)
         met = lcs = None
         if metrics is not None:
-            met = np.frombuffer(np.full(n * abi.episode_metrics.itemsize, 0xAB, np.uint8).tobytes(), abi.episode_metrics).copy()
-        if agent_model is None:
-            name, tail = "jo_run_closed_loop_metrics", (C.byref(metrics), abi.ptr(met))
-        else:
-            am, v0 = agent_model
+            met = np.frombuffer(np.full(hdr.shape[0] * abi.episode_metrics.itemsize, 0xAB, np.uint8).tobytes(), abi.episode_metrics).copy()
+        if v0 is not None:
             v0 = np.ascontiguousarray(v0, np.float64)
             assert v0.shape == agents.shape
-            name = "jo_run_closed_loop_agents"
-            tail = (C.byref(metrics) if metrics is not None else None, abi.ptr(met), C.byref(am), abi.ptr(v0))
-            if lane_change is not None:
-                lcs = np.frombuffer(np.full(agents.size * abi.lane_change_state.itemsize, 0xAB, np.uint8).tobytes(),
-                                    abi.lane_change_state).reshape(agents.shape).copy()
-                name = "jo_run_closed_loop_lanechg"
-                tail = tail + (C.byref(lane_change), abi.ptr(lcs))
-        f = getattr(self.lib, name)
+        if lane_change is not None:
+            lcs = np.frombuffer(np.full(agents.size * abi.lane_change_state.itemsize, 0xAB, np.uint8).tobytes(),
+                                abi.lane_change_state).reshape(agents.shape).copy()
+        ref = lambda p: None if p is None else C.byref(p)
+        models = (ref(metrics), abi.ptr(met), ref(am), abi.ptr(v0), ref(lane_change), abi.ptr(lcs))
+        f = self.lib.jo_run_closed_loop
         f.restype = C.c_longlong
-
-        class _Lib:                                         # ob._closed_loop's call, with the params and the rows appended
-            pass
-        setattr(_Lib, name, staticmethod(lambda *a: f(*a, *tail)))
-        o = ob._closed_loop(_Lib, name, self.params, wp, hdr, agents, cycles, paths, threads)
+        # ob._closed_loop passes the arrays every closed loop has; the model arguments follow them
+        o = ob._closed_loop(types.SimpleNamespace(jo_run_closed_loop=lambda *a: f(*a, *models)), "jo_run_closed_loop", self.params,
+                            wp or self.world_params(), hdr, agents, cycles, paths, threads)
         if met is not None:
             o["metrics"] = met
         if lcs is not None:

@@ -1,9 +1,8 @@
 // tools/junction_oracle/junction_api.cpp -- TEST INFRASTRUCTURE. C API of libjunction_oracle.so: the restated cycle of oracle/
 // (planner_oracle.cpp, compiled in unchanged) with the junction world step of world_junction.cpp between its cycles; the
-// same arrays as oracle_world_step / oracle_run_closed_loop of oracle/oracle_api.cpp; the episode metrics of
-// episode_metrics.cpp after every world step (jo_run_closed_loop_metrics, jo_metrics_step); the reactive agents of
-// agent_model.cpp before every world step (jo_run_closed_loop_agents, jo_react_step); and their lane changes of lane_change.cpp
-// (jo_run_closed_loop_lanechg, jo_lane_change_step).
+// same arrays as oracle_world_step / oracle_run_closed_loop of oracle/oracle_api.cpp; in jo_run_closed_loop, the models each
+// world step may carry: the episode metrics of episode_metrics.cpp (alone: jo_metrics_step), the reactive agents of
+// agent_model.cpp (alone: jo_react_step) and their lane changes of lane_change.cpp (alone: jo_lane_change_step).
 #include <algorithm>
 #include <atomic>
 #include <cstring>
@@ -38,18 +37,17 @@ int jo_world_step(const dp_params* p, const dp_world_params* wp, int n, int max_
     return 0;
 }
 
-}  // extern "C"
-
-namespace {
-// the closed loop of jo_run_closed_loop; mp / met non-null: the episode metrics accumulated after every world step; am / v0
-// non-null: the agents react (v0[n][max_obs]) before every world step; lp / lcs non-null (with am): and change lanes, states
-// lcs[n][max_obs]
-long long closed_loop(const dp_params* p, const dp_world_params* wp, int n, int cycles, int max_obs, dp_scene_hdr* hdr, dp_agent* agents,
-                      double* ox, double* oy, dp_plan_record* rec, dp_scene_hdr* hdr_log, double* obs_log_x, double* obs_log_y,
-                      double* path_xy, dp_carry* carry_out, double* last_path_out, int threads, int32_t* ub_scene,
-                      const dp_metrics_params* mp, dp_episode_metrics* met, const dp_agent_model_params* am, const double* v0,
-                      const dp_lane_change_params* lp, dp_lane_change_state* lcs) {
+// the closed loop: the junction world step between the cycles of oracle/, the same arrays as oracle_run_closed_loop.  Each model is
+// armed by a non-null pair, or off with both NULL: mp / met[n] the episode metrics of include/dmpp_b200.h section 11, accumulated
+// after every world step; am / v0[n][max_obs] the reactive agents of section 12, before every world step; lp / lcs[n][max_obs]
+// (with am) their lane changes of section 13, states initialised by the placement step and holding the final states
+long long jo_run_closed_loop(const dp_params* p, const dp_world_params* wp, int n, int cycles, int max_obs, dp_scene_hdr* hdr,
+                             dp_agent* agents, double* ox, double* oy, dp_plan_record* rec, dp_scene_hdr* hdr_log, double* obs_log_x,
+                             double* obs_log_y, double* path_xy, dp_carry* carry_out, double* last_path_out, int threads,
+                             int32_t* ub_scene, const dp_metrics_params* mp, dp_episode_metrics* met, const dp_agent_model_params* am,
+                             const double* v0, const dp_lane_change_params* lp, dp_lane_change_state* lcs) {
     if (!g_have_map) return -1;
+    if ((!mp) != (!met) || (!am) != (!v0) || (!lp) != (!lcs) || (lcs && !v0)) return -1;
     if (threads < 1) threads = 1;
     std::atomic<long long> ub(0);
     auto work = [&](int s0, int s1) {
@@ -97,39 +95,6 @@ long long closed_loop(const dp_params* p, const dp_world_params* wp, int n, int 
     }
     return ub.load();
 }
-}  // namespace
-
-extern "C" {
-
-long long jo_run_closed_loop(const dp_params* p, const dp_world_params* wp, int n, int cycles, int max_obs, dp_scene_hdr* hdr,
-                             dp_agent* agents, double* ox, double* oy, dp_plan_record* rec, dp_scene_hdr* hdr_log, double* obs_log_x,
-                             double* obs_log_y, double* path_xy, dp_carry* carry_out, double* last_path_out, int threads,
-                             int32_t* ub_scene) {
-    return closed_loop(p, wp, n, cycles, max_obs, hdr, agents, ox, oy, rec, hdr_log, obs_log_x, obs_log_y, path_xy, carry_out, last_path_out,
-                       threads, ub_scene, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr);
-}
-
-// jo_run_closed_loop with the episode metrics of every world in met[n] (include/dmpp_b200.h section 11)
-long long jo_run_closed_loop_metrics(const dp_params* p, const dp_world_params* wp, int n, int cycles, int max_obs, dp_scene_hdr* hdr,
-                                     dp_agent* agents, double* ox, double* oy, dp_plan_record* rec, dp_scene_hdr* hdr_log, double* obs_log_x,
-                                     double* obs_log_y, double* path_xy, dp_carry* carry_out, double* last_path_out, int threads,
-                                     int32_t* ub_scene, const dp_metrics_params* mp, dp_episode_metrics* met) {
-    if (!mp || !met) return -1;
-    return closed_loop(p, wp, n, cycles, max_obs, hdr, agents, ox, oy, rec, hdr_log, obs_log_x, obs_log_y, path_xy, carry_out, last_path_out,
-                       threads, ub_scene, mp, met, nullptr, nullptr, nullptr, nullptr);
-}
-
-// jo_run_closed_loop with the reactive agents of include/dmpp_b200.h section 12 (am, v0[n][max_obs]); mp / met: the episode
-// metrics as in jo_run_closed_loop_metrics, or both NULL
-long long jo_run_closed_loop_agents(const dp_params* p, const dp_world_params* wp, int n, int cycles, int max_obs, dp_scene_hdr* hdr,
-                                    dp_agent* agents, double* ox, double* oy, dp_plan_record* rec, dp_scene_hdr* hdr_log, double* obs_log_x,
-                                    double* obs_log_y, double* path_xy, dp_carry* carry_out, double* last_path_out, int threads,
-                                    int32_t* ub_scene, const dp_metrics_params* mp, dp_episode_metrics* met, const dp_agent_model_params* am,
-                                    const double* v0) {
-    if (!am || !v0 || (!mp) != (!met)) return -1;
-    return closed_loop(p, wp, n, cycles, max_obs, hdr, agents, ox, oy, rec, hdr_log, obs_log_x, obs_log_y, path_xy, carry_out, last_path_out,
-                       threads, ub_scene, mp, met, am, v0, nullptr, nullptr);
-}
 
 // the react phase alone, for every scene (agents[n][max_obs], v0[n][max_obs], k < min(n_obs, max_obs)), as the armed kernel runs
 // it at the start of a step with a record; a header that names no lane leaves its agents alone
@@ -142,18 +107,6 @@ int jo_react_step(const dp_world_params* wp, const dp_agent_model_params* am, in
 }
 
 int jo_agent_model_sizeof(void) { return (int)sizeof(dp_agent_model_params); }
-
-// jo_run_closed_loop_agents with the lane changes of include/dmpp_b200.h section 13 (lp, states lcs[n][max_obs], initialised by
-// the placement step and holding the final states)
-long long jo_run_closed_loop_lanechg(const dp_params* p, const dp_world_params* wp, int n, int cycles, int max_obs, dp_scene_hdr* hdr,
-                                     dp_agent* agents, double* ox, double* oy, dp_plan_record* rec, dp_scene_hdr* hdr_log, double* obs_log_x,
-                                     double* obs_log_y, double* path_xy, dp_carry* carry_out, double* last_path_out, int threads,
-                                     int32_t* ub_scene, const dp_metrics_params* mp, dp_episode_metrics* met, const dp_agent_model_params* am,
-                                     const double* v0, const dp_lane_change_params* lp, dp_lane_change_state* lcs) {
-    if (!am || !v0 || !lp || !lcs || (!mp) != (!met)) return -1;
-    return closed_loop(p, wp, n, cycles, max_obs, hdr, agents, ox, oy, rec, hdr_log, obs_log_x, obs_log_y, path_xy, carry_out, last_path_out,
-                       threads, ub_scene, mp, met, am, v0, lp, lcs);
-}
 
 // the react and lane-change phases alone, for every scene, in place (agents and lcs [n][max_obs], k < min(n_obs, max_obs)), as the
 // armed kernel runs them at the start of a step with a record; a header that names no lane leaves its agents and states alone
