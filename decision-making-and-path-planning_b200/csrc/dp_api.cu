@@ -71,120 +71,87 @@ struct dp_ctx {
     long long ep_launches = 0;
     int ep_graph = 1;                                       // DP_EPISODE_GRAPH=0: enqueue the launches directly
     int ep_last_graph = 0;
-    int split = 1;                                          // Decision / Planning halves as two launches (DP_SPLIT=0: one fused launch)
-    int zero_copy = 0;                                      // DP_ZERO_COPY=1: the kernels read pinned host inputs directly over PCIe (slower than the DMA route)
     // pipelined submit / wait: inputs of cycle k+1 cross PCIe on the copy stream while cycle k computes
     cudaStream_t cp[3] = {nullptr, nullptr, nullptr};       // one copy stream per input array: the three DMAs overlap
-    cudaStream_t cp_out = nullptr;                          // records device -> host by DMA behind the kernels of a pipelined submit
-    cudaEvent_t kdone[2] = {nullptr, nullptr};
-    int rec_dma = 0;                                        // DP_REC_DMA=1: records of dp_cycle_submit return by DMA behind the kernels instead of
-                                                            // stores from the Planning warps (measured slower with two cycles in flight: see profiles/README.md)
-    cudaEvent_t in_ready[2][3] = {{nullptr, nullptr, nullptr}, {nullptr, nullptr, nullptr}}, done[2] = {nullptr, nullptr};
+    cudaEvent_t in_ready[2][3] = {{nullptr, nullptr, nullptr}, {nullptr, nullptr, nullptr}};
     unsigned long long submitted = 0, waited = 0;
-    // overlapped split launch (split == 2): per-scene hand-off flags and the epoch of the next cycle
+    // overlapped launch of the two halves: per-scene hand-off flags and the epoch of the next cycle
     unsigned* d_done = nullptr;
     unsigned epoch = 0;
-    // chained submits (dp_cycle_submit, DP_CHAIN=0 switches back to events): no event or stream wait sits between the launches,
-    // so cycle k+1's Decision launch can be a programmatic dependent of cycle k's Planning launch; inputs and completion are
-    // signalled through flags instead
-    int chain = 1;
+    // submitted cycles (dp_cycle_submit): no event or stream wait sits between the launches; inputs and completion are signalled
+    // through flags instead
     unsigned* d_inflag = nullptr;                           // [2] "inputs of the cycle in staging set s are on the device"
-    unsigned* d_pdone = nullptr;                            // [max_scenes] per-scene "Planning finished" epoch
     unsigned* d_tally = nullptr;                            // [2] finished Planning warps
     unsigned* h_done = nullptr;                             // [2] page-locked: the last Planning warp of a cycle stores its epoch here
                                                             // [2..3] page-locked source words of the in_flag copies
     unsigned wait_epoch[2] = {0, 0};
-    unsigned chain_prev_epoch = 0; int chain_first = -1, chain_n = -1;
-    // record mirrors (dp_set_record_mirrors): device-accessible bases indexed by carry slot
-    dp_plan_record* mirror[DP_MAX_MIRRORS - 1] = {};
-    int n_mirror = 0;
-    // fused gather (dp_gather_*): flags the next cycle launch raises on every rank when its last record is out
-    unsigned* peer_flag[DP_MAX_MIRRORS] = {};
-    int n_peer_flag = 0; unsigned flag_value = 0;
-    const unsigned* wait_flag = nullptr; int n_wait = 0; unsigned wait_value = 0;
-    // deferred gather (dp_gather_arm_deferred): the next launch forwards the records of the last one; one-shot
-    dp_plan_record* fwd_dst[DP_MAX_MIRRORS] = {};
-    int n_fwd = 0; bool deferred = false;
+    // what the next cycle launch carries besides its own plumbing: the record mirrors (dp_set_record_mirrors) and the armed gather
+    // (dp_gather_*: mirrors, peer flags, the folded wait, the deferred forward), mirror / fwd_dst indexed by carry slot (make_io)
+    DpIo armed = {};
+    bool deferred = false;                                  // armed by dp_gather_arm_deferred: one-shot
     dp_plan_record* last_rec = nullptr; int last_first = -1, last_n = 0;   // record array (device) and slot range of the last cycle launch
     unsigned* d_tally_g = nullptr;                          // [2]: launch tally, Decision-half tally of the deferred gather
 };
 
 namespace {
-// launch plumbing of one cycle call: hand-off flags, then the caller's pinned record buffer (if any) and the context's mirrors
+// launch plumbing of one cycle call: hand-off flags, then the caller's pinned record buffer (if any), the context's mirrors and
+// armed gather offset by the first slot
 DpIo make_io(dp_ctx* c, int first, dp_plan_record* host_rec) {
-    DpIo io = dp_io_none();
+    DpIo io = c->armed;
     if (++c->epoch == 0) ++c->epoch;                        // (0 is what never-written flags hold)
     io.done = c->d_done + first; io.epoch = c->epoch;
-    c->chain_prev_epoch = 0;                                // (dp_cycle_submit re-arms the chain after its own launch)
+    io.n_mirror = 0;
     if (host_rec) io.mirror[io.n_mirror++] = host_rec;
-    for (int k = 0; k < c->n_mirror; ++k) io.mirror[io.n_mirror++] = c->mirror[k] + first;
-    for (int k = 0; k < c->n_peer_flag; ++k) io.peer_flag[k] = c->peer_flag[k];
-    io.n_peer_flag = c->n_peer_flag; io.flag_value = c->flag_value;
-    io.wait_flag = c->wait_flag; io.n_wait = c->n_wait; io.wait_value = c->wait_value;
-    if (c->n_fwd && c->last_rec) {
-        io.fwd_src = c->last_rec; io.n_fwd = c->n_fwd;
-        for (int k = 0; k < c->n_fwd; ++k) io.fwd_dst[k] = c->fwd_dst[k] + first;
+    for (int k = 0; k < c->armed.n_mirror; ++k) io.mirror[io.n_mirror++] = c->armed.mirror[k] + first;
+    if (io.n_fwd && c->last_rec) {
+        io.fwd_src = c->last_rec;
+        for (int k = 0; k < io.n_fwd; ++k) io.fwd_dst[k] += first;
         io.tally2 = c->d_tally_g + 1;
-    }
+    } else io.n_fwd = 0;
     return io;
 }
-// one cycle of n scenes (carry slots first ..) on stream st
+// record mirrors or a gather armed for the next launch?
+bool armed_any(const DpIo& a) { return a.n_mirror || a.n_peer_flag || a.wait.n || a.n_fwd; }
 // bookkeeping of every cycle launch: remember its record array (the deferred gather of the NEXT launch forwards it) and drop the
 // one-shot deferred state
 struct LaunchDone {
     dp_ctx* c; dp_plan_record* rec; int first, n;
     ~LaunchDone() {
         c->last_rec = rec; c->last_first = first; c->last_n = n;
-        if (c->deferred) { c->n_fwd = 0; c->n_peer_flag = 0; c->n_wait = 0; c->wait_flag = nullptr; c->deferred = false; }
+        if (c->deferred) { c->armed = {}; c->deferred = false; }
     }
 };
-// the warp-per-scene kernel pair (dp_cycle.cu) for slots first .. first + n
-cudaError_t launch_warp(dp_ctx* c, int first, int n, const dp_scene_hdr* hdr, const double* ox, const double* oy, dp_plan_record* rec,
-                        dp_trace_record* trace, double* path_xy, double* path_ll, cudaStream_t st, const DpIo& io) {
+// one cycle of n scenes (carry slots first ..) on stream st: the group kernel (dp_group.cuh), or the warp-per-scene kernel pair
+// (dp_cycle.cu)
+cudaError_t run_cycle(dp_ctx* c, int first, int n, const dp_scene_hdr* hdr, const double* ox, const double* oy, dp_plan_record* rec,
+                      dp_trace_record* trace, double* path_xy, double* path_ll, cudaStream_t st, DpIo io) {
     if (io.n_fwd && (first != c->last_first || n != c->last_n)) return cudaErrorInvalidValue;   // deferred gather: same slot range as the launch before
     LaunchDone done_{c, rec, first, n};
-    c->launches += c->split ? 2 : 1;
-    DpIo iow = io;
-    if (!iow.tally) {
-        // deferred gather with split launches: the Decision half forwards, flags and waits by itself (tally2): the Planning half ends as
-        // it does without a gather; otherwise the launch's last warp does it and needs the tally
-        if (iow.n_fwd && iow.tally2 && c->split) iow.tally_n = (unsigned)n;
-        else if (iow.n_peer_flag || iow.n_wait) { iow.tally = c->d_tally_g; iow.tally_n = (unsigned)n; }
+    const bool group = c->kernel == 1 || c->tracks_T > 0;  // (track tiles are only read by the group kernel)
+    if (!io.tally) {
+        // deferred gather on the warp kernel: the Decision half forwards, flags and waits by itself (tally2), the Planning half ends as
+        // it does without a gather; otherwise the launch's last warp / CTA does it and needs the tally
+        if (!group && io.n_fwd && io.tally2) io.tally_n = (unsigned)n;
+        else if (io.n_peer_flag || io.wait.n) { io.tally = c->d_tally_g; io.tally_n = (unsigned)n; }
     }
-    return dp_launch_cycle(c->gmap, c->p, n, hdr, ox, oy, c->max_obs, c->d_carry + first, c->d_last + (size_t)first * DP_PATH_POINTS, rec, trace,
-                           path_xy, path_ll, st, c->split, iow, c->lc);
-}
-// one cycle of n scenes (carry slots first ..) on stream st
-cudaError_t run_cycle(dp_ctx* c, int first, int n, const dp_scene_hdr* hdr, const double* ox, const double* oy, dp_plan_record* rec,
-                      dp_trace_record* trace, double* path_xy, double* path_ll, cudaStream_t st, const DpIo& io) {
-    if (c->kernel == 1 || c->tracks_T > 0) {                // (track tiles are only read by the group kernel)
-        if (io.n_fwd && (first != c->last_first || n != c->last_n)) return cudaErrorInvalidValue;
-        LaunchDone done_{c, rec, first, n};
-        DgIo g = {};
-        if (c->tracks_T > 0) {
-            const size_t tb = (size_t)first * c->max_obs;
-            g.trk_vx = c->trk_vx + tb; g.trk_vy = c->trk_vy + tb; g.trk_dth = c->trk_dth + tb; g.trk_T = c->tracks_T;
-        }
-        for (int k = 0; k < io.n_mirror; ++k) g.mirror[k] = io.mirror[k];
-        g.n_mirror = io.n_mirror; g.tally = io.tally; g.tally_n = io.tally_n; g.host_done = io.host_done; g.epoch = io.epoch;
-        for (int k = 0; k < io.n_peer_flag; ++k) g.peer_flag[k] = io.peer_flag[k];
-        g.n_peer_flag = io.n_peer_flag; g.flag_value = io.flag_value;
-        g.wait_flag = io.wait_flag; g.n_wait = io.n_wait; g.wait_value = io.wait_value;
-        g.fwd_src = io.fwd_src; g.n_fwd = io.n_fwd;
-        for (int k = 0; k < io.n_fwd; ++k) g.fwd_dst[k] = io.fwd_dst[k];
-        if ((g.n_peer_flag || g.n_wait) && !g.tally) { g.tally = c->d_tally_g; g.tally_n = (unsigned)n; }
-        g.timeline = (n <= 8192) ? c->d_timeline : nullptr;
-        if (g.timeline) cudaMemsetAsync(c->d_timeline, 0, (size_t)8192 * 32 * 8, st);
-        c->launches += 1;
-        return dp_launch_group(c->gmap, c->p, n, hdr, ox, oy, c->max_obs, c->d_carry + first, c->d_last + (size_t)first * DP_PATH_POINTS, rec,
-                               trace, path_xy, path_ll, st, g, c->lc);
+    dp_carry* carry = c->d_carry + first;
+    double2* last_path = c->d_last + (size_t)first * DP_PATH_POINTS;
+    if (!group) {
+        c->launches += 2;
+        return dp_launch_cycle(c->gmap, c->p, n, hdr, ox, oy, c->max_obs, carry, last_path, rec, trace, path_xy, path_ll, st, io, c->lc);
     }
-    return launch_warp(c, first, n, hdr, ox, oy, rec, trace, path_xy, path_ll, st, io);
+    if (c->tracks_T > 0) {
+        const size_t tb = (size_t)first * c->max_obs;
+        io.trk_vx = c->trk_vx + tb; io.trk_vy = c->trk_vy + tb; io.trk_dth = c->trk_dth + tb; io.trk_T = c->tracks_T;
+    }
+    io.timeline = (n <= 8192) ? c->d_timeline : nullptr;
+    if (io.timeline) cudaMemsetAsync(c->d_timeline, 0, (size_t)8192 * 32 * 8, st);
+    c->launches += 1;
+    return dp_launch_group(c->gmap, c->p, n, hdr, ox, oy, c->max_obs, carry, last_path, rec, trace, path_xy, path_ll, st, io, c->lc);
 }
 }  // namespace
 
 namespace {
-int cycle_submit(dp_ctx* c, int first, int n, const dp_scene_hdr* hdr, const double* ox, const double* oy, dp_plan_record* rec, bool dma);
 bool is_pinned(const void* p, void** dev = nullptr) {
     cudaPointerAttributes a;
     if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
@@ -302,9 +269,6 @@ int dp_create(dp_ctx** out, int device, const dp_params* params, int max_scenes,
     c->device = device;
     if (params) c->p = *params; else dp_default_params(&c->p);
     c->max_scenes = max_scenes; c->max_obs = max_obs;
-    c->split = 2;
-    if (const char* e = getenv("DP_SPLIT")) c->split = atoi(e);   // 0: one fused launch, 1: two launches back to back, 2: overlapped
-    if (const char* e = getenv("DP_ZERO_COPY")) c->zero_copy = atoi(e) != 0;
     if (const char* e = getenv("DP_EPISODE_GRAPH")) c->ep_graph = atoi(e) != 0;
     dp_world_default_params(&c->world.wp);
     dp_metrics_default_params(&c->world.mp);
@@ -316,9 +280,7 @@ int dp_create(dp_ctx** out, int device, const dp_params* params, int max_scenes,
     c->kernel = (max_obs >= 32) ? 1 : 0;
     if (const char* e = getenv("DP_KERNEL")) c->kernel = (strcmp(e, "warp") == 0) ? 0 : (strcmp(e, "group") == 0) ? 1 : c->kernel;
     CK(cudaDeviceGetAttribute(&c->lc.sm_count, cudaDevAttrMultiProcessorCount, device));
-    if (const char* e = getenv("DP_WPB")) c->lc.force_wpb = atoi(e);
     if (const char* e = getenv("DP_GROUP_CFG")) c->lc.group_cfg = atoi(e);
-    if (const char* e = getenv("DP_GROUP_G")) c->lc.group_g = atoi(e);
     if (const char* e = getenv("DP_TIMELINE")) {
         if (atoi(e)) { int rt = dev_alloc(&c->d_timeline, (size_t)8192 * 32); if (rt) { delete c; return rt; } cudaMemset(c->d_timeline, 0, (size_t)8192 * 32 * 8); }
     }
@@ -327,14 +289,11 @@ int dp_create(dp_ctx** out, int device, const dp_params* params, int max_scenes,
     if ((r = dev_alloc(&c->d_carry, (size_t)max_scenes))) { delete c; return r; }
     if ((r = dev_alloc(&c->d_last, (size_t)max_scenes * DP_PATH_POINTS))) { delete c; return r; }
     if ((r = dev_alloc(&c->d_done, (size_t)max_scenes))) { delete c; return r; }
-    if ((r = dev_alloc(&c->d_pdone, (size_t)max_scenes)) || (r = dev_alloc(&c->d_inflag, 2)) || (r = dev_alloc(&c->d_tally, 2)) ||
-        (r = dev_alloc(&c->d_tally_g, 2))) { delete c; return r; }
+    if ((r = dev_alloc(&c->d_inflag, 2)) || (r = dev_alloc(&c->d_tally, 2)) || (r = dev_alloc(&c->d_tally_g, 2))) { delete c; return r; }
     CK(cudaMemset(c->d_tally_g, 0, 2 * sizeof(unsigned)));
-    CK(cudaMemset(c->d_pdone, 0, (size_t)max_scenes * sizeof(unsigned)));
     CK(cudaMemset(c->d_inflag, 0, 2 * sizeof(unsigned))); CK(cudaMemset(c->d_tally, 0, 2 * sizeof(unsigned)));
     CK(cudaHostAlloc((void**)&c->h_done, 4 * sizeof(unsigned), cudaHostAllocMapped));
     c->h_done[0] = c->h_done[1] = c->h_done[2] = c->h_done[3] = 0;
-    if (const char* e = getenv("DP_CHAIN")) c->chain = atoi(e);   // 0: events, 1: flags only, 2: flags + chained Decision launch
     CK(cudaMemset(c->d_done, 0, (size_t)max_scenes * sizeof(unsigned)));
     for (int s = 0; s < 2; ++s) {
         CK(cudaStreamCreateWithFlags(&c->st[s], cudaStreamNonBlocking));
@@ -347,12 +306,8 @@ int dp_create(dp_ctx** out, int device, const dp_params* params, int max_scenes,
         CK(cudaMallocHost((void**)&c->h_oy[s], (size_t)c->chunk * max_obs * sizeof(double)));
         CK(cudaMallocHost((void**)&c->h_rec[s], (size_t)c->chunk * sizeof(dp_plan_record)));
         for (int k = 0; k < 3; ++k) CK(cudaEventCreateWithFlags(&c->in_ready[s][k], cudaEventDisableTiming));
-        CK(cudaEventCreateWithFlags(&c->done[s], cudaEventDisableTiming));
     }
     for (int k = 0; k < 3; ++k) CK(cudaStreamCreateWithFlags(&c->cp[k], cudaStreamNonBlocking));
-    CK(cudaStreamCreateWithFlags(&c->cp_out, cudaStreamNonBlocking));
-    for (int s = 0; s < 2; ++s) CK(cudaEventCreateWithFlags(&c->kdone[s], cudaEventDisableTiming));
-    if (const char* e = getenv("DP_REC_DMA")) c->rec_dma = atoi(e);
     *out = c;
     return dp_reset(c, 0, max_scenes);
 }
@@ -366,7 +321,7 @@ int dp_destroy(dp_ctx* c) {
     if (c->ep_exec) cudaGraphExecDestroy(c->ep_exec);
     if (c->ep_stream) cudaStreamDestroy(c->ep_stream);
     cudaFree(c->d_timeline); cudaFree(c->d_trk);
-    cudaFree(c->d_carry); cudaFree(c->d_last); cudaFree(c->d_done); cudaFree(c->d_pdone); cudaFree(c->d_inflag); cudaFree(c->d_tally); cudaFree(c->d_tally_g);
+    cudaFree(c->d_carry); cudaFree(c->d_last); cudaFree(c->d_done); cudaFree(c->d_inflag); cudaFree(c->d_tally); cudaFree(c->d_tally_g);
     if (c->h_done) cudaFreeHost(c->h_done);
     for (int s = 0; s < 2; ++s) {
         cudaFree(c->d_hdr[s]); cudaFree(c->d_ox[s]); cudaFree(c->d_oy[s]); cudaFree(c->d_rec[s]);
@@ -374,11 +329,8 @@ int dp_destroy(dp_ctx* c) {
         cudaFreeHost(c->h_hdr[s]); cudaFreeHost(c->h_ox[s]); cudaFreeHost(c->h_oy[s]); cudaFreeHost(c->h_rec[s]);
         if (c->st[s]) cudaStreamDestroy(c->st[s]);
         for (int k = 0; k < 3; ++k) if (c->in_ready[s][k]) cudaEventDestroy(c->in_ready[s][k]);
-        if (c->done[s]) cudaEventDestroy(c->done[s]);
     }
     for (int k = 0; k < 3; ++k) if (c->cp[k]) cudaStreamDestroy(c->cp[k]);
-    if (c->cp_out) cudaStreamDestroy(c->cp_out);
-    for (int s = 0; s < 2; ++s) if (c->kdone[s]) cudaEventDestroy(c->kdone[s]);
     delete c;
     return DP_OK;
 }
@@ -491,7 +443,6 @@ int dp_map_upload(dp_ctx* c, const dp_map_desc* m) {
 int dp_reset(dp_ctx* c, int first, int count) {
     if (!c || first < 0 || count < 0 || first + count > c->max_scenes) return fail(DP_ERR_ARG, "dp_reset: range");
     if (c->submitted != c->waited) return fail(DP_ERR_STATE, "dp_reset: submitted cycles in flight, call dp_cycle_wait first");
-    c->chain_prev_epoch = 0;
     CK(cudaSetDevice(c->device));
     CK(dp_launch_reset(c->d_carry, c->d_last, first, count, c->st[0]));
     ++c->launches;
@@ -502,7 +453,6 @@ int dp_reset(dp_ctx* c, int first, int count) {
 int dp_reset_dev(dp_ctx* c, int first, int count, void* stream) {
     if (!c || first < 0 || count < 0 || first + count > c->max_scenes) return fail(DP_ERR_ARG, "dp_reset_dev: range");
     if (c->submitted != c->waited) return fail(DP_ERR_STATE, "dp_reset_dev: submitted cycles in flight, call dp_cycle_wait first");
-    c->chain_prev_epoch = 0;
     CK(cudaSetDevice(c->device));
     CK(dp_launch_reset(c->d_carry, c->d_last, first, count, (cudaStream_t)stream));
     ++c->launches;
@@ -529,7 +479,6 @@ int dp_carry_download(dp_ctx* c, int first, int count, dp_carry* hc, double* hl)
 int dp_carry_upload(dp_ctx* c, int first, int count, const dp_carry* hc, const double* hl) {
     if (!c || first < 0 || count < 0 || first + count > c->max_scenes) return fail(DP_ERR_ARG, "dp_carry_upload: range");
     if (c->submitted != c->waited) return fail(DP_ERR_STATE, "dp_carry_upload: submitted cycles in flight, call dp_cycle_wait first");
-    c->chain_prev_epoch = 0;
     CK(cudaSetDevice(c->device));
     CK(cudaDeviceSynchronize());
     if (hc) CK(cudaMemcpy(c->d_carry + first, hc, (size_t)count * sizeof(dp_carry), cudaMemcpyHostToDevice));
@@ -561,9 +510,9 @@ int dp_run_episode_dev(dp_ctx* c, int first, int n, int cycles, const dp_scene_h
     if (c->submitted != c->waited) return fail(DP_ERR_STATE, "dp_run_episode_dev: submitted cycles in flight, call dp_cycle_wait first");
     CK(cudaSetDevice(c->device));
     const size_t mo = (size_t)c->max_obs;
-    // back-to-back launch pairs, no host involvement in between.  (Chaining cycle k+1's Decision launch to cycle k's Planning
-    // launch as dp_cycle_submit does was measured here too: 84 vs 66 us per 4096-scene cycle -- the early Decision CTAs spin in
-    // slots the Planning launch needs -- so the episode runner keeps the plain stream order.)
+    // back-to-back launch pairs, no host involvement in between.  (Cycle k+1's Decision launch as a programmatic dependent of
+    // cycle k's Planning launch was measured here too: 84 vs 66 us per 4096-scene cycle -- the early Decision CTAs spin in slots
+    // the Planning launch needs -- so the episode runner keeps the plain stream order.)
     for (int k = 0; k < cycles; ++k) {
         const DpIo io = make_io(c, first, nullptr);
         CK(run_cycle(c, first, n, hdr + (size_t)k * n, ox + (size_t)k * n * mo, oy + (size_t)k * n * mo, rec + (size_t)k * n, nullptr, nullptr,
@@ -583,28 +532,15 @@ int dp_cycle_batch(dp_ctx* c, int first, int n, const dp_scene_hdr* hdr, const d
     if (path_xy && (r = ensure_optional(c, 1))) return r;
     if (path_ll && (r = ensure_optional(c, 2))) return r;
     const size_t mo = (size_t)c->max_obs;
-    void *dv_hdr = nullptr, *dv_ox = nullptr, *dv_oy = nullptr, *dv_rec = nullptr;
-    const bool pin_in = is_pinned(hdr, &dv_hdr) && is_pinned(ox, &dv_ox) && is_pinned(oy, &dv_oy);
-    const bool pin_rec = is_pinned(rec, &dv_rec);
+    const bool pin_in = is_pinned(hdr) && is_pinned(ox) && is_pinned(oy);
+    const bool pin_rec = is_pinned(rec);
     const bool plain = n <= c->chunk && !trace && !path_xy && !path_ll;
-    if (plain && pin_in && pin_rec && !c->zero_copy) {
+    if (plain && pin_in && pin_rec) {
         // Page-locked buffers: the pipelined machinery with one cycle in flight -- three overlapping input DMAs, the two
         // launches, and the Planning launch storing each finished 128-byte record straight into the caller's buffer.
-        int rs = cycle_submit(c, first, n, hdr, ox, oy, rec, false);   // one call in flight: the kernel stores the records itself
+        int rs = dp_cycle_submit(c, first, n, hdr, ox, oy, rec);
         if (rs != DP_OK) return rs;
         return dp_cycle_wait(c);
-    }
-    if (plain && c->zero_copy && c->split && c->kernel == 0 && pin_in && pin_rec && dv_hdr && dv_ox && dv_oy && dv_rec) {
-        // DP_ZERO_COPY=1: the Decision launch pulls the 128-byte headers and the obstacle rows straight out of the caller's
-        // pinned buffers over PCIe (one coalesced load per scene) and leaves device copies for the Planning launch, which
-        // pushes each finished record into the caller's pinned result buffer.  No copy engines -- but GPU-issued PCIe reads
-        // are slower than the DMA route above (163 vs 120 us per 4096-scene call), so this is not the default.
-        cudaStream_t st = c->st[0];
-        DpIo io = make_io(c, first, (dp_plan_record*)dv_rec);
-        io.hdr_stage = c->d_hdr[0]; io.ox_stage = c->d_ox[0]; io.oy_stage = c->d_oy[0];
-        CK(launch_warp(c, first, n, (const dp_scene_hdr*)dv_hdr, (const double*)dv_ox, (const double*)dv_oy, c->d_rec[0], nullptr, nullptr, nullptr, st, io));
-        CK(cudaStreamSynchronize(st));
-        return DP_OK;
     }
     int nchunks = (n + c->chunk - 1) / c->chunk;
     for (int k = 0; k < nchunks; ++k) {
@@ -641,11 +577,9 @@ int dp_cycle_batch(dp_ctx* c, int first, int n, const dp_scene_hdr* hdr, const d
     return DP_OK;
 }
 
-}  // extern "C"
-namespace {
-// dma: the records reach the caller's buffer by a device->host copy behind the kernels (pipelined use: it overlaps the next cycle);
-// otherwise the Planning warps store them there themselves (one call in flight: no copy in the tail of the call)
-int cycle_submit(dp_ctx* c, int first, int n, const dp_scene_hdr* hdr, const double* ox, const double* oy, dp_plan_record* rec, bool dma) {
+// The records reach the caller's buffer by stores of the kernel (the Planning warps, or the group kernel's CTAs): no copy in the
+// tail of a call
+int dp_cycle_submit(dp_ctx* c, int first, int n, const dp_scene_hdr* hdr, const double* ox, const double* oy, dp_plan_record* rec) {
     if (!c || !hdr || !ox || !oy || !rec || n < 0 || first < 0 || first + n > c->max_scenes || n > c->chunk)
         return fail(DP_ERR_ARG, "dp_cycle_submit: bad argument");
     if (!c->have_map) return fail(DP_ERR_STATE, "dp_cycle_submit: map not uploaded");
@@ -658,10 +592,15 @@ int cycle_submit(dp_ctx* c, int first, int n, const dp_scene_hdr* hdr, const dou
     const int s = (int)(c->submitted & 1);
     const size_t mo = (size_t)c->max_obs;
     cudaStream_t st = c->st[0];                             // one compute stream: cycle k+1 reads the carry cycle k wrote
+    DpIo io = make_io(c, first, (dp_plan_record*)dv_rec);
+    void* dv_done = nullptr;
+    CK(cudaHostGetDevicePointer(&dv_done, c->h_done, 0));
+    // the last Planning warp / CTA of the cycle stores its epoch to page-locked host memory (dp_cycle_wait polls it: no event round
+    // trip) and re-arms the tally word itself, no memset
+    io.tally = c->d_tally + s; io.tally_n = (unsigned)n; io.host_done = (unsigned*)dv_done + s;
+    c->wait_epoch[s] = n > 0 ? io.epoch : 0u;
     if (c->kernel == 1 || c->tracks_T > 0) {
-        // group kernel: the three input DMAs overlap on their own copy streams, the launch waits for their events; the kernel
-        // stores every record into the caller's page-locked buffer itself and its last CTA raises a flag in page-locked memory
-        // (dp_cycle_wait polls it: no event round trip).  The tally word is re-armed by that last CTA, not by a memset.
+        // group kernel: the three input DMAs overlap on their own copy streams, the launch waits for their events
         CK(cudaMemcpyAsync(c->d_hdr[s], hdr, (size_t)n * sizeof(dp_scene_hdr), cudaMemcpyHostToDevice, c->cp[0]));
         CK(cudaMemcpyAsync(c->d_ox[s], ox, (size_t)n * mo * 8, cudaMemcpyHostToDevice, c->cp[1]));
         CK(cudaMemcpyAsync(c->d_oy[s], oy, (size_t)n * mo * 8, cudaMemcpyHostToDevice, c->cp[2]));
@@ -669,21 +608,9 @@ int cycle_submit(dp_ctx* c, int first, int n, const dp_scene_hdr* hdr, const dou
             CK(cudaEventRecord(c->in_ready[s][k], c->cp[k]));
             CK(cudaStreamWaitEvent(st, c->in_ready[s][k], 0));
         }
-        DpIo io = make_io(c, first, (dp_plan_record*)dv_rec);
-        void* dv_done = nullptr;
-        CK(cudaHostGetDevicePointer(&dv_done, c->h_done, 0));
-        io.tally = c->d_tally + s; io.tally_n = (unsigned)n; io.host_done = (unsigned*)dv_done + s;
-        c->wait_epoch[s] = n > 0 ? io.epoch : 0u;
-        CK(run_cycle(c, first, n, c->d_hdr[s], c->d_ox[s], c->d_oy[s], c->d_rec[s], nullptr, nullptr, nullptr, st, io));
-        ++c->submitted;
-        return DP_OK;
-    }
-    if (c->chain && c->split == 2) {
-        // Chained: nothing but kernels goes into the compute stream.  The copy stream carries the three input DMAs and then a
-        // four-byte copy that raises in_flag; the Decision warps wait for that flag, and per scene for the previous cycle's
-        // Planning warp; the last Planning warp of the batch stores the epoch to page-locked host memory (dp_cycle_wait).
-        const unsigned prev = (c->chain >= 2 && c->chain_prev_epoch && c->chain_first == first && c->chain_n == n) ? c->chain_prev_epoch : 0u;
-        DpIo io = make_io(c, first, dma ? nullptr : (dp_plan_record*)dv_rec);
+    } else {
+        // warp kernel: nothing but kernels goes into the compute stream.  The copy stream carries the three input DMAs and then a
+        // four-byte copy that raises in_flag; the Decision warps wait for that flag
         CK(cudaMemcpyAsync(c->d_hdr[s], hdr, (size_t)n * sizeof(dp_scene_hdr), cudaMemcpyHostToDevice, c->cp[0]));
         CK(cudaMemcpyAsync(c->d_ox[s], ox, (size_t)n * mo * 8, cudaMemcpyHostToDevice, c->cp[0]));
         CK(cudaMemcpyAsync(c->d_oy[s], oy, (size_t)n * mo * 8, cudaMemcpyHostToDevice, c->cp[0]));
@@ -691,69 +618,30 @@ int cycle_submit(dp_ctx* c, int first, int n, const dp_scene_hdr* hdr, const dou
         // CTAs that are waiting for exactly this flag
         c->h_done[2 + s] = io.epoch;
         CK(cudaMemcpyAsync(c->d_inflag + s, c->h_done + 2 + s, sizeof(unsigned), cudaMemcpyHostToDevice, c->cp[0]));
-        void* dv_done = nullptr;
-        CK(cudaHostGetDevicePointer(&dv_done, c->h_done, 0));
         io.in_flag = c->d_inflag + s;
-        io.pdone = c->d_pdone + first; io.prev_epoch = prev;
-        if (!dma) { io.tally = c->d_tally + s; io.tally_n = (unsigned)n; io.host_done = (unsigned*)dv_done + s; }
-        c->wait_epoch[s] = n > 0 ? io.epoch : 0u;
-        CK(launch_warp(c, first, n, c->d_hdr[s], c->d_ox[s], c->d_oy[s], c->d_rec[s], nullptr, nullptr, nullptr, st, io));
-        if (dma) {
-            // behind the kernels, on its own stream: the records, then the completion word (the epoch the input copies left in
-            // d_inflag[s]) -- two DMAs that run beside the next cycle's kernels; dp_cycle_wait polls the same page-locked word
-            CK(cudaEventRecord(c->kdone[s], st));
-            CK(cudaStreamWaitEvent(c->cp_out, c->kdone[s], 0));
-            CK(cudaMemcpyAsync(rec, c->d_rec[s], (size_t)n * sizeof(dp_plan_record), cudaMemcpyDeviceToHost, c->cp_out));
-            CK(cudaMemcpyAsync(c->h_done + s, c->d_inflag + s, sizeof(unsigned), cudaMemcpyDeviceToHost, c->cp_out));
-        }
-        c->chain_prev_epoch = io.epoch; c->chain_first = first; c->chain_n = n;
-    } else {
-        CK(cudaMemcpyAsync(c->d_hdr[s], hdr, (size_t)n * sizeof(dp_scene_hdr), cudaMemcpyHostToDevice, c->cp[0]));
-        CK(cudaMemcpyAsync(c->d_ox[s], ox, (size_t)n * mo * 8, cudaMemcpyHostToDevice, c->cp[1]));
-        CK(cudaMemcpyAsync(c->d_oy[s], oy, (size_t)n * mo * 8, cudaMemcpyHostToDevice, c->cp[2]));
-        for (int k = 0; k < 3; ++k) {
-            CK(cudaEventRecord(c->in_ready[s][k], c->cp[k]));
-            CK(cudaStreamWaitEvent(st, c->in_ready[s][k], 0));
-        }
-        CK(launch_warp(c, first, n, c->d_hdr[s], c->d_ox[s], c->d_oy[s], c->d_rec[s], nullptr, nullptr, nullptr, st,
-                       make_io(c, first, (dp_plan_record*)dv_rec)));
-        CK(cudaEventRecord(c->done[s], st));
-        c->wait_epoch[s] = 0;
     }
+    CK(run_cycle(c, first, n, c->d_hdr[s], c->d_ox[s], c->d_oy[s], c->d_rec[s], nullptr, nullptr, nullptr, st, io));
     ++c->submitted;
     return DP_OK;
-}
-}  // namespace
-extern "C" {
-int dp_cycle_submit(dp_ctx* c, int first, int n, const dp_scene_hdr* hdr, const double* ox, const double* oy, dp_plan_record* rec) {
-    return cycle_submit(c, first, n, hdr, ox, oy, rec, c && c->rec_dma != 0);
 }
 int dp_cycle_wait(dp_ctx* c) {
     if (!c) return fail(DP_ERR_ARG, "dp_cycle_wait: null context");
     if (c->submitted == c->waited) return fail(DP_ERR_STATE, "dp_cycle_wait: nothing in flight");
     CK(cudaSetDevice(c->device));
     const int s = (int)(c->waited & 1);
-    if (c->kernel == 1 || c->tracks_T > 0 || (c->chain && c->split == 2)) {
-        const unsigned want = c->wait_epoch[s];
-        const volatile unsigned* flag = c->h_done + s;
-        if (want) {
-            const auto t0 = std::chrono::steady_clock::now();
-            for (unsigned long long spin = 0; *flag != want; ++spin) {
-                if ((spin & 0xfff) == 0xfff) {              // a kernel that trapped never raises the flag: ask the stream now and then
-                    const cudaError_t q = cudaStreamQuery(c->st[0]);
-                    if (q != cudaSuccess && q != cudaErrorNotReady) return fail(DP_ERR_CUDA, "dp_cycle_wait", q);
-                    if (q == cudaSuccess) {                  // (the flag may still be on its way behind the record copy, on the output stream)
-                        const cudaError_t q2 = cudaStreamQuery(c->cp_out);
-                        if (q2 != cudaSuccess && q2 != cudaErrorNotReady) return fail(DP_ERR_CUDA, "dp_cycle_wait", q2);
-                        if (q2 == cudaSuccess && *flag != want) return fail(DP_ERR_CUDA, "dp_cycle_wait: the streams drained without the completion flag");
-                    }
-                    if (std::chrono::steady_clock::now() - t0 > std::chrono::seconds(30)) return fail(DP_ERR_CUDA, "dp_cycle_wait: timed out");
-                }
+    const unsigned want = c->wait_epoch[s];
+    const volatile unsigned* flag = c->h_done + s;
+    if (want) {
+        const auto t0 = std::chrono::steady_clock::now();
+        for (unsigned long long spin = 0; *flag != want; ++spin) {
+            if ((spin & 0xfff) == 0xfff) {                  // a kernel that trapped never raises the flag: ask the stream now and then
+                const cudaError_t q = cudaStreamQuery(c->st[0]);
+                if (q != cudaSuccess && q != cudaErrorNotReady) return fail(DP_ERR_CUDA, "dp_cycle_wait", q);
+                if (q == cudaSuccess && *flag != want) return fail(DP_ERR_CUDA, "dp_cycle_wait: the stream drained without the completion flag");
+                if (std::chrono::steady_clock::now() - t0 > std::chrono::seconds(30)) return fail(DP_ERR_CUDA, "dp_cycle_wait: timed out");
             }
-            std::atomic_thread_fence(std::memory_order_acquire);
         }
-    } else {
-        CK(cudaEventSynchronize(c->done[s]));
+        std::atomic_thread_fence(std::memory_order_acquire);
     }
     ++c->waited;
     return DP_OK;
@@ -764,9 +652,9 @@ int dp_set_record_mirrors(dp_ctx* c, int n, void* const* bases) {
     if (c->submitted != c->waited) return fail(DP_ERR_STATE, "dp_set_record_mirrors: submitted cycles in flight, call dp_cycle_wait first");
     for (int k = 0; k < n; ++k) {
         if (!bases[k]) return fail(DP_ERR_ARG, "dp_set_record_mirrors: null base");
-        c->mirror[k] = (dp_plan_record*)bases[k];
+        c->armed.mirror[k] = (dp_plan_record*)bases[k];
     }
-    c->n_mirror = n;
+    c->armed.n_mirror = n;
     return DP_OK;
 }
 
@@ -816,14 +704,14 @@ struct dp_gather {
     int lag = 1;                                            // a launch awaits the flags of the step `lag` launches back (dp_gather_set_lag)
 };
 namespace {
-// deferred gather: point the context (or a flush launch) at the buffers / flags of step `step`
-void gather_route(dp_gather* g, unsigned step, dp_plan_record** dst, unsigned** flag, const unsigned** wait) {
+// the buffers / flags of step `step`: this rank's slice and flag word in every rank's buffer, and this rank's flag words of the step
+void gather_route(dp_gather* g, unsigned step, dp_plan_record** dst, unsigned** flag, DpWait* wait) {
     const size_t b = step % (unsigned)g->depth;
     for (int r = 0; r < g->world; ++r) {
         dst[r] = reinterpret_cast<dp_plan_record*>(g->base[r]) + (b * g->world + g->rank) * g->slots;
         flag[r] = reinterpret_cast<unsigned*>(g->base[r] + g->rec_bytes) + b * g->world + g->rank;
     }
-    *wait = reinterpret_cast<const unsigned*>(g->base[g->rank] + g->rec_bytes) + b * g->world;
+    if (wait) *wait = {reinterpret_cast<const unsigned*>(g->base[g->rank] + g->rec_bytes) + b * g->world, g->world, step};
 }
 }  // namespace
 static_assert(DP_IPC_BYTES >= sizeof(cudaIpcMemHandle_t), "DP_IPC_BYTES");
@@ -861,36 +749,34 @@ int dp_gather_attach(dp_gather* g, const void* handles) {
 int dp_gather_arm(dp_gather* g, unsigned step) {
     if (!g || step == 0) return fail(DP_ERR_ARG, "dp_gather_arm: bad argument (steps count from 1)");
     dp_ctx* c = g->c;                                       // (only read by the NEXT launch call of this thread: fine between pipelined submits)
-    const size_t b = step % (unsigned)g->depth;
-    c->n_mirror = 0; c->n_peer_flag = 0;
-    for (int r = 0; r < g->world; ++r) {
-        if (!g->base[r]) return fail(DP_ERR_STATE, "dp_gather_arm: dp_gather_attach first");
-        c->mirror[c->n_mirror++] = reinterpret_cast<dp_plan_record*>(g->base[r]) + (b * g->world + g->rank) * g->slots;
-        c->peer_flag[c->n_peer_flag++] = reinterpret_cast<unsigned*>(g->base[r] + g->rec_bytes) + b * g->world + g->rank;
-    }
-    c->flag_value = step;
+    for (int r = 0; r < g->world; ++r) if (!g->base[r]) return fail(DP_ERR_STATE, "dp_gather_arm: dp_gather_attach first");
+    DpIo a = {};                                            // replaces the mirrors and any armed gather; a wait folded in by dp_gather_chain stays
+    a.wait = c->armed.wait;
+    gather_route(g, step, a.mirror, a.peer_flag, nullptr);
+    a.n_mirror = a.n_peer_flag = g->world;
+    a.flag_value = step;
+    c->armed = a; c->deferred = false;
     return DP_OK;
 }
 int dp_gather_arm_deferred(dp_gather* g, unsigned step) {
     if (!g || step == 0) return fail(DP_ERR_ARG, "dp_gather_arm_deferred: bad argument (steps count from 1)");
     dp_ctx* c = g->c;
     for (int r = 0; r < g->world; ++r) if (!g->base[r]) return fail(DP_ERR_STATE, "dp_gather_arm_deferred: dp_gather_attach first");
-    c->n_mirror = 0; c->n_fwd = 0; c->n_peer_flag = 0; c->n_wait = 0; c->wait_flag = nullptr;
+    DpIo a = {};
     if (g->pending && c->last_rec) {                        // the launch that follows forwards and flags the step before ...
-        gather_route(g, g->pending, c->fwd_dst, c->peer_flag, &c->wait_flag);
-        c->n_fwd = c->n_peer_flag = g->world;
-        c->flag_value = g->pending;
+        gather_route(g, g->pending, a.fwd_dst, a.peer_flag, nullptr);
+        a.n_fwd = a.n_peer_flag = g->world;
+        a.flag_value = g->pending;
         // ... and awaits every rank's flags of that step (lag 1) or of the one before it (lag 2: a full step of slack between the
         // ranks; that step was forwarded by the launch before, so only launches that have one to wait for do)
         const unsigned w = (g->lag == 1) ? g->pending : g->forwarded;
         if (w) {
             dp_plan_record* d_[DP_MAX_MIRRORS]; unsigned* f_[DP_MAX_MIRRORS];
-            gather_route(g, w, d_, f_, &c->wait_flag);
-            c->n_wait = g->world; c->wait_value = w;
-        } else c->wait_flag = nullptr;
+            gather_route(g, w, d_, f_, &a.wait);
+        }
         g->forwarded = g->pending;
     }
-    c->deferred = true;
+    c->armed = a; c->deferred = true;
     g->pending = step;
     return DP_OK;
 }
@@ -904,11 +790,11 @@ int dp_gather_flush(dp_gather* g, void* stream) {
     dp_ctx* c = g->c;
     if (!g->pending || !c->last_rec) return DP_OK;
     CK(cudaSetDevice(c->device));
-    DpIo io = dp_io_none();
-    gather_route(g, g->pending, io.fwd_dst, io.peer_flag, &io.wait_flag);
+    DpIo io = {};
+    gather_route(g, g->pending, io.fwd_dst, io.peer_flag, &io.wait);
     for (int r = 0; r < g->world; ++r) io.fwd_dst[r] += c->last_first;
-    io.n_fwd = io.n_peer_flag = io.n_wait = g->world;
-    io.flag_value = io.wait_value = g->pending;
+    io.n_fwd = io.n_peer_flag = g->world;
+    io.flag_value = g->pending;
     if (g->lag == 2 && g->forwarded) {                      // the step before may not have been awaited by any launch yet
         CK(dp_launch_gather_wait(reinterpret_cast<const unsigned*>(g->base[g->rank] + g->rec_bytes) + (size_t)(g->forwarded % (unsigned)g->depth) * g->world,
                                  g->world, g->forwarded, (cudaStream_t)stream));
@@ -922,17 +808,16 @@ int dp_gather_flush(dp_gather* g, void* stream) {
 int dp_gather_chain(dp_gather* g, unsigned prev_step) {
     if (!g) return fail(DP_ERR_ARG, "dp_gather_chain: null");
     dp_ctx* c = g->c;
-    if (prev_step == 0) { c->wait_flag = nullptr; c->n_wait = 0; c->wait_value = 0; return DP_OK; }
+    if (prev_step == 0) { c->armed.wait = {}; return DP_OK; }
     if (!g->base[g->rank]) return fail(DP_ERR_STATE, "dp_gather_chain: dp_gather_attach first");
-    c->wait_flag = reinterpret_cast<const unsigned*>(g->base[g->rank] + g->rec_bytes) + (size_t)(prev_step % (unsigned)g->depth) * g->world;
-    c->n_wait = g->world; c->wait_value = prev_step;
+    c->armed.wait = {reinterpret_cast<const unsigned*>(g->base[g->rank] + g->rec_bytes) + (size_t)(prev_step % (unsigned)g->depth) * g->world,
+                     g->world, prev_step};
     return DP_OK;
 }
 int dp_gather_disarm(dp_gather* g) {
     if (!g) return fail(DP_ERR_ARG, "dp_gather_disarm: null");
-    g->c->n_mirror = 0; g->c->n_peer_flag = 0;
-    g->c->wait_flag = nullptr; g->c->n_wait = 0; g->c->wait_value = 0;
-    g->c->n_fwd = 0; g->c->deferred = false; g->pending = 0; g->forwarded = 0;
+    g->c->armed = {}; g->c->deferred = false;
+    g->pending = 0; g->forwarded = 0;
     return DP_OK;
 }
 int dp_gather_wait(dp_gather* g, unsigned step, void* stream) {
@@ -1531,7 +1416,7 @@ int dp_run_closed_loop_dev(dp_ctx* c, int first, int n, int cycles, dp_scene_hdr
     c->ep_last_graph = 0;
     if (n == 0) return DP_OK;
     // the graph holds the warp-kernel launches of a plain context (no gather armed, no record mirrors, no predicted tracks)
-    const bool plain = c->kernel == 0 && c->tracks_T == 0 && !c->n_mirror && !c->n_peer_flag && !c->n_wait && !c->n_fwd;
+    const bool plain = c->kernel == 0 && c->tracks_T == 0 && !armed_any(c->armed);
     if (c->ep_graph && plain) {
         const void* key[8] = {hdr, agents, ox, oy, rec, hdr_log, olx, oly};
         const int dims[3] = {first, n, cycles};

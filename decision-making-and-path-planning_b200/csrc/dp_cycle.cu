@@ -1,5 +1,5 @@
 // csrc/dp_cycle.cu -- the Decision + Planning cycle kernel (sm_100a): dp_cycle_kernel<PHASE, WPB>, launched as a Decision
-// half and a Planning half that overlap scene by scene (PHASE 1 / 2; PHASE 0 = both halves in one launch), see below.
+// half and a Planning half that overlap scene by scene (PHASE 1 / 2), see below.
 //
 // One WARP owns one scene for the whole cycle: LoadRefPath -> AroundObstacle -> BehaviorDecision
 // (with the in-lane avoid sweep) -> SpeedDecision/RefPath  (Decision.cpp:216-315, 323-486), then
@@ -200,9 +200,9 @@ template <class T> __device__ __forceinline__ T dp_l2(const T* p) { return __ldc
 #endif
 #define DP_MIN_BLOCKS(WPB) ((WPB) == 1 ? DP_MIN_BLOCKS_W1 : 7)
 
-// PHASE 0: whole cycle in one launch.  PHASE 1 / 2: Decision half / Planning half as two back-to-back launches -- the
-// same work with half the code per kernel: with 28 warps per SM in different places of a ~11 k-instruction kernel the
-// instruction cache thrashes (ncu: 25 % `no_instruction` stalls); each half alone fits.  The hand-off between the two
+// PHASE 1 / 2: Decision half / Planning half as two launches -- the same work with half the code per kernel: with 28 warps
+// per SM in different places of a ~11 k-instruction kernel the instruction cache thrashes (ncu: 25 % `no_instruction` stalls);
+// each half alone fits.  The hand-off between the two
 // halves is what the reference hands from CDecisionThread to CPlanningThread (DecisionOut, Decision.cpp:187-205),
 // already stored in dp_carry / dp_plan_record.
 #ifdef DP_DEBUG_CLOCK
@@ -246,19 +246,17 @@ dp_cycle_kernel(DevMap m, dp_params p, int n_scenes, const dp_scene_hdr* __restr
 #endif
     WarpSmem& sm = smem[wib];
     if (PHASE == 1 && io.done) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");   // Planning CTAs may start filling in
-    if (PHASE == 2 && io.pdone) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");  // ... and the next cycle's Decision CTAs
     if (PHASE == 1 && io.in_flag) dp_await(io.in_flag, io.epoch);                                // chained submit: inputs staged?
     if (PHASE == 2 && io.done) dp_await(io.done + scene, io.epoch);
     // while the header is on its way: ask L2 for the lines the warp needs next and whose addresses do not depend on it -- the two
     // obstacle rows and the carry (otherwise three DRAM round trips in a row at the start of every scene after an L2 flush)
-    if (PHASE == 1 && !io.in_flag && !io.hdr_stage && lane < 5) {
+    if (PHASE == 1 && !io.in_flag && lane < 5) {
         const size_t row = (size_t)scene * max_obs, last = (size_t)(max_obs > 0 ? max_obs - 1 : 0);
         const void* a = lane == 0 ? (const void*)(obs_x + row) : lane == 1 ? (const void*)(obs_x + row + last)
                       : lane == 2 ? (const void*)(obs_y + row) : lane == 3 ? (const void*)(obs_y + row + last) : (const void*)(carry + scene);
         asm volatile("prefetch.global.L2 [%0];" ::"l"(a));
     }
-    // the 128-byte scene header comes in with one coalesced warp load (from HBM, or straight from pinned host memory
-    // over PCIe in the zero-copy mode of dp_cycle_batch) and is read from shared memory afterwards
+    // the 128-byte scene header comes in with one coalesced warp load and is read from shared memory afterwards
     sm.hdr[lane] = (PHASE == 2 || io.in_flag) ? dp_l2(reinterpret_cast<const uint32_t*>(hdr + scene) + lane)   // (staged by a concurrent launch / copy)
                                               : reinterpret_cast<const uint32_t*>(hdr + scene)[lane];
     __syncwarp();
@@ -266,32 +264,22 @@ dp_cycle_kernel(DevMap m, dp_params p, int n_scenes, const dp_scene_hdr* __restr
     const double* ox = obs_x + (size_t)scene * max_obs;
     const double* oy = obs_y + (size_t)scene * max_obs;
     const int N = min((int)h.n_obs, max_obs);
-    if (PHASE != 2 && io.hdr_stage) {                       // zero-copy ingest: keep a device copy for the Planning launch
-        reinterpret_cast<uint32_t*>(io.hdr_stage + scene)[lane] = sm.hdr[lane];
-        for (int k = lane; k < N; k += 32) {
-            io.ox_stage[(size_t)scene * max_obs + k] = ox[k];
-            io.oy_stage[(size_t)scene * max_obs + k] = oy[k];
-        }
-    }
     double2* lastp = last_path + (size_t)scene * DP_PATH_POINTS;
     dp_carry* const cg = carry + scene;
     dp_plan_record* const out = rec + scene;                // the record is assembled in place: fields are stored when final
-    // chained submit: the previous cycle's Planning warp of THIS scene may still be running (it reads the hand-off in the
-    // carry this warp is about to overwrite): wait for it, scene by scene
-    if (PHASE == 1 && io.prev_epoch) dp_await(io.pdone + scene, io.prev_epoch);
-    // deferred gather: last cycle's record of this scene (DgIo) is picked up here, before this cycle overwrites it, and sent
+    // deferred gather: last cycle's record of this scene (DpIo) is picked up here, before this cycle overwrites it, and sent
     // when the Decision half of the scene is done: the warps of a launch START together (28 per SM x 148 SMs x world stores at
     // once is a 4 us NVLink burst that every warp then sits behind: +3.9 us per step at 8 GPUs), but they FINISH spread over
     // 15-50 us
     uint32_t fwd_w = 0;
-    if (PHASE != 2 && io.n_fwd) fwd_w = __ldcg(reinterpret_cast<const uint32_t*>(io.fwd_src + scene) + lane);
+    if (PHASE == 1 && io.n_fwd) fwd_w = __ldcg(reinterpret_cast<const uint32_t*>(io.fwd_src + scene) + lane);
     const LaneMap lm = dp_lane_map(N, lane);
     // this lane's obstacle stays in registers for the whole cycle when N < 32
     const bool lm_act = (lm.nchunk > 1) && (lane < N * lm.nchunk);
     const bool via_l2 = PHASE == 2 || io.in_flag != nullptr;
     const double mx = lm_act ? (via_l2 ? dp_l2(ox + lm.o) : ox[lm.o]) : 0.0, my = lm_act ? (via_l2 ? dp_l2(oy + lm.o) : oy[lm.o]) : 0.0;
     dp_trace_record* tr = trace ? trace + scene : nullptr;
-    if (tr && PHASE != 2) {                                 // zero the trace record cooperatively
+    if (tr && PHASE == 1) {                                 // zero the trace record cooperatively
         uint32_t* w = reinterpret_cast<uint32_t*>(tr);
         for (int i = lane; i < (int)(sizeof(dp_trace_record) / 4); i += 32) w[i] = 0;
         __syncwarp();
@@ -406,13 +394,13 @@ dp_cycle_kernel(DevMap m, dp_params p, int n_scenes, const dp_scene_hdr* __restr
         DBG_MARK(0, 4);
 
         // ---- BehaviorDecision (Decision.cpp:898-1773) ----
-        dp_carry c;
-        if (PHASE == 1) {                                   // through L2: in a chain the line was written by launches that may still be running
+        dp_carry c;                                         // (read through L2, 16 bytes at a time)
+        {
             const int4* src = reinterpret_cast<const int4*>(cg);
             int4* dst = reinterpret_cast<int4*>(&c);
 #pragma unroll
             for (int k = 0; k < (int)(sizeof(dp_carry) / 16); ++k) dst[k] = __ldcg(src + k);
-        } else c = *cg;
+        }
         Beh cur;
         cur.behavior = c.behavior; cur.target = c.target_lanenum; cur.light = c.light_status;
         cur.lanechg = c.lanechg_status != 0; cur.obsavoid = c.obsavoid_status != 0; cur.dlg = c.behavior_to_dlg;
@@ -674,7 +662,7 @@ dp_cycle_kernel(DevMap m, dp_params p, int n_scenes, const dp_scene_hdr* __restr
         }
     }
     DBG_T(0);
-    if (PHASE != 2 && tr && lane == 0) tr->refpath_len = (uint16_t)(rp_n0 + rp_n1);
+    if (PHASE == 1 && tr && lane == 0) tr->refpath_len = (uint16_t)(rp_n0 + rp_n1);
     if (PHASE == 1) {                                       // hand the counters over and stop: the Planning launch follows
         if (lane == 0) {
             out->n_traj = (uint16_t)n_traj;
@@ -689,32 +677,16 @@ dp_cycle_kernel(DevMap m, dp_params p, int n_scenes, const dp_scene_hdr* __restr
         }
         if (io.flag_mode == 1 && io.tally2) {               // deferred gather: every forwarded record is out when the last Decision warp retires
             __threadfence(); __syncwarp();                  // (every lane: its forwarded words before the tally)
-            if (lane == 0 && atomicAdd(io.tally2, 1u) == io.tally_n - 1u) {
-                *io.tally2 = 0;
-                __threadfence_system();
-#pragma unroll
-                for (int k = 0; k < DP_MAX_MIRRORS; ++k)
-                    if (k < io.n_peer_flag) asm volatile("st.relaxed.sys.global.u32 [%0], %1;" ::"l"(io.peer_flag[k]), "r"(io.flag_value) : "memory");
-                // ... and this warp stays until every rank's flag of that step is here: the pair of launches is complete only
-                // when the gathered buffer of the step before is (the Planning half needs no tally for it)
-                dg_wait_flags(io.wait_flag, io.n_wait, io.wait_value);
-            }
+            // ... and that warp stays until every rank's flag of that step is here: the pair of launches is complete only when the
+            // gathered buffer of the step before is (the Planning half needs no tally for it)
+            if (lane == 0 && atomicAdd(io.tally2, 1u) == io.tally_n - 1u) dg_complete(io.tally2, io, true, false);
         }
         return;
-    }
-
-    if (PHASE == 0 && io.n_fwd) {                           // one launch for both halves: the forward goes here, the end-of-launch tally covers it
-#pragma unroll
-        for (int k = 0; k < DP_MAX_MIRRORS; ++k)
-            if (k < io.n_fwd) reinterpret_cast<uint32_t*>(io.fwd_dst[k] + scene)[lane] = fwd_w;
     }
     // ================================ Planning thread iteration ================================
     // last_Bpoints (Planning.cpp:6) -> sm.plan by one TMA bulk copy; the staging area of the decision half is free now and
     // the copy lands while the aim point is searched
     __syncwarp();
-    // chained submits: the previous cycle's Planning warp of this scene wrote last_path with generic stores and may belong to a launch
-    // that is still running: order those writes (seen through the pdone acquire) before the async-proxy read of the bulk copy
-    if (PHASE == 2 && io.pdone) asm volatile("fence.proxy.async.global;" ::: "memory");
     dp_bulk_prefetch(sm.plan, lastp, DP_PATH_POINTS * (uint32_t)sizeof(double2), &sm.mbar, lane);
     const int plan_his_behavior = dp_l2(&cg->plan_his_behavior), carried_near_id = dp_l2(&cg->path_near_id), plan_count = dp_l2(&cg->plan_count);
     double aim_x = dp_l2(&cg->aim_x), aim_y = dp_l2(&cg->aim_y), aim_dir = dp_l2(&cg->aim_dir);
@@ -1000,35 +972,20 @@ dp_cycle_kernel(DevMap m, dp_params p, int n_scenes, const dp_scene_hdr* __restr
         for (int k = 0; k < DP_MAX_MIRRORS; ++k)             // (static indices: the parameter array stays in the constant bank)
             if (k < io.n_mirror) reinterpret_cast<uint32_t*>(io.mirror[k] + scene)[lane] = w;
     }
-    if (PHASE != 1 && io.tally && !io.pdone) {
-        // completion of the whole launch without the chain: the last warp tells the host (page-locked flag) and / or the peers
+    // completion: the last warp of the launch tells the host (page-locked flag) and / or the peers.  Two copies of the same
+    // sequence, one per way of launching: a launch call (io.tally set by the caller or for a gather) and a submitted cycle
+    // (io.in_flag).  Written as one `if (io.tally)` block it costs the one-wave Planning half 24 B more stack and twice the
+    // spill traffic: ptxas allocates registers differently.
+    if (io.tally && !io.in_flag) {
         __threadfence();                                    // (every lane: its stores, the mirrors included, before the tally)
         __syncwarp();
-        if (lane == 0 && atomicAdd(io.tally, 1u) == io.tally_n - 1u) {
-            *io.tally = 0;
-            __threadfence_system();                         // cumulative: everything the other warps fenced before their tally increment
-#pragma unroll
-            for (int k = 0; k < DP_MAX_MIRRORS; ++k)
-                if (k < io.n_peer_flag && io.flag_mode == 0) asm volatile("st.relaxed.sys.global.u32 [%0], %1;" ::"l"(io.peer_flag[k]), "r"(io.flag_value) : "memory");
-            dg_wait_flags(io.wait_flag, io.n_wait, io.wait_value);
-            if (io.host_done) *reinterpret_cast<volatile unsigned*>(io.host_done) = io.epoch;
-        }
+        if (lane == 0 && atomicAdd(io.tally, 1u) == io.tally_n - 1u) dg_complete(io.tally, io, io.flag_mode == 0, true);
     }
-    if (PHASE == 2 && io.pdone) {
-        // chained submit: this scene's cycle is complete -- its next Decision warp may go; the last warp of the batch tells the host
-        __threadfence();                                    // (every lane: its stores, the mirrors included, before the flags)
+    if (io.in_flag) {
+        __threadfence();                                    // (every lane: its stores, the mirrors included, before the tally)
         __syncwarp();
         if (lane == 0) {
-            asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(io.pdone + scene), "r"(io.epoch) : "memory");
-            if (io.tally && atomicAdd(io.tally, 1u) == io.tally_n - 1u) {
-                *io.tally = 0;                              // re-armed here: a memset on the copy stream could run as a kernel and find no SM slot
-                __threadfence_system();                     // cumulative: everything the other warps fenced before their tally increment
-#pragma unroll
-                for (int k = 0; k < DP_MAX_MIRRORS; ++k)     // fused gather: this rank's slice of the step is complete on every rank
-                    if (k < io.n_peer_flag && io.flag_mode == 0) asm volatile("st.relaxed.sys.global.u32 [%0], %1;" ::"l"(io.peer_flag[k]), "r"(io.flag_value) : "memory");
-                dg_wait_flags(io.wait_flag, io.n_wait, io.wait_value);
-                if (io.host_done) *reinterpret_cast<volatile unsigned*>(io.host_done) = io.epoch;
-            }
+            if (io.tally && atomicAdd(io.tally, 1u) == io.tally_n - 1u) dg_complete(io.tally, io, io.flag_mode == 0, true);
         }
     }
 }
@@ -1116,7 +1073,7 @@ __global__ void __launch_bounds__(TPB, (G <= 8) ? 4 : 2)   // G 16: 2 CTAs x 256
 dp_group_kernel(DgMap m, dp_params p, int n_scenes, int g, const dp_scene_hdr* __restrict__ hdr, const double* __restrict__ obs_x,
                 const double* __restrict__ obs_y, int max_obs, dp_carry* __restrict__ carry, double2* __restrict__ last_path,
                 dp_plan_record* __restrict__ rec, dp_trace_record* __restrict__ trace, double* __restrict__ path_xy,
-                double* __restrict__ path_ll, DgIo io) {
+                double* __restrict__ path_ll, DpIo io) {
     extern __shared__ __align__(16) unsigned char dg_raw[];
     DgSmem<G>& sm = *reinterpret_cast<DgSmem<G>*>(dg_raw);
     const int first = blockIdx.x * g;
@@ -1137,7 +1094,6 @@ static void dp_l2_window(cudaLaunchAttribute& a, const DpLaunchCfg& lc) {
 }
 void dp_launch_prepare(DpLaunchCfg& lc) {
     if (lc.attr_warp) return;                               // 196 of 256 KB as shared memory, the rest stays L1 (per context: no process-wide state)
-    cudaFuncSetAttribute(dp_cycle_kernel<0, 4>, cudaFuncAttributePreferredSharedMemoryCarveout, DP_CARVEOUT);
     cudaFuncSetAttribute(dp_cycle_kernel<1, 4>, cudaFuncAttributePreferredSharedMemoryCarveout, DP_CARVEOUT);
     cudaFuncSetAttribute(dp_cycle_kernel<2, 4>, cudaFuncAttributePreferredSharedMemoryCarveout, DP_CARVEOUT);
     cudaFuncSetAttribute(dp_cycle_kernel<1, 1>, cudaFuncAttributePreferredSharedMemoryCarveout, DP_CARVEOUT);
@@ -1146,62 +1102,38 @@ void dp_launch_prepare(DpLaunchCfg& lc) {
 }
 cudaError_t dp_launch_cycle(const DevMap& m, const dp_params& p, int n, const dp_scene_hdr* hdr, const double* ox, const double* oy,
                             int max_obs, dp_carry* carry, double2* last_path, dp_plan_record* rec, dp_trace_record* trace,
-                            double* path_xy, double* path_ll, cudaStream_t st, int split, const DpIo& io, DpLaunchCfg& lc) {
+                            double* path_xy, double* path_ll, cudaStream_t st, const DpIo& io, DpLaunchCfg& lc) {
     if (n <= 0) return cudaSuccess;
     dp_launch_prepare(lc);
-    const int sm_count = lc.sm_count;
-    if (!split) {
-        DpIo io0 = io; io0.done = nullptr; io0.in_flag = nullptr; io0.pdone = nullptr; io0.prev_epoch = 0; io0.flag_mode = 0;
-        const int blocks = (n + 3) / 4;
-        dp_cycle_kernel<0, 4><<<blocks, 128, 0, st>>>(m, p, n, hdr, ox, oy, max_obs, carry, last_path, rec, trace, path_xy, path_ll, io0);
-    } else {
-        // batches of at most one wave of 4-warp CTAs stay one wave; larger ones run one warp per CTA (see DP_MIN_BLOCKS)
-        const int force_wpb = lc.force_wpb;                 // DP_WPB=1|4 overrides the choice (experiments)
-        const bool wide = force_wpb ? force_wpb == 4 : n <= sm_count * DP_MIN_BLOCKS(4) * 4;
-        const int wpb = wide ? 4 : 1;
-        const int blocks = (n + wpb - 1) / wpb, threads = wpb * 32;
-        // Decision launch ingests (hdr/ox/oy may be pinned host memory); Planning launch reads the staged device copies
-        DpIo io1 = io; io1.n_mirror = 0;
-        DpIo io2 = io; io2.hdr_stage = nullptr; io2.ox_stage = nullptr; io2.oy_stage = nullptr;
-        if (split != 2) { io1.done = io2.done = nullptr; io1.in_flag = io2.in_flag = nullptr; io1.pdone = io2.pdone = nullptr; io1.prev_epoch = 0; }
-        io1.flag_mode = io2.flag_mode = (io.n_fwd && io.tally2) ? 1 : 0;   // deferred gather: the Decision half forwards and raises the flags
-        {
-            // chained submit: the Decision half is a programmatic dependent of the previous cycle's Planning half (which triggers
-            // at entry); its warps wait per scene for that cycle's Planning warp (io.prev_epoch) and for the staged inputs
-            cudaLaunchConfig_t cfg1 = {};
-            cfg1.gridDim = dim3(blocks); cfg1.blockDim = dim3(threads); cfg1.dynamicSmemBytes = 0; cfg1.stream = st;
-            cudaLaunchAttribute at1[2];
-            int na1 = 0;
-            if (io1.prev_epoch) {
-                at1[na1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-                at1[na1].val.programmaticStreamSerializationAllowed = 1;
-                ++na1;
-            }
-            if (lc.l2_bytes) dp_l2_window(at1[na1++], lc);
-            cfg1.attrs = at1; cfg1.numAttrs = na1;
-            cudaError_t e1 = wide ? cudaLaunchKernelEx(&cfg1, dp_cycle_kernel<1, 4>, m, p, n, hdr, ox, oy, max_obs, carry, last_path, rec, trace, path_xy, path_ll, io1)
-                                  : cudaLaunchKernelEx(&cfg1, dp_cycle_kernel<1, 1>, m, p, n, hdr, ox, oy, max_obs, carry, last_path, rec, trace, path_xy, path_ll, io1);
-            if (e1 != cudaSuccess) return e1;
-        }
-        const dp_scene_hdr* hdr2 = io.hdr_stage ? io.hdr_stage : hdr;
-        const double* ox2 = io.ox_stage ? io.ox_stage : ox; const double* oy2 = io.oy_stage ? io.oy_stage : oy;
+    // batches of at most one wave of 4-warp CTAs stay one wave; larger ones run one warp per CTA (see DP_MIN_BLOCKS)
+    const bool wide = n <= lc.sm_count * DP_MIN_BLOCKS(4) * 4;
+    const int wpb = wide ? 4 : 1;
+    const int blocks = (n + wpb - 1) / wpb, threads = wpb * 32;
+    DpIo io1 = io; io1.n_mirror = 0;                        // the records are final in the Planning half
+    DpIo io2 = io;
+    io1.flag_mode = io2.flag_mode = (io.n_fwd && io.tally2) ? 1 : 0;   // deferred gather: the Decision half forwards and raises the flags
+    auto launch = [&](void (*kernel)(DevMap, dp_params, int, const dp_scene_hdr*, const double*, const double*, int, dp_carry*, double2*,
+                                     dp_plan_record*, dp_trace_record*, double*, double*, DpIo),
+                      const DpIo& hio, bool pdl) {
         cudaLaunchConfig_t cfg = {};
         cfg.gridDim = dim3(blocks); cfg.blockDim = dim3(threads); cfg.dynamicSmemBytes = 0; cfg.stream = st;
         cudaLaunchAttribute at[2];
         int na = 0;
-        // programmatic dependent launch WITHOUT a grid-wide dependency wait in the kernel: scenes hand over one by one
-        // (dp_publish / dp_await), so Planning CTAs run in the slots the Decision launch frees while its tail finishes
-        if (io2.done) {
+        if (pdl) {
             at[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
             at[na].val.programmaticStreamSerializationAllowed = 1;
             ++na;
         }
         if (lc.l2_bytes) dp_l2_window(at[na++], lc);
         cfg.attrs = at; cfg.numAttrs = na;
-        cudaError_t e = wide ? cudaLaunchKernelEx(&cfg, dp_cycle_kernel<2, 4>, m, p, n, hdr2, ox2, oy2, max_obs, carry, last_path, rec, trace, path_xy, path_ll, io2)
-                             : cudaLaunchKernelEx(&cfg, dp_cycle_kernel<2, 1>, m, p, n, hdr2, ox2, oy2, max_obs, carry, last_path, rec, trace, path_xy, path_ll, io2);
-        if (e != cudaSuccess) return e;
-    }
+        return cudaLaunchKernelEx(&cfg, kernel, m, p, n, hdr, ox, oy, max_obs, carry, last_path, rec, trace, path_xy, path_ll, hio);
+    };
+    cudaError_t e = launch(wide ? dp_cycle_kernel<1, 4> : dp_cycle_kernel<1, 1>, io1, false);
+    if (e != cudaSuccess) return e;
+    // the Planning half as a programmatic dependent launch WITHOUT a grid-wide dependency wait in the kernel: scenes hand over one
+    // by one (dp_publish / dp_await), so Planning CTAs run in the slots the Decision launch frees while its tail finishes
+    e = launch(wide ? dp_cycle_kernel<2, 4> : dp_cycle_kernel<2, 1>, io2, io.done != nullptr);
+    if (e != cudaSuccess) return e;
     return cudaGetLastError();
 }
 cudaError_t dp_launch_gather_wait(const unsigned* flags, int world, unsigned step, cudaStream_t st) {
@@ -1217,10 +1149,11 @@ __global__ void dp_gather_forward_kernel(const dp_plan_record* __restrict__ src,
     for (int k = 0; k < DP_MAX_MIRRORS; ++k)
         if (k < io.n_fwd) reinterpret_cast<uint4*>(io.fwd_dst[k])[i] = w;
 }
+// (the sequence of dg_complete without a tally or host flag, written out: the helper's unrolled flag loop takes 2 registers more here)
 __global__ void dp_gather_raise_kernel(DpIo io) {           // (after the forward kernel in stream order: its stores are complete)
     __threadfence_system();
     for (int k = 0; k < io.n_peer_flag; ++k) asm volatile("st.relaxed.sys.global.u32 [%0], %1;" ::"l"(io.peer_flag[k]), "r"(io.flag_value) : "memory");
-    dg_wait_flags(io.wait_flag, io.n_wait, io.wait_value);
+    dg_wait_flags(io.wait.flag, io.wait.n, io.wait.value);
 }
 cudaError_t dp_launch_gather_flush(const dp_plan_record* src, int n, const DpIo& io, cudaStream_t st) {
     dp_gather_forward_kernel<<<(n * 8 + 255) / 256, 256, 0, st>>>(src, n, io);
@@ -1252,7 +1185,7 @@ cudaError_t dp_launch_map_prep(const double* x, const double* y, const uint16_t*
 template <int G, int TPB>
 static cudaError_t dp_launch_group_t(const DgMap& m, const dp_params& p, int n, const dp_scene_hdr* hdr, const double* ox, const double* oy,
                                      int max_obs, dp_carry* carry, double2* last_path, dp_plan_record* rec, dp_trace_record* trace,
-                                     double* path_xy, double* path_ll, cudaStream_t st, const DgIo& io, int sm_count, int force_g, bool& configured) {
+                                     double* path_xy, double* path_ll, cudaStream_t st, const DpIo& io, int sm_count, bool& configured) {
     const size_t smem = sizeof(DgSmem<G>);
     if (!configured) {
         cudaError_t e = cudaFuncSetAttribute(dp_group_kernel<G, TPB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -1261,21 +1194,19 @@ static cudaError_t dp_launch_group_t(const DgMap& m, const dp_params& p, int n, 
         configured = true;
     }
     const int per_sm = (G <= 8) ? 4 : 2;
-    (void)0;
     int g = (n + sm_count * per_sm - 1) / (sm_count * per_sm);
     if (g < 1) g = 1;
     if (g > G) g = G;
-    if (force_g > 0 && force_g <= G) g = force_g;
     const int blocks = (n + g - 1) / g;
     dp_group_kernel<G, TPB><<<blocks, TPB, smem, st>>>(m, p, n, g, hdr, ox, oy, max_obs, carry, last_path, rec, trace, path_xy, path_ll, io);
     return cudaGetLastError();
 }
 cudaError_t dp_launch_group(const DgMap& m, const dp_params& p, int n, const dp_scene_hdr* hdr, const double* ox, const double* oy,
                             int max_obs, dp_carry* carry, double2* last_path, dp_plan_record* rec, dp_trace_record* trace,
-                            double* path_xy, double* path_ll, cudaStream_t st, const DgIo& io, DpLaunchCfg& lc) {
+                            double* path_xy, double* path_ll, cudaStream_t st, const DpIo& io, DpLaunchCfg& lc) {
     if (n <= 0) return cudaSuccess;
-    const int cfg = lc.group_cfg, force_g = lc.group_g, sm_count = lc.sm_count;
-    if (cfg == 1) return dp_launch_group_t<8, 128>(m, p, n, hdr, ox, oy, max_obs, carry, last_path, rec, trace, path_xy, path_ll, st, io, sm_count, force_g, lc.attr_group[1]);
-    if (cfg == 2) return dp_launch_group_t<8, 256>(m, p, n, hdr, ox, oy, max_obs, carry, last_path, rec, trace, path_xy, path_ll, st, io, sm_count, force_g, lc.attr_group[2]);
-    return dp_launch_group_t<16, 256>(m, p, n, hdr, ox, oy, max_obs, carry, last_path, rec, trace, path_xy, path_ll, st, io, sm_count, force_g, lc.attr_group[0]);
+    const int cfg = lc.group_cfg, sm_count = lc.sm_count;
+    if (cfg == 1) return dp_launch_group_t<8, 128>(m, p, n, hdr, ox, oy, max_obs, carry, last_path, rec, trace, path_xy, path_ll, st, io, sm_count, lc.attr_group[1]);
+    if (cfg == 2) return dp_launch_group_t<8, 256>(m, p, n, hdr, ox, oy, max_obs, carry, last_path, rec, trace, path_xy, path_ll, st, io, sm_count, lc.attr_group[2]);
+    return dp_launch_group_t<16, 256>(m, p, n, hdr, ox, oy, max_obs, carry, last_path, rec, trace, path_xy, path_ll, st, io, sm_count, lc.attr_group[0]);
 }

@@ -91,26 +91,34 @@ struct DgMap {
     int n_roads, n_lanes, n_conn;
 };
 
-// plumbing of one launch (see dp_kernels.h): record mirrors and the completion flag in page-locked host memory
-#define DG_MAX_MIRRORS 9
-struct DgIo {
-    dp_plan_record* mirror[DG_MAX_MIRRORS]; int n_mirror;
+// plumbing of one cycle launch, both kernels (dp_cycle.cu: the warp kernel's two halves and the group kernel)
+#define DP_MAX_MIRRORS 9
+struct DpWait { const unsigned* flag; int n; unsigned value; };
+struct DpIo {
+    // every finished 128-byte plan record is ALSO stored (one coalesced store each) at mirror[k][scene]: the caller's pinned result
+    // buffer (no D2H copy), and/or the gathered-records buffers of the peer GPUs mapped over NVLink (dp_set_record_mirrors, dp_gather_arm)
+    dp_plan_record* mirror[DP_MAX_MIRRORS]; int n_mirror;
+    // finished Planning warps / scenes of the launch; the last one stores epoch to *host_done (page-locked host memory)
     unsigned* tally; unsigned tally_n; unsigned* host_done; unsigned epoch;
     // fused record gather of a multi-GPU job (dp_gather_*): when the LAST record of the launch is out, flag_value is stored to
     // peer_flag[k] of every rank (one system fence, then relaxed system-scope stores): "rank's slice of this step is complete in your buffer"
-    unsigned* peer_flag[DG_MAX_MIRRORS]; int n_peer_flag; unsigned flag_value;
+    unsigned* peer_flag[DP_MAX_MIRRORS]; int n_peer_flag; unsigned flag_value;
     // ... and the barrier of the PREVIOUS step folded into this launch: after raising its own flags the last warp / CTA waits
-    // until wait_flag[0..n_wait) (this rank's flag words of that step, one per rank) all hold wait_value, and only then tells the
+    // until wait.flag[0..wait.n) (this rank's flag words of that step, one per rank) all hold wait.value, and only then tells the
     // host -- "this launch is complete" implies "every rank's records of the step before are in my gathered buffer"
-    const unsigned* wait_flag; int n_wait; unsigned wait_value;
+    DpWait wait;
     // deferred gather (dp_gather_arm_deferred): the records of the PREVIOUS launch (fwd_src, indexed like rec) are copied to
     // fwd_dst[0..n_fwd) by the warps / CTAs as they START -- the NVLink round trips hide under the cycle -- and the flags above
     // then stand for THAT step: nothing of the gather is left at the end of the launch but one fence, the flags and the wait
-    const dp_plan_record* fwd_src; dp_plan_record* fwd_dst[DG_MAX_MIRRORS]; int n_fwd;
-    unsigned* tally2; int flag_mode;                        // warp kernel, split launches: flags raised at the end of the Decision half (mode 1)
-    long long* timeline;                           // instrumented runs only (tools/group_timeline.py): [block][32] globaltimer stamps
-    // predicted agent tracks (BASELINE config 5, dp_set_tracks): constant-turn-rate parameters [scene][max_obs] -- displacement of
-    // step 0 (vx, vy) and heading change per step (deg) -- and the horizon T; null = static obstacles (the reference's semantics)
+    const dp_plan_record* fwd_src; dp_plan_record* fwd_dst[DP_MAX_MIRRORS]; int n_fwd;
+    unsigned* tally2; int flag_mode;                        // warp kernel: flags raised at the end of the Decision half (mode 1)
+    // warp kernel: per-scene hand-off flags of the overlapped halves (the Decision warp of a scene publishes epoch in done[scene]
+    // when its outputs are in memory, the Planning warp of that scene waits for it), and of a submitted cycle's inputs
+    // (*in_flag == epoch once they are in the staging set, dp_cycle_submit)
+    unsigned* done; const unsigned* in_flag;
+    long long* timeline;                           // group kernel, instrumented runs only (tools/group_timeline.py): [block][32] globaltimer stamps
+    // group kernel: predicted agent tracks (BASELINE config 5, dp_set_tracks): constant-turn-rate parameters [scene][max_obs] --
+    // displacement of step 0 (vx, vy) and heading change per step (deg) -- and the horizon T; null = static obstacles (the reference's semantics)
     const double* trk_vx; const double* trk_vy; const double* trk_dth; int trk_T;
 };
 
@@ -126,6 +134,19 @@ __device__ __forceinline__ void dg_wait_flags(const unsigned* flags, int n, unsi
         }
         if (v != value) __trap();                           // never spin forever on a rank that is not there
     }
+}
+// one thread, the last warp / CTA of a launch (or of the warp kernel's Decision half) once every other one has counted itself
+// in *tally: re-arm the tally (here: a memset on the copy stream could run as a kernel and find no SM slot), one system fence
+// (cumulative: everything the other warps fenced before their increment), this rank's gather flags on every rank (when `raise`),
+// the previous step's flags, then the host flag (when `host`)
+__device__ __forceinline__ void dg_complete(unsigned* tally, const DpIo& io, bool raise, bool host) {
+    *tally = 0;
+    __threadfence_system();
+#pragma unroll
+    for (int k = 0; k < DP_MAX_MIRRORS; ++k)
+        if (k < io.n_peer_flag && raise) asm volatile("st.relaxed.sys.global.u32 [%0], %1;" ::"l"(io.peer_flag[k]), "r"(io.flag_value) : "memory");
+    dg_wait_flags(io.wait.flag, io.wait.n, io.wait.value);
+    if (host && io.host_done) *reinterpret_cast<volatile unsigned*>(io.host_done) = io.epoch;
 }
 #endif
 
@@ -795,7 +816,7 @@ DG_FN DgRes dg_selected(const DgView& v, int P, unsigned key, const double* ox, 
 template <int G, int TPB>
 DG_BODY dg_group_cycle(const DgMap& m, const dp_params& p, const int first, const int S, const dp_scene_hdr* hdr, const double* obs_x,
                        const double* obs_y, const int max_obs, dp_carry* carry, double2* last_path, dp_plan_record* rec,
-                       dp_trace_record* trace, double* path_xy, double* path_ll, const DgIo& io, DgSmem<G>& sm) {
+                       dp_trace_record* trace, double* path_xy, double* path_ll, const DpIo& io, DgSmem<G>& sm) {
     const double Vw = p.vehicle_width;
     DG_MARK(0);
 
@@ -812,7 +833,7 @@ DG_BODY dg_group_cycle(const DgMap& m, const dp_params& p, const int first, cons
             for (int i = tid; i < S * 8; i += TPB) {
                 const uint4 w = __ldcg(fs + i);
 #pragma unroll
-                for (int q = 0; q < DG_MAX_MIRRORS; ++q)
+                for (int q = 0; q < DP_MAX_MIRRORS; ++q)
                     if (q < io.n_fwd) reinterpret_cast<uint4*>(io.fwd_dst[q] + first)[i] = w;
             }
         }
@@ -1895,7 +1916,7 @@ DG_BODY dg_group_cycle(const DgMap& m, const dp_params& p, const int first, cons
             const uint4 w = sr[i];
             gr[i] = w; gc[i] = sc[i];
 #pragma unroll
-            for (int q = 0; q < DG_MAX_MIRRORS; ++q)
+            for (int q = 0; q < DP_MAX_MIRRORS; ++q)
                 if (q < io.n_mirror) reinterpret_cast<uint4*>(io.mirror[q] + first)[i] = w;
         }
     }
@@ -1905,15 +1926,7 @@ DG_BODY dg_group_cycle(const DgMap& m, const dp_params& p, const int first, cons
         __syncthreads();
         if (threadIdx.x == 0) {
             __threadfence();                                // cumulative: the CTA's stores (ordered before the barrier) before the tally
-            if (atomicAdd(io.tally, (unsigned)S) + (unsigned)S == io.tally_n) {
-                *io.tally = 0;                              // re-armed for the next cycle that uses this word
-                __threadfence_system();
-#pragma unroll
-                for (int q = 0; q < DG_MAX_MIRRORS; ++q)
-                    if (q < io.n_peer_flag) asm volatile("st.relaxed.sys.global.u32 [%0], %1;" ::"l"(io.peer_flag[q]), "r"(io.flag_value) : "memory");
-                dg_wait_flags(io.wait_flag, io.n_wait, io.wait_value);
-                if (io.host_done) *reinterpret_cast<volatile unsigned*>(io.host_done) = io.epoch;
-            }
+            if (atomicAdd(io.tally, (unsigned)S) + (unsigned)S == io.tally_n) dg_complete(io.tally, io, true, true);
         }
     }
 #endif

@@ -2,42 +2,14 @@
 #pragma once
 #include <cuda_runtime.h>
 #include "dp_device.cuh"
-#include "dp_group.cuh"
-
-// optional plumbing of the cycle launches:
-//   *_stage   zero-copy ingest (DP_ZERO_COPY=1): the Decision launch reads hdr/obstacles from pinned host memory and leaves
-//             device copies here for the Planning launch;
-//   mirror    every finished 128-byte plan record is ALSO stored (one coalesced warp store each) at mirror[k][scene]:
-//             the caller's pinned result buffer (no D2H copy), and/or the gathered-records buffers of the peer GPUs
-//             mapped over NVLink -- the per-step record gather fused into the Planning launch (dp_set_record_mirrors);
-//   done / epoch  per-scene hand-off flags of the overlapped split launch (dp_cycle.cu): the Decision warp of a scene
-//             publishes `epoch` in done[scene] when its outputs are in memory, the Planning warp of that scene waits for it
-#define DP_MAX_MIRRORS 9
-struct DpIo {
-    dp_scene_hdr* hdr_stage; double* ox_stage; double* oy_stage;
-    dp_plan_record* mirror[DP_MAX_MIRRORS]; int n_mirror;
-    unsigned* done; unsigned epoch;
-    // chained submits (dp_cycle_submit): consecutive cycles of the same scenes overlap as well, see dp_cycle.cu
-    const unsigned* in_flag;                   // *in_flag == epoch once this cycle's inputs are in the staging set
-    unsigned* pdone; unsigned prev_epoch;      // pdone[scene] = epoch of the last cycle whose Planning warp finished; the Decision warp
-                                               // of a scene waits for prev_epoch before it touches the carry (0: nothing to wait for)
-    unsigned* tally; unsigned tally_n;         // finished Planning warps of this cycle; the last one stores epoch to *host_done
-    unsigned* host_done;                       // (page-locked host memory)
-    unsigned* peer_flag[DP_MAX_MIRRORS]; int n_peer_flag; unsigned flag_value;   // fused gather (dp_gather_*), see DgIo
-    const unsigned* wait_flag; int n_wait; unsigned wait_value;                  // the previous step's barrier, folded in (DgIo)
-    const dp_plan_record* fwd_src; dp_plan_record* fwd_dst[DP_MAX_MIRRORS]; int n_fwd;   // deferred gather (DgIo)
-    unsigned* tally2; int flag_mode;
-};
-inline DpIo dp_io_none() { DpIo io = {}; return io; }
+#include "dp_group.cuh"                        // (DpIo: the plumbing of one cycle launch)
 
 // launch-time state of ONE context (no process-wide statics: two threads may own two contexts): device properties, which
-// kernels already carry their shared-memory attributes, and the experiment switches read from the environment by dp_create
+// kernels already carry their shared-memory attributes, and the experiment switch read from the environment by dp_create
 struct DpLaunchCfg {
     int sm_count = 0;
     bool attr_warp = false, attr_group[3] = {false, false, false};
-    int force_wpb = 0;                         // DP_WPB = 1 | 4: CTA size of the warp kernel (0: by batch size)
     int group_cfg = 0;                         // DP_GROUP_CFG = 0 | 1 | 2: CTA shape of the group kernel (16 x 256, 8 x 128, 8 x 256)
-    int group_g = 0;                           // DP_GROUP_G: scenes per CTA (0: spread one wave evenly)
     // L2 persistence for the map arena (dp_map_upload): the warp-kernel launches carry an access-policy window over it, so the
     // ~3 MB of map tables every scene gathers from stay resident in the L2 set-aside whatever streams through in between
     void* l2_base = nullptr; size_t l2_bytes = 0;
@@ -45,8 +17,7 @@ struct DpLaunchCfg {
 
 cudaError_t dp_launch_cycle(const DevMap& m, const dp_params& p, int n, const dp_scene_hdr* hdr, const double* ox, const double* oy,
                             int max_obs, dp_carry* carry, double2* last_path, dp_plan_record* rec, dp_trace_record* trace,
-                            double* path_xy, double* path_ll, cudaStream_t st, int split, const DpIo& io, DpLaunchCfg& lc);   // split: 0 fused, 1 two launches, 2 overlapped
-// (io.prev_epoch != 0 additionally launches the Decision half as a programmatic dependent of the previous cycle's Planning half)
+                            double* path_xy, double* path_ll, cudaStream_t st, const DpIo& io, DpLaunchCfg& lc);   // Decision + Planning half, overlapped
 // set the shared-memory attributes of the warp kernels (done lazily by dp_launch_cycle; called up front before a stream capture)
 void dp_launch_prepare(DpLaunchCfg& lc);
 // the closed-loop world step (dp_world_step.cuh): the buffers of one launch, and the option set a context arms.  A model is armed
@@ -81,7 +52,7 @@ cudaError_t dp_launch_map_prep(const double* x, const double* y, const uint16_t*
 // the group kernel (dp_group.cuh): ONE launch per cycle, a CTA walks a group of scenes through the cycle phase by phase
 cudaError_t dp_launch_group(const DgMap& m, const dp_params& p, int n, const dp_scene_hdr* hdr, const double* ox, const double* oy,
                             int max_obs, dp_carry* carry, double2* last_path, dp_plan_record* rec, dp_trace_record* trace,
-                            double* path_xy, double* path_ll, cudaStream_t st, const DgIo& io, DpLaunchCfg& lc);
+                            double* path_xy, double* path_ll, cudaStream_t st, const DpIo& io, DpLaunchCfg& lc);
 
 // operator-level kernels (dp_ops.cu)
 // operator kernels take polylines as AoS double2 (the host entry points interleave x/y)

@@ -207,14 +207,9 @@ int dp_cycle_batch(dp_ctx* ctx, int first_scene, int n_scenes, const dp_scene_hd
  * cycle on a copy stream and its kernels on the compute stream and returns at once; dp_cycle_wait blocks until the
  * OLDEST submitted cycle has written its records into `rec`.  At most two cycles may be in flight; all four buffers
  * must be page-locked (dp_host_alloc) and must not be touched between submit and the matching wait; n_scenes is
- * limited to 32768 per call.  Cycles execute in submission order (each reads the carry the previous one wrote).  By default
- * (DP_CHAIN=1) the inputs are announced to the Decision warps by a flag that a four-byte copy raises behind the input DMAs, and
- * completion reaches the host as a flag in page-locked memory instead of a stream event (DP_CHAIN=0 restores the event-based
- * path).  DP_CHAIN=2 additionally chains the launches: when two consecutive submits cover the same scene slots, the second
- * cycle's Decision launch becomes a programmatic dependent of the first one's Planning launch and waits scene by scene (it
- * starts while the other is still draining): measured 77.5 vs 78.5 us per step, not the default (tests/test_gpu_parity.py
- * runs the pipelined test under both).  DP_REC_DMA=1 returns the records by a device->host copy behind the kernels instead of
- * stores from the Planning warps (measured slower with two cycles in flight; under test as well).
+ * limited to 32768 per call.  Cycles execute in submission order (each reads the carry the previous one wrote).  The inputs
+ * are announced to the Decision warps by a flag that a four-byte copy raises behind the input DMAs, the Planning warps store
+ * the records into `rec` themselves, and completion reaches the host as a flag in page-locked memory instead of a stream event.
  * dp_cycle_batch / dp_reset / dp_carry_* return DP_ERR_STATE while cycles are in flight. */
 int dp_cycle_submit(dp_ctx* ctx, int first_scene, int n_scenes, const dp_scene_hdr* hdr,
                     const double* obs_x, const double* obs_y, dp_plan_record* rec);

@@ -357,13 +357,11 @@ def test_library_is_the_cuda_path(planner):
     assert fp64 > 5 and fp32 > 20, (fp64, fp32)
 
 
-def test_pinned_host_paths(planner, oracle, the_map, monkeypatch):
-    """dp_cycle_batch with PINNED host buffers: the default route (three input DMAs, records stored straight into the
-    caller's buffer) and the DP_ZERO_COPY=1 route (kernels read the inputs from host memory over PCIe) must both give
+def test_pinned_host_paths(planner, oracle, the_map):
+    """dp_cycle_batch with PINNED host buffers (three input DMAs, records stored straight into the caller's buffer) must give
     byte-identical records to the staged-copy route used with pageable buffers."""
     import torch
     from dmpp_b200 import abi, scenes
-    from dmpp_b200.planner import Planner
     n, cycles = 512, 12
     ep = scenes.Episodes(the_map, np.arange(4242, 4242 + n), cycles=cycles, n_obs=10)
     H, OX, OY = ep.all_cycles()
@@ -383,13 +381,6 @@ def test_pinned_host_paths(planner, oracle, the_map, monkeypatch):
         assert o["rec"].tobytes() == got[c].tobytes(), "cycle %d" % c
     want = oracle.run(H, OX, OY, paths=False, calls=False, trace=False, exhaustive=False)
     assert_records_equal(np.stack(got), want["rec"], REC_EXACT, close=DIR_ERR_TOL, what="pinned")
-    monkeypatch.setenv("DP_ZERO_COPY", "1")                     # read by dp_create
-    zc = Planner(max_scenes=n, max_obs=planner.max_obs)
-    zc.upload_map(the_map)
-    for c in range(cycles):
-        zc.cycle(Hp[c], PXp[c], PYp[c], out={"rec": rec_p})
-        assert rec_p.tobytes() == got[c].tobytes(), "zero-copy cycle %d" % c
-    zc.close()
 
 
 def test_pipelined_submit_wait(planner, oracle, the_map):
@@ -432,19 +423,13 @@ def test_pipelined_submit_wait(planner, oracle, the_map):
         assert o["rec"].tobytes() == got[c].tobytes(), "cycle %d" % c
 
 
-@pytest.mark.parametrize("chain", ["0", "2", "dma"])
-def test_pipelined_submit_wait_chain_levels(oracle, the_map, monkeypatch, chain):
-    """the pipelined pair under the other DP_CHAIN levels (read by dp_create): 0 = stream events, 2 = the next cycle's Decision
-    launch as a programmatic dependent of the previous Planning launch with per-scene flags.  Same records as the oracle; level 2
-    also with 4096 scenes (one full wave: early Decision CTAs and the Planning launch compete for the slots)."""
+def test_pipelined_submit_wait_one_wave(oracle, the_map):
+    """the pipelined pair on a context of its own, 512 scenes and 4096 scenes (one full wave: the Decision CTAs waiting for the
+    input flag and the Planning launch compete for the slots).  Same records as the oracle."""
     import torch
     from dmpp_b200 import abi, scenes
     from dmpp_b200.planner import Planner
-    if chain == "dma":                                       # default flags, records returned by a device->host copy behind the kernels
-        monkeypatch.setenv("DP_REC_DMA", "1")
-    else:
-        monkeypatch.setenv("DP_CHAIN", chain)
-    for n, cycles in ((512, 10), (4096, 6)) if chain != "0" else ((512, 10),):
+    for n, cycles in ((512, 10), (4096, 6)):
         p = Planner(n, 10)
         p.upload_map(the_map)
         ep = scenes.Episodes(the_map, np.arange(31000, 31000 + n), cycles=cycles, n_obs=10)
@@ -463,7 +448,7 @@ def test_pipelined_submit_wait_chain_levels(oracle, the_map, monkeypatch, chain)
         while pend:
             p.wait(); got.append(recs[pend.pop(0) & 1].copy())
         want = oracle.run(H, OX, OY, paths=False, calls=False, trace=False, exhaustive=False)
-        assert_records_equal(np.stack(got), want["rec"], REC_EXACT, close=DIR_ERR_TOL, what="pipelined, DP_CHAIN=%s, %d scenes" % (chain, n))
+        assert_records_equal(np.stack(got), want["rec"], REC_EXACT, close=DIR_ERR_TOL, what="pipelined, %d scenes" % n)
         p.close()
 
 
@@ -536,11 +521,10 @@ def test_multi_wave_batch_one_warp_ctas(oracle, the_map):
         p.close()
 
 
-@pytest.mark.parametrize("split", ["0", "1", "warp", "group", "group1", "group2"])
+@pytest.mark.parametrize("split", ["warp", "group", "group1", "group2"])
 def test_launch_modes_agree(planner, the_map, monkeypatch, split):
     """Every way the cycle can be launched must produce the same bytes (records, traces, paths, carried state) as the
-    module's default planner: the warp-per-scene kernel as one fused launch (DP_SPLIT=0), as two launches back to back
-    (DP_SPLIT=1) or overlapped (default), and the group kernel in its three CTA shapes (DP_GROUP_CFG 0/1/2)."""
+    module's default planner: the warp-per-scene kernel, and the group kernel in its three CTA shapes (DP_GROUP_CFG 0/1/2)."""
     from dmpp_b200 import scenes
     from dmpp_b200.planner import Planner
     n, cycles = 384, 10
@@ -549,8 +533,7 @@ def test_launch_modes_agree(planner, the_map, monkeypatch, split):
         H, OX, OY = ep.all_cycles()
         PX, PY = pad_obs(OX, OY, planner.max_obs)
         want = planner.run_episodes(H, PX, PY)
-        env = {"0": {"DP_KERNEL": "warp", "DP_SPLIT": "0"}, "1": {"DP_KERNEL": "warp", "DP_SPLIT": "1"}, "warp": {"DP_KERNEL": "warp"},
-               "group": {"DP_KERNEL": "group"}, "group1": {"DP_KERNEL": "group", "DP_GROUP_CFG": "1"},
+        env = {"warp": {"DP_KERNEL": "warp"}, "group": {"DP_KERNEL": "group"}, "group1": {"DP_KERNEL": "group", "DP_GROUP_CFG": "1"},
                "group2": {"DP_KERNEL": "group", "DP_GROUP_CFG": "2"}}[split]
         for k, v in env.items():
             monkeypatch.setenv(k, v)                           # read by dp_create (DP_GROUP_CFG: at the first group launch of the process)

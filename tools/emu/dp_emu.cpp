@@ -104,7 +104,7 @@ int emu_run_batch_tracks(const dp_params* p, int n, int cycles, int max_obs, con
         carry[s].behavior = 1; carry[s].velocity_expect = 10; carry[s].his_behavior = 1; carry[s].plan_his_behavior = 1;
     }
     DgSmem<G>* sm = new DgSmem<G>();
-    DgIo io; std::memset(&io, 0, sizeof(io));
+    DpIo io; std::memset(&io, 0, sizeof(io));
     for (int c = 0; c < cycles; ++c) {
         const size_t e = (size_t)c * n;
         if (vx) { io.trk_vx = vx + e * max_obs; io.trk_vy = vy + e * max_obs; io.trk_dth = dth + e * max_obs; io.trk_T = T; }
