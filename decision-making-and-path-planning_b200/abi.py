@@ -165,6 +165,32 @@ lane_change_state = np.dtype([("lat_goal", "<f8"), ("hold", "<f8"), ("changes_le
 assert lane_change_state.itemsize == 24
 
 
+v2x_event_spec = np.dtype(
+    [
+        ("sig_cycle", "<f8"), ("sig_green", "<f8"), ("sig_yellow", "<f8"), ("sig_red", "<f8"), ("sig_offset", "<f8"), ("sig_range", "<f8"),
+        ("ped_x", "<f8"), ("ped_y", "<f8"), ("ped_vx", "<f8"), ("ped_vy", "<f8"), ("ped_t_on", "<f8"), ("ped_t_off", "<f8"),
+        ("ped_range", "<f8"), ("rw_x", "<f8"), ("rw_y", "<f8"), ("rw_range", "<f8"),
+        ("sig_road", "<i4"), ("sig_stop", "<i4"), ("has_ped", "<i4"), ("ped_direction", "<i4"), ("has_works", "<i4"), ("rw_rsi", "<i4"),
+        ("wp_first", "<i4"), ("wp_count", "<i4"),
+    ]
+)
+assert v2x_event_spec.itemsize == 160
+
+v2x_episode_stats = np.dtype(
+    [
+        ("min_ped_distance", "<f8"), ("last_d", "<f8"), ("cycles", "<i4"), ("light_cycles", "<i4", (3,)),
+        ("construction_cycles", "<i4", (2,)), ("pedestrian_cycles", "<i4", (2,)), ("stop_cmds", "<i4"), ("creep_cmds", "<i4"),
+        ("ub_cycles", "<i4"), ("red_crossings", "<i4"), ("first_red_crossing", "<i4"), ("last_phase", "<i4"), ("last_on", "<i4"),
+        ("pad", "<i4"),
+    ]
+)
+assert v2x_episode_stats.itemsize == 80
+
+
+class V2xWorldParams(C.Structure):
+    _fields_ = [("mode", C.c_int32), ("apply", C.c_int32)]
+
+
 class MapDesc(C.Structure):
     _fields_ = [
         ("n_roads", C.c_int32), ("road_lane_base", C.c_void_p),

@@ -65,6 +65,7 @@ struct dp_ctx {
     // closed-loop episodes (dp_run_closed_loop_dev): world-step parameters, the capture stream, the cached episode graph and its key
     DpWorldOpts world;                                      // dp_world_set_params and the armed models (dp_world_set_metrics,
                                                             // dp_world_set_agent_model, dp_world_set_lane_change)
+    DpV2xOpts v2x;                                          // dp_world_set_v2x: the V2X launch between cycle and world step
     cudaStream_t ep_stream = nullptr;
     cudaGraphExec_t ep_exec = nullptr;
     const void* ep_key[8] = {}; int ep_dims[3] = {-1, -1, -1};
@@ -1371,6 +1372,47 @@ int dp_world_set_lane_change(dp_ctx* c, const dp_lane_change_params* p, dp_lane_
     c->world.lcs = st;
     return drop_episode_graph(c);
 }
+int dp_world_set_v2x(dp_ctx* c, const dp_v2x_world_params* vp, int n, const dp_v2x_event_spec* spec, const double* wp_x, const double* wp_y,
+                     int n_wp, dp_v2x_flags* flags, dp_v2x_episode_stats* stats) {
+    if (!c) return fail(DP_ERR_ARG, "dp_world_set_v2x: bad argument");
+    if (!spec) {
+        c->v2x = DpV2xOpts{};
+        return drop_episode_graph(c);
+    }
+    if (!vp || !stats || n < 0 || n_wp < 0 || (n_wp > 0 && (!wp_x || !wp_y)) || (vp->mode != 0 && vp->mode != 1) ||
+        (vp->apply != 0 && vp->apply != 1))
+        return fail(DP_ERR_ARG, "dp_world_set_v2x: bad argument");
+    if (!c->have_map) return fail(DP_ERR_STATE, "dp_world_set_v2x: map not uploaded");
+    CK(cudaSetDevice(c->device));
+    std::vector<dp_v2x_event_spec> h((size_t)n);
+    if (n > 0) CK(cudaMemcpy(h.data(), spec, (size_t)n * sizeof(dp_v2x_event_spec), cudaMemcpyDeviceToHost));
+    for (const dp_v2x_event_spec& e : h) {
+        if (!all_finite({e.sig_cycle, e.sig_green, e.sig_yellow, e.sig_red, e.sig_offset, e.sig_range, e.ped_x, e.ped_y, e.ped_vx, e.ped_vy,
+                         e.ped_t_on, e.ped_t_off, e.ped_range, e.rw_x, e.rw_y, e.rw_range}))
+            return fail(DP_ERR_ARG, "dp_world_set_v2x: specifications must be finite");
+        if (!(e.sig_range >= 0) || !(e.ped_range >= 0) || !(e.rw_range >= 0))
+            return fail(DP_ERR_ARG, "dp_world_set_v2x: ranges must be >= 0");
+        if (e.sig_road < 0 || e.sig_road > c->gmap.n_roads || e.sig_stop < -1)
+            return fail(DP_ERR_ARG, "dp_world_set_v2x: sig_road outside [0, n_roads] or sig_stop < -1");
+        if (e.sig_road > 0 && (!(e.sig_green > 0) || !(e.sig_yellow > 0) || !(e.sig_red > 0) || !(e.sig_cycle > 0) ||
+                               !(std::fabs(e.sig_green + e.sig_yellow + e.sig_red - e.sig_cycle) <= 1e-9 * e.sig_cycle)))
+            return fail(DP_ERR_ARG, "dp_world_set_v2x: signal durations must be > 0 and sum to the cycle");
+        if (e.has_works && (e.wp_count < 0 || (e.wp_count > 0 && (e.wp_first < 0 || e.wp_first > n_wp - e.wp_count))))
+            return fail(DP_ERR_ARG, "dp_world_set_v2x: warning-point slice out of range");
+    }
+    c->v2x.vp = *vp; c->v2x.spec = spec; c->v2x.wp_x = wp_x; c->v2x.wp_y = wp_y; c->v2x.flags = flags; c->v2x.stats = stats; c->v2x.n = n;
+    return drop_episode_graph(c);
+}
+int dp_v2x_world_dev(dp_ctx* c, int first, int n, const dp_scene_hdr* hdr, dp_plan_record* rec, int cycle, void* stream) {
+    if (!c || !hdr || n < 0 || first < 0 || first + n > c->max_scenes || cycle < 0) return fail(DP_ERR_ARG, "dp_v2x_world_dev: bad argument");
+    if (!c->have_map) return fail(DP_ERR_STATE, "dp_v2x_world_dev: map not uploaded");
+    if (!c->v2x.spec) return fail(DP_ERR_STATE, "dp_v2x_world_dev: V2X is not armed (dp_world_set_v2x)");
+    if (n > c->v2x.n) return fail(DP_ERR_ARG, "dp_v2x_world_dev: more scenes than the armed specifications");
+    CK(cudaSetDevice(c->device));
+    c->launches += n > 0 ? 1 : 0;
+    CK(dp_launch_world_v2x(c->gmap, c->p, c->v2x, n, hdr, rec, cycle, (cudaStream_t)stream));
+    return DP_OK;
+}
 int dp_world_step_dev(dp_ctx* c, int first, int n, dp_scene_hdr* hdr, dp_agent* agents, double* ox, double* oy, const dp_plan_record* rec,
                       void* stream) {
     if (!c || !hdr || !agents || !ox || !oy || n < 0 || first < 0 || first + n > c->max_scenes)
@@ -1399,9 +1441,17 @@ cudaError_t enqueue_closed_loop(dp_ctx* c, int first, int n, int cycles, dp_scen
         if (oly && (e = cudaMemcpyAsync(oly + (size_t)k * n * mo, oy, (size_t)n * mo * sizeof(double), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
         const DpIo io = make_io(c, first, nullptr);
         if ((e = run_cycle(c, first, n, hdr, ox, oy, rec + (size_t)k * n, nullptr, nullptr, nullptr, st, io)) != cudaSuccess) return e;
+        if (c->v2x.spec) {                                  // V2X armed: the flags act on the records before the world step reads them
+            c->launches += 1;
+            if ((e = dp_launch_world_v2x(c->gmap, c->p, c->v2x, n, hdr, rec + (size_t)k * n, k, st)) != cudaSuccess) return e;
+        }
         c->launches += 1;
         b.rec = rec + (size_t)k * n;
         if ((e = dp_launch_world(c->gmap, c->p, c->world, b, st)) != cudaSuccess) return e;
+    }
+    if (c->v2x.spec) {                                      // the tally: closes the red-crossing check of the last world step
+        c->launches += 1;
+        if ((e = dp_launch_world_v2x(c->gmap, c->p, c->v2x, n, hdr, nullptr, cycles, st)) != cudaSuccess) return e;
     }
     return cudaSuccess;
 }
@@ -1412,6 +1462,7 @@ int dp_run_closed_loop_dev(dp_ctx* c, int first, int n, int cycles, dp_scene_hdr
         return fail(DP_ERR_ARG, "dp_run_closed_loop_dev: bad argument");
     if (!c->have_map) return fail(DP_ERR_STATE, "dp_run_closed_loop_dev: map not uploaded");
     if (c->submitted != c->waited) return fail(DP_ERR_STATE, "dp_run_closed_loop_dev: submitted cycles in flight, call dp_cycle_wait first");
+    if (c->v2x.spec && n > c->v2x.n) return fail(DP_ERR_ARG, "dp_run_closed_loop_dev: more scenes than the armed V2X specifications");
     CK(cudaSetDevice(c->device));
     c->ep_last_graph = 0;
     if (n == 0) return DP_OK;

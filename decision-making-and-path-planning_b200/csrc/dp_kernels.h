@@ -38,6 +38,17 @@ struct DpWorldOpts {
 cudaError_t dp_launch_world(const DevMap& m, const dp_params& p, const DpWorldOpts& o, const DpWorldBufs& b, cudaStream_t st);
 // allow the reactive instances the dynamic shared memory of DP_AGENT_MODEL_MAX_OBS agent slots (current device; set before a capture)
 cudaError_t dp_world_prepare();
+// the V2X events of a closed-loop episode (include/dmpp_b200.h section 14), armed by spec != nullptr; n: the worlds the specs cover
+struct DpV2xOpts {
+    dp_v2x_world_params vp = {0, 0};
+    const dp_v2x_event_spec* spec = nullptr;
+    const double* wp_x = nullptr; const double* wp_y = nullptr;
+    dp_v2x_flags* flags = nullptr; dp_v2x_episode_stats* stats = nullptr;
+    int n = 0;
+};
+// one V2X launch of cycle `cycle` (dp_world_v2x.cu); rec == nullptr: the tally after the last world step
+cudaError_t dp_launch_world_v2x(const DevMap& m, const dp_params& p, const DpV2xOpts& o, int n, const dp_scene_hdr* hdr, dp_plan_record* rec,
+                                int cycle, cudaStream_t st);
 cudaError_t dp_launch_v2x(const DevMap& m, const dp_params& p, int n, const dp_scene_hdr* hdr, const dp_v2x_data* v2x, const double* wp_lat,
                           const double* wp_lng, int mode, dp_v2x_flags* out, cudaStream_t st);
 cudaError_t dp_launch_v2x_apply(int n, const dp_v2x_flags* flags, dp_plan_record* rec, cudaStream_t st);

@@ -27,7 +27,7 @@ SYMBOLS = [
     "dp_pack_frames_dev", "dp_pack_frames", "dp_world_default_params", "dp_world_set_params", "dp_world_step_dev",
     "dp_run_closed_loop_dev", "dp_closed_loop_is_graph", "dp_v2x_event_batch", "dp_v2x_event_batch_dev", "dp_v2x_apply", "dp_v2x_apply_dev",
     "dp_metrics_default_params", "dp_world_set_metrics", "dp_agent_model_default_params", "dp_world_set_agent_model",
-    "dp_lane_change_default_params", "dp_world_set_lane_change",
+    "dp_lane_change_default_params", "dp_world_set_lane_change", "dp_world_set_v2x", "dp_v2x_world_dev",
     "dp_gather_create", "dp_gather_attach", "dp_gather_arm", "dp_gather_chain", "dp_gather_arm_deferred", "dp_gather_set_lag", "dp_gather_flush", "dp_gather_disarm", "dp_gather_wait", "dp_gather_buffer", "dp_gather_destroy",
 ]
 
@@ -258,6 +258,19 @@ class Planner:
         _ck(self.lib.dp_world_set_lane_change(self.ctx, C.byref(params) if params is not None else None, C.c_void_p(d_state or 0)),
             "dp_world_set_lane_change")
 
+    def set_v2x_world(self, params, n, d_spec, d_wp_x=None, d_wp_y=None, n_wp=0, d_flags=None, d_stats=None):
+        """arm the V2X events of closed-loop episodes (include/dmpp_b200.h section 14): params = V2xWorldParams (mode, apply);
+        device addresses of spec[n] (dp_v2x_event_spec, indexed like hdr), the warning points wp_x / wp_y[n_wp], flags[n]
+        (nullable) and stats[n]; d_spec None / 0 disarms"""
+        _ck(self.lib.dp_world_set_v2x(self.ctx, C.byref(params) if params is not None else None, C.c_int(n), C.c_void_p(d_spec or 0),
+                                      C.c_void_p(d_wp_x or 0), C.c_void_p(d_wp_y or 0), C.c_int(n_wp), C.c_void_p(d_flags or 0),
+                                      C.c_void_p(d_stats or 0)), "dp_world_set_v2x")
+
+    def v2x_world_dev(self, n, d_hdr, d_rec, cycle, first=0, stream=0):
+        """one V2X launch of cycle `cycle` between cycle_dev and world_step_dev; d_rec None: the tally after the last step"""
+        _ck(self.lib.dp_v2x_world_dev(self.ctx, C.c_int(first), C.c_int(n), C.c_void_p(d_hdr), C.c_void_p(d_rec or 0), C.c_int(cycle),
+                                      C.c_void_p(stream)), "dp_v2x_world_dev")
+
     def world_step_dev(self, n, d_hdr, d_agents, d_ox, d_oy, d_rec=None, first=0, stream=0):
         _ck(self.lib.dp_world_step_dev(self.ctx, C.c_int(first), C.c_int(n), C.c_void_p(d_hdr), C.c_void_p(d_agents), C.c_void_p(d_ox),
                                        C.c_void_p(d_oy), C.c_void_p(d_rec or 0), C.c_void_p(stream)), "dp_world_step_dev")
@@ -272,13 +285,15 @@ class Planner:
     def closed_loop_is_graph(self):
         return bool(self.lib.dp_closed_loop_is_graph(self.ctx))
 
-    def run_closed_loop(self, hdr, agents, cycles, log=True, repeat=1, metrics=None, agent_model=None, lane_change=None):
+    def run_closed_loop(self, hdr, agents, cycles, log=True, repeat=1, metrics=None, agent_model=None, lane_change=None, v2x=None):
         """host arrays in, host arrays out (the same dictionary as oracle.binding's run_closed_loop); `repeat` > 1 replays the
         episode from the same initial world (same device buffers, i.e. the cached graph) and returns the last run.
         metrics: None, or MetricsParams: the episode metrics are armed for this call (and disarmed after it) and the rows are
         returned under the key "metrics".  agent_model: None, or (AgentModelParams, v0[n][max_obs] desired speeds in m/s): the
         reactive agents are armed for this call (and disarmed after it).  lane_change: None, or LaneChangeParams (needs
-        agent_model): the agents also change lanes for this call, and their final states are returned under "lane_change_state"."""
+        agent_model): the agents also change lanes for this call, and their final states are returned under "lane_change_state".
+        v2x: None, or (V2xWorldParams, events) with events.spec[n] / wp_x / wp_y (scenes.V2xEvents): the V2X events are armed for
+        this call, the rows are returned under "v2x_stats" and the flags of the last launch under "v2x_flags"."""
         n, mo = agents.shape
         assert lane_change is None or agent_model is not None, "lane changes run on the reactive agents"
         assert mo == self.max_obs and hdr.shape == (n,)
@@ -293,6 +308,12 @@ class Planner:
             sizes["v0"] = n * mo * 8
         if lane_change is not None:
             sizes["lane_change_state"] = n * mo * abi.lane_change_state.itemsize
+        if v2x is not None:
+            vp, ev = v2x
+            spec, wx, wy = np.ascontiguousarray(ev.spec), np.ascontiguousarray(ev.wp_x, np.float64), np.ascontiguousarray(ev.wp_y, np.float64)
+            assert spec.dtype == abi.v2x_event_spec and spec.shape == (n,) and wx.shape == wy.shape
+            sizes.update(v2x_spec=n * spec.itemsize, v2x_wp_x=max(wx.nbytes, 8), v2x_wp_y=max(wy.nbytes, 8),
+                         v2x_flags=n * abi.v2x_flags.itemsize, v2x_stats=n * abi.v2x_episode_stats.itemsize)
         d = {}
         try:
             for k, b in sizes.items():
@@ -307,6 +328,11 @@ class Planner:
                 self.set_agent_model(am, d["v0"])
             if lane_change is not None:
                 self.set_lane_change(lane_change, d["lane_change_state"])
+            if v2x is not None:
+                for k, a in (("v2x_spec", spec), ("v2x_wp_x", wx), ("v2x_wp_y", wy)):
+                    _ck(self.lib.dp_memcpy_h2d(self.ctx, C.c_void_p(d[k]), abi.ptr(a), C.c_size_t(a.nbytes), None), "h2d")
+                _ck(self.lib.dp_stream_sync(self.ctx, None), "sync")
+                self.set_v2x_world(vp, n, d["v2x_spec"], d["v2x_wp_x"], d["v2x_wp_y"], wx.size, d["v2x_flags"], d["v2x_stats"])
             h0, a0 = np.ascontiguousarray(hdr), np.ascontiguousarray(agents)
             for _ in range(repeat):
                 self.reset(0, n)
@@ -324,6 +350,8 @@ class Planner:
                 o["metrics"] = np.zeros(n, abi.episode_metrics)
             if lane_change is not None:
                 o["lane_change_state"] = np.zeros((n, mo), abi.lane_change_state)
+            if v2x is not None:
+                o["v2x_flags"], o["v2x_stats"] = np.zeros(n, abi.v2x_flags), np.zeros(n, abi.v2x_episode_stats)
             for k in o:
                 _ck(self.lib.dp_memcpy_d2h(self.ctx, abi.ptr(o[k]), C.c_void_p(d[k]), C.c_size_t(sizes[k]), None), "d2h")
             _ck(self.lib.dp_stream_sync(self.ctx, None), "sync")
@@ -331,6 +359,8 @@ class Planner:
             o["graph"] = self.closed_loop_is_graph()
             return o
         finally:
+            if v2x is not None:
+                self.set_v2x_world(None, 0, None)
             if metrics is not None:
                 self.set_metrics(None, None)
             if lane_change is not None:

@@ -496,6 +496,73 @@ def v2x_events(m: Map, hdr, seed=0, p_far=0.12):
     return v, np.ascontiguousarray(la[keep]), np.ascontiguousarray(lo[keep])
 
 
+# streams of the V2X events of closed-loop worlds
+(V_OFF, V_RANGE, V_KIND, V_PED_S, V_PED_D, V_PED_V, V_PED_T, V_PED_R, V_PED_DIR, V_RW_LANE, V_RW_S, V_RW_D, V_RW_RSI,
+ V_RW_N) = range(300, 314)
+
+
+class V2xEvents:
+    """Seeded V2X events for the closed-loop worlds of `World` (include/dmpp_b200.h section 14), one dp_v2x_event_spec per world in
+    map coordinates: `spec[n]`, and the warning points `wp_x` / `wp_y` the road-works zones index.  `seeds` are the worlds' seeds.
+      junction / urban worlds: a signal at the end of the approach (road 6, stop index -1) with a seeded phase offset, cycle
+          SIGNAL = (cycle, green, yellow, red) seconds, and a seeded range of 25-60 m, so that some worlds start beyond it;
+      highway worlds: half of them a pedestrian who crosses the ego's road from its right at a seeded station 15-70 m ahead of the
+          ego's start, from 4 m right to 1 m left of its lane at 0.8-2 m/s, active from a seeded instant in the first second, with
+          a seeded range of 40-120 m; the other half a road-works zone 20-90 m ahead on a seeded lane of the ego's road, up to
+          1.5 m off its centre line, an RSI point in 70 % of them and 0-3 warning points 5 m apart along that lane.
+    Between them the seeded worlds reach every flag value of the handlers and every warn_status."""
+    SIGNAL = (14.0, 6.0, 2.0, 6.0)
+
+    def __init__(self, world, seeds, seed=0):
+        m, h, n = world.m, world.hdr, world.n
+        sd = np.asarray(seeds, np.uint64) + np.uint64(seed) * np.uint64(1000003)
+        assert sd.shape == (n,)
+        spec = np.zeros(n, abi.v2x_event_spec)
+        self.wp_x, self.wp_y = np.zeros(0), np.zeros(0)
+        if world.kind != "highway":
+            cyc, g, y, r = self.SIGNAL
+            spec["sig_road"], spec["sig_stop"] = 6, -1
+            spec["sig_cycle"], spec["sig_green"], spec["sig_yellow"], spec["sig_red"] = cyc, g, y, r
+            spec["sig_offset"] = rnd(sd, V_OFF) * cyc
+            spec["sig_range"] = 25.0 + rnd(sd, V_RANGE) * 35.0
+            self.spec = spec
+            return
+        road, lane = h["road_num"].astype(np.int64), h["lane_num"].astype(np.int64)
+        base = m.road_lane_base[road - 1].astype(np.int64)
+        nl = (m.road_lane_base[road] - m.road_lane_base[road - 1]).astype(np.int64)
+        eid = np.take_along_axis(h["id"].astype(np.int64), (lane - 1)[:, None], axis=1)[:, 0]
+
+        def point(gl, ahead_m, left_m):
+            off, cnt = m.lane_pt_off[gl].astype(np.int64), (m.lane_pt_off[gl + 1] - m.lane_pt_off[gl]).astype(np.int64)
+            i = np.clip(eid + np.rint(ahead_m / SPACING).astype(np.int64), 0, cnt - 2)
+            hr = np.radians(m.dir[off + i])
+            nx, ny = -np.sin(hr), np.cos(hr)                # left normal of the lane
+            return m.x[off + i] + left_m * nx, m.y[off + i] + left_m * ny, nx, ny
+
+        ped = rnd(sd, V_KIND) < 0.5
+        x, y, nx, ny = point(base + lane - 1, 15.0 + rnd(sd, V_PED_S) * 55.0, -4.0 + rnd(sd, V_PED_D) * 5.0)
+        v = 0.8 + rnd(sd, V_PED_V) * 1.2
+        spec["has_ped"] = ped
+        spec["ped_x"], spec["ped_y"], spec["ped_vx"], spec["ped_vy"] = x, y, v * nx, v * ny
+        spec["ped_t_on"] = rnd(sd, V_PED_T)
+        spec["ped_t_off"] = spec["ped_t_on"] + 30.0
+        spec["ped_range"] = 40.0 + rnd(sd, V_PED_R) * 80.0
+        spec["ped_direction"] = rnd(sd, V_PED_DIR) < 0.3
+        gw = base + (rnd(sd, V_RW_LANE) * nl).astype(np.int64)
+        ahead = 20.0 + rnd(sd, V_RW_S) * 70.0
+        rx, ry, _, _ = point(gw, ahead, -0.5 + rnd(sd, V_RW_D) * 2.0)
+        works = ~ped
+        spec["has_works"], spec["rw_rsi"] = works, works & (rnd(sd, V_RW_RSI) < 0.7)
+        spec["rw_x"], spec["rw_y"], spec["rw_range"] = rx, ry, 150.0
+        cnt = np.where(works, (rnd(sd, V_RW_N) * 4).astype(np.int64), 0)
+        spec["wp_count"], spec["wp_first"] = cnt, np.concatenate([[0], np.cumsum(cnt)[:-1]])
+        cols = [point(gw, ahead + 5.0 * k, 0.0)[:2] for k in range(3)]
+        keep = np.arange(3)[None, :] < cnt[:, None]
+        self.wp_x = np.ascontiguousarray(np.stack([c[0] for c in cols], axis=1)[keep])
+        self.wp_y = np.ascontiguousarray(np.stack([c[1] for c in cols], axis=1)[keep])
+        self.spec = spec
+
+
 # streams of the directed families
 (D_FAM, D_LANE, D_ID, D_GAP, D_LAT, D_SPEED, D_NAV, D_STALL, D_YAW, D_PERIOD, D_OTHER_S, D_OTHER_L, D_MOVE, D_WOB) = range(100, 114)
 

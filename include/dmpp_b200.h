@@ -671,6 +671,91 @@ void dp_lane_change_default_params(dp_lane_change_params* p);
  * ego_b_safe <= 0, politeness, cooldown, end_guard, ego_front < 0, or arming while the agent model is disarmed. */
 int dp_world_set_lane_change(dp_ctx* ctx, const dp_lane_change_params* p, dp_lane_change_state* st);
 
+/* (14) V2X events in closed-loop episodes (opt-in): each world carries one traffic signal, one crossing pedestrian and one
+ * road-works zone, placed in map coordinates; every cycle a V2X launch between the cycle and the world step builds the cycle's
+ * dp_v2x_data from the world, runs the handlers of section 10 on it (the same device code as dp_v2x_event_batch) and, with
+ * apply = 1, lets the flags act on the cycle's record with the rule of dp_v2x_apply, so the world step of section 9 moves the
+ * ego with the adjusted speed command.  Armed, an episode is: placement, then per cycle Decision + Planning -> V2X -> world
+ * step, then one tally-only V2X launch (1 + cycles * 4 + 1 kernels).  Disarmed (the default) the episode is that of section 9,
+ * launch for launch.  The rules are frozen in tools/junction_oracle/v2x_world.h.  Out of scope: agents that obey signals or
+ * yield to pedestrians, pedestrians as obstacle points, V2X in pos 1 / 2.
+ *
+ * IEEE binary64, operations in the order written, no contraction.  World s at cycle k (k = 0 .. cycles-1 the cycle launches,
+ * k = cycles the tally), with its cycle's header h (before the world step) and t = k * period_ms / 1000:
+ *   row       the launch with k == 0 first initialises the world's row (also for a header that names no lane), so a replayed
+ *             episode graph starts clean; a header that names no lane then gets zero flags and leaves its row alone
+ *   GPS       GlobalToWGS84 as dp_frames_kernel: lat = fma(y, k_lat, lat0), lng = fma(x, k_lng, lng0)
+ *   signal    sig_road > 0: phase ph = fmod(t + sig_offset, sig_cycle), ph += sig_cycle when ph < 0; state 6 (green) when
+ *             ph < sig_green, else 7 (yellow) when ph < sig_green + sig_yellow, else 3 (red); sig_road == 0: state 0.
+ *             on = sig_road > 0, h.road_num == sig_road and h.pos != 2 (the approach, pos 0 / 1); then on the ego's lane gl
+ *             (off, cnt): stop = sig_stop < 0 || sig_stop > cnt - 1 ? cnt - 1 : sig_stop (-1: the stop line at the end of a
+ *             junction approach), i = id[lane_num-1] clamped to [0, cnt-1], d = cump[off + stop] - cump[off + i]
+ *             (cump: the prefix table of dp_map_upload, section 12); off the approach d = 0.
+ *             spat_state = state, spat_lane_occupied = on && d >= 0 && d <= sig_range
+ *   pedestrian ped_on = has_ped && ped_t_on <= t && t <= ped_t_off; then px = ped_x + ped_vx * (t - ped_t_on), py likewise;
+ *             dx = px - h.x, dy = py - h.y, ped_distance = sqrt(dx * dx + dy * dy), (ped_lat, ped_lng) = GPS(px, py);
+ *             otherwise ped_distance = ped_lat = ped_lng = 0.  ped_direction = the specification's
+ *   road works has_works: (rsi_lat, rsi_lng) = GPS(rw_x, rw_y) when rw_rsi, else 0 / 0 (no RSI point: the warning list
+ *             alone); wp_first / wp_count = the specification's slice of the caller's list, whose entries pass as
+ *             GPS(wp_x, wp_y); rw_dx = rw_x - h.x, rw_dy = rw_y - h.y, near_works = sqrt(rw_dx * rw_dx + rw_dy * rw_dy) <= rw_range.
+ *             !has_works: rsi 0 / 0, an empty slice, near_works false
+ *   ego       (ego_lat, ego_lng) = GPS(h.x, h.y)
+ *   warn_status  5 when ped_on && ped_distance <= ped_range, else 3 when on, else 4 when near_works, else 0
+ *   handlers  only on headers with h.pos == 0 (SegmentDecision is their only caller, Decision.cpp:283) and k < cycles: the
+ *             flags of section 10 with the world's mode; in pos 1 / 2 and on the tally the flags are zero (distances 9999)
+ *   apply     stop  = pedestrian_flag || light_flag == 1; creep = !stop && construction_flag && rec.brakespeed > 3; with
+ *             apply = 1 the record is adjusted as dp_v2x_apply does (stop: brakespeed 0, acc_flag 1, des_acc -3; creep:
+ *             brakespeed 3); with apply = 0 the record is left alone and the row still counts both.  So with apply = 1,
+ *             replaying hdr_log through dp_run_episode_dev gives the planner's own records, which differ from the logged ones
+ *             in brakespeed / acc_flag / des_acc on the cycles with a stop or creep command, and nowhere else
+ *   red crossing  a world step that starts with last_on && last_d >= 0 && last_phase == 3 and ends past the stop line: the
+ *             header of the next launch has !on or d < 0.  The row carries (d, state, on) of the previous launch.
+ * Row (initial value): min_ped_distance min of ped_distance over launches k < cycles with ped_on, any pos (+inf); cycles:
+ * launches that ran the handlers; light_cycles[f] / construction_cycles[f] / pedestrian_cycles[f]: of those, the cycles with
+ * that flag value; stop_cmds, creep_cmds, ub_cycles (flags.ub); red_crossings and first_red_crossing (k of the step, -1). */
+typedef struct dp_v2x_event_spec {
+    double sig_cycle, sig_green, sig_yellow, sig_red;  /* seconds; each > 0 and green + yellow + red == cycle (to 1e-9 of it) */
+    double sig_offset;                 /* seconds added to t before the phase */
+    double sig_range;                  /* metres before the stop index within which the approach counts as occupied */
+    double ped_x, ped_y, ped_vx, ped_vy;               /* map metres at t = ped_t_on, m/s */
+    double ped_t_on, ped_t_off;        /* active window, seconds */
+    double ped_range;                  /* metres */
+    double rw_x, rw_y, rw_range;       /* the road-works point (map metres) and its range */
+    int32_t sig_road;                  /* governed road, 1-based; 0 = no signal */
+    int32_t sig_stop;                  /* stop index on the governed road's lanes; -1 = the last point of the lane */
+    int32_t has_ped, ped_direction;    /* ped_direction: PedesDirection as the handler reads it */
+    int32_t has_works, rw_rsi;         /* rw_rsi: the RSI broadcasts (rw_x, rw_y) */
+    int32_t wp_first, wp_count;        /* the zone's warning points: wp_x / wp_y[wp_first .. wp_first + wp_count) */
+} dp_v2x_event_spec;                   /* 160 bytes */
+typedef struct dp_v2x_world_params {
+    int32_t mode;                      /* 0 / 1 as in dp_v2x_event_batch */
+    int32_t apply;                     /* 1: the flags act on the records; 0: observe only (the row still counts) */
+} dp_v2x_world_params;
+typedef struct dp_v2x_episode_stats {
+    double min_ped_distance;
+    double last_d;                     /* carried from the previous launch (0) */
+    int32_t cycles;
+    int32_t light_cycles[3], construction_cycles[2], pedestrian_cycles[2];
+    int32_t stop_cmds, creep_cmds, ub_cycles;
+    int32_t red_crossings, first_red_crossing;
+    int32_t last_phase, last_on;       /* carried from the previous launch (0 / 0) */
+    int32_t pad;                       /* zero */
+} dp_v2x_episode_stats;                /* 80 bytes */
+/* spec[n] (device): one specification per world, indexed like hdr (the s-th scene of every later dp_run_closed_loop_dev /
+ * dp_v2x_world_dev call, which may name at most n scenes); wp_x / wp_y[n_wp] (device, nullable when n_wp is 0): the warning
+ * points; flags[n] (device, nullable): every V2X launch of a cycle stores the world's flags (the tally leaves them); stats[n] (device): the rows.  spec == NULL
+ * disarms (everything else may then be NULL).  The setter copies the specifications to the host once to validate them:
+ * DP_ERR_ARG for a mode other than 0 / 1, apply other than 0 / 1, non-finite values, signal durations that are not > 0 or do
+ * not sum to the cycle, ranges < 0, sig_road outside [0, n_roads], sig_stop < -1, a warning-point slice outside [0, n_wp), or
+ * NULL stats.  Context state like dp_world_set_metrics: the cached episode graph is rebuilt on its next call. */
+int dp_world_set_v2x(dp_ctx* ctx, const dp_v2x_world_params* params, int n, const dp_v2x_event_spec* spec, const double* wp_x,
+                     const double* wp_y, int n_wp, dp_v2x_flags* flags, dp_v2x_episode_stats* stats);
+/* one V2X launch of cycle `cycle` for callers that step by hand: after dp_cycle_batch_dev wrote rec[n] for hdr[n], before
+ * dp_world_step_dev(rec) moves the world; rec == NULL: the tally after the last world step (cycle = the number of cycles).
+ * DP_ERR_STATE when V2X is disarmed. */
+int dp_v2x_world_dev(dp_ctx* ctx, int first_scene, int n_scenes, const dp_scene_hdr* hdr, dp_plan_record* rec, int cycle,
+                     void* stream);
+
 /* diagnostic: phase time stamps (globaltimer, ns) of the most recent cycle launch, one row of 32 per CTA (row b = scenes
  * [b*g, (b+1)*g) of the batch; stamp 0 = CTA start, stamp i = end of phase i of csrc/dp_group.cuh).  Only contexts created
  * with DP_TIMELINE=1 in the environment record them; used by tools/group_timeline.py, never by the product path. */

@@ -13,7 +13,12 @@ SM clock read in the same run.
                of it, another lane).
   lane_change  lane changes (section 13) on top of the reactive agents, against the reactive agents alone: the highway episode,
                the collision table and the lane changes made, and dp_world_step_dev alone (4096 highway worlds with 10 agents, 1024
-               with 200)."""
+               with 200).
+  v2x          V2X events in closed-loop episodes (section 14): the highway and junction episodes (4096 worlds) disarmed, observe-only
+               (apply = 0: the records must equal the disarmed ones, the delta is the V2X launches alone) and applied; the V2X launch
+               alone (dp_v2x_world_dev, 4096 worlds, apply = 0, on the world and records the last episode left); and the effect of
+               applying the flags on seeds 0-511 (red crossings, stop cycles, worlds that stopped on a red and left on green, the
+               minimum ego-pedestrian distance while the pedestrian is active)."""
 import argparse
 import json
 import os
@@ -49,7 +54,7 @@ def cump_of():
 class Arm:
     """one planner + world of one kind, with the models asked for armed"""
 
-    def __init__(self, kind, n, n_obs, cycles, metrics=False, react=False, lanechg=False):
+    def __init__(self, kind, n, n_obs, cycles, metrics=False, react=False, lanechg=False, v2x=None):
         self.n = n
         self.p = Planner(n, n_obs); self.p.upload_map(m)
         wp = self.p.world_params(); wp.pre_junction_pts = scenes.World.PRE_JUNCTION_PTS[kind]
@@ -69,6 +74,13 @@ class Arm:
             self.p.set_agent_model(pl.agent_model_params(), self.d_v0.data_ptr())
         if lanechg:
             self.p.set_lane_change(pl.lane_change_params(), self.d_s.data_ptr())
+        if v2x is not None:                                 # v2x = apply (0 / 1)
+            self.ev = scenes.V2xEvents(self.w, np.arange(n))
+            self.d_spec, self.d_wx, self.d_wy = u8(self.ev.spec), u8(np.append(self.ev.wp_x, 0.0)), u8(np.append(self.ev.wp_y, 0.0))
+            self.d_vf = torch.zeros((n, abi.v2x_flags.itemsize), dtype=torch.uint8, device=dev)
+            self.d_vs = torch.zeros((n, abi.v2x_episode_stats.itemsize), dtype=torch.uint8, device=dev)
+            self.p.set_v2x_world(abi.V2xWorldParams(0, v2x), n, self.d_spec.data_ptr(), self.d_wx.data_ptr(), self.d_wy.data_ptr(),
+                                 self.ev.wp_x.size, self.d_vf.data_ptr(), self.d_vs.data_ptr())
 
     def episode_ms(self, graph=True):
         st = torch.cuda.current_stream()
@@ -100,8 +112,18 @@ class Arm:
         self.d_h.copy_(h); self.d_a.copy_(a); self.d_s.copy_(s)
         return e0.elapsed_time(e1) * 1e3 / launches
 
+    def v2x_us(self, launches=50):
+        """dp_v2x_world_dev alone (cycle 5) on the world and the last records the last episode left"""
+        st = torch.cuda.current_stream()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record(st)
+        for _ in range(launches):
+            self.p.v2x_world_dev(self.n, self.d_h.data_ptr(), self.d_r[-1].data_ptr(), 5, stream=st.cuda_stream)
+        e1.record(st); torch.cuda.synchronize()
+        return e0.elapsed_time(e1) * 1e3 / launches
+
     def close(self):
-        self.p.set_lane_change(None, None); self.p.set_agent_model(None, None); self.p.set_metrics(None, None); self.p.close()
+        self.p.set_v2x_world(None, 0, None); self.p.set_lane_change(None, None); self.p.set_agent_model(None, None); self.p.set_metrics(None, None); self.p.close()
 
 
 def alternate(arms, *measures):
@@ -255,8 +277,66 @@ def bench_lane_change():
     return out
 
 
+def v2x_effect(kind, cycles, n=512):
+    """seeds 0 .. n-1, apply 0 against 1: what the flags do to the episode"""
+    out = {}
+    w = scenes.World(m, np.arange(n), 10, kind=kind)
+    ev = scenes.V2xEvents(w, np.arange(n))
+    for apply in (0, 1):
+        p = Planner(n, 10); p.upload_map(m)
+        wp = p.world_params(); wp.pre_junction_pts = scenes.World.PRE_JUNCTION_PTS[kind]; p.set_world_params(wp)
+        o = p.run_closed_loop(w.hdr, w.agents, cycles, v2x=(abi.V2xWorldParams(0, apply), ev))
+        p.close()
+        st, hl = o["v2x_stats"], o["hdr_log"]
+        r = {"stop_cycles": int(st["stop_cmds"].sum()), "creep_cycles": int(st["creep_cmds"].sum()),
+             "worlds_with_a_stop_command": int((st["stop_cmds"] > 0).sum()), "handler_cycles": int(st["cycles"].sum())}
+        if kind == "junction":
+            s = ev.spec
+            t = np.arange(cycles)[:, None] * hl["period_ms"] / 1000.0
+            ph = np.fmod(t + s["sig_offset"][None, :], s["sig_cycle"][None, :])
+            ph = np.where(ph < 0, ph + s["sig_cycle"][None, :], ph)
+            state = np.where(ph < s["sig_green"], 6, np.where(ph < s["sig_green"] + s["sig_yellow"], 7, 3))
+            on = (hl["road_num"] == 6) & (hl["pos"] != 2)
+            stopped_red = on & (hl["velocity"] == 0) & (state == 3)
+            left = on[:-1] & ~on[1:]                           # the step from cycle k left the approach
+            left_green = left & (state[:-1] == 6)
+            sr = stopped_red.any(axis=0)
+            later_green = np.array([left_green[np.argmax(stopped_red[:, i]):, i].any() if sr[i] else False for i in range(n)])
+            r.update(red_crossings=int(st["red_crossings"].sum()), worlds_crossing_on_red=int((st["red_crossings"] > 0).sum()),
+                     worlds_stopped_on_red=int(sr.sum()), worlds_stopped_on_red_then_left_on_green=int(later_green.sum()),
+                     worlds_crossed=int(left.any(axis=0).sum()))
+        else:
+            d = st["min_ped_distance"][ev.spec["has_ped"] == 1]
+            r.update(worlds_with_pedestrian=int(d.size), min_ped_distance_median=float(np.median(d)), min_ped_distance_min=float(d.min()),
+                     worlds_within_1m=int((d < 1.0).sum()), worlds_within_2m=int((d < 2.0).sum()))
+        out["apply_%d" % apply] = r
+    return out
+
+
+def bench_v2x():
+    N = 4096
+    out = {"scenes": N, "card": card(), "episode": {}, "v2x_launch": {}, "effect": {}}
+    for kind, cycles in (("highway", 25), ("junction", 120)):
+        arms = {"off": Arm(kind, N, 10, cycles), "observe": Arm(kind, N, 10, cycles, v2x=0), "apply": Arm(kind, N, 10, cycles, v2x=1)}
+        warm(arms)
+        ep, = alternate(arms, Arm.episode_ms)
+        same = arms["off"].d_r.cpu().numpy().tobytes() == arms["observe"].d_r.cpu().numpy().tobytes()
+        assert same, kind + ": observe-only records differ from the disarmed ones"
+        out["episode"]["%s_%dx%d" % (kind, N, cycles)] = {
+            "cycles": cycles, "ms_off": summary(ep["off"]), "ms_observe": summary(ep["observe"]), "ms_apply": summary(ep["apply"]),
+            "observe_over_off": ratio(ep["observe"], ep["off"]), "apply_over_off": ratio(ep["apply"], ep["off"]),
+            "records_identical_off_observe": same}
+        a = arms["observe"]
+        a.v2x_us()
+        us = [a.v2x_us() for _ in range(REPS * ROUNDS)]
+        out["v2x_launch"]["%s_%d" % (kind, N)] = {"us_per_launch": summary(us), "launches_per_window": 50}
+        close(arms)
+        out["effect"]["%s_512x%d" % (kind, cycles)] = v2x_effect(kind, cycles)
+    return out
+
+
 if __name__ == "__main__":
-    benches = {"metrics": bench_metrics, "agents": bench_agents, "lane_change": bench_lane_change}
+    benches = {"metrics": bench_metrics, "agents": bench_agents, "lane_change": bench_lane_change, "v2x": bench_v2x}
     ap = argparse.ArgumentParser(description=__doc__.split("\n")[0])
     ap.add_argument("model", choices=list(benches))
     print(json.dumps(benches[ap.parse_args().model]()))

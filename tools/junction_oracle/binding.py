@@ -50,10 +50,13 @@ class JunctionOracle:
         assert self.lib.jo_world_step(C.byref(self.params), C.byref(wp), C.c_int(n), C.c_int(max_obs), abi.ptr(hdr), abi.ptr(agents),
                                       abi.ptr(ox), abi.ptr(oy), abi.ptr(rec), abi.ptr(last_path)) == 0
 
-    def run_closed_loop(self, hdr, agents, cycles, wp=None, paths=False, threads=1, metrics=None, agent_model=None, lane_change=None):
+    def run_closed_loop(self, hdr, agents, cycles, wp=None, paths=False, threads=1, metrics=None, agent_model=None, lane_change=None,
+                        v2x=None):
         """hdr[n], agents[n][max_obs] (copied; the final world is returned), through jo_run_closed_loop; metrics = MetricsParams: the
         episode metrics of every world under "metrics"; agent_model = (AgentModelParams, v0[n][max_obs]): the reactive agents;
-        lane_change = LaneChangeParams (with agent_model): their lane changes, the final states under "lane_change_state"
+        lane_change = LaneChangeParams (with agent_model): their lane changes, the final states under "lane_change_state";
+        v2x = (V2xWorldParams, events with spec / wp_x / wp_y): the V2X events, the rows under "v2x_stats" and the flags of the last
+        launch under "v2x_flags"
         """
         assert lane_change is None or agent_model is not None
         am, v0 = agent_model if agent_model is not None else (None, None)
@@ -68,6 +71,17 @@ class JunctionOracle:
                                 abi.lane_change_state).reshape(agents.shape).copy()
         ref = lambda p: None if p is None else C.byref(p)
         models = (ref(metrics), abi.ptr(met), ref(am), abi.ptr(v0), ref(lane_change), abi.ptr(lcs))
+        vflags = vstats = None
+        if v2x is not None:
+            vp, ev = v2x
+            spec, wx, wy = self._v2x_inputs(ev)
+            n = hdr.shape[0]
+            assert spec.shape == (n,)
+            vflags = np.frombuffer(np.full(n * abi.v2x_flags.itemsize, 0xAB, np.uint8).tobytes(), abi.v2x_flags).copy()
+            vstats = np.frombuffer(np.full(n * abi.v2x_episode_stats.itemsize, 0xAB, np.uint8).tobytes(), abi.v2x_episode_stats).copy()
+            models += (C.byref(vp), abi.ptr(spec), abi.ptr(wx), abi.ptr(wy), C.c_int(wx.size), abi.ptr(vflags), abi.ptr(vstats))
+        else:
+            models += (None,) * 4 + (C.c_int(0), None, None)
         f = self.lib.jo_run_closed_loop
         f.restype = C.c_longlong
         # ob._closed_loop passes the arrays every closed loop has; the model arguments follow them
@@ -77,7 +91,45 @@ class JunctionOracle:
             o["metrics"] = met
         if lcs is not None:
             o["lane_change_state"] = lcs
+        if vstats is not None:
+            o["v2x_flags"], o["v2x_stats"] = vflags, vstats
         return o
+
+    @staticmethod
+    def _v2x_inputs(ev):
+        spec, wx, wy = np.ascontiguousarray(ev.spec), np.ascontiguousarray(ev.wp_x, np.float64), np.ascontiguousarray(ev.wp_y, np.float64)
+        assert spec.dtype == abi.v2x_event_spec and wx.shape == wy.shape
+        return spec, wx, wy
+
+    def v2x_data(self, spec, hdr, k):
+        """the V2X data builder alone (jo_v2x_data): data[n], aux[n][3] = (d, spat_state, on + 2 * ped_on)"""
+        spec, hdr = np.ascontiguousarray(spec), np.ascontiguousarray(hdr)
+        n = hdr.shape[0]
+        data, aux = np.zeros(n, abi.v2x_data), np.zeros((n, 3))
+        assert self.lib.jo_v2x_data(C.byref(self.params), C.c_int(n), abi.ptr(spec), abi.ptr(hdr), C.c_int(k), abi.ptr(data), abi.ptr(aux)) == 0
+        return data, aux
+
+    def v2x_cycle(self, vp, ev, hdr, rec, k, stats):
+        """one V2X launch for every world (jo_v2x_cycle): rec (adjusted in place; None: the tally) and stats in place, returns the flags"""
+        spec, wx, wy = self._v2x_inputs(ev)
+        hdr = np.ascontiguousarray(hdr)
+        n = hdr.shape[0]
+        assert stats.dtype == abi.v2x_episode_stats and stats.shape == (n,) and (rec is None or rec.flags["C_CONTIGUOUS"])
+        flags = np.zeros(n, abi.v2x_flags)
+        assert self.lib.jo_v2x_cycle(C.byref(self.params), C.byref(vp), C.c_int(n), abi.ptr(spec), abi.ptr(wx), abi.ptr(wy), C.c_int(wx.size),
+                                     abi.ptr(hdr), abi.ptr(rec), C.c_int(k), abi.ptr(flags), abi.ptr(stats)) == 0
+        return flags
+
+    def gps(self, x, y):
+        """GlobalToWGS84 of the points (x, y): (lat, lng)"""
+        x, y = np.ascontiguousarray(x, np.float64), np.ascontiguousarray(y, np.float64)
+        la, lo = np.zeros(x.size), np.zeros(x.size)
+        self.lib.jo_gps(C.byref(self.params), C.c_int(x.size), abi.ptr(x), abi.ptr(y), abi.ptr(la), abi.ptr(lo))
+        return la, lo
+
+    def v2x_sizeof(self):
+        """sizeof(dp_v2x_event_spec), sizeof(dp_v2x_episode_stats)"""
+        return int(self.lib.jo_v2x_sizeof(0)), int(self.lib.jo_v2x_sizeof(1))
 
     def react_step(self, hdr, agents, v0, am, wp=None):
         """the react phase alone, agents[n][max_obs] in place (jo_react_step)"""

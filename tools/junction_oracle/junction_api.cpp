@@ -2,7 +2,8 @@
 // (planner_oracle.cpp, compiled in unchanged) with the junction world step of world_junction.cpp between its cycles; the
 // same arrays as oracle_world_step / oracle_run_closed_loop of oracle/oracle_api.cpp; in jo_run_closed_loop, the models each
 // world step may carry: the episode metrics of episode_metrics.cpp (alone: jo_metrics_step), the reactive agents of
-// agent_model.cpp (alone: jo_react_step) and their lane changes of lane_change.cpp (alone: jo_lane_change_step).
+// agent_model.cpp (alone: jo_react_step) and their lane changes of lane_change.cpp (alone: jo_lane_change_step); and the V2X launch
+// of v2x_world.cpp between a cycle and its world step (alone: jo_v2x_cycle, its data builder: jo_v2x_data).
 #include <algorithm>
 #include <atomic>
 #include <cstring>
@@ -11,10 +12,18 @@
 #include "agent_model.h"
 #include "episode_metrics.h"
 #include "lane_change.h"
+#include "v2x_world.h"
 #include "world_junction.h"
 #include "../../oracle/cshare_spec.h"
 
-namespace { junction::JMap g_map; bool g_have_map = false; }
+namespace {
+junction::JMap g_map; bool g_have_map = false;
+// the warning list through GlobalToWGS84, as the handlers read it
+void wp_gps(const dp_params& p, const double* wp_x, const double* wp_y, int n_wp, std::vector<double>& la, std::vector<double>& lo) {
+    la.resize((size_t)n_wp); lo.resize((size_t)n_wp);
+    for (int i = 0; i < n_wp; ++i) spec::global_to_wgs84(spec::Datum{p.lat0, p.lng0, p.k_lat, p.k_lng}, wp_x[i], wp_y[i], &la[i], &lo[i]);
+}
+}  // namespace
 
 extern "C" {
 
@@ -40,15 +49,20 @@ int jo_world_step(const dp_params* p, const dp_world_params* wp, int n, int max_
 // the closed loop: the junction world step between the cycles of oracle/, the same arrays as oracle_run_closed_loop.  Each model is
 // armed by a non-null pair, or off with both NULL: mp / met[n] the episode metrics of include/dmpp_b200.h section 11, accumulated
 // after every world step; am / v0[n][max_obs] the reactive agents of section 12, before every world step; lp / lcs[n][max_obs]
-// (with am) their lane changes of section 13, states initialised by the placement step and holding the final states
+// (with am) their lane changes of section 13, states initialised by the placement step and holding the final states; vp / spec[n]
+// (wp_x / wp_y[n_wp], flags[n] nullable, stats[n]) the V2X events of section 14 between every cycle and its world step
 long long jo_run_closed_loop(const dp_params* p, const dp_world_params* wp, int n, int cycles, int max_obs, dp_scene_hdr* hdr,
                              dp_agent* agents, double* ox, double* oy, dp_plan_record* rec, dp_scene_hdr* hdr_log, double* obs_log_x,
                              double* obs_log_y, double* path_xy, dp_carry* carry_out, double* last_path_out, int threads,
                              int32_t* ub_scene, const dp_metrics_params* mp, dp_episode_metrics* met, const dp_agent_model_params* am,
-                             const double* v0, const dp_lane_change_params* lp, dp_lane_change_state* lcs) {
+                             const double* v0, const dp_lane_change_params* lp, dp_lane_change_state* lcs, const dp_v2x_world_params* vp,
+                             const dp_v2x_event_spec* spec, const double* wp_x, const double* wp_y, int n_wp, dp_v2x_flags* flags,
+                             dp_v2x_episode_stats* stats) {
     if (!g_have_map) return -1;
-    if ((!mp) != (!met) || (!am) != (!v0) || (!lp) != (!lcs) || (lcs && !v0)) return -1;
+    if ((!mp) != (!met) || (!am) != (!v0) || (!lp) != (!lcs) || (lcs && !v0) || (!vp) != (!spec) || (spec && !stats)) return -1;
     if (threads < 1) threads = 1;
+    std::vector<double> wla, wlo;
+    if (spec) wp_gps(*p, wp_x, wp_y, n_wp, wla, wlo);
     std::atomic<long long> ub(0);
     auto work = [&](int s0, int s1) {
         long long lub = 0;
@@ -71,6 +85,7 @@ long long jo_run_closed_loop(const dp_params* p, const dp_world_params* wp, int 
                 o.path_xy = path_xy ? path_xy + e * 400 : nullptr;
                 oracle::cycle(g_map.m, *p, hdr[s], sx, sy, st, o, false);
                 lub += o.ub_hits;
+                if (spec) v2x::cycle(g_map, *p, *vp, spec[s], wla.data(), wlo.data(), hdr[s], c, rec + e, stats[s], flags ? flags + s : nullptr);
                 const dp_scene_hdr h0 = hdr[s];
                 if (lcs) lanechg::step(g_map, *wp, *am, *lp, h0, ag, std::min((int)h0.n_obs, max_obs), v0 + (size_t)s * max_obs,
                                        lcs + (size_t)s * max_obs);
@@ -78,6 +93,7 @@ long long jo_run_closed_loop(const dp_params* p, const dp_world_params* wp, int 
                 junction::world_step(g_map, *p, *wp, hdr[s], ag, sx, sy, rec + e, st.last_x, st.last_y);
                 if (met) metrics::update(g_map, *wp, *mp, met[s], h0, hdr[s], ag, sx, sy, std::min((int)h0.n_obs, max_obs), rec[e]);
             }
+            if (spec) v2x::cycle(g_map, *p, *vp, spec[s], wla.data(), wlo.data(), hdr[s], cycles, nullptr, stats[s], flags ? flags + s : nullptr);
             if (ub_scene) ub_scene[s] = (int32_t)(lub - lub0);
             if (carry_out) carry_out[s] = st.c;
             if (last_path_out) {
@@ -142,5 +158,36 @@ int jo_metrics_step(const dp_params* p, const dp_world_params* wp, const dp_metr
 int jo_metrics_sizeof(void) { return (int)sizeof(dp_episode_metrics); }
 
 void jo_sincos_deg(double a, double* c, double* s) { spec::spec_sincos_deg(a, c, s); }
+
+// the V2X data builder alone for every world at cycle k: data[n], and aux[n][3] = (d, spat_state, on + 2 * ped_on); headers must
+// name a lane
+int jo_v2x_data(const dp_params* p, int n, const dp_v2x_event_spec* spec, const dp_scene_hdr* hdr, int k, dp_v2x_data* data, double* aux) {
+    if (!g_have_map) return -1;
+    for (int s = 0; s < n; ++s) {
+        if (!metrics::header_valid(g_map.m, hdr[s])) return -1;
+        const v2x::World w = v2x::build(g_map, *p, spec[s], hdr[s], k);
+        data[s] = w.v;
+        aux[3 * s] = w.d; aux[3 * s + 1] = w.state; aux[3 * s + 2] = (w.on ? 1 : 0) + (w.ped_on ? 2 : 0);
+    }
+    return 0;
+}
+
+// one V2X launch for every world, in place (rec[n] nullable: the tally), as dp_v2x_world_dev runs it
+int jo_v2x_cycle(const dp_params* p, const dp_v2x_world_params* vp, int n, const dp_v2x_event_spec* spec, const double* wp_x, const double* wp_y,
+                 int n_wp, const dp_scene_hdr* hdr, dp_plan_record* rec, int k, dp_v2x_flags* flags, dp_v2x_episode_stats* stats) {
+    if (!g_have_map) return -1;
+    std::vector<double> wla, wlo;
+    wp_gps(*p, wp_x, wp_y, n_wp, wla, wlo);
+    for (int s = 0; s < n; ++s)
+        v2x::cycle(g_map, *p, *vp, spec[s], wla.data(), wlo.data(), hdr[s], k, rec ? rec + s : nullptr, stats[s], flags ? flags + s : nullptr);
+    return 0;
+}
+
+// GlobalToWGS84 of n points
+void jo_gps(const dp_params* p, int n, const double* x, const double* y, double* lat, double* lng) {
+    for (int i = 0; i < n; ++i) spec::global_to_wgs84(spec::Datum{p->lat0, p->lng0, p->k_lat, p->k_lng}, x[i], y[i], lat + i, lng + i);
+}
+
+int jo_v2x_sizeof(int which) { return which ? (int)sizeof(dp_v2x_episode_stats) : (int)sizeof(dp_v2x_event_spec); }
 
 }  // extern "C"
