@@ -191,6 +191,16 @@ class V2xWorldParams(C.Structure):
     _fields_ = [("mode", C.c_int32), ("apply", C.c_int32)]
 
 
+class V2xTrafficParams(C.Structure):
+    _fields_ = [("b_commit", C.c_double), ("ped_half_width", C.c_double), ("obey", C.c_int32), ("pad", C.c_int32)]
+
+
+v2x_traffic_stats = np.dtype(
+    [("min_ped_dist", "<f8"), ("red_runs", "<i4"), ("line_steps", "<i4"), ("ped_steps", "<i4"), ("ped_hits", "<i4"), ("pad", "<i4", (2,))]
+)
+assert v2x_traffic_stats.itemsize == 32
+
+
 class MapDesc(C.Structure):
     _fields_ = [
         ("n_roads", C.c_int32), ("road_lane_base", C.c_void_p),

@@ -66,6 +66,8 @@ struct dp_ctx {
     DpWorldOpts world;                                      // dp_world_set_params and the armed models (dp_world_set_metrics,
                                                             // dp_world_set_agent_model, dp_world_set_lane_change)
     DpV2xOpts v2x;                                          // dp_world_set_v2x: the V2X launch between cycle and world step
+    int v2x_cycle = 0;                                      // the cycle of the last dp_v2x_world_dev call: section 15's t of a
+                                                            // hand-stepped world step
     cudaStream_t ep_stream = nullptr;
     cudaGraphExec_t ep_exec = nullptr;
     const void* ep_key[8] = {}; int ep_dims[3] = {-1, -1, -1};
@@ -1345,7 +1347,7 @@ int dp_world_set_agent_model(dp_ctx* c, const dp_agent_model_params* p, const do
         c->world.amp = *p;
     }
     c->world.v0 = v0;
-    if (!v0) c->world.lcs = nullptr;                        // lane changes run on the react phase
+    if (!v0) { c->world.lcs = nullptr; c->world.ts = nullptr; }   // lane changes and the V2X events act on the react phase
     return drop_episode_graph(c);
 }
 void dp_lane_change_default_params(dp_lane_change_params* p) {
@@ -1377,6 +1379,7 @@ int dp_world_set_v2x(dp_ctx* c, const dp_v2x_world_params* vp, int n, const dp_v
     if (!c) return fail(DP_ERR_ARG, "dp_world_set_v2x: bad argument");
     if (!spec) {
         c->v2x = DpV2xOpts{};
+        c->world.ts = nullptr; c->world.spec = nullptr;     // the agents cannot obey events that are not there
         return drop_episode_graph(c);
     }
     if (!vp || !stats || n < 0 || n_wp < 0 || (n_wp > 0 && (!wp_x || !wp_y)) || (vp->mode != 0 && vp->mode != 1) ||
@@ -1401,6 +1404,29 @@ int dp_world_set_v2x(dp_ctx* c, const dp_v2x_world_params* vp, int n, const dp_v
             return fail(DP_ERR_ARG, "dp_world_set_v2x: warning-point slice out of range");
     }
     c->v2x.vp = *vp; c->v2x.spec = spec; c->v2x.wp_x = wp_x; c->v2x.wp_y = wp_y; c->v2x.flags = flags; c->v2x.stats = stats; c->v2x.n = n;
+    if (c->world.ts) c->world.spec = spec;
+    return drop_episode_graph(c);
+}
+void dp_v2x_traffic_default_params(dp_v2x_traffic_params* p) {
+    if (!p) return;
+    memset(p, 0, sizeof(*p));
+    p->b_commit = 4.0; p->ped_half_width = 2.0; p->obey = 1;
+}
+int dp_world_set_v2x_traffic(dp_ctx* c, const dp_v2x_traffic_params* p, dp_v2x_traffic_stats* stats) {
+    if (!c || (stats && !p)) return fail(DP_ERR_ARG, "dp_world_set_v2x_traffic: bad argument");
+    if (p) {
+        if (!all_finite({p->b_commit, p->ped_half_width})) return fail(DP_ERR_ARG, "dp_world_set_v2x_traffic: parameters must be finite");
+        if (!(p->b_commit > 0) || !(p->ped_half_width >= 0) || (p->obey != 0 && p->obey != 1))
+            return fail(DP_ERR_ARG, "dp_world_set_v2x_traffic: b_commit > 0, ped_half_width >= 0 and obey 0 / 1");
+    }
+    if (stats) {
+        if (!c->world.v0) return fail(DP_ERR_ARG, "dp_world_set_v2x_traffic: the agent model is not armed (dp_world_set_agent_model)");
+        if (!c->v2x.spec) return fail(DP_ERR_ARG, "dp_world_set_v2x_traffic: the V2X events are not armed (dp_world_set_v2x)");
+        CK(cudaSetDevice(c->device));
+        CK(dp_world_prepare());                             // function attributes are set before any launch or capture of the armed step
+        c->world.tp = *p; c->world.spec = c->v2x.spec;
+    } else c->world.spec = nullptr;
+    c->world.ts = stats;
     return drop_episode_graph(c);
 }
 int dp_v2x_world_dev(dp_ctx* c, int first, int n, const dp_scene_hdr* hdr, dp_plan_record* rec, int cycle, void* stream) {
@@ -1410,6 +1436,7 @@ int dp_v2x_world_dev(dp_ctx* c, int first, int n, const dp_scene_hdr* hdr, dp_pl
     if (n > c->v2x.n) return fail(DP_ERR_ARG, "dp_v2x_world_dev: more scenes than the armed specifications");
     CK(cudaSetDevice(c->device));
     c->launches += n > 0 ? 1 : 0;
+    c->v2x_cycle = cycle;
     CK(dp_launch_world_v2x(c->gmap, c->p, c->v2x, n, hdr, rec, cycle, (cudaStream_t)stream));
     return DP_OK;
 }
@@ -1418,9 +1445,10 @@ int dp_world_step_dev(dp_ctx* c, int first, int n, dp_scene_hdr* hdr, dp_agent* 
     if (!c || !hdr || !agents || !ox || !oy || n < 0 || first < 0 || first + n > c->max_scenes)
         return fail(DP_ERR_ARG, "dp_world_step_dev: bad argument");
     if (!c->have_map) return fail(DP_ERR_STATE, "dp_world_step_dev: map not uploaded");
+    if (c->world.ts && n > c->v2x.n) return fail(DP_ERR_ARG, "dp_world_step_dev: more scenes than the armed V2X specifications");
     CK(cudaSetDevice(c->device));
     c->launches += n > 0 ? 1 : 0;
-    const DpWorldBufs b = {n, c->max_obs, hdr, agents, ox, oy, rec, c->d_last + (size_t)first * DP_PATH_POINTS};
+    const DpWorldBufs b = {n, c->max_obs, hdr, agents, ox, oy, rec, c->d_last + (size_t)first * DP_PATH_POINTS, c->v2x_cycle};
     CK(dp_launch_world(c->gmap, c->p, c->world, b, (cudaStream_t)stream));
     return DP_OK;
 }
@@ -1446,7 +1474,7 @@ cudaError_t enqueue_closed_loop(dp_ctx* c, int first, int n, int cycles, dp_scen
             if ((e = dp_launch_world_v2x(c->gmap, c->p, c->v2x, n, hdr, rec + (size_t)k * n, k, st)) != cudaSuccess) return e;
         }
         c->launches += 1;
-        b.rec = rec + (size_t)k * n;
+        b.rec = rec + (size_t)k * n; b.cycle = k;
         if ((e = dp_launch_world(c->gmap, c->p, c->world, b, st)) != cudaSuccess) return e;
     }
     if (c->v2x.spec) {                                      // the tally: closes the red-crossing check of the last world step

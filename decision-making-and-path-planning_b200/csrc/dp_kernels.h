@@ -22,18 +22,22 @@ cudaError_t dp_launch_cycle(const DevMap& m, const dp_params& p, int n, const dp
 void dp_launch_prepare(DpLaunchCfg& lc);
 // the closed-loop world step (dp_world_step.cuh): the buffers of one launch, and the option set a context arms.  A model is armed
 // by its pointer: met != nullptr episode metrics (include/dmpp_b200.h section 11), v0 != nullptr reactive agents (section 12),
-// lcs != nullptr with v0 lane changes (section 13); its parameters are read only while it is armed
+// lcs != nullptr with v0 lane changes (section 13), ts != nullptr with v0 and spec agents that obey the V2X events (section 15);
+// its parameters are read only while it is armed
 struct DpWorldBufs {
     int n, max_obs;
     dp_scene_hdr* hdr; dp_agent* agents; double* ox; double* oy;
     const dp_plan_record* rec;                 // nullptr: the placement step
     const double2* last_path;
+    int cycle = 0;                             // the cycle whose record the step applies (section 15's t)
 };
 struct DpWorldOpts {
     dp_world_params wp;
     dp_metrics_params mp; dp_episode_metrics* met = nullptr;
     dp_agent_model_params amp; const double* v0 = nullptr;
     dp_lane_change_params lcp; dp_lane_change_state* lcs = nullptr;
+    dp_v2x_traffic_params tp; dp_v2x_traffic_stats* ts = nullptr;
+    const dp_v2x_event_spec* spec = nullptr;   // section 14's specifications, while ts is armed
 };
 cudaError_t dp_launch_world(const DevMap& m, const dp_params& p, const DpWorldOpts& o, const DpWorldBufs& b, cudaStream_t st);
 // allow the reactive instances the dynamic shared memory of DP_AGENT_MODEL_MAX_OBS agent slots (current device; set before a capture)

@@ -4,8 +4,9 @@
 //                     (arithmetic frozen in oracle/world_spec.cpp, junction transitions in tools/junction_oracle/world_junction.cpp;
 //                     IEEE binary64, -fmad=false, operations in that order); the kernel and its launcher are in
 //                     dp_world_step.cuh, its disarmed instances here, its episode-metrics instances in dp_world_metrics.cu,
-//                     its reactive-agent instances in dp_world_agents.cu, its lane-changing instances in dp_world_lanechange.cu;
-//                     dp_launch_world picks the instance set from the armed options;
+//                     its reactive-agent instances in dp_world_agents.cu, its lane-changing instances in dp_world_lanechange.cu,
+//                     the instances whose agents obey the V2X events in dp_world_traffic.cu; dp_launch_world picks the instance
+//                     set from the armed options;
 //   dp_v2x_kernel     the V2X event handlers (Decision.cpp:1824-2434, dp_v2x.cuh) as a batch operator next to the cycle (their
 //                     closed-loop launch is dp_world_v2x.cu);
 //   dp_frames_kernel  the output stage: PlanningOut / PlanningStatus (Planning.cpp:173-214) packed into fixed-layout frames
@@ -92,13 +93,19 @@ template struct WorldStep<false, false, false>;
 
 cudaError_t dp_launch_world(const DevMap& m, const dp_params& p, const DpWorldOpts& o, const DpWorldBufs& b, cudaStream_t st) {
     if (b.n <= 0) return cudaSuccess;
+    if (o.v0 && o.ts && o.lcs)
+        return o.met ? WorldStep<true, true, true, true>::launch(m, p, o, b, st) : WorldStep<false, true, true, true>::launch(m, p, o, b, st);
+    if (o.v0 && o.ts)
+        return o.met ? WorldStep<true, true, false, true>::launch(m, p, o, b, st) : WorldStep<false, true, false, true>::launch(m, p, o, b, st);
     if (o.v0 && o.lcs) return o.met ? WorldStep<true, true, true>::launch(m, p, o, b, st) : WorldStep<false, true, true>::launch(m, p, o, b, st);
     if (o.v0) return o.met ? WorldStep<true, true, false>::launch(m, p, o, b, st) : WorldStep<false, true, false>::launch(m, p, o, b, st);
     return o.met ? WorldStep<true, false, false>::launch(m, p, o, b, st) : WorldStep<false, false, false>::launch(m, p, o, b, st);
 }
 cudaError_t dp_world_prepare() {
     for (auto prepare : {WorldStep<false, true, false>::prepare, WorldStep<true, true, false>::prepare, WorldStep<false, true, true>::prepare,
-                         WorldStep<true, true, true>::prepare})
+                         WorldStep<true, true, true>::prepare, WorldStep<false, true, false, true>::prepare,
+                         WorldStep<true, true, false, true>::prepare, WorldStep<false, true, true, true>::prepare,
+                         WorldStep<true, true, true, true>::prepare})
         if (const cudaError_t e = prepare(); e != cudaSuccess) return e;
     return cudaSuccess;
 }

@@ -1,9 +1,10 @@
 // csrc/dp_world_step.cuh -- the world step of the closed-loop episode runner (dp_world_kernel, see dp_world.cu), with the
-// episode metrics of include/dmpp_b200.h section 11, the reactive agents of section 12 and their lane changes (section 13) as
-// compile-time options, and its launcher WorldStep<METRICS, REACT, LANECHG>.  dp_world.cu instantiates the disarmed kernels
-// (METRICS = REACT = false), dp_world_metrics.cu the metrics instances, dp_world_agents.cu the reactive ones and
-// dp_world_lanechange.cu the lane-changing ones: kept in separate translation units, the disarmed instances compile to exactly
-// what they compiled to before the options existed.
+// episode metrics of include/dmpp_b200.h section 11, the reactive agents of section 12, their lane changes (section 13) and the
+// agents that obey the V2X events (section 15) as compile-time options, and its launcher WorldStep<METRICS, REACT, LANECHG,
+// TRAFFIC>.  dp_world.cu instantiates the disarmed kernels (METRICS = REACT = false), dp_world_metrics.cu the metrics instances,
+// dp_world_agents.cu the reactive ones, dp_world_lanechange.cu the lane-changing ones and dp_world_traffic.cu the ones that obey
+// the V2X events: kept in separate translation units, the disarmed instances compile to exactly what they compiled to before the
+// options existed.
 #pragma once
 #include <type_traits>
 
@@ -209,13 +210,127 @@ __device__ __forceinline__ void lc_relax(const dp_lane_change_params& c, double 
     }
 }
 
+// ---- the V2X events of a world at time t (include/dmpp_b200.h section 14), shared by the V2X launch and the world step ----
+__device__ __forceinline__ double v2x_time(int k, const dp_scene_hdr& h) { return (double)k * h.period_ms / 1000.0; }
+// spat_state: 6 green, 7 yellow, 3 red, 0 without a signal
+__device__ __forceinline__ int v2x_signal_state(const dp_v2x_event_spec& s, double t) {
+    int state = 0;
+    if (s.sig_road > 0) {
+        double ph = fmod(t + s.sig_offset, s.sig_cycle);
+        if (ph < 0) ph += s.sig_cycle;
+        state = ph < s.sig_green ? 6 : (ph < s.sig_green + s.sig_yellow ? 7 : 3);
+    }
+    return state;
+}
+// ped_on; (px, py) only when it is
+__device__ __forceinline__ bool v2x_pedestrian(const dp_v2x_event_spec& s, double t, double* px, double* py) {
+    const bool on = s.has_ped && s.ped_t_on <= t && t <= s.ped_t_off;
+    if (on) {
+        const double tp = t - s.ped_t_on;
+        *px = s.ped_x + s.ped_vx * tp; *py = s.ped_y + s.ped_vy * tp;
+    }
+    return on;
+}
+
+// ---- agents obey the V2X events (include/dmpp_b200.h section 15): two more leaders, standing still ----
+static_assert(sizeof(dp_v2x_traffic_params) == 24, "dp_v2x_traffic_params is 24 bytes");
+static_assert(sizeof(dp_v2x_traffic_stats) == 32, "dp_v2x_traffic_stats is 32 bytes");
+// the model of the TRAFFIC instances: the agent (and lane-change) model plus the parameters, the V2X specifications, the rows and
+// the cycle of the step.  A type of its own, so that the kernel parameters of the other instances stay what they were
+template <class Base>
+struct TrafficModel : Base {
+    dp_v2x_traffic_params tp;
+    const dp_v2x_event_spec* spec;     // [n], section 14's
+    dp_v2x_traffic_stats* ts;          // [n]
+    int cycle;
+};
+template <class M> struct IsTraffic : std::false_type {};
+template <class B> struct IsTraffic<TrafficModel<B>> : std::true_type {};
+
+// the world's events at this step (warp-uniform) and this lane's share of the row update
+struct TrafficWorld {
+    double px = 0, py = 0;             // the pedestrian (ped_on)
+    double b_commit = 0, half = 0;     // the parameters
+    int gb = 0, ge = 0;                // the governed lanes [gb, ge) (empty without a signal)
+    int sig_stop = -1;
+    bool line = false, red = false, ped_on = false, obey = false;   // line: state 7 or 3; red: state 3
+    int line_n = 0, ped_n = 0, red_n = 0, hit_n = 0;
+    double dmin = __builtin_huge_val();
+};
+struct NoTraffic {};
+
+__device__ __forceinline__ bool tw_governed(const TrafficWorld& w, int l) { return l >= w.gb && l < w.ge; }
+// S(l): the station of the stop line on governed lane l
+__device__ __forceinline__ double tw_stop(const DevMap& m, const TrafficWorld& w, int l) {
+    const int off = m.lane_pt_off[l], cnt = m.lane_pt_off[l + 1] - off;
+    const int stop = w.sig_stop < 0 || w.sig_stop > cnt - 1 ? cnt - 1 : w.sig_stop;
+    return m.cump[off + stop];
+}
+// the line ds ahead: within look, and stoppable within b_commit (the commit test); *g its gap
+__device__ __forceinline__ bool tw_line(const TrafficWorld& w, const dp_agent_model_params& p, double ds, double v, double* g) {
+    if (!(ds <= p.look)) return false;
+    const double gg = ds - p.length;
+    if (!(gg > 0 && v * v <= 2.0 * w.b_commit * gg)) return false;
+    *g = gg;
+    return true;
+}
+// the pedestrian in the frame of segment (i, i + 1) of lane l at offset u; false when the segment has no length
+__device__ __forceinline__ bool tw_ped_frame(const DevMap& m, const TrafficWorld& w, int l, int i, double u, double* lon, double* lat) {
+    const int off = m.lane_pt_off[l];
+    const double2 Q = m.xy[off + i], R = m.xy[off + i + 1];
+    const double dx = R.x - Q.x, dy = R.y - Q.y, L = sqrt(dx * dx + dy * dy);
+    if (!(L > 0)) return false;
+    const double q = u / L, Px = Q.x + q * dx, Py = Q.y + q * dy, tx = dx / L, ty = dy / L;
+    const double ex = w.px - Px, ey = w.py - Py;
+    *lon = ex * tx + ey * ty; *lat = ey * tx - ex * ty;
+    return true;
+}
+// the pedestrian as a leader candidate of an agent at (l, i, u); *g its gap
+__device__ __forceinline__ bool tw_ped(const DevMap& m, const TrafficWorld& w, const dp_agent_model_params& p, int l, int i, double u, double* g) {
+    double lon, lat;
+    if (!w.ped_on || !tw_ped_frame(m, w, l, i, u, &lon, &lat)) return false;
+    if (!(0 < lon && lon <= p.look && fabs(lat) <= w.half)) return false;
+    *g = lon - p.length;
+    return true;
+}
+// the events of world `scene` at the step of the model's cycle
+template <class Model>
+__device__ __forceinline__ void traffic_world(TrafficWorld& w, const DevMap& m, const Model& am, const dp_scene_hdr& h, int scene) {
+    const dp_v2x_event_spec& s = am.spec[scene];
+    const double t = v2x_time(am.cycle, h);
+    const int state = v2x_signal_state(s, t);
+    w.line = state == 7 || state == 3; w.red = state == 3;
+    if (s.sig_road > 0) { w.gb = m.road_lane_base[s.sig_road - 1]; w.ge = m.road_lane_base[s.sig_road]; w.sig_stop = s.sig_stop; }
+    w.ped_on = v2x_pedestrian(s, t, &w.px, &w.py);
+    w.b_commit = am.tp.b_commit; w.half = am.tp.ped_half_width; w.obey = am.tp.obey != 0;
+}
+__device__ __forceinline__ void traffic_init(dp_v2x_traffic_stats& r) {
+    r.min_ped_dist = __longlong_as_double(0x7ff0000000000000LL);
+    r.red_runs = 0; r.line_steps = 0; r.ped_steps = 0; r.ped_hits = 0; r.pad[0] = 0; r.pad[1] = 0;
+}
+// the end of a step: the warp's sums and minimum (order-free: no NaN and no -0 among the distances), lane 0 updates the row
+__device__ __forceinline__ void traffic_step(TrafficWorld& w, dp_v2x_traffic_stats* row, int lane) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) w.dmin = fmin(w.dmin, __shfl_xor_sync(DP_FULL, w.dmin, o));
+    const int red = (int)__reduce_add_sync(DP_FULL, (unsigned)w.red_n), line = (int)__reduce_add_sync(DP_FULL, (unsigned)w.line_n);
+    const int ped = (int)__reduce_add_sync(DP_FULL, (unsigned)w.ped_n), hit = (int)__reduce_add_sync(DP_FULL, (unsigned)w.hit_n);
+    if (lane == 0) {
+        dp_v2x_traffic_stats r = *row;
+        r.red_runs += red; r.line_steps += line; r.ped_steps += ped; r.ped_hits += hit;
+        if (w.dmin < r.min_ped_dist) r.min_ped_dist = w.dmin;
+        *row = r;
+    }
+}
+
 struct LcSide { bool ok; double delta, atc; int im; };
 
 // one side of agent k: target lane ml, abeam station, leader and follower on ml alone, safety and incentive.  (i, u): the agent's
-// point and offset; (v, vd, ac): its start-of-step speed, desired speed and react-phase acceleration; (le, se, ve): the ego candidate
+// point and offset; (v, vd, ac): its start-of-step speed, desired speed and react-phase acceleration; (le, se, ve): the ego candidate.
+// TrafficWorld: the line and the pedestrian on ml join the leader of at_c and of the safety test (section 15)
+template <class TW>
 __device__ __forceinline__ LcSide lc_side(const DevMap& m, const LaneChangeModel& am, double sab, const double2* SV, const int* L, int n_obs,
                                           const double* v0, int le, double se, double ve, int ml, int i, double u, double v, double vd,
-                                          double ac) {
+                                          double ac, const TW& tw) {
     const dp_agent_model_params& p = am.p;
     const dp_lane_change_params& c = am.lc;
     LcSide r;
@@ -251,8 +366,20 @@ __device__ __forceinline__ LcSide lc_side(const DevMap& m, const LaneChangeModel
             }
         }
     }
-    if (overlap || (lead && !(gl > 0)) || (foll && !(gf > 0))) return r;
-    r.atc = idm_accel(p, sab, v, vd, lead, gl, vl);
+    bool clead = lead;                                      // the leader of at_c and of the safety test
+    double cg = gl, cv = vl;
+    if constexpr (std::is_same_v<TW, TrafficWorld>) {
+        bool tl = lead, won = false;
+        double tg = gl, g;
+        if (tw.line && tw_governed(tw, ml)) {
+            const double S = tw_stop(m, tw, ml);
+            if (S > sm && tw_line(tw, p, S - sm, v, &g) && (!tl || g < tg)) { tg = g; tl = won = true; }
+        }
+        if (tw_ped(m, tw, p, ml, r.im, u, &g) && (!tl || g < tg)) { tg = g; tl = won = true; }
+        if (tw.obey && won) { clead = true; cg = tg; cv = 0.0; }
+    }
+    if (overlap || (clead && !(cg > 0)) || (foll && !(gf > 0))) return r;
+    r.atc = idm_accel(p, sab, v, vd, clead, cg, cv);
     double af = 0, atf = 0;
     if (fego) {
         af = lc_ego_idm(p, sab, vf, lead, (sl - sf) - c.ego_front, vl);
@@ -273,9 +400,10 @@ __device__ __forceinline__ LcSide lc_side(const DevMap& m, const LaneChangeModel
 
 // agent k after its react phase (acc = a_c, vn = section 12's new speed): MOBIL, then the change or the relaxation; writes the
 // agent and its lane-change state once
+template <class TW>
 __device__ __forceinline__ void lane_change_agent(const DevMap& m, const LaneChangeModel& am, double sab, const double2* SV, const int* L,
                                                   int n_obs, const double* v0, int le, double se, double ve, double dt, int k, double v,
-                                                  double vd, double acc, double vn, dp_agent* ag, dp_lane_change_state* lcs) {
+                                                  double vd, double acc, double vn, dp_agent* ag, dp_lane_change_state* lcs, const TW& tw) {
     const dp_lane_change_params& c = am.lc;
     dp_agent a = ag[k];
     dp_lane_change_state s = lcs[k];
@@ -293,11 +421,11 @@ __device__ __forceinline__ void lane_change_agent(const DevMap& m, const LaneCha
         best.ok = false;
         int side = 0;
         if (q >= 1 && (attr == 1 || attr == 3)) {
-            best = lc_side(m, am, sab, SV, L, n_obs, v0, le, se, ve, l0 - 1, a.i, a.u, v, vd, acc);
+            best = lc_side(m, am, sab, SV, L, n_obs, v0, le, se, ve, l0 - 1, a.i, a.u, v, vd, acc, tw);
             side = -1;
         }
         if (q + 1 < nl && (attr == 2 || attr == 3)) {
-            const LcSide rs = lc_side(m, am, sab, SV, L, n_obs, v0, le, se, ve, l0 + 1, a.i, a.u, v, vd, acc);
+            const LcSide rs = lc_side(m, am, sab, SV, L, n_obs, v0, le, se, ve, l0 + 1, a.i, a.u, v, vd, acc, tw);
             if (rs.ok && (!best.ok || rs.delta > best.delta)) { best = rs; side = 1; }
         }
         if (best.ok) {
@@ -323,10 +451,11 @@ __device__ __forceinline__ void lane_change_agent(const DevMap& m, const LaneCha
 
 // rewrite agents[].v of one scene from the state at the start of the step (Jacobi): stage (lane, s, v) of every agent in the
 // warp's slice of dynamic shared memory, then each lane scans the staged candidates for each of its agents (broadcast reads).
-// LANECHG: each agent's lane change (section 13) follows its IDM step on the same staging.
-template <bool LANECHG, class Model>
+// LANECHG: each agent's lane change (section 13) follows its IDM step on the same staging.  TW = TrafficWorld: the line and the
+// pedestrian join the leader choice (section 15) and the lane counts the steps they lead.
+template <bool LANECHG, class Model, class TW>
 __device__ __forceinline__ void react_step(const DevMap& m, const Model& am, const dp_scene_hdr& h, int pos, int n_obs, double dt,
-                                           dp_agent* ag, const double* v0, unsigned char* stage, int max_obs, int lane) {
+                                           dp_agent* ag, const double* v0, unsigned char* stage, int max_obs, int lane, TW& tw) {
     double2* SV = reinterpret_cast<double2*>(stage);
     int* L = reinterpret_cast<int*>(SV + max_obs);
     for (int k = lane; k < n_obs; k += 32) {
@@ -391,10 +520,29 @@ __device__ __forceinline__ void react_step(const DevMap& m, const Model& am, con
                 if (!lead || g < best) { best = g; vl = c2.y; lead = true; }
             }
         }
+        if constexpr (std::is_same_v<TW, TrafficWorld>) {
+            bool tl = lead;
+            double tb = best, g;
+            int kind = 0;                                   // 1: the line leads, 2: the pedestrian
+            if (tw.line) {
+                double ds = 0;
+                bool have = false;
+                if (tw_governed(tw, l0)) { const double S = tw_stop(m, tw, l0); if (S > sk) { ds = S - sk; have = true; } }
+                else if (l1 >= 0 && tw_governed(tw, l1)) { ds = D1 + tw_stop(m, tw, l1); have = true; }
+                else if (l2 >= 0 && tw_governed(tw, l2)) { ds = D2 + tw_stop(m, tw, l2); have = true; }
+                if (have && tw_line(tw, p, ds, v, &g) && (!tl || g < tb)) { tb = g; tl = true; kind = 1; }
+            }
+            if (tw.ped_on) {
+                const dp_agent a = ag[k];
+                if (tw_ped(m, tw, p, l0, a.i, a.u, &g) && (!tl || g < tb)) { tb = g; tl = true; kind = 2; }
+            }
+            tw.line_n += kind == 1; tw.ped_n += kind == 2;
+            if (tw.obey && kind != 0) { best = tb; vl = 0.0; lead = tl; }
+        }
         const double acc = idm_accel(p, sab, v, vd, lead, best, vl);
         double vn = v + acc * dt;
         if (vn < 0) vn = 0;
-        if constexpr (LANECHG) lane_change_agent(m, am, sab, SV, L, n_obs, v0, le, se, ve, dt, k, v, vd, acc, vn, ag, am.lcs + (v0 - am.v0));
+        if constexpr (LANECHG) lane_change_agent(m, am, sab, SV, L, n_obs, v0, le, se, ve, dt, k, v, vd, acc, vn, ag, am.lcs + (v0 - am.v0), tw);
         else ag[k].v = vn;
     }
 }
@@ -406,13 +554,19 @@ __device__ __forceinline__ void react_step(const DevMap& m, const Model& am, con
 // staging max_obs * REACT_SLOT_BYTES of dynamic shared memory per warp.
 // LANECHG = lane changes armed (am.lcs != nullptr, REACT instances only): the react phase is followed per agent by the lane
 // change of section 13 on the same staging; the placement step initialises the states.
-template <bool JUNC, bool METRICS, bool REACT, bool LANECHG = false>
+// TRAFFIC = the agents obey the V2X events (am.ts != nullptr, REACT instances only, section 15): the react and lane-change phases
+// see the line and the pedestrian, the agent loop counts red runs, pedestrian hits and distances; the placement step initialises
+// the rows.
+template <bool LANECHG, bool TRAFFIC>
+using WorldModel = std::conditional_t<TRAFFIC, TrafficModel<std::conditional_t<LANECHG, LaneChangeModel, AgentModel>>,
+                                      std::conditional_t<LANECHG, LaneChangeModel, AgentModel>>;
+template <bool JUNC, bool METRICS, bool REACT, bool LANECHG = false, bool TRAFFIC = false>
 __global__ void __launch_bounds__(WPB * 32, (METRICS || REACT) ? 8 : 0) dp_world_kernel(DevMap m, dp_params p, dp_world_params wp, int n, int max_obs,
                                                             dp_scene_hdr* __restrict__ hdr, dp_agent* __restrict__ agents,
                                                             double* __restrict__ obs_x, double* __restrict__ obs_y,
                                                             const dp_plan_record* __restrict__ rec, const double2* __restrict__ last_path,
                                                             dp_metrics_params mp, dp_episode_metrics* __restrict__ met,
-                                                            std::conditional_t<LANECHG, LaneChangeModel, AgentModel> am) {
+                                                            WorldModel<LANECHG, TRAFFIC> am) {
     __shared__ __align__(16) uint32_t sh[WPB][METRICS ? 32 + 2 * MET_WORDS : 32];
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     const int scene = blockIdx.x * WPB + wib;
@@ -439,6 +593,10 @@ __global__ void __launch_bounds__(WPB * 32, (METRICS || REACT) ? 8 : 0) dp_world
                 am.lcs[e] = s;
             }
         }
+    }
+    if constexpr (TRAFFIC) {
+        static_assert(REACT, "the V2X events act on the react phase");
+        if (rec == nullptr && lane == 0) traffic_init(am.ts[scene]);   // placement step: a clean row, whatever the header names
     }
     // a header that does not name a lane of the map (device-pointer callers are not validated on the host) leaves its world untouched
     if (h.road_num < 1 || h.road_num > m.n_roads || h.lane_num < 1 ||
@@ -511,11 +669,16 @@ __global__ void __launch_bounds__(WPB * 32, (METRICS || REACT) ? 8 : 0) dp_world
             ml.c = c; ml.s = sn;
         }
     }
+    // the V2X events of this step; an empty object in the other instances
+    std::conditional_t<TRAFFIC, TrafficWorld, NoTraffic> tw;
+    if constexpr (TRAFFIC) {
+        if (step) traffic_world(tw, m, am, h, scene);
+    }
     if constexpr (REACT) {
         if (step) {
             extern __shared__ __align__(16) unsigned char react_stage[];
             react_step<LANECHG>(m, am, h, pos, n_obs, dt, agents + (size_t)scene * max_obs, am.v0 + (size_t)scene * max_obs,
-                                react_stage + wib * react_stage_bytes(max_obs), max_obs, lane);
+                                react_stage + wib * react_stage_bytes(max_obs), max_obs, lane, tw);
         }
     }
     // ---- agents: constant speed along their lanes (junctions on: and on into the lane's successor), then their obstacle points ----
@@ -523,6 +686,12 @@ __global__ void __launch_bounds__(WPB * 32, (METRICS || REACT) ? 8 : 0) dp_world
         dp_agent a = agents[(size_t)scene * max_obs + k];
         int off = m.lane_pt_off[a.lane], cntk = m.lane_pt_off[a.lane + 1] - off;
         double ddx, ddy;
+        std::conditional_t<TRAFFIC, int, NoTraffic> l_s;     // (TRAFFIC) the lane and station the motion starts from
+        std::conditional_t<TRAFFIC, double, NoTraffic> s_s;
+        if constexpr (TRAFFIC) {
+            l_s = a.lane; s_s = 0;
+            if (step && tw.red && tw_governed(tw, l_s)) s_s = m.cump[off + a.i] + a.u;
+        }
         if (step) {
             double u = a.u + a.v * dt;
             int i = a.i;
@@ -557,6 +726,22 @@ __global__ void __launch_bounds__(WPB * 32, (METRICS || REACT) ? 8 : 0) dp_world
         }
         obs_x[(size_t)scene * max_obs + k] = ox;
         obs_y[(size_t)scene * max_obs + k] = oy;
+        if constexpr (TRAFFIC) {
+            if (step) {                                     // red run, pedestrian hit and distance of this agent's step
+                if (tw.red && tw_governed(tw, l_s)) {
+                    const double S = tw_stop(m, tw, l_s);
+                    if (s_s < S && (a.lane != l_s || m.cump[off + a.i] + a.u >= S)) tw.red_n += 1;
+                }
+                if (tw.ped_on) {
+                    double lon, lat;
+                    if (tw_ped_frame(m, tw, a.lane, a.i, a.u, &lon, &lat) && 0 <= lon && lon <= am.p.length &&
+                        fabs(lat) <= p.vehicle_width / 2.0)
+                        tw.hit_n += 1;
+                    const double dx = ox - tw.px, dy = oy - tw.py, d = sqrt(dx * dx + dy * dy);
+                    if (d < tw.dmin) tw.dmin = d;
+                }
+            }
+        }
         if constexpr (METRICS) {
             if (step) {                                     // the agent in the ego frame: box, clearance, lead gap and ttc
                 const double dx = ox - x, dy = oy - y;
@@ -583,6 +768,9 @@ __global__ void __launch_bounds__(WPB * 32, (METRICS || REACT) ? 8 : 0) dp_world
     }
     if constexpr (METRICS) {
         if (step) metrics_step(ml, reinterpret_cast<double*>(&sh[wib][32]), met + scene, lane, mp, rec[scene], h.velocity, vn, dt);
+    }
+    if constexpr (TRAFFIC) {
+        if (step) traffic_step(tw, am.ts + scene, lane);
     }
     // ---- localisation: nearest point per lane inside a window around the previous index (pos 2: the departure road from its
     // start), nearest lane ----
@@ -654,26 +842,29 @@ __global__ void __launch_bounds__(WPB * 32, (METRICS || REACT) ? 8 : 0) dp_world
 
 // the launches of one instance set, both JUNC instances: each set is instantiated in its own translation unit (the extern
 // declarations below name it), and dp_launch_world (dp_world.cu) picks the set from the armed options
-template <bool METRICS, bool REACT, bool LANECHG>
+template <bool METRICS, bool REACT, bool LANECHG, bool TRAFFIC = false>
 struct WorldStep {
     static cudaError_t launch(const DevMap& m, const dp_params& p, const DpWorldOpts& o, const DpWorldBufs& b, cudaStream_t st);
     static cudaError_t prepare();              // REACT: allow the dynamic shared memory of DP_AGENT_MODEL_MAX_OBS agent slots
-    static auto kernel(bool junc) { return junc ? dp_world_kernel<true, METRICS, REACT, LANECHG> : dp_world_kernel<false, METRICS, REACT, LANECHG>; }
+    static auto kernel(bool junc) {
+        return junc ? dp_world_kernel<true, METRICS, REACT, LANECHG, TRAFFIC> : dp_world_kernel<false, METRICS, REACT, LANECHG, TRAFFIC>;
+    }
 };
 // (defined outside the class: not inline, so the extern declarations below keep the other translation units from instantiating them)
-template <bool METRICS, bool REACT, bool LANECHG>
-cudaError_t WorldStep<METRICS, REACT, LANECHG>::launch(const DevMap& m, const dp_params& p, const DpWorldOpts& o, const DpWorldBufs& b,
-                                                       cudaStream_t st) {
-    std::conditional_t<LANECHG, LaneChangeModel, AgentModel> am;
+template <bool METRICS, bool REACT, bool LANECHG, bool TRAFFIC>
+cudaError_t WorldStep<METRICS, REACT, LANECHG, TRAFFIC>::launch(const DevMap& m, const dp_params& p, const DpWorldOpts& o, const DpWorldBufs& b,
+                                                                cudaStream_t st) {
+    WorldModel<LANECHG, TRAFFIC> am;
     am.p = o.amp; am.v0 = o.v0;
     if constexpr (LANECHG) { am.lc = o.lcp; am.lcs = o.lcs; }
+    if constexpr (TRAFFIC) { am.tp = o.tp; am.spec = o.spec; am.ts = o.ts; am.cycle = b.cycle; }
     const size_t smem = REACT ? WPB * react_stage_bytes(b.max_obs) : 0;
     kernel(o.wp.pre_junction_pts > 0)<<<(b.n + WPB - 1) / WPB, WPB * 32, smem, st>>>(
         m, p, o.wp, b.n, b.max_obs, b.hdr, b.agents, b.ox, b.oy, b.rec, b.last_path, o.mp, o.met, am);
     return cudaGetLastError();
 }
-template <bool METRICS, bool REACT, bool LANECHG>
-cudaError_t WorldStep<METRICS, REACT, LANECHG>::prepare() {
+template <bool METRICS, bool REACT, bool LANECHG, bool TRAFFIC>
+cudaError_t WorldStep<METRICS, REACT, LANECHG, TRAFFIC>::prepare() {
     const int bytes = (int)(WPB * react_stage_bytes(DP_AGENT_MODEL_MAX_OBS));
     for (const bool junc : {false, true}) {
         const cudaError_t e = cudaFuncSetAttribute(kernel(junc), cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
@@ -687,3 +878,7 @@ extern template struct WorldStep<false, true, false>;    // dp_world_agents.cu
 extern template struct WorldStep<true, true, false>;
 extern template struct WorldStep<false, true, true>;     // dp_world_lanechange.cu
 extern template struct WorldStep<true, true, true>;
+extern template struct WorldStep<false, true, false, true>;   // dp_world_traffic.cu
+extern template struct WorldStep<true, true, false, true>;
+extern template struct WorldStep<false, true, true, true>;
+extern template struct WorldStep<true, true, true, true>;

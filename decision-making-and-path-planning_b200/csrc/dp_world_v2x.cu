@@ -22,15 +22,10 @@ struct V2xWpGlobal {
 // (scalar work on broadcast loads), so the handlers need no shuffle of the inputs.
 struct V2xWorld { dp_v2x_data v; double d; int state; bool on, ped_on; };
 __device__ __forceinline__ V2xWorld v2x_world_data(const DevMap& m, const dp_params& p, const dp_v2x_event_spec& s, const dp_scene_hdr& h, int k) {
-    const double t = (double)k * h.period_ms / 1000.0;
+    const double t = v2x_time(k, h);
     V2xWorld w;
     dp_v2x_data& v = w.v;
-    w.state = 0;
-    if (s.sig_road > 0) {
-        double ph = fmod(t + s.sig_offset, s.sig_cycle);
-        if (ph < 0) ph += s.sig_cycle;
-        w.state = ph < s.sig_green ? 6 : (ph < s.sig_green + s.sig_yellow ? 7 : 3);
-    }
+    w.state = v2x_signal_state(s, t);
     w.on = s.sig_road > 0 && h.road_num == s.sig_road && h.pos != 2;
     w.d = 0;
     if (w.on) {
@@ -44,11 +39,10 @@ __device__ __forceinline__ V2xWorld v2x_world_data(const DevMap& m, const dp_par
     }
     v.spat_state = w.state;
     v.spat_lane_occupied = (w.on && w.d >= 0 && w.d <= s.sig_range) ? 1 : 0;
-    w.ped_on = s.has_ped && s.ped_t_on <= t && t <= s.ped_t_off;
+    double px, py;
+    w.ped_on = v2x_pedestrian(s, t, &px, &py);
     v.ped_distance = 0; v.ped_lat = 0; v.ped_lng = 0;
     if (w.ped_on) {
-        const double tp = t - s.ped_t_on;
-        const double px = s.ped_x + s.ped_vx * tp, py = s.ped_y + s.ped_vy * tp;
         const double dx = px - h.x, dy = py - h.y;
         v.ped_distance = sqrt(dx * dx + dy * dy);
         v.ped_lat = fma(py, p.k_lat, p.lat0); v.ped_lng = fma(px, p.k_lng, p.lng0);

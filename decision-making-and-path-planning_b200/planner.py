@@ -28,6 +28,7 @@ SYMBOLS = [
     "dp_run_closed_loop_dev", "dp_closed_loop_is_graph", "dp_v2x_event_batch", "dp_v2x_event_batch_dev", "dp_v2x_apply", "dp_v2x_apply_dev",
     "dp_metrics_default_params", "dp_world_set_metrics", "dp_agent_model_default_params", "dp_world_set_agent_model",
     "dp_lane_change_default_params", "dp_world_set_lane_change", "dp_world_set_v2x", "dp_v2x_world_dev",
+    "dp_v2x_traffic_default_params", "dp_world_set_v2x_traffic",
     "dp_gather_create", "dp_gather_attach", "dp_gather_arm", "dp_gather_chain", "dp_gather_arm_deferred", "dp_gather_set_lag", "dp_gather_flush", "dp_gather_disarm", "dp_gather_wait", "dp_gather_buffer", "dp_gather_destroy",
 ]
 
@@ -74,6 +75,15 @@ def lane_change_params():
     """dp_lane_change_default_params (no GPU needed)"""
     p = abi.LaneChangeParams()
     load().dp_lane_change_default_params(C.byref(p))
+    return p
+
+
+def v2x_traffic_params(**kw):
+    """dp_v2x_traffic_default_params (no GPU needed), then the keyword fields"""
+    p = abi.V2xTrafficParams()
+    load().dp_v2x_traffic_default_params(C.byref(p))
+    for k, v in kw.items():
+        setattr(p, k, v)
     return p
 
 
@@ -266,6 +276,12 @@ class Planner:
                                       C.c_void_p(d_wp_x or 0), C.c_void_p(d_wp_y or 0), C.c_int(n_wp), C.c_void_p(d_flags or 0),
                                       C.c_void_p(d_stats or 0)), "dp_world_set_v2x")
 
+    def set_v2x_traffic(self, params, d_stats):
+        """let the agents obey the V2X events (include/dmpp_b200.h section 15; the agent model and the V2X events must be armed):
+        d_stats = device address of dp_v2x_traffic_stats [n] indexed like hdr, initialised by the placement step; None / 0 disarms"""
+        _ck(self.lib.dp_world_set_v2x_traffic(self.ctx, C.byref(params) if params is not None else None, C.c_void_p(d_stats or 0)),
+            "dp_world_set_v2x_traffic")
+
     def v2x_world_dev(self, n, d_hdr, d_rec, cycle, first=0, stream=0):
         """one V2X launch of cycle `cycle` between cycle_dev and world_step_dev; d_rec None: the tally after the last step"""
         _ck(self.lib.dp_v2x_world_dev(self.ctx, C.c_int(first), C.c_int(n), C.c_void_p(d_hdr), C.c_void_p(d_rec or 0), C.c_int(cycle),
@@ -285,7 +301,8 @@ class Planner:
     def closed_loop_is_graph(self):
         return bool(self.lib.dp_closed_loop_is_graph(self.ctx))
 
-    def run_closed_loop(self, hdr, agents, cycles, log=True, repeat=1, metrics=None, agent_model=None, lane_change=None, v2x=None):
+    def run_closed_loop(self, hdr, agents, cycles, log=True, repeat=1, metrics=None, agent_model=None, lane_change=None, v2x=None,
+                        traffic=None):
         """host arrays in, host arrays out (the same dictionary as oracle.binding's run_closed_loop); `repeat` > 1 replays the
         episode from the same initial world (same device buffers, i.e. the cached graph) and returns the last run.
         metrics: None, or MetricsParams: the episode metrics are armed for this call (and disarmed after it) and the rows are
@@ -293,9 +310,12 @@ class Planner:
         reactive agents are armed for this call (and disarmed after it).  lane_change: None, or LaneChangeParams (needs
         agent_model): the agents also change lanes for this call, and their final states are returned under "lane_change_state".
         v2x: None, or (V2xWorldParams, events) with events.spec[n] / wp_x / wp_y (scenes.V2xEvents): the V2X events are armed for
-        this call, the rows are returned under "v2x_stats" and the flags of the last launch under "v2x_flags"."""
+        this call, the rows are returned under "v2x_stats" and the flags of the last launch under "v2x_flags".  traffic: None, or
+        V2xTrafficParams (needs agent_model and v2x): the agents obey the V2X events for this call, and their rows are returned
+        under "v2x_traffic"."""
         n, mo = agents.shape
         assert lane_change is None or agent_model is not None, "lane changes run on the reactive agents"
+        assert traffic is None or (agent_model is not None and v2x is not None), "the agents obey the V2X events on the reactive agents"
         assert mo == self.max_obs and hdr.shape == (n,)
         sizes = {"hdr": n * 128, "agents": n * mo * 32, "ox": n * mo * 8, "oy": n * mo * 8, "rec": cycles * n * 128,
                  "hdr_log": cycles * n * 128, "obs_log_x": cycles * n * mo * 8, "obs_log_y": cycles * n * mo * 8}
@@ -314,6 +334,8 @@ class Planner:
             assert spec.dtype == abi.v2x_event_spec and spec.shape == (n,) and wx.shape == wy.shape
             sizes.update(v2x_spec=n * spec.itemsize, v2x_wp_x=max(wx.nbytes, 8), v2x_wp_y=max(wy.nbytes, 8),
                          v2x_flags=n * abi.v2x_flags.itemsize, v2x_stats=n * abi.v2x_episode_stats.itemsize)
+        if traffic is not None:
+            sizes["v2x_traffic"] = n * abi.v2x_traffic_stats.itemsize
         d = {}
         try:
             for k, b in sizes.items():
@@ -333,6 +355,8 @@ class Planner:
                     _ck(self.lib.dp_memcpy_h2d(self.ctx, C.c_void_p(d[k]), abi.ptr(a), C.c_size_t(a.nbytes), None), "h2d")
                 _ck(self.lib.dp_stream_sync(self.ctx, None), "sync")
                 self.set_v2x_world(vp, n, d["v2x_spec"], d["v2x_wp_x"], d["v2x_wp_y"], wx.size, d["v2x_flags"], d["v2x_stats"])
+            if traffic is not None:
+                self.set_v2x_traffic(traffic, d["v2x_traffic"])
             h0, a0 = np.ascontiguousarray(hdr), np.ascontiguousarray(agents)
             for _ in range(repeat):
                 self.reset(0, n)
@@ -352,6 +376,8 @@ class Planner:
                 o["lane_change_state"] = np.zeros((n, mo), abi.lane_change_state)
             if v2x is not None:
                 o["v2x_flags"], o["v2x_stats"] = np.zeros(n, abi.v2x_flags), np.zeros(n, abi.v2x_episode_stats)
+            if traffic is not None:
+                o["v2x_traffic"] = np.zeros(n, abi.v2x_traffic_stats)
             for k in o:
                 _ck(self.lib.dp_memcpy_d2h(self.ctx, abi.ptr(o[k]), C.c_void_p(d[k]), C.c_size_t(sizes[k]), None), "d2h")
             _ck(self.lib.dp_stream_sync(self.ctx, None), "sync")
@@ -359,6 +385,8 @@ class Planner:
             o["graph"] = self.closed_loop_is_graph()
             return o
         finally:
+            if traffic is not None:
+                self.set_v2x_traffic(None, None)
             if v2x is not None:
                 self.set_v2x_world(None, 0, None)
             if metrics is not None:

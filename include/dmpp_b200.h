@@ -677,8 +677,8 @@ int dp_world_set_lane_change(dp_ctx* ctx, const dp_lane_change_params* p, dp_lan
  * apply = 1, lets the flags act on the cycle's record with the rule of dp_v2x_apply, so the world step of section 9 moves the
  * ego with the adjusted speed command.  Armed, an episode is: placement, then per cycle Decision + Planning -> V2X -> world
  * step, then one tally-only V2X launch (1 + cycles * 4 + 1 kernels).  Disarmed (the default) the episode is that of section 9,
- * launch for launch.  The rules are frozen in tools/junction_oracle/v2x_world.h.  Out of scope: agents that obey signals or
- * yield to pedestrians, pedestrians as obstacle points, V2X in pos 1 / 2.
+ * launch for launch.  The rules are frozen in tools/junction_oracle/v2x_world.h.  Agents that stop for the signal and yield to
+ * the pedestrian are section 15.  Out of scope: pedestrians as obstacle points, V2X in pos 1 / 2.
  *
  * IEEE binary64, operations in the order written, no contraction.  World s at cycle k (k = 0 .. cycles-1 the cycle launches,
  * k = cycles the tally), with its cycle's header h (before the world step) and t = k * period_ms / 1000:
@@ -755,6 +755,65 @@ int dp_world_set_v2x(dp_ctx* ctx, const dp_v2x_world_params* params, int n, cons
  * DP_ERR_STATE when V2X is disarmed. */
 int dp_v2x_world_dev(dp_ctx* ctx, int first_scene, int n_scenes, const dp_scene_hdr* hdr, dp_plan_record* rec, int cycle,
                      void* stream);
+
+/* (15) Agents obey the V2X events (opt-in, on top of the reactive agents of section 12 and the V2X events of section 14, both of
+ * which must be armed; disarming either disarms this model, as disarming the agent model disarms lane changes).  The stop line of
+ * a red or yellow signal and the active pedestrian become two more leader candidates of section 12's IDM and of section 13's
+ * target lane, both standing still.  Disarmed (the default) nothing changes: the same launches, the same graph, the same bytes.
+ * The arithmetic is frozen in tools/junction_oracle/v2x_traffic.h.  Out of scope: the pedestrian as an obstacle point the planner
+ * sees; agents reacting to road works (the ego only creeps past them, so "stop" would be the wrong rule); V2X in pos 1 / 2; any
+ * change to how the ego moves.
+ *
+ * IEEE binary64, operations in the order written, no contraction.  World s at the world step of cycle k:
+ *   time      t = k * period_ms / 1000 with the header's period_ms, the t of that cycle's V2X launch.  dp_run_closed_loop_dev passes
+ *             k to its world steps; a caller who steps by hand gets the cycle of the context's most recent dp_v2x_world_dev call
+ *             (which section 14 already requires before every hand-stepped world step)
+ *   events    state (6 / 7 / 3, 0 without a signal), ped_on and (px, py): section 14's, from the same device functions
+ *   governed  the lanes l of road sig_road (sig_road > 0); with (off, cnt) of l, stop = sig_stop < 0 || sig_stop > cnt - 1 ?
+ *             cnt - 1 : sig_stop and S(l) = cump[off + stop]
+ * Section 12, agent k with v0[k] > 0, with its s_k, v, chain l0 / l1 / l2, D1, D2, point i and offset u:
+ *   line      state 7 or 3: the first governed lane of the chain decides -- l0: ds = S(l0) - s_k, counting only when
+ *             S(l0) > s_k; l1: ds = D1 + S(l1); l2: ds = D2 + S(l2).  A candidate when ds <= look and, with g = ds - length,
+ *             g > 0 && v * v <= 2.0 * b_commit * g (an agent that cannot stop within b_commit continues: the yellow-light
+ *             dilemma, on red too); leader speed 0
+ *   pedestrian ped_on: Q, R = points i, i + 1 of l0, dx = R.x - Q.x, dy = R.y - Q.y, L = sqrt(dx * dx + dy * dy); when L > 0:
+ *             q = u / L, Px = Q.x + q * dx, Py = Q.y + q * dy, tx = dx / L, ty = dy / L, ex = px - Px, ey = py - Py,
+ *             lon = ex * tx + ey * ty, lat = ey * tx - ex * ty; a candidate when 0 < lon <= look and fabs(lat) <=
+ *             ped_half_width, g = lon - length, leader speed 0 (the agent's own lat is ignored; on curves the segment frame is an
+ *             approximation, frozen as such)
+ *   leader    after section 12's scan, the line and then the pedestrian replace the leader with `if (!lead || g < best)`: the
+ *             smallest g, vehicles first on a tie (ego, agents by index), then the line, then the pedestrian
+ * Section 13, target lane m at (i_m, s_m): the line when m is governed, state 7 or 3 and S(m) > s_m, ds = S(m) - s_m, with the
+ *   same look, g and commit test (the agent's own v); the pedestrian in the frame of segment (i_m, i_m + 1) of m at u.  They
+ *   replace the leader of at_c as above, and the safety test reads that leader (a virtual leader with g <= 0 makes the side
+ *   unsafe: agents do not change lanes to escape a red light).  a_f and at_f keep section 13's vehicle-only leaders.
+ * obey = 0: the candidates are evaluated and counted but never used (records, world, logs, carry and the other rows are those of
+ *   the model disarmed); obey = 1: the agents act on them.
+ * Row (initialised by the placement step, whatever the header names; updated on every step with a record on a header that names
+ *   a lane, over agents k < min(n_obs, max_obs), with the agent's lane / station as the motion of section 9 starts -- after a
+ *   lane change of section 13, so a change to a neighbouring lane is no run -- and its state after the motion):
+ *   red_runs     state 3, the start lane governed with s < S(lane), and the end on another lane or at s >= S(that lane)
+ *   line_steps, ped_steps  reacting agents whose section 12 leader (obey = 0: would-be leader) was the line / the pedestrian
+ *   ped_hits     ped_on and, in the end segment's frame as above (L > 0, (px, py) of the start of the step),
+ *                0 <= lon <= length and fabs(lat) <= vehicle_width / 2 (dp_params)
+ *   min_ped_dist ped_on: min over steps and agents of sqrt(dx * dx + dy * dy), (dx, dy) = the agent's new obstacle point - (px, py)
+ *                (+inf) */
+typedef struct dp_v2x_traffic_params {
+    double b_commit;                   /* m/s^2, default 4.0 (= dp_lane_change_params.b_safe): the hardest stop an agent commits to */
+    double ped_half_width;             /* m, default 2.0 (this library's choice): the band around the lane centre an agent yields in */
+    int32_t obey;                      /* 1 (default): the agents act on the candidates; 0: evaluated and counted only */
+    int32_t pad;                       /* zero */
+} dp_v2x_traffic_params;               /* 24 bytes */
+typedef struct dp_v2x_traffic_stats {
+    double min_ped_dist;
+    int32_t red_runs, line_steps, ped_steps, ped_hits;
+    int32_t pad[2];                    /* zero */
+} dp_v2x_traffic_stats;                /* 32 bytes, [n] indexed like hdr */
+void dp_v2x_traffic_default_params(dp_v2x_traffic_params* p);
+/* stats == NULL disarms (p may then be NULL).  Context state like dp_world_set_lane_change: the cached episode graph is rebuilt on
+ * its next call.  DP_ERR_ARG for non-finite parameters, b_commit <= 0, ped_half_width < 0, obey other than 0 / 1, or arming while
+ * the agent model or the V2X events are disarmed.  The world step then needs at most as many scenes as the armed V2X specifications. */
+int dp_world_set_v2x_traffic(dp_ctx* ctx, const dp_v2x_traffic_params* p, dp_v2x_traffic_stats* stats);
 
 /* diagnostic: phase time stamps (globaltimer, ns) of the most recent cycle launch, one row of 32 per CTA (row b = scenes
  * [b*g, (b+1)*g) of the batch; stamp 0 = CTA start, stamp i = end of phase i of csrc/dp_group.cuh).  Only contexts created

@@ -18,7 +18,12 @@ SM clock read in the same run.
                (apply = 0: the records must equal the disarmed ones, the delta is the V2X launches alone) and applied; the V2X launch
                alone (dp_v2x_world_dev, 4096 worlds, apply = 0, on the world and records the last episode left); and the effect of
                applying the flags on seeds 0-511 (red crossings, stop cycles, worlds that stopped on a red and left on green, the
-               minimum ego-pedestrian distance while the pedestrian is active)."""
+               minimum ego-pedestrian distance while the pedestrian is active).
+  traffic      agents that obey the V2X events (section 15), with the reactive agents and the V2X events (apply = 1) armed in every
+               arm: disarmed, obey = 0 (the records must equal the disarmed ones: the delta is the candidates' cost alone) and
+               obey = 1, for the highway and junction episodes (4096 worlds) and dp_world_step_dev alone (4096 junction worlds with 10
+               agents, 1024 urban worlds with 200); and the effect of obey 0 -> 1 on seeds 0-511 (agent red runs, ego red crossings,
+               collisions and where they started, ego stopped steps; pedestrian hits and distances, ego collisions)."""
 import argparse
 import json
 import os
@@ -54,7 +59,7 @@ def cump_of():
 class Arm:
     """one planner + world of one kind, with the models asked for armed"""
 
-    def __init__(self, kind, n, n_obs, cycles, metrics=False, react=False, lanechg=False, v2x=None):
+    def __init__(self, kind, n, n_obs, cycles, metrics=False, react=False, lanechg=False, v2x=None, traffic=None):
         self.n = n
         self.p = Planner(n, n_obs); self.p.upload_map(m)
         wp = self.p.world_params(); wp.pre_junction_pts = scenes.World.PRE_JUNCTION_PTS[kind]
@@ -81,6 +86,9 @@ class Arm:
             self.d_vs = torch.zeros((n, abi.v2x_episode_stats.itemsize), dtype=torch.uint8, device=dev)
             self.p.set_v2x_world(abi.V2xWorldParams(0, v2x), n, self.d_spec.data_ptr(), self.d_wx.data_ptr(), self.d_wy.data_ptr(),
                                  self.ev.wp_x.size, self.d_vf.data_ptr(), self.d_vs.data_ptr())
+        if traffic is not None:                             # traffic = obey (0 / 1)
+            self.d_ts = torch.zeros((n, abi.v2x_traffic_stats.itemsize), dtype=torch.uint8, device=dev)
+            self.p.set_v2x_traffic(pl.v2x_traffic_params(obey=traffic), self.d_ts.data_ptr())
 
     def episode_ms(self, graph=True):
         st = torch.cuda.current_stream()
@@ -123,7 +131,7 @@ class Arm:
         return e0.elapsed_time(e1) * 1e3 / launches
 
     def close(self):
-        self.p.set_v2x_world(None, 0, None); self.p.set_lane_change(None, None); self.p.set_agent_model(None, None); self.p.set_metrics(None, None); self.p.close()
+        self.p.set_v2x_traffic(None, None); self.p.set_v2x_world(None, 0, None); self.p.set_lane_change(None, None); self.p.set_agent_model(None, None); self.p.set_metrics(None, None); self.p.close()
 
 
 def alternate(arms, *measures):
@@ -335,8 +343,69 @@ def bench_v2x():
     return out
 
 
+def traffic_effect(kind, cycles, n=512):
+    """seeds 0 .. n-1 with metrics, reactive agents and V2X (apply = 1) armed, obey 0 against 1"""
+    out, cump = {}, cump_of()
+    w = scenes.World(m, np.arange(n), 10, kind=kind)
+    ev = scenes.V2xEvents(w, np.arange(n))
+    for obey in (0, 1):
+        p = Planner(n, 10); p.upload_map(m)
+        wp = p.world_params(); wp.pre_junction_pts = scenes.World.PRE_JUNCTION_PTS[kind]; p.set_world_params(wp)
+        o = p.run_closed_loop(w.hdr, w.agents, cycles, metrics=pl.metrics_params(), agent_model=(pl.agent_model_params(), w.v0),
+                              v2x=(abi.V2xWorldParams(0, 1), ev), traffic=pl.v2x_traffic_params(obey=obey))
+        p.close()
+        ts, vs, met = o["v2x_traffic"], o["v2x_stats"], o["metrics"]
+        r = {"line_steps": int(ts["line_steps"].sum()), "ped_steps": int(ts["ped_steps"].sum())}
+        if kind == "junction":
+            r.update(agent_red_runs=int(ts["red_runs"].sum()), worlds_with_agent_red_run=int((ts["red_runs"] > 0).sum()),
+                     ego_red_crossings=int(vs["red_crossings"].sum()), ego_stopped_steps=int(met["stopped_steps"].sum()),
+                     first_strikes=first_strikes(w, met, cump))
+        else:
+            ped = ev.spec["has_ped"] == 1
+            d = ts["min_ped_dist"][ped]
+            r.update(ped_hits=int(ts["ped_hits"].sum()), worlds_with_ped_hit=int((ts["ped_hits"] > 0).sum()), worlds_with_pedestrian=int(d.size),
+                     min_ped_dist_median=float(np.median(d)), worlds_min_ped_dist_below_2m=int((d < 2.0).sum()),
+                     ego_collision_worlds=int((met["first_collision_step"] > 0).sum()), ego_collision_steps=int(met["collision_steps"].sum()))
+        out["obey_%d" % obey] = r
+    return out
+
+
+def bench_traffic():
+    out = {"card": card(), "episode": {}, "world_step": {}, "effect": {}}
+    for kind, cycles in (("highway", 25), ("junction", 120)):
+        N = 4096
+        mk = lambda t: Arm(kind, N, 10, cycles, react=True, v2x=1, traffic=t)   # noqa: E731
+        arms = {"off": mk(None), "obey0": mk(0), "obey1": mk(1)}
+        warm(arms)
+        ep, = alternate(arms, Arm.episode_ms)
+        same = arms["off"].d_r.cpu().numpy().tobytes() == arms["obey0"].d_r.cpu().numpy().tobytes()
+        assert same, kind + ": obey = 0 records differ from the disarmed ones"
+        out["episode"]["%s_%dx%d" % (kind, N, cycles)] = {
+            "cycles": cycles, "ms_off": summary(ep["off"]), "ms_obey0": summary(ep["obey0"]), "ms_obey1": summary(ep["obey1"]),
+            "obey0_over_off": ratio(ep["obey0"], ep["off"]), "obey1_over_off": ratio(ep["obey1"], ep["off"]),
+            "records_identical_off_obey0": same}
+        close(arms)
+    for kind, N, n_obs in (("junction", 4096, 10), ("urban", 1024, 200)):
+        mk = lambda t: Arm(kind, N, n_obs, 2, react=True, v2x=1, traffic=t)    # noqa: E731
+        arms = {"off": mk(None), "obey0": mk(0), "obey1": mk(1)}
+        for a in arms.values():                             # (from 32 agents up the cycle runs on the group kernel: no graph)
+            a.episode_ms(graph=n_obs < 32)
+        h, a_, rec, s = arms["off"].state()
+        for a in arms.values():                             # the V2X launch that sets the hand-stepped cycle (section 15's t)
+            a.p.v2x_world_dev(N, h.data_ptr(), rec.data_ptr(), 40)
+            a.step_us(h, a_, rec, s)
+        st, = alternate(arms, lambda x: x.step_us(h, a_, rec, s))
+        out["world_step"]["%s_%dx%d" % (kind, N, n_obs)] = {
+            "us_off": summary(st["off"]), "us_obey0": summary(st["obey0"]), "us_obey1": summary(st["obey1"]),
+            "obey0_over_off": ratio(st["obey0"], st["off"]), "obey1_over_off": ratio(st["obey1"], st["off"]), "launches_per_window": 50}
+        close(arms)
+    for kind, cycles in (("junction", 120), ("highway", 25)):
+        out["effect"]["%s_512x%d" % (kind, cycles)] = traffic_effect(kind, cycles)
+    return out
+
+
 if __name__ == "__main__":
-    benches = {"metrics": bench_metrics, "agents": bench_agents, "lane_change": bench_lane_change, "v2x": bench_v2x}
+    benches = {"metrics": bench_metrics, "agents": bench_agents, "lane_change": bench_lane_change, "v2x": bench_v2x, "traffic": bench_traffic}
     ap = argparse.ArgumentParser(description=__doc__.split("\n")[0])
     ap.add_argument("model", choices=list(benches))
     print(json.dumps(benches[ap.parse_args().model]()))

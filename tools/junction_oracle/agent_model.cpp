@@ -30,7 +30,7 @@ int ego_lane(const junction::JMap& jm, const dp_world_params& wp, const dp_scene
 }
 
 void react(const junction::JMap& jm, const dp_world_params& wp, const dp_agent_model_params& mp, const dp_scene_hdr& h0, dp_agent* ag,
-           int n, const double* v0, double* acc_out) {
+           int n, const double* v0, double* acc_out, const traffic::World* tw, int* kind_out) {
     const oracle::MapView& m = jm.m;
     if (!metrics::header_valid(m, h0)) return;
     const double inf = std::numeric_limits<double>::infinity();
@@ -46,6 +46,8 @@ void react(const junction::JMap& jm, const dp_world_params& wp, const dp_agent_m
     double se = 0;
     const int le = ego_lane(jm, wp, h0, &se);
     const double ve = h0.velocity / 3.6;
+    if (kind_out)
+        for (int k = 0; k < n; ++k) kind_out[k] = 0;
     for (int k = 0; k < n; ++k) {
         const double vd = v0[k];
         if (!(vd > 0)) continue;
@@ -72,6 +74,13 @@ void react(const junction::JMap& jm, const dp_world_params& wp, const dp_agent_m
                 const double g = ds - mp.length;
                 if (!lead || g < best) { best = g; vl = V[j]; lead = true; }
             }
+        }
+        if (tw) {                                           // section 15: the line and the pedestrian, standing still
+            bool tl = lead;
+            double tb = best;
+            const int kind = traffic::leader(jm, *tw, mp, l0, l1, l2, D1, D2, sk, v, ag[k].i, ag[k].u, &tl, &tb);
+            if (kind_out) kind_out[k] = kind;
+            if (tw->tp.obey && kind != 0) { best = tb; vl = 0.0; lead = tl; }
         }
         // IDM, delta = 4
         const double r = v / vd;

@@ -51,14 +51,16 @@ class JunctionOracle:
                                       abi.ptr(ox), abi.ptr(oy), abi.ptr(rec), abi.ptr(last_path)) == 0
 
     def run_closed_loop(self, hdr, agents, cycles, wp=None, paths=False, threads=1, metrics=None, agent_model=None, lane_change=None,
-                        v2x=None):
+                        v2x=None, traffic=None):
         """hdr[n], agents[n][max_obs] (copied; the final world is returned), through jo_run_closed_loop; metrics = MetricsParams: the
         episode metrics of every world under "metrics"; agent_model = (AgentModelParams, v0[n][max_obs]): the reactive agents;
         lane_change = LaneChangeParams (with agent_model): their lane changes, the final states under "lane_change_state";
         v2x = (V2xWorldParams, events with spec / wp_x / wp_y): the V2X events, the rows under "v2x_stats" and the flags of the last
-        launch under "v2x_flags"
+        launch under "v2x_flags"; traffic = V2xTrafficParams (with agent_model and v2x): the agents obey the V2X events, the rows
+        under "v2x_traffic"
         """
         assert lane_change is None or agent_model is not None
+        assert traffic is None or (agent_model is not None and v2x is not None)
         am, v0 = agent_model if agent_model is not None else (None, None)
         met = lcs = None
         if metrics is not None:
@@ -82,6 +84,10 @@ class JunctionOracle:
             models += (C.byref(vp), abi.ptr(spec), abi.ptr(wx), abi.ptr(wy), C.c_int(wx.size), abi.ptr(vflags), abi.ptr(vstats))
         else:
             models += (None,) * 4 + (C.c_int(0), None, None)
+        tstats = None
+        if traffic is not None:
+            tstats = np.frombuffer(np.full(hdr.shape[0] * abi.v2x_traffic_stats.itemsize, 0xAB, np.uint8).tobytes(), abi.v2x_traffic_stats).copy()
+        models += (ref(traffic), abi.ptr(tstats))
         f = self.lib.jo_run_closed_loop
         f.restype = C.c_longlong
         # ob._closed_loop passes the arrays every closed loop has; the model arguments follow them
@@ -93,7 +99,48 @@ class JunctionOracle:
             o["lane_change_state"] = lcs
         if vstats is not None:
             o["v2x_flags"], o["v2x_stats"] = vflags, vstats
+        if tstats is not None:
+            o["v2x_traffic"] = tstats
         return o
+
+    def traffic_step(self, tp, ev, k, hdr, agents, ox, oy, v0, am, ts, rec=None, last_path=None, lp=None, lcs=None, wp=None):
+        """one world step of cycle k with the agents obeying the V2X events (jo_traffic_step), everything in place; rec None: the
+        placement step (the rows initialised); returns the leader kinds [n][max_obs]"""
+        wp = wp or self.world_params()
+        n, max_obs = agents.shape
+        spec = np.ascontiguousarray(ev.spec)
+        v0 = np.ascontiguousarray(v0, np.float64)
+        assert spec.shape == (n,) and v0.shape == agents.shape and ts.dtype == abi.v2x_traffic_stats and ts.shape == (n,)
+        assert (lp is None) == (lcs is None) and agents.flags["C_CONTIGUOUS"] and hdr.flags["C_CONTIGUOUS"]
+        kinds = np.zeros((n, max_obs), np.int32)
+        assert self.lib.jo_traffic_step(C.byref(self.params), C.byref(wp), C.byref(am), None if lp is None else C.byref(lp), C.byref(tp),
+                                        C.c_int(n), C.c_int(max_obs), abi.ptr(spec), C.c_int(k), abi.ptr(hdr), abi.ptr(agents), abi.ptr(ox),
+                                        abi.ptr(oy), abi.ptr(v0), abi.ptr(lcs), abi.ptr(rec), abi.ptr(last_path), abi.ptr(ts),
+                                        abi.ptr(kinds)) == 0
+        return kinds
+
+    def traffic_leader(self, tp, am, spec, hdr, k, lanes, x, iv):
+        """section 15's candidates after a vehicle scan (jo_traffic_leader): lanes[n][3] = (l0, l1, l2), x[n][6] = (D1, D2, sk, v, u,
+        best), iv[n][2] = (i, lead) -> [n][3] = (best, lead, kind)"""
+        n = len(spec)
+        out = np.zeros((n, 3))
+        args = [np.ascontiguousarray(a, t) for a, t in ((spec, abi.v2x_event_spec), (hdr, abi.scene_hdr), (k, np.int32), (lanes, np.int32),
+                                                        (x, np.float64), (iv, np.int32))]
+        assert self.lib.jo_traffic_leader(C.byref(tp), C.byref(am), C.c_int(n), *[abi.ptr(a) for a in args], abi.ptr(out)) == 0
+        return out
+
+    def traffic_side(self, tp, am, spec, hdr, k, lanes, x, lead):
+        """... on a target lane (jo_traffic_side): lanes[n][2] = (m, i_m), x[n][4] = (s_m, u, v, g), lead[n] -> [n][3] = (g, lead, won)"""
+        n = len(spec)
+        out = np.zeros((n, 3))
+        args = [np.ascontiguousarray(a, t) for a, t in ((spec, abi.v2x_event_spec), (hdr, abi.scene_hdr), (k, np.int32), (lanes, np.int32),
+                                                        (x, np.float64), (lead, np.int32))]
+        assert self.lib.jo_traffic_side(C.byref(tp), C.byref(am), C.c_int(n), *[abi.ptr(a) for a in args], abi.ptr(out)) == 0
+        return out
+
+    def traffic_sizeof(self):
+        """sizeof(dp_v2x_traffic_params), sizeof(dp_v2x_traffic_stats)"""
+        return int(self.lib.jo_traffic_sizeof(0)), int(self.lib.jo_traffic_sizeof(1))
 
     @staticmethod
     def _v2x_inputs(ev):

@@ -3,7 +3,8 @@
 // same arrays as oracle_world_step / oracle_run_closed_loop of oracle/oracle_api.cpp; in jo_run_closed_loop, the models each
 // world step may carry: the episode metrics of episode_metrics.cpp (alone: jo_metrics_step), the reactive agents of
 // agent_model.cpp (alone: jo_react_step) and their lane changes of lane_change.cpp (alone: jo_lane_change_step); and the V2X launch
-// of v2x_world.cpp between a cycle and its world step (alone: jo_v2x_cycle, its data builder: jo_v2x_data).
+// of v2x_world.cpp between a cycle and its world step (alone: jo_v2x_cycle, its data builder: jo_v2x_data); and the agents that
+// obey the V2X events of v2x_traffic.cpp (alone: jo_traffic_step, its candidates: jo_traffic_leader / jo_traffic_side).
 #include <algorithm>
 #include <atomic>
 #include <cstring>
@@ -12,12 +13,20 @@
 #include "agent_model.h"
 #include "episode_metrics.h"
 #include "lane_change.h"
+#include "v2x_traffic.h"
 #include "v2x_world.h"
 #include "world_junction.h"
 #include "../../oracle/cshare_spec.h"
 
 namespace {
 junction::JMap g_map; bool g_have_map = false;
+// section 15's row update of one world after its motion, with the step's leader kinds
+void traffic_update(const dp_params& p, const dp_agent_model_params& am, const traffic::World& tw, dp_v2x_traffic_stats& r, const dp_agent* a1,
+                    const dp_agent* a2, const double* ox, const double* oy, int n, const int* kinds) {
+    int line_n = 0, ped_n = 0;
+    for (int k = 0; k < n; ++k) { line_n += kinds[k] == 1; ped_n += kinds[k] == 2; }
+    traffic::update(g_map, tw, am, p.vehicle_width, r, a1, a2, ox, oy, n, line_n, ped_n);
+}
 // the warning list through GlobalToWGS84, as the handlers read it
 void wp_gps(const dp_params& p, const double* wp_x, const double* wp_y, int n_wp, std::vector<double>& la, std::vector<double>& lo) {
     la.resize((size_t)n_wp); lo.resize((size_t)n_wp);
@@ -50,16 +59,18 @@ int jo_world_step(const dp_params* p, const dp_world_params* wp, int n, int max_
 // armed by a non-null pair, or off with both NULL: mp / met[n] the episode metrics of include/dmpp_b200.h section 11, accumulated
 // after every world step; am / v0[n][max_obs] the reactive agents of section 12, before every world step; lp / lcs[n][max_obs]
 // (with am) their lane changes of section 13, states initialised by the placement step and holding the final states; vp / spec[n]
-// (wp_x / wp_y[n_wp], flags[n] nullable, stats[n]) the V2X events of section 14 between every cycle and its world step
+// (wp_x / wp_y[n_wp], flags[n] nullable, stats[n]) the V2X events of section 14 between every cycle and its world step; tp / ts[n]
+// (with am and vp) the agents that obey them, section 15
 long long jo_run_closed_loop(const dp_params* p, const dp_world_params* wp, int n, int cycles, int max_obs, dp_scene_hdr* hdr,
                              dp_agent* agents, double* ox, double* oy, dp_plan_record* rec, dp_scene_hdr* hdr_log, double* obs_log_x,
                              double* obs_log_y, double* path_xy, dp_carry* carry_out, double* last_path_out, int threads,
                              int32_t* ub_scene, const dp_metrics_params* mp, dp_episode_metrics* met, const dp_agent_model_params* am,
                              const double* v0, const dp_lane_change_params* lp, dp_lane_change_state* lcs, const dp_v2x_world_params* vp,
                              const dp_v2x_event_spec* spec, const double* wp_x, const double* wp_y, int n_wp, dp_v2x_flags* flags,
-                             dp_v2x_episode_stats* stats) {
+                             dp_v2x_episode_stats* stats, const dp_v2x_traffic_params* tp, dp_v2x_traffic_stats* ts) {
     if (!g_have_map) return -1;
     if ((!mp) != (!met) || (!am) != (!v0) || (!lp) != (!lcs) || (lcs && !v0) || (!vp) != (!spec) || (spec && !stats)) return -1;
+    if ((!tp) != (!ts) || (ts && (!v0 || !spec))) return -1;
     if (threads < 1) threads = 1;
     std::vector<double> wla, wlo;
     if (spec) wp_gps(*p, wp_x, wp_y, n_wp, wla, wlo);
@@ -75,6 +86,9 @@ long long jo_run_closed_loop(const dp_params* p, const dp_world_params* wp, int 
             junction::world_step(g_map, *p, *wp, hdr[s], ag, sx, sy, nullptr, nullptr, nullptr);
             if (met) metrics::init(met[s]);
             if (lcs) lanechg::init(ag, std::min((int)hdr[s].n_obs, max_obs), lcs + (size_t)s * max_obs);
+            if (ts) traffic::init(ts[s]);
+            std::vector<int> kinds((size_t)max_obs);
+            std::vector<dp_agent> a1((size_t)max_obs);
             for (int c = 0; c < cycles; ++c) {
                 const size_t e = (size_t)c * n + s;
                 if (hdr_log) hdr_log[e] = hdr[s];
@@ -87,10 +101,15 @@ long long jo_run_closed_loop(const dp_params* p, const dp_world_params* wp, int 
                 lub += o.ub_hits;
                 if (spec) v2x::cycle(g_map, *p, *vp, spec[s], wla.data(), wlo.data(), hdr[s], c, rec + e, stats[s], flags ? flags + s : nullptr);
                 const dp_scene_hdr h0 = hdr[s];
-                if (lcs) lanechg::step(g_map, *wp, *am, *lp, h0, ag, std::min((int)h0.n_obs, max_obs), v0 + (size_t)s * max_obs,
-                                       lcs + (size_t)s * max_obs);
-                else if (am) agents::react(g_map, *wp, *am, h0, ag, std::min((int)h0.n_obs, max_obs), v0 + (size_t)s * max_obs);
+                const int na = std::min((int)h0.n_obs, max_obs);
+                traffic::World tw;
+                if (ts) tw = traffic::world(g_map, *tp, spec[s], h0, c);
+                const traffic::World* twp = ts ? &tw : nullptr;
+                if (lcs) lanechg::step(g_map, *wp, *am, *lp, h0, ag, na, v0 + (size_t)s * max_obs, lcs + (size_t)s * max_obs, twp, kinds.data());
+                else if (am) agents::react(g_map, *wp, *am, h0, ag, na, v0 + (size_t)s * max_obs, nullptr, twp, kinds.data());
+                if (ts) std::copy(ag, ag + na, a1.begin());
                 junction::world_step(g_map, *p, *wp, hdr[s], ag, sx, sy, rec + e, st.last_x, st.last_y);
+                if (ts && metrics::header_valid(g_map.m, h0)) traffic_update(*p, *am, tw, ts[s], a1.data(), ag, sx, sy, na, kinds.data());
                 if (met) metrics::update(g_map, *wp, *mp, met[s], h0, hdr[s], ag, sx, sy, std::min((int)h0.n_obs, max_obs), rec[e]);
             }
             if (spec) v2x::cycle(g_map, *p, *vp, spec[s], wla.data(), wlo.data(), hdr[s], cycles, nullptr, stats[s], flags ? flags + s : nullptr);
@@ -189,5 +208,74 @@ void jo_gps(const dp_params* p, int n, const double* x, const double* y, double*
 }
 
 int jo_v2x_sizeof(int which) { return which ? (int)sizeof(dp_v2x_episode_stats) : (int)sizeof(dp_v2x_event_spec); }
+
+// one world step of cycle k with the agents obeying the V2X events, for every scene, in place, as the TRAFFIC kernel runs it: the
+// react phase (with lp / lcs non-null: and the lane changes), the world step, the row update; kinds[n][max_obs] (nullable) the leader
+// kinds.  rec == NULL initialises the rows and runs the placement step.  The ego walks its last_path[n][400] with rec
+int jo_traffic_step(const dp_params* p, const dp_world_params* wp, const dp_agent_model_params* am, const dp_lane_change_params* lp,
+                    const dp_v2x_traffic_params* tp, int n, int max_obs, const dp_v2x_event_spec* spec, int k, dp_scene_hdr* hdr, dp_agent* agents,
+                    double* ox, double* oy, const double* v0, dp_lane_change_state* lcs, const dp_plan_record* rec, const double* last_path,
+                    dp_v2x_traffic_stats* ts, int32_t* kinds) {
+    if (!g_have_map || (!lp) != (!lcs)) return -1;
+    std::vector<int> kd((size_t)max_obs);
+    std::vector<dp_agent> a1((size_t)max_obs);
+    for (int s = 0; s < n; ++s) {
+        dp_agent* ag = agents + (size_t)s * max_obs;
+        double* sx = ox + (size_t)s * max_obs; double* sy = oy + (size_t)s * max_obs;
+        const double* lx = last_path ? last_path + (size_t)s * 400 : nullptr;
+        if (!rec) {
+            traffic::init(ts[s]);
+            if (lcs) lanechg::init(ag, std::min((int)hdr[s].n_obs, max_obs), lcs + (size_t)s * max_obs);
+            junction::world_step(g_map, *p, *wp, hdr[s], ag, sx, sy, nullptr, nullptr, nullptr);
+            continue;
+        }
+        const dp_scene_hdr h0 = hdr[s];
+        const int na = std::min((int)h0.n_obs, max_obs);
+        const traffic::World tw = traffic::world(g_map, *tp, spec[s], h0, k);
+        std::fill(kd.begin(), kd.end(), 0);
+        if (lcs) lanechg::step(g_map, *wp, *am, *lp, h0, ag, na, v0 + (size_t)s * max_obs, lcs + (size_t)s * max_obs, &tw, kd.data());
+        else agents::react(g_map, *wp, *am, h0, ag, na, v0 + (size_t)s * max_obs, nullptr, &tw, kd.data());
+        std::copy(ag, ag + na, a1.begin());
+        junction::world_step(g_map, *p, *wp, hdr[s], ag, sx, sy, rec + s, lx, lx ? lx + 200 : nullptr);
+        if (metrics::header_valid(g_map.m, h0)) traffic_update(*p, *am, tw, ts[s], a1.data(), ag, sx, sy, na, kd.data());
+        if (kinds)
+            for (int j = 0; j < max_obs; ++j) kinds[(size_t)s * max_obs + j] = j < na ? kd[j] : 0;
+    }
+    return 0;
+}
+
+// section 15's candidates alone, for n independent agents of world s (spec[s], hdr[s] at cycle k[s]): the section 12 leader after a
+// vehicle scan, lanes[s] = (l0, l1, l2), x[s] = (D1, D2, sk, v, u, best), iv[s] = (i, lead) -> out[s] = (best, lead, kind)
+int jo_traffic_leader(const dp_v2x_traffic_params* tp, const dp_agent_model_params* am, int n, const dp_v2x_event_spec* spec,
+                      const dp_scene_hdr* hdr, const int32_t* k, const int32_t* lanes, const double* x, const int32_t* iv, double* out) {
+    if (!g_have_map) return -1;
+    for (int s = 0; s < n; ++s) {
+        const traffic::World w = traffic::world(g_map, *tp, spec[s], hdr[s], k[s]);
+        const double* a = x + 6 * s;
+        bool lead = iv[2 * s + 1] != 0;
+        double best = a[5];
+        const int kind = traffic::leader(g_map, w, *am, lanes[3 * s], lanes[3 * s + 1], lanes[3 * s + 2], a[0], a[1], a[2], a[3], iv[2 * s],
+                                         a[4], &lead, &best);
+        out[3 * s] = best; out[3 * s + 1] = lead; out[3 * s + 2] = kind;
+    }
+    return 0;
+}
+
+// ... and on a target lane: lanes[s] = (m, i_m), x[s] = (s_m, u, v, g), lead[s] -> out[s] = (g, lead, won)
+int jo_traffic_side(const dp_v2x_traffic_params* tp, const dp_agent_model_params* am, int n, const dp_v2x_event_spec* spec, const dp_scene_hdr* hdr,
+                    const int32_t* k, const int32_t* lanes, const double* x, const int32_t* lead_in, double* out) {
+    if (!g_have_map) return -1;
+    for (int s = 0; s < n; ++s) {
+        const traffic::World w = traffic::world(g_map, *tp, spec[s], hdr[s], k[s]);
+        const double* a = x + 4 * s;
+        bool lead = lead_in[s] != 0;
+        double g = a[3];
+        const bool won = traffic::side(g_map, w, *am, lanes[2 * s], lanes[2 * s + 1], a[0], a[1], a[2], &lead, &g);
+        out[3 * s] = g; out[3 * s + 1] = lead; out[3 * s + 2] = won;
+    }
+    return 0;
+}
+
+int jo_traffic_sizeof(int which) { return which ? (int)sizeof(dp_v2x_traffic_stats) : (int)sizeof(dp_v2x_traffic_params); }
 
 }  // extern "C"

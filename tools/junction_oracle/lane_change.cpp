@@ -53,7 +53,7 @@ struct Snapshot {
 };
 
 Side side(const junction::JMap& jm, const dp_agent_model_params& p, const dp_lane_change_params& c, const Snapshot& w, const double* v0,
-          int ml, int i, double u, double v, double vd, double ac) {
+          int ml, int i, double u, double v, double vd, double ac, const traffic::World* tw) {
     const oracle::MapView& m = jm.m;
     Side r;
     const int off = m.d.lane_pt_off[ml], cnt = m.lane_size(ml);
@@ -92,8 +92,15 @@ Side side(const junction::JMap& jm, const dp_agent_model_params& p, const dp_lan
             }
         }
     }
-    if (overlap || (lead && !(gl > 0)) || (foll && !(gf > 0))) return r;
-    r.atc = idm(p, v, vd, lead, gl, vl);
+    bool clead = lead;                                      // the leader of at_c and of the safety test
+    double cg = gl, cv = vl;
+    if (tw) {                                               // section 15: the line and the pedestrian on ml
+        bool tl = lead;
+        double tg = gl;
+        if (traffic::side(jm, *tw, p, ml, r.im, sm, u, v, &tl, &tg) && tw->tp.obey) { clead = true; cg = tg; cv = 0.0; }
+    }
+    if (overlap || (clead && !(cg > 0)) || (foll && !(gf > 0))) return r;
+    r.atc = idm(p, v, vd, clead, cg, cv);
     double af = 0, atf = 0;
     if (fego) {
         af = ego_idm(p, vf, lead, (sl - sf) - c.ego_front, vl);
@@ -128,7 +135,8 @@ void init(const dp_agent* ag, int n, dp_lane_change_state* st) {
 }
 
 void step(const junction::JMap& jm, const dp_world_params& wp, const dp_agent_model_params& am, const dp_lane_change_params& lp,
-          const dp_scene_hdr& h0, dp_agent* ag, int n, const double* v0, dp_lane_change_state* st) {
+          const dp_scene_hdr& h0, dp_agent* ag, int n, const double* v0, dp_lane_change_state* st, const traffic::World* tw,
+          int* kind_out) {
     const oracle::MapView& m = jm.m;
     if (!metrics::header_valid(m, h0)) return;
     const double dt = h0.period_ms / 1000.0;
@@ -142,7 +150,7 @@ void step(const junction::JMap& jm, const dp_world_params& wp, const dp_agent_mo
     w.le = agents::ego_lane(jm, wp, h0, &w.se);
     w.ve = h0.velocity / 3.6;
     std::vector<double> acc(n, 0.0);
-    agents::react(jm, wp, am, h0, ag, n, v0, acc.data());    // ag[k].v = section 12's speed; acc[k] = a_c
+    agents::react(jm, wp, am, h0, ag, n, v0, acc.data(), tw, kind_out);   // ag[k].v = section 12's speed; acc[k] = a_c
     const int road_lanes = m.d.road_lane_base[m.d.n_roads];
     for (int k = 0; k < n; ++k) {
         dp_agent& a = ag[k];
@@ -156,11 +164,11 @@ void step(const junction::JMap& jm, const dp_world_params& wp, const dp_agent_mo
             Side best;
             int dir = 0;
             if (q >= 1 && (attr == 1 || attr == 3)) {
-                best = side(jm, am, lp, w, v0, l0 - 1, a.i, a.u, w.V[k], v0[k], acc[k]);
+                best = side(jm, am, lp, w, v0, l0 - 1, a.i, a.u, w.V[k], v0[k], acc[k], tw);
                 dir = -1;
             }
             if (q + 1 < nl && (attr == 2 || attr == 3)) {
-                const Side rs = side(jm, am, lp, w, v0, l0 + 1, a.i, a.u, w.V[k], v0[k], acc[k]);
+                const Side rs = side(jm, am, lp, w, v0, l0 + 1, a.i, a.u, w.V[k], v0[k], acc[k], tw);
                 if (rs.ok && (!best.ok || rs.delta > best.delta)) { best = rs; dir = 1; }
             }
             if (best.ok) {

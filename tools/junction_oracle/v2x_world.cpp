@@ -17,17 +17,32 @@ void gps(const dp_params& p, double x, double y, double* lat, double* lng) {
 }
 }  // namespace
 
+int signal_state(const dp_v2x_event_spec& s, double t) {
+    int state = 0;
+    if (s.sig_road > 0) {
+        double ph = std::fmod(t + s.sig_offset, s.sig_cycle);
+        if (ph < 0) ph += s.sig_cycle;
+        state = ph < s.sig_green ? 6 : (ph < s.sig_green + s.sig_yellow ? 7 : 3);
+    }
+    return state;
+}
+
+bool pedestrian(const dp_v2x_event_spec& s, double t, double* px, double* py) {
+    const bool on = s.has_ped && s.ped_t_on <= t && t <= s.ped_t_off;
+    if (on) {
+        const double tp = t - s.ped_t_on;
+        *px = s.ped_x + s.ped_vx * tp; *py = s.ped_y + s.ped_vy * tp;
+    }
+    return on;
+}
+
 World build(const junction::JMap& jm, const dp_params& p, const dp_v2x_event_spec& s, const dp_scene_hdr& h, int k) {
     const oracle::MapView& m = jm.m;
     const double t = (double)k * h.period_ms / 1000.0;
     World w;
     std::memset(&w, 0, sizeof(w));
     dp_v2x_data& v = w.v;
-    if (s.sig_road > 0) {
-        double ph = std::fmod(t + s.sig_offset, s.sig_cycle);
-        if (ph < 0) ph += s.sig_cycle;
-        w.state = ph < s.sig_green ? 6 : (ph < s.sig_green + s.sig_yellow ? 7 : 3);
-    }
+    w.state = signal_state(s, t);
     w.on = s.sig_road > 0 && h.road_num == s.sig_road && h.pos != 2;
     if (w.on) {
         const int gl = m.lane_index(h.road_num, h.lane_num), off = m.d.lane_pt_off[gl], cnt = m.lane_size(gl);
@@ -39,10 +54,9 @@ World build(const junction::JMap& jm, const dp_params& p, const dp_v2x_event_spe
     }
     v.spat_state = w.state;
     v.spat_lane_occupied = (w.on && w.d >= 0 && w.d <= s.sig_range) ? 1 : 0;
-    w.ped_on = s.has_ped && s.ped_t_on <= t && t <= s.ped_t_off;
+    double px = 0, py = 0;
+    w.ped_on = pedestrian(s, t, &px, &py);
     if (w.ped_on) {
-        const double tp = t - s.ped_t_on;
-        const double px = s.ped_x + s.ped_vx * tp, py = s.ped_y + s.ped_vy * tp;
         const double dx = px - h.x, dy = py - h.y;
         v.ped_distance = std::sqrt(dx * dx + dy * dy);
         gps(p, px, py, &v.ped_lat, &v.ped_lng);

@@ -19,6 +19,9 @@ struct World {
     int state;                         // spat_state: 6 / 7 / 3, 0 without a signal
     bool on, ped_on;                   // on the governed approach (pos 0 / 1); the pedestrian is active
 };
+// the pieces of build that the agents of section 15 share: the spat_state at t, and ped_on with (px, py) when it is
+int signal_state(const dp_v2x_event_spec& s, double t);
+bool pedestrian(const dp_v2x_event_spec& s, double t, double* px, double* py);
 World build(const junction::JMap& jm, const dp_params& p, const dp_v2x_event_spec& s, const dp_scene_hdr& h, int k);
 void init(dp_v2x_episode_stats& r);
 // flags (nullable) receives the flags of a launch with rec (the tally leaves them); a header that names no lane gets zero flags and leaves the row alone
