@@ -201,6 +201,22 @@ v2x_traffic_stats = np.dtype(
 assert v2x_traffic_stats.itemsize == 32
 
 
+class V2xObstacleParams(C.Structure):
+    _fields_ = [("range", C.c_double), ("front", C.c_double), ("rear", C.c_double), ("half_width", C.c_double), ("what", C.c_int32),
+                ("pad", C.c_int32)]
+
+
+v2x_obstacle_stats = np.dtype(
+    [
+        ("min_ped_clearance", "<f8"), ("min_works_clearance", "<f8"), ("views", "<i4"), ("ped_cycles", "<i4"), ("works_cycles", "<i4"),
+        ("dropped", "<i4"), ("ped_bound_cycles", "<i4"), ("works_bound_cycles", "<i4"), ("ped_hits", "<i4"), ("first_ped_hit", "<i4"),
+        ("works_hits", "<i4"), ("first_works_hit", "<i4"), ("last_ped_slot", "<i4"), ("last_works_first", "<i4"), ("last_works_end", "<i4"),
+        ("pad", "<i4", (3,)),
+    ]
+)
+assert v2x_obstacle_stats.itemsize == 80
+
+
 class MapDesc(C.Structure):
     _fields_ = [
         ("n_roads", C.c_int32), ("road_lane_base", C.c_void_p),

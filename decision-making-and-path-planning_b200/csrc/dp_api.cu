@@ -68,6 +68,7 @@ struct dp_ctx {
     DpV2xOpts v2x;                                          // dp_world_set_v2x: the V2X launch between cycle and world step
     int v2x_cycle = 0;                                      // the cycle of the last dp_v2x_world_dev call: section 15's t of a
                                                             // hand-stepped world step
+    DpObstOpts obst;                                        // dp_world_set_v2x_obstacles: the views every cycle runs on
     cudaStream_t ep_stream = nullptr;
     cudaGraphExec_t ep_exec = nullptr;
     const void* ep_key[8] = {}; int ep_dims[3] = {-1, -1, -1};
@@ -1380,6 +1381,7 @@ int dp_world_set_v2x(dp_ctx* c, const dp_v2x_world_params* vp, int n, const dp_v
     if (!spec) {
         c->v2x = DpV2xOpts{};
         c->world.ts = nullptr; c->world.spec = nullptr;     // the agents cannot obey events that are not there
+        c->obst = DpObstOpts{};                             // ... nor the planner see them
         return drop_episode_graph(c);
     }
     if (!vp || !stats || n < 0 || n_wp < 0 || (n_wp > 0 && (!wp_x || !wp_y)) || (vp->mode != 0 && vp->mode != 1) ||
@@ -1429,6 +1431,39 @@ int dp_world_set_v2x_traffic(dp_ctx* c, const dp_v2x_traffic_params* p, dp_v2x_t
     c->world.ts = stats;
     return drop_episode_graph(c);
 }
+void dp_v2x_obstacle_default_params(dp_v2x_obstacle_params* p) {
+    if (!p) return;
+    memset(p, 0, sizeof(*p));
+    p->range = 100.0; p->front = 4.0; p->rear = 1.0; p->half_width = 0.9; p->what = 7;
+}
+int dp_world_set_v2x_obstacles(dp_ctx* c, const dp_v2x_obstacle_params* p, dp_scene_hdr* hv, double* vx, double* vy, dp_v2x_obstacle_stats* stats) {
+    if (!c || (stats && !p)) return fail(DP_ERR_ARG, "dp_world_set_v2x_obstacles: bad argument");
+    if (!stats) {
+        c->obst = DpObstOpts{};
+        return drop_episode_graph(c);
+    }
+    if (!all_finite({p->range, p->front, p->rear, p->half_width}))
+        return fail(DP_ERR_ARG, "dp_world_set_v2x_obstacles: parameters must be finite");
+    if (!(p->range >= 0) || !(p->half_width > 0) || !(p->front >= 0) || !(p->rear >= 0) || p->what < 0 || p->what > 7)
+        return fail(DP_ERR_ARG, "dp_world_set_v2x_obstacles: range, front, rear >= 0, half_width > 0 and what in 0 .. 7");
+    if (!hv || !vx || !vy) return fail(DP_ERR_ARG, "dp_world_set_v2x_obstacles: NULL view buffers");
+    if (!c->v2x.spec) return fail(DP_ERR_ARG, "dp_world_set_v2x_obstacles: the V2X events are not armed (dp_world_set_v2x)");
+    if (c->tracks_T > 0) return fail(DP_ERR_STATE, "dp_world_set_v2x_obstacles: predicted tracks are set (dp_clear_tracks first)");
+    c->obst.op = *p; c->obst.hv = hv; c->obst.vx = vx; c->obst.vy = vy; c->obst.stats = stats;
+    return drop_episode_graph(c);
+}
+int dp_v2x_obstacles_dev(dp_ctx* c, int first, int n, const dp_scene_hdr* hdr, const double* ox, const double* oy, const dp_plan_record* prev,
+                         int cycle, int tally, void* stream) {
+    if (!c || !hdr || !ox || !oy || n < 0 || first < 0 || first + n > c->max_scenes || cycle < 0 || (tally != 0 && tally != 1))
+        return fail(DP_ERR_ARG, "dp_v2x_obstacles_dev: bad argument");
+    if (!c->have_map) return fail(DP_ERR_STATE, "dp_v2x_obstacles_dev: map not uploaded");
+    if (!c->obst.stats) return fail(DP_ERR_STATE, "dp_v2x_obstacles_dev: the model is not armed (dp_world_set_v2x_obstacles)");
+    if (n > c->v2x.n) return fail(DP_ERR_ARG, "dp_v2x_obstacles_dev: more scenes than the armed V2X specifications");
+    CK(cudaSetDevice(c->device));
+    c->launches += n > 0 ? 1 : 0;
+    CK(dp_launch_world_obstacles(c->gmap, c->v2x, c->obst, n, c->max_obs, hdr, ox, oy, prev, cycle, tally != 0, (cudaStream_t)stream));
+    return DP_OK;
+}
 int dp_v2x_world_dev(dp_ctx* c, int first, int n, const dp_scene_hdr* hdr, dp_plan_record* rec, int cycle, void* stream) {
     if (!c || !hdr || n < 0 || first < 0 || first + n > c->max_scenes || cycle < 0) return fail(DP_ERR_ARG, "dp_v2x_world_dev: bad argument");
     if (!c->have_map) return fail(DP_ERR_STATE, "dp_v2x_world_dev: map not uploaded");
@@ -1463,12 +1498,22 @@ cudaError_t enqueue_closed_loop(dp_ctx* c, int first, int n, int cycles, dp_scen
     if (rearm && (e = cudaMemsetAsync(c->d_done + first, 0, (size_t)n * sizeof(unsigned), st)) != cudaSuccess) return e;
     c->launches += 1;
     if ((e = dp_launch_world(c->gmap, c->p, c->world, b, st)) != cudaSuccess) return e;
+    // with the V2X road users armed (section 16) every cycle runs on, and the logs record, the view an obstacles launch builds
+    const bool obst = c->obst.stats != nullptr;
+    dp_scene_hdr* ch = obst ? c->obst.hv : hdr;
+    double* cx = obst ? c->obst.vx : ox;
+    double* cy = obst ? c->obst.vy : oy;
     for (int k = 0; k < cycles; ++k) {
-        if (hdr_log && (e = cudaMemcpyAsync(hdr_log + (size_t)k * n, hdr, (size_t)n * sizeof(dp_scene_hdr), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
-        if (olx && (e = cudaMemcpyAsync(olx + (size_t)k * n * mo, ox, (size_t)n * mo * sizeof(double), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
-        if (oly && (e = cudaMemcpyAsync(oly + (size_t)k * n * mo, oy, (size_t)n * mo * sizeof(double), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
+        if (obst) {
+            c->launches += 1;
+            const dp_plan_record* prev = k > 0 ? rec + (size_t)(k - 1) * n : nullptr;
+            if ((e = dp_launch_world_obstacles(c->gmap, c->v2x, c->obst, n, c->max_obs, hdr, ox, oy, prev, k, false, st)) != cudaSuccess) return e;
+        }
+        if (hdr_log && (e = cudaMemcpyAsync(hdr_log + (size_t)k * n, ch, (size_t)n * sizeof(dp_scene_hdr), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
+        if (olx && (e = cudaMemcpyAsync(olx + (size_t)k * n * mo, cx, (size_t)n * mo * sizeof(double), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
+        if (oly && (e = cudaMemcpyAsync(oly + (size_t)k * n * mo, cy, (size_t)n * mo * sizeof(double), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
         const DpIo io = make_io(c, first, nullptr);
-        if ((e = run_cycle(c, first, n, hdr, ox, oy, rec + (size_t)k * n, nullptr, nullptr, nullptr, st, io)) != cudaSuccess) return e;
+        if ((e = run_cycle(c, first, n, ch, cx, cy, rec + (size_t)k * n, nullptr, nullptr, nullptr, st, io)) != cudaSuccess) return e;
         if (c->v2x.spec) {                                  // V2X armed: the flags act on the records before the world step reads them
             c->launches += 1;
             if ((e = dp_launch_world_v2x(c->gmap, c->p, c->v2x, n, hdr, rec + (size_t)k * n, k, st)) != cudaSuccess) return e;
@@ -1481,6 +1526,11 @@ cudaError_t enqueue_closed_loop(dp_ctx* c, int first, int n, int cycles, dp_scen
         c->launches += 1;
         if ((e = dp_launch_world_v2x(c->gmap, c->p, c->v2x, n, hdr, nullptr, cycles, st)) != cudaSuccess) return e;
     }
+    if (obst) {                                             // the tally: the last cycle's bound check, the hits of the final world
+        c->launches += 1;
+        const dp_plan_record* prev = cycles > 0 ? rec + (size_t)(cycles - 1) * n : nullptr;
+        if ((e = dp_launch_world_obstacles(c->gmap, c->v2x, c->obst, n, c->max_obs, hdr, ox, oy, prev, cycles, true, st)) != cudaSuccess) return e;
+    }
     return cudaSuccess;
 }
 }  // namespace
@@ -1491,6 +1541,8 @@ int dp_run_closed_loop_dev(dp_ctx* c, int first, int n, int cycles, dp_scene_hdr
     if (!c->have_map) return fail(DP_ERR_STATE, "dp_run_closed_loop_dev: map not uploaded");
     if (c->submitted != c->waited) return fail(DP_ERR_STATE, "dp_run_closed_loop_dev: submitted cycles in flight, call dp_cycle_wait first");
     if (c->v2x.spec && n > c->v2x.n) return fail(DP_ERR_ARG, "dp_run_closed_loop_dev: more scenes than the armed V2X specifications");
+    if (c->obst.stats && c->tracks_T > 0)
+        return fail(DP_ERR_STATE, "dp_run_closed_loop_dev: the V2X road users are armed and predicted tracks are set");
     CK(cudaSetDevice(c->device));
     c->ep_last_graph = 0;
     if (n == 0) return DP_OK;

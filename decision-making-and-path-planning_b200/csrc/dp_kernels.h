@@ -53,6 +53,16 @@ struct DpV2xOpts {
 // one V2X launch of cycle `cycle` (dp_world_v2x.cu); rec == nullptr: the tally after the last world step
 cudaError_t dp_launch_world_v2x(const DevMap& m, const dp_params& p, const DpV2xOpts& o, int n, const dp_scene_hdr* hdr, dp_plan_record* rec,
                                 int cycle, cudaStream_t st);
+// the planner sees the V2X road users (include/dmpp_b200.h section 16), armed by stats != nullptr: the views every cycle runs on
+struct DpObstOpts {
+    dp_v2x_obstacle_params op = {};
+    dp_scene_hdr* hv = nullptr; double* vx = nullptr; double* vy = nullptr;
+    dp_v2x_obstacle_stats* stats = nullptr;
+};
+// one obstacles launch of cycle `cycle` (dp_world_v2x_obstacles.cu) on the world hdr / ox / oy, with section 14's specifications;
+// prev: the records of cycle - 1 (nullptr at cycle 0); tally: the row only
+cudaError_t dp_launch_world_obstacles(const DevMap& m, const DpV2xOpts& v, const DpObstOpts& o, int n, int max_obs, const dp_scene_hdr* hdr,
+                                      const double* ox, const double* oy, const dp_plan_record* prev, int cycle, bool tally, cudaStream_t st);
 cudaError_t dp_launch_v2x(const DevMap& m, const dp_params& p, int n, const dp_scene_hdr* hdr, const dp_v2x_data* v2x, const double* wp_lat,
                           const double* wp_lng, int mode, dp_v2x_flags* out, cudaStream_t st);
 cudaError_t dp_launch_v2x_apply(int n, const dp_v2x_flags* flags, dp_plan_record* rec, cudaStream_t st);

@@ -28,7 +28,8 @@ SYMBOLS = [
     "dp_run_closed_loop_dev", "dp_closed_loop_is_graph", "dp_v2x_event_batch", "dp_v2x_event_batch_dev", "dp_v2x_apply", "dp_v2x_apply_dev",
     "dp_metrics_default_params", "dp_world_set_metrics", "dp_agent_model_default_params", "dp_world_set_agent_model",
     "dp_lane_change_default_params", "dp_world_set_lane_change", "dp_world_set_v2x", "dp_v2x_world_dev",
-    "dp_v2x_traffic_default_params", "dp_world_set_v2x_traffic",
+    "dp_v2x_traffic_default_params", "dp_world_set_v2x_traffic", "dp_v2x_obstacle_default_params", "dp_world_set_v2x_obstacles",
+    "dp_v2x_obstacles_dev",
     "dp_gather_create", "dp_gather_attach", "dp_gather_arm", "dp_gather_chain", "dp_gather_arm_deferred", "dp_gather_set_lag", "dp_gather_flush", "dp_gather_disarm", "dp_gather_wait", "dp_gather_buffer", "dp_gather_destroy",
 ]
 
@@ -82,6 +83,15 @@ def v2x_traffic_params(**kw):
     """dp_v2x_traffic_default_params (no GPU needed), then the keyword fields"""
     p = abi.V2xTrafficParams()
     load().dp_v2x_traffic_default_params(C.byref(p))
+    for k, v in kw.items():
+        setattr(p, k, v)
+    return p
+
+
+def v2x_obstacle_params(**kw):
+    """dp_v2x_obstacle_default_params (no GPU needed), then the keyword fields"""
+    p = abi.V2xObstacleParams()
+    load().dp_v2x_obstacle_default_params(C.byref(p))
     for k, v in kw.items():
         setattr(p, k, v)
     return p
@@ -282,6 +292,21 @@ class Planner:
         _ck(self.lib.dp_world_set_v2x_traffic(self.ctx, C.byref(params) if params is not None else None, C.c_void_p(d_stats or 0)),
             "dp_world_set_v2x_traffic")
 
+    def set_v2x_obstacles(self, params, d_hdr_view, d_ox_view, d_oy_view, d_stats):
+        """let the planner see the V2X road users (include/dmpp_b200.h section 16; the V2X events must be armed): device addresses of
+        the views hdr_view[n] / ox_view / oy_view[n][max_obs] every cycle runs on and of dp_v2x_obstacle_stats [n], all indexed like
+        hdr; d_stats None / 0 disarms"""
+        _ck(self.lib.dp_world_set_v2x_obstacles(self.ctx, C.byref(params) if params is not None else None, C.c_void_p(d_hdr_view or 0),
+                                                C.c_void_p(d_ox_view or 0), C.c_void_p(d_oy_view or 0), C.c_void_p(d_stats or 0)),
+            "dp_world_set_v2x_obstacles")
+
+    def v2x_obstacles_dev(self, n, d_hdr, d_ox, d_oy, d_prev_rec, cycle, tally=False, first=0, stream=0):
+        """one obstacles launch of cycle `cycle` into the armed views, before cycle_dev runs on them; d_prev_rec = the records of cycle
+        - 1 (None at cycle 0); tally=True: the row only, after the last world step and V2X tally"""
+        _ck(self.lib.dp_v2x_obstacles_dev(self.ctx, C.c_int(first), C.c_int(n), C.c_void_p(d_hdr), C.c_void_p(d_ox), C.c_void_p(d_oy),
+                                          C.c_void_p(d_prev_rec or 0), C.c_int(cycle), C.c_int(int(tally)), C.c_void_p(stream)),
+            "dp_v2x_obstacles_dev")
+
     def v2x_world_dev(self, n, d_hdr, d_rec, cycle, first=0, stream=0):
         """one V2X launch of cycle `cycle` between cycle_dev and world_step_dev; d_rec None: the tally after the last step"""
         _ck(self.lib.dp_v2x_world_dev(self.ctx, C.c_int(first), C.c_int(n), C.c_void_p(d_hdr), C.c_void_p(d_rec or 0), C.c_int(cycle),
@@ -302,7 +327,7 @@ class Planner:
         return bool(self.lib.dp_closed_loop_is_graph(self.ctx))
 
     def run_closed_loop(self, hdr, agents, cycles, log=True, repeat=1, metrics=None, agent_model=None, lane_change=None, v2x=None,
-                        traffic=None):
+                        traffic=None, obstacles=None):
         """host arrays in, host arrays out (the same dictionary as oracle.binding's run_closed_loop); `repeat` > 1 replays the
         episode from the same initial world (same device buffers, i.e. the cached graph) and returns the last run.
         metrics: None, or MetricsParams: the episode metrics are armed for this call (and disarmed after it) and the rows are
@@ -312,10 +337,12 @@ class Planner:
         v2x: None, or (V2xWorldParams, events) with events.spec[n] / wp_x / wp_y (scenes.V2xEvents): the V2X events are armed for
         this call, the rows are returned under "v2x_stats" and the flags of the last launch under "v2x_flags".  traffic: None, or
         V2xTrafficParams (needs agent_model and v2x): the agents obey the V2X events for this call, and their rows are returned
-        under "v2x_traffic"."""
+        under "v2x_traffic".  obstacles: None, or V2xObstacleParams (needs v2x): every cycle runs on a view of the world with the V2X
+        road users in it for this call (the logs record the views), and the rows are returned under "v2x_obstacles"."""
         n, mo = agents.shape
         assert lane_change is None or agent_model is not None, "lane changes run on the reactive agents"
         assert traffic is None or (agent_model is not None and v2x is not None), "the agents obey the V2X events on the reactive agents"
+        assert obstacles is None or v2x is not None, "the planner sees the V2X road users of the armed V2X events"
         assert mo == self.max_obs and hdr.shape == (n,)
         sizes = {"hdr": n * 128, "agents": n * mo * 32, "ox": n * mo * 8, "oy": n * mo * 8, "rec": cycles * n * 128,
                  "hdr_log": cycles * n * 128, "obs_log_x": cycles * n * mo * 8, "obs_log_y": cycles * n * mo * 8}
@@ -336,6 +363,8 @@ class Planner:
                          v2x_flags=n * abi.v2x_flags.itemsize, v2x_stats=n * abi.v2x_episode_stats.itemsize)
         if traffic is not None:
             sizes["v2x_traffic"] = n * abi.v2x_traffic_stats.itemsize
+        if obstacles is not None:
+            sizes.update(v2x_hdr_view=n * 128, v2x_ox_view=n * mo * 8, v2x_oy_view=n * mo * 8, v2x_obstacles=n * abi.v2x_obstacle_stats.itemsize)
         d = {}
         try:
             for k, b in sizes.items():
@@ -357,6 +386,8 @@ class Planner:
                 self.set_v2x_world(vp, n, d["v2x_spec"], d["v2x_wp_x"], d["v2x_wp_y"], wx.size, d["v2x_flags"], d["v2x_stats"])
             if traffic is not None:
                 self.set_v2x_traffic(traffic, d["v2x_traffic"])
+            if obstacles is not None:
+                self.set_v2x_obstacles(obstacles, d["v2x_hdr_view"], d["v2x_ox_view"], d["v2x_oy_view"], d["v2x_obstacles"])
             h0, a0 = np.ascontiguousarray(hdr), np.ascontiguousarray(agents)
             for _ in range(repeat):
                 self.reset(0, n)
@@ -378,6 +409,8 @@ class Planner:
                 o["v2x_flags"], o["v2x_stats"] = np.zeros(n, abi.v2x_flags), np.zeros(n, abi.v2x_episode_stats)
             if traffic is not None:
                 o["v2x_traffic"] = np.zeros(n, abi.v2x_traffic_stats)
+            if obstacles is not None:
+                o["v2x_obstacles"] = np.zeros(n, abi.v2x_obstacle_stats)
             for k in o:
                 _ck(self.lib.dp_memcpy_d2h(self.ctx, abi.ptr(o[k]), C.c_void_p(d[k]), C.c_size_t(sizes[k]), None), "d2h")
             _ck(self.lib.dp_stream_sync(self.ctx, None), "sync")
@@ -385,6 +418,8 @@ class Planner:
             o["graph"] = self.closed_loop_is_graph()
             return o
         finally:
+            if obstacles is not None:
+                self.set_v2x_obstacles(None, None, None, None, None)
             if traffic is not None:
                 self.set_v2x_traffic(None, None)
             if v2x is not None:

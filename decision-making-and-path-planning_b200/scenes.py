@@ -415,10 +415,12 @@ class World:
     kind 'junction' / 'urban': the agents sit on the approach lane, the connector or the departure lane by arclength, as
     `Episodes.obstacles` spreads them; the ego crosses the junction only with dp_world_params.pre_junction_pts > 0
     (`PRE_JUNCTION_PTS[kind]` matches the scripted episodes).  `v0`: the agents' desired speeds for the reactive agents of
-    include/dmpp_b200.h section 12, by default their initial speeds."""
+    include/dmpp_b200.h section 12, by default their initial speeds.  `max_obs` (default n_obs): the width of `agents` / `v0`,
+    zero-padded beyond the n_obs agents (hdr.n_obs stays n_obs), for contexts with room for more obstacle points than agents --
+    the V2X road users of include/dmpp_b200.h section 16 are appended in those slots."""
     PRE_JUNCTION_PTS = {"highway": 0, "junction": 60, "urban": 400}
 
-    def __init__(self, m: Map, seeds, n_obs=10, roads=None, kind="highway"):
+    def __init__(self, m: Map, seeds, n_obs=10, roads=None, kind="highway", max_obs=None):
         ep = Episodes(m, seeds, n_obs=n_obs, kind=kind, cycles=1, roads=roads)
         self.m, self.n, self.n_obs, self.kind = m, ep.n, int(n_obs), kind
         self.hdr = ep.hdr(0)
@@ -445,6 +447,11 @@ class World:
         a["u"] = (f - i) * SPACING
         a["v"] = ep.ob_v
         a["lat"] = ep.ob_lat
+        if max_obs is not None and int(max_obs) != self.n_obs:
+            assert int(max_obs) > self.n_obs
+            pad = np.zeros((self.n, int(max_obs)), abi.agent)
+            pad[:, :self.n_obs] = a
+            a = pad
         self.agents = np.ascontiguousarray(a)
         self.v0 = np.ascontiguousarray(a["v"])
 

@@ -678,7 +678,8 @@ int dp_world_set_lane_change(dp_ctx* ctx, const dp_lane_change_params* p, dp_lan
  * ego with the adjusted speed command.  Armed, an episode is: placement, then per cycle Decision + Planning -> V2X -> world
  * step, then one tally-only V2X launch (1 + cycles * 4 + 1 kernels).  Disarmed (the default) the episode is that of section 9,
  * launch for launch.  The rules are frozen in tools/junction_oracle/v2x_world.h.  Agents that stop for the signal and yield to
- * the pedestrian are section 15.  Out of scope: pedestrians as obstacle points, V2X in pos 1 / 2.
+ * the pedestrian are section 15; the pedestrian and the road works as obstacle points the planner sees are section 16.  Out of
+ * scope: V2X in pos 1 / 2.
  *
  * IEEE binary64, operations in the order written, no contraction.  World s at cycle k (k = 0 .. cycles-1 the cycle launches,
  * k = cycles the tally), with its cycle's header h (before the world step) and t = k * period_ms / 1000:
@@ -760,9 +761,9 @@ int dp_v2x_world_dev(dp_ctx* ctx, int first_scene, int n_scenes, const dp_scene_
  * which must be armed; disarming either disarms this model, as disarming the agent model disarms lane changes).  The stop line of
  * a red or yellow signal and the active pedestrian become two more leader candidates of section 12's IDM and of section 13's
  * target lane, both standing still.  Disarmed (the default) nothing changes: the same launches, the same graph, the same bytes.
- * The arithmetic is frozen in tools/junction_oracle/v2x_traffic.h.  Out of scope: the pedestrian as an obstacle point the planner
- * sees; agents reacting to road works (the ego only creeps past them, so "stop" would be the wrong rule); V2X in pos 1 / 2; any
- * change to how the ego moves.
+ * The arithmetic is frozen in tools/junction_oracle/v2x_traffic.h.  The pedestrian as an obstacle point the planner sees is
+ * section 16.  Out of scope: agents reacting to road works (the ego only creeps past them, so "stop" would be the wrong rule);
+ * V2X in pos 1 / 2; any change to how the ego moves.
  *
  * IEEE binary64, operations in the order written, no contraction.  World s at the world step of cycle k:
  *   time      t = k * period_ms / 1000 with the header's period_ms, the t of that cycle's V2X launch.  dp_run_closed_loop_dev passes
@@ -814,6 +815,83 @@ void dp_v2x_traffic_default_params(dp_v2x_traffic_params* p);
  * its next call.  DP_ERR_ARG for non-finite parameters, b_commit <= 0, ped_half_width < 0, obey other than 0 / 1, or arming while
  * the agent model or the V2X events are disarmed.  The world step then needs at most as many scenes as the armed V2X specifications. */
 int dp_world_set_v2x_traffic(dp_ctx* ctx, const dp_v2x_traffic_params* p, dp_v2x_traffic_stats* stats);
+
+/* (16) The planner sees the V2X road users (opt-in, on top of the V2X events of section 14, which must be armed; disarming them
+ * disarms this model).  Each cycle of an episode runs on a VIEW of the world: the world's header and obstacle points, followed
+ * by the active pedestrian, the road-works point and the zone's warning points within `range` of the ego, as perception would
+ * hand them to the planner (ObPoint, Decision.cpp:343).  The view is built by an "obstacles" launch just before the cycle, into
+ * caller-owned buffers; the world state (hdr, agents, obs_x / obs_y) is never written by this model, so the world step, the
+ * metrics and every agent model keep seeing the agents only (k < min(hdr.n_obs, max_obs)).  The planner itself is unchanged: the
+ * points enter the obstacle list it already reads (SearchObstacle, the region gaps, the avoid sweep, SpeedPlanning's stop).
+ * Armed, an episode is: placement, then per cycle obstacles -> Decision + Planning on the view -> V2X -> world step, then the V2X
+ * tally and the obstacles tally (1 + cycles * 5 + 2 kernels); hdr_log / obs_log_* record the views, i.e. what every cycle ran
+ * on.  Disarmed (the default) the episode is that of section 14, launch for launch.  The rules are frozen in
+ * tools/junction_oracle/v2x_obstacles.h.  A record's ob_index >= the world's agent count names an event point (the cycle reads no
+ * obstacle type).  Out of scope: agents reacting to the points; the stop line as a virtual obstacle; pedestrians in junction
+ * worlds; any change to the cycle, the world step or how the ego moves.
+ *
+ * IEEE binary64, operations in the order written, no contraction.  World s at launch k (k = 0 .. cycles-1 before cycle k,
+ * k = cycles the tally), with the world's header h and obstacle row, t = k * period_ms / 1000 (the t of cycle k's V2X launch),
+ * na = min(h.n_obs, max_obs):
+ *   row       the launch with k == 0 first initialises the world's row (also for a header that names no lane), so a replayed
+ *             episode graph starts clean
+ *   no lane   a header that names no lane (section 14's test): the view is a plain copy (header, slots 0 .. na-1) and the row
+ *             is left alone
+ *   view      (not on the tally) header = h; slots 0 .. na-1 = the world's points; then appended in this order, each at the next
+ *             slot while that slot is < max_obs (else dropped and counted):
+ *               the pedestrian (px, py)  when what & 1, ped_on (section 14's pedestrian at t) and sqrt(dx * dx + dy * dy) <= range,
+ *                                        dx = px - h.x, dy = py - h.y;
+ *               the works point (rw_x, rw_y)  when what & 2, has_works and within range (the same distance);
+ *               the warning points wp[wp_first .. wp_first + wp_count) in list order  when what & 4, has_works and each within range.
+ *             n_obs = na + appended (the world's n_obs when nothing is appended: with what = 0 the view IS the world).  Slots at
+ *             and beyond the view's n_obs are not written
+ *   box       section 11's: (c, s) = spec_sincos_deg(h.dir); for a point (ox, oy): dx = ox - h.x, dy = oy - h.y,
+ *             lon = dx*c + dy*s, lat = dy*c - dx*s; inside: -rear <= lon <= front && -half_width <= lat <= half_width;
+ *             clearance ex = lon > front ? lon - front : (lon < -rear ? -rear - lon : 0), ey = |lat| > half_width ? |lat| - half_width
+ *             : 0, d = sqrt(ex*ex + ey*ey)
+ * Row (initial value), updated on every launch on a header that names a lane, the tally included:
+ *   views                     views built (0)
+ *   ped_cycles / works_cycles views with the pedestrian / with at least one works or warning point in them (0)
+ *   dropped                   points dropped for want of a slot (0)
+ *   ped_bound_cycles /        prev_rec (the record of cycle k-1; NULL at k == 0) has ob_flag set and ob_index == last_ped_slot /
+ *   works_bound_cycles        last_works_first <= ob_index < last_works_end: the previous cycle's local path was bounded by that point (0)
+ *   ped_hits, first_ped_hit   launches with the active pedestrian inside the ego box, and the k of the first one (0 / -1)
+ *   works_hits, first_works_hit  launches with the works point or any warning point (has_works) inside the box (0 / -1)
+ *   min_ped_clearance / min_works_clearance  min of d over launches with ped_on / with has_works, over those points (+inf)
+ *   last_ped_slot, last_works_first, last_works_end  the slot layout of the last view: the pedestrian's slot (-1 when not in it),
+ *                             the works and warning points' slots [first, end) (-1 / 0 / 0)
+ * Hits and clearances are counted whether or not the point is in the view, so that the arms of `what` compare fairly. */
+typedef struct dp_v2x_obstacle_params {
+    double range;                      /* m, default 100 (this library's choice) */
+    double front, rear, half_width;    /* the ego box of the row, default 4.0 / 1.0 / 0.9 (dp_metrics_params) */
+    int32_t what;                      /* bit mask of the appended points: 1 pedestrian, 2 works point, 4 warning points; default 7;
+                                          0 = observe only (the view is the world, the row still counts) */
+    int32_t pad;                       /* zero */
+} dp_v2x_obstacle_params;              /* 40 bytes */
+typedef struct dp_v2x_obstacle_stats {
+    double min_ped_clearance, min_works_clearance;
+    int32_t views, ped_cycles, works_cycles, dropped;
+    int32_t ped_bound_cycles, works_bound_cycles;
+    int32_t ped_hits, first_ped_hit, works_hits, first_works_hit;
+    int32_t last_ped_slot, last_works_first, last_works_end;   /* carried from the previous view (-1 / 0 / 0) */
+    int32_t pad[3];                    /* zero */
+} dp_v2x_obstacle_stats;               /* 80 bytes, [n] indexed like hdr */
+void dp_v2x_obstacle_default_params(dp_v2x_obstacle_params* p);
+/* hdr_view[n], obs_x_view / obs_y_view[n][max_obs], stats[n]: caller-owned device buffers indexed like hdr, for at least as many
+ * scenes as the armed V2X specifications.  stats == NULL disarms (everything else may then be NULL).  Context state like
+ * dp_world_set_v2x: the cached episode graph is rebuilt on its next call.  DP_ERR_ARG for non-finite parameters, range < 0,
+ * half_width <= 0, front or rear < 0, what outside 0 .. 7, NULL view buffers, or arming while the V2X events are disarmed;
+ * DP_ERR_STATE while predicted tracks are set (dp_set_tracks: their tiles are indexed by obstacle slot), which
+ * dp_run_closed_loop_dev refuses as well. */
+int dp_world_set_v2x_obstacles(dp_ctx* ctx, const dp_v2x_obstacle_params* p, dp_scene_hdr* hdr_view, double* obs_x_view,
+                               double* obs_y_view, dp_v2x_obstacle_stats* stats);
+/* one obstacles launch for callers that step by hand: the view of cycle `cycle` of the world hdr / obs_x / obs_y (device pointers)
+ * into the armed view buffers, and the row; prev_rec = the records of cycle - 1 (NULL at cycle 0); tally = 1: the row only, after
+ * the last world step (cycle = the number of cycles).  Per cycle: dp_v2x_obstacles_dev -> dp_cycle_batch_dev on the view ->
+ * dp_v2x_world_dev -> dp_world_step_dev; after the last one dp_v2x_world_dev(rec NULL) -> dp_v2x_obstacles_dev(tally).
+ * DP_ERR_STATE when the model is disarmed. */
+int dp_v2x_obstacles_dev(dp_ctx* ctx, int first_scene, int n_scenes, const dp_scene_hdr* hdr, const double* obs_x, const double* obs_y,
+                         const dp_plan_record* prev_rec, int cycle, int tally, void* stream);
 
 /* diagnostic: phase time stamps (globaltimer, ns) of the most recent cycle launch, one row of 32 per CTA (row b = scenes
  * [b*g, (b+1)*g) of the batch; stamp 0 = CTA start, stamp i = end of phase i of csrc/dp_group.cuh).  Only contexts created

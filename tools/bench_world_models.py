@@ -23,7 +23,12 @@ SM clock read in the same run.
                arm: disarmed, obey = 0 (the records must equal the disarmed ones: the delta is the candidates' cost alone) and
                obey = 1, for the highway and junction episodes (4096 worlds) and dp_world_step_dev alone (4096 junction worlds with 10
                agents, 1024 urban worlds with 200); and the effect of obey 0 -> 1 on seeds 0-511 (agent red runs, ego red crossings,
-               collisions and where they started, ego stopped steps; pedestrian hits and distances, ego collisions)."""
+               collisions and where they started, ego stopped steps; pedestrian hits and distances, ego collisions).
+  obstacles    the planner sees the V2X road users (section 16), with the V2X events (apply = 1) armed in every arm and 14 obstacle
+               slots for 10 agents: disarmed, what = 0 (the view is the world: the records must equal the disarmed ones, the delta is
+               the obstacles launches alone) and what = 7, for 4096 highway worlds x 25 cycles as ONE graph launch; and
+               dp_v2x_obstacles_dev alone (4096 worlds, what = 0 and 7, on the world and records the last episode left).  The effect
+               on seeds 0-511 is the checker's, in tests/test_v2x_obstacles.py."""
 import argparse
 import json
 import os
@@ -59,20 +64,22 @@ def cump_of():
 class Arm:
     """one planner + world of one kind, with the models asked for armed"""
 
-    def __init__(self, kind, n, n_obs, cycles, metrics=False, react=False, lanechg=False, v2x=None, traffic=None):
+    def __init__(self, kind, n, n_obs, cycles, metrics=False, react=False, lanechg=False, v2x=None, traffic=None, obstacles=None,
+                 max_obs=None):
         self.n = n
-        self.p = Planner(n, n_obs); self.p.upload_map(m)
+        mo = max_obs or n_obs
+        self.p = Planner(n, mo); self.p.upload_map(m)
         wp = self.p.world_params(); wp.pre_junction_pts = scenes.World.PRE_JUNCTION_PTS[kind]
         self.p.set_world_params(wp)
-        self.w = scenes.World(m, np.arange(n), n_obs, kind=kind)
+        self.w = scenes.World(m, np.arange(n), n_obs, kind=kind, max_obs=mo)
         self.cycles = cycles
         self.h0, self.a0 = u8(self.w.hdr), u8(self.w.agents)
         self.d_h, self.d_a = torch.empty_like(self.h0), torch.empty_like(self.a0)
-        self.d_x = torch.zeros((n, n_obs), dtype=torch.float64, device=dev); self.d_y = torch.zeros_like(self.d_x)
+        self.d_x = torch.zeros((n, mo), dtype=torch.float64, device=dev); self.d_y = torch.zeros_like(self.d_x)
         self.d_r = torch.zeros((cycles, n, 128), dtype=torch.uint8, device=dev)
         self.d_v0 = u8(self.w.v0)
         self.d_m = torch.zeros((n, 192), dtype=torch.uint8, device=dev)
-        self.d_s = torch.zeros((n, n_obs, abi.lane_change_state.itemsize), dtype=torch.uint8, device=dev)
+        self.d_s = torch.zeros((n, mo, abi.lane_change_state.itemsize), dtype=torch.uint8, device=dev)
         if metrics:
             self.p.set_metrics(pl.metrics_params(), self.d_m.data_ptr())
         if react:
@@ -89,6 +96,12 @@ class Arm:
         if traffic is not None:                             # traffic = obey (0 / 1)
             self.d_ts = torch.zeros((n, abi.v2x_traffic_stats.itemsize), dtype=torch.uint8, device=dev)
             self.p.set_v2x_traffic(pl.v2x_traffic_params(obey=traffic), self.d_ts.data_ptr())
+        if obstacles is not None:                           # obstacles = what (0 .. 7)
+            self.d_hv = torch.zeros((n, 128), dtype=torch.uint8, device=dev)
+            self.d_vx, self.d_vy = torch.zeros_like(self.d_x), torch.zeros_like(self.d_x)
+            self.d_os = torch.zeros((n, abi.v2x_obstacle_stats.itemsize), dtype=torch.uint8, device=dev)
+            self.p.set_v2x_obstacles(pl.v2x_obstacle_params(what=obstacles), self.d_hv.data_ptr(), self.d_vx.data_ptr(), self.d_vy.data_ptr(),
+                                     self.d_os.data_ptr())
 
     def episode_ms(self, graph=True):
         st = torch.cuda.current_stream()
@@ -130,8 +143,19 @@ class Arm:
         e1.record(st); torch.cuda.synchronize()
         return e0.elapsed_time(e1) * 1e3 / launches
 
+    def obstacles_us(self, launches=50):
+        """dp_v2x_obstacles_dev alone (cycle 5) on the world and the last records the last episode left"""
+        st = torch.cuda.current_stream()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record(st)
+        for _ in range(launches):
+            self.p.v2x_obstacles_dev(self.n, self.d_h.data_ptr(), self.d_x.data_ptr(), self.d_y.data_ptr(), self.d_r[-1].data_ptr(), 5,
+                                     stream=st.cuda_stream)
+        e1.record(st); torch.cuda.synchronize()
+        return e0.elapsed_time(e1) * 1e3 / launches
+
     def close(self):
-        self.p.set_v2x_traffic(None, None); self.p.set_v2x_world(None, 0, None); self.p.set_lane_change(None, None); self.p.set_agent_model(None, None); self.p.set_metrics(None, None); self.p.close()
+        self.p.set_v2x_obstacles(None, None, None, None, None); self.p.set_v2x_traffic(None, None); self.p.set_v2x_world(None, 0, None); self.p.set_lane_change(None, None); self.p.set_agent_model(None, None); self.p.set_metrics(None, None); self.p.close()
 
 
 def alternate(arms, *measures):
@@ -404,8 +428,33 @@ def bench_traffic():
     return out
 
 
+def bench_obstacles():
+    N, kind, cycles = 4096, "highway", 25
+    out = {"scenes": N, "max_obs": 14, "agents": 10, "card": card(), "episode": {}, "obstacles_launch": {}}
+    mk = lambda what: Arm(kind, N, 10, cycles, v2x=1, obstacles=what, max_obs=14)   # noqa: E731
+    arms = {"off": mk(None), "what0": mk(0), "what7": mk(7)}
+    warm(arms)
+    ep, = alternate(arms, Arm.episode_ms)
+    same = arms["off"].d_r.cpu().numpy().tobytes() == arms["what0"].d_r.cpu().numpy().tobytes()
+    assert same, "what = 0 records differ from the disarmed ones"
+    differ = arms["off"].d_r.cpu().numpy().tobytes() != arms["what7"].d_r.cpu().numpy().tobytes()
+    out["episode"]["%s_%dx%d" % (kind, N, cycles)] = {
+        "cycles": cycles, "ms_off": summary(ep["off"]), "ms_what0": summary(ep["what0"]), "ms_what7": summary(ep["what7"]),
+        "what0_over_off": ratio(ep["what0"], ep["off"]), "what7_over_off": ratio(ep["what7"], ep["off"]),
+        "records_identical_off_what0": same, "records_differ_off_what7": differ, "target_what0_over_off": 1.05,
+        "target_met": ratio(ep["what0"], ep["off"]) <= 1.05}
+    for name in ("what0", "what7"):
+        a = arms[name]
+        a.obstacles_us()
+        us = [a.obstacles_us() for _ in range(REPS * ROUNDS)]
+        out["obstacles_launch"]["%s_%s_%d" % (name, kind, N)] = {"us_per_launch": summary(us), "launches_per_window": 50}
+    close(arms)
+    return out
+
+
 if __name__ == "__main__":
-    benches = {"metrics": bench_metrics, "agents": bench_agents, "lane_change": bench_lane_change, "v2x": bench_v2x, "traffic": bench_traffic}
+    benches = {"metrics": bench_metrics, "agents": bench_agents, "lane_change": bench_lane_change, "v2x": bench_v2x, "traffic": bench_traffic,
+               "obstacles": bench_obstacles}
     ap = argparse.ArgumentParser(description=__doc__.split("\n")[0])
     ap.add_argument("model", choices=list(benches))
     print(json.dumps(benches[ap.parse_args().model]()))

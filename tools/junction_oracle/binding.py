@@ -51,16 +51,18 @@ class JunctionOracle:
                                       abi.ptr(ox), abi.ptr(oy), abi.ptr(rec), abi.ptr(last_path)) == 0
 
     def run_closed_loop(self, hdr, agents, cycles, wp=None, paths=False, threads=1, metrics=None, agent_model=None, lane_change=None,
-                        v2x=None, traffic=None):
+                        v2x=None, traffic=None, obstacles=None):
         """hdr[n], agents[n][max_obs] (copied; the final world is returned), through jo_run_closed_loop; metrics = MetricsParams: the
         episode metrics of every world under "metrics"; agent_model = (AgentModelParams, v0[n][max_obs]): the reactive agents;
         lane_change = LaneChangeParams (with agent_model): their lane changes, the final states under "lane_change_state";
         v2x = (V2xWorldParams, events with spec / wp_x / wp_y): the V2X events, the rows under "v2x_stats" and the flags of the last
         launch under "v2x_flags"; traffic = V2xTrafficParams (with agent_model and v2x): the agents obey the V2X events, the rows
-        under "v2x_traffic"
+        under "v2x_traffic"; obstacles = V2xObstacleParams (with v2x): every cycle runs on the view of the V2X road users, the logs
+        record the views, the rows under "v2x_obstacles"
         """
         assert lane_change is None or agent_model is not None
         assert traffic is None or (agent_model is not None and v2x is not None)
+        assert obstacles is None or v2x is not None
         am, v0 = agent_model if agent_model is not None else (None, None)
         met = lcs = None
         if metrics is not None:
@@ -88,6 +90,10 @@ class JunctionOracle:
         if traffic is not None:
             tstats = np.frombuffer(np.full(hdr.shape[0] * abi.v2x_traffic_stats.itemsize, 0xAB, np.uint8).tobytes(), abi.v2x_traffic_stats).copy()
         models += (ref(traffic), abi.ptr(tstats))
+        ostats = None
+        if obstacles is not None:
+            ostats = np.frombuffer(np.full(hdr.shape[0] * abi.v2x_obstacle_stats.itemsize, 0xAB, np.uint8).tobytes(), abi.v2x_obstacle_stats).copy()
+        models += (ref(obstacles), abi.ptr(ostats))
         f = self.lib.jo_run_closed_loop
         f.restype = C.c_longlong
         # ob._closed_loop passes the arrays every closed loop has; the model arguments follow them
@@ -101,7 +107,27 @@ class JunctionOracle:
             o["v2x_flags"], o["v2x_stats"] = vflags, vstats
         if tstats is not None:
             o["v2x_traffic"] = tstats
+        if ostats is not None:
+            o["v2x_obstacles"] = ostats
         return o
+
+    def v2x_obstacles_view(self, op, ev, hdr, ox, oy, k, stats, prev=None, tally=False, view=None):
+        """one obstacles launch of cycle k for every world (jo_v2x_obstacles_view): stats in place; returns the view (hdr, ox, oy),
+        built into `view` when given (slots beyond the view's n_obs keep what they held), fresh zero arrays otherwise"""
+        spec, wx, wy = self._v2x_inputs(ev)
+        hdr, ox, oy = np.ascontiguousarray(hdr), np.ascontiguousarray(ox, np.float64), np.ascontiguousarray(oy, np.float64)
+        n, max_obs = ox.shape
+        assert spec.shape == hdr.shape == (n,) and oy.shape == ox.shape and stats.dtype == abi.v2x_obstacle_stats and stats.shape == (n,)
+        prev = None if prev is None else np.ascontiguousarray(prev)
+        hv, vx, vy = view if view is not None else (np.zeros(n, abi.scene_hdr), np.zeros((n, max_obs)), np.zeros((n, max_obs)))
+        assert self.lib.jo_v2x_obstacles_view(C.byref(op), C.c_int(max_obs), C.c_int(n), abi.ptr(spec), abi.ptr(wx), abi.ptr(wy), abi.ptr(hdr),
+                                              abi.ptr(ox), abi.ptr(oy), abi.ptr(prev), C.c_int(k), C.c_int(int(tally)), abi.ptr(hv),
+                                              abi.ptr(vx), abi.ptr(vy), abi.ptr(stats)) == 0
+        return hv, vx, vy
+
+    def v2x_obstacles_sizeof(self):
+        """sizeof(dp_v2x_obstacle_params), sizeof(dp_v2x_obstacle_stats)"""
+        return int(self.lib.jo_v2x_obstacles_sizeof(0)), int(self.lib.jo_v2x_obstacles_sizeof(1))
 
     def traffic_step(self, tp, ev, k, hdr, agents, ox, oy, v0, am, ts, rec=None, last_path=None, lp=None, lcs=None, wp=None):
         """one world step of cycle k with the agents obeying the V2X events (jo_traffic_step), everything in place; rec None: the

@@ -4,7 +4,8 @@
 // world step may carry: the episode metrics of episode_metrics.cpp (alone: jo_metrics_step), the reactive agents of
 // agent_model.cpp (alone: jo_react_step) and their lane changes of lane_change.cpp (alone: jo_lane_change_step); and the V2X launch
 // of v2x_world.cpp between a cycle and its world step (alone: jo_v2x_cycle, its data builder: jo_v2x_data); and the agents that
-// obey the V2X events of v2x_traffic.cpp (alone: jo_traffic_step, its candidates: jo_traffic_leader / jo_traffic_side).
+// obey the V2X events of v2x_traffic.cpp (alone: jo_traffic_step, its candidates: jo_traffic_leader / jo_traffic_side); and the view of
+// the V2X road users every cycle runs on, v2x_obstacles.cpp (alone: jo_v2x_obstacles_view).
 #include <algorithm>
 #include <atomic>
 #include <cstring>
@@ -13,6 +14,7 @@
 #include "agent_model.h"
 #include "episode_metrics.h"
 #include "lane_change.h"
+#include "v2x_obstacles.h"
 #include "v2x_traffic.h"
 #include "v2x_world.h"
 #include "world_junction.h"
@@ -60,17 +62,20 @@ int jo_world_step(const dp_params* p, const dp_world_params* wp, int n, int max_
 // after every world step; am / v0[n][max_obs] the reactive agents of section 12, before every world step; lp / lcs[n][max_obs]
 // (with am) their lane changes of section 13, states initialised by the placement step and holding the final states; vp / spec[n]
 // (wp_x / wp_y[n_wp], flags[n] nullable, stats[n]) the V2X events of section 14 between every cycle and its world step; tp / ts[n]
-// (with am and vp) the agents that obey them, section 15
+// (with am and vp) the agents that obey them, section 15; op / os[n] (with vp) the V2X road users the planner sees, section 16: every
+// cycle runs on the view its obstacles launch builds, and hdr_log / obs_log_* record the views
 long long jo_run_closed_loop(const dp_params* p, const dp_world_params* wp, int n, int cycles, int max_obs, dp_scene_hdr* hdr,
                              dp_agent* agents, double* ox, double* oy, dp_plan_record* rec, dp_scene_hdr* hdr_log, double* obs_log_x,
                              double* obs_log_y, double* path_xy, dp_carry* carry_out, double* last_path_out, int threads,
                              int32_t* ub_scene, const dp_metrics_params* mp, dp_episode_metrics* met, const dp_agent_model_params* am,
                              const double* v0, const dp_lane_change_params* lp, dp_lane_change_state* lcs, const dp_v2x_world_params* vp,
                              const dp_v2x_event_spec* spec, const double* wp_x, const double* wp_y, int n_wp, dp_v2x_flags* flags,
-                             dp_v2x_episode_stats* stats, const dp_v2x_traffic_params* tp, dp_v2x_traffic_stats* ts) {
+                             dp_v2x_episode_stats* stats, const dp_v2x_traffic_params* tp, dp_v2x_traffic_stats* ts,
+                             const dp_v2x_obstacle_params* op, dp_v2x_obstacle_stats* os) {
     if (!g_have_map) return -1;
     if ((!mp) != (!met) || (!am) != (!v0) || (!lp) != (!lcs) || (lcs && !v0) || (!vp) != (!spec) || (spec && !stats)) return -1;
     if ((!tp) != (!ts) || (ts && (!v0 || !spec))) return -1;
+    if ((!op) != (!os) || (os && !spec)) return -1;
     if (threads < 1) threads = 1;
     std::vector<double> wla, wlo;
     if (spec) wp_gps(*p, wp_x, wp_y, n_wp, wla, wlo);
@@ -89,15 +94,23 @@ long long jo_run_closed_loop(const dp_params* p, const dp_world_params* wp, int 
             if (ts) traffic::init(ts[s]);
             std::vector<int> kinds((size_t)max_obs);
             std::vector<dp_agent> a1((size_t)max_obs);
+            // the cycle's inputs: the world, or with os the view of it (slots beyond the view's n_obs keep what they held)
+            dp_scene_hdr hv{};
+            std::vector<double> vx((size_t)max_obs), vy((size_t)max_obs);
             for (int c = 0; c < cycles; ++c) {
                 const size_t e = (size_t)c * n + s;
-                if (hdr_log) hdr_log[e] = hdr[s];
-                if (obs_log_x) std::memcpy(obs_log_x + e * max_obs, sx, sizeof(double) * max_obs);
-                if (obs_log_y) std::memcpy(obs_log_y + e * max_obs, sy, sizeof(double) * max_obs);
+                if (os) v2xobs::launch(g_map, *op, max_obs, spec[s], wp_x, wp_y, hdr[s], sx, sy, c > 0 ? rec + e - n : nullptr, c, false, &hv,
+                                       vx.data(), vy.data(), os[s]);
+                const dp_scene_hdr& ch = os ? hv : hdr[s];
+                const double* cx = os ? vx.data() : sx;
+                const double* cy = os ? vy.data() : sy;
+                if (hdr_log) hdr_log[e] = ch;
+                if (obs_log_x) std::memcpy(obs_log_x + e * max_obs, cx, sizeof(double) * max_obs);
+                if (obs_log_y) std::memcpy(obs_log_y + e * max_obs, cy, sizeof(double) * max_obs);
                 oracle::CycleOut o{};
                 o.rec = rec + e;
                 o.path_xy = path_xy ? path_xy + e * 400 : nullptr;
-                oracle::cycle(g_map.m, *p, hdr[s], sx, sy, st, o, false);
+                oracle::cycle(g_map.m, *p, ch, cx, cy, st, o, false);
                 lub += o.ub_hits;
                 if (spec) v2x::cycle(g_map, *p, *vp, spec[s], wla.data(), wlo.data(), hdr[s], c, rec + e, stats[s], flags ? flags + s : nullptr);
                 const dp_scene_hdr h0 = hdr[s];
@@ -113,6 +126,8 @@ long long jo_run_closed_loop(const dp_params* p, const dp_world_params* wp, int 
                 if (met) metrics::update(g_map, *wp, *mp, met[s], h0, hdr[s], ag, sx, sy, std::min((int)h0.n_obs, max_obs), rec[e]);
             }
             if (spec) v2x::cycle(g_map, *p, *vp, spec[s], wla.data(), wlo.data(), hdr[s], cycles, nullptr, stats[s], flags ? flags + s : nullptr);
+            if (os) v2xobs::launch(g_map, *op, max_obs, spec[s], wp_x, wp_y, hdr[s], sx, sy, cycles > 0 ? rec + (size_t)(cycles - 1) * n + s : nullptr,
+                                   cycles, true, nullptr, nullptr, nullptr, os[s]);
             if (ub_scene) ub_scene[s] = (int32_t)(lub - lub0);
             if (carry_out) carry_out[s] = st.c;
             if (last_path_out) {
@@ -275,6 +290,22 @@ int jo_traffic_side(const dp_v2x_traffic_params* tp, const dp_agent_model_params
     }
     return 0;
 }
+
+// one obstacles launch of cycle k for every world, as dp_v2x_obstacles_dev runs it: hdr[n] / ox / oy[n][max_obs] the world,
+// prev[n] (nullable) the records of cycle k - 1, views hv[n] / vx / vy[n][max_obs] (not written on the tally), stats[n] in place
+int jo_v2x_obstacles_view(const dp_v2x_obstacle_params* op, int max_obs, int n, const dp_v2x_event_spec* spec, const double* wp_x,
+                          const double* wp_y, const dp_scene_hdr* hdr, const double* ox, const double* oy, const dp_plan_record* prev, int k,
+                          int tally, dp_scene_hdr* hv, double* vx, double* vy, dp_v2x_obstacle_stats* stats) {
+    if (!g_have_map) return -1;
+    for (int s = 0; s < n; ++s) {
+        const size_t o = (size_t)s * max_obs;
+        v2xobs::launch(g_map, *op, max_obs, spec[s], wp_x, wp_y, hdr[s], ox + o, oy + o, prev ? prev + s : nullptr, k, tally != 0,
+                       tally ? nullptr : hv + s, tally ? nullptr : vx + o, tally ? nullptr : vy + o, stats[s]);
+    }
+    return 0;
+}
+
+int jo_v2x_obstacles_sizeof(int which) { return which ? (int)sizeof(dp_v2x_obstacle_stats) : (int)sizeof(dp_v2x_obstacle_params); }
 
 int jo_traffic_sizeof(int which) { return which ? (int)sizeof(dp_v2x_traffic_stats) : (int)sizeof(dp_v2x_traffic_params); }
 
