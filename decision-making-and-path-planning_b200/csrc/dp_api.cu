@@ -9,6 +9,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <initializer_list>
+#include <memory>
 #include <string>
 #include <algorithm>
 #include <atomic>
@@ -70,9 +71,13 @@ struct dp_ctx {
                                                             // hand-stepped world step
     DpObstOpts obst;                                        // dp_world_set_v2x_obstacles: the views every cycle runs on
     cudaStream_t ep_stream = nullptr;
-    cudaGraphExec_t ep_exec = nullptr;
-    const void* ep_key[8] = {}; int ep_dims[3] = {-1, -1, -1};
-    long long ep_launches = 0;
+    // one cached graph per kind of part, (k0 > 0) * 2 + finish: the parts of a long episode update theirs in place, and a
+    // one-call episode (k0 = 0, finish = 1) keeps its own
+    struct EpGraph {
+        cudaGraphExec_t exec = nullptr;
+        const void* key[9] = {}; int dims[5] = {-1, -1, -1, -1, -1};
+        long long launches = 0;
+    } ep[4];
     int ep_graph = 1;                                       // DP_EPISODE_GRAPH=0: enqueue the launches directly
     int ep_last_graph = 0;
     // pipelined submit / wait: inputs of cycle k+1 cross PCIe on the copy stream while cycle k computes
@@ -322,7 +327,7 @@ int dp_destroy(dp_ctx* c) {
     cudaDeviceSynchronize();
     if (c->lc.l2_bytes) { cudaCtxResetPersistingL2Cache(); cudaGetLastError(); }   // hand the map's lines in the L2 set-aside back
     for (void* p : c->map_allocs) cudaFree(p);
-    if (c->ep_exec) cudaGraphExecDestroy(c->ep_exec);
+    for (auto& g : c->ep) if (g.exec) cudaGraphExecDestroy(g.exec);
     if (c->ep_stream) cudaStreamDestroy(c->ep_stream);
     cudaFree(c->d_timeline); cudaFree(c->d_trk);
     cudaFree(c->d_carry); cudaFree(c->d_last); cudaFree(c->d_done); cudaFree(c->d_inflag); cudaFree(c->d_tally); cudaFree(c->d_tally_g);
@@ -345,7 +350,8 @@ int dp_map_upload(dp_ctx* c, const dp_map_desc* m) {
     for (void* p : c->map_allocs) cudaFree(p);
     c->map_allocs.clear();
     c->have_map = false; c->lc.l2_base = nullptr; c->lc.l2_bytes = 0;   // (until the new tables are complete)
-    if (c->ep_exec) { cudaGraphExecDestroy(c->ep_exec); c->ep_exec = nullptr; }   // (a cached episode graph points into the old map)
+    for (auto& g : c->ep)                                   // (a cached episode graph points into the old map)
+        if (g.exec) { cudaGraphExecDestroy(g.exec); g.exec = nullptr; }
     // every map table lives in ONE arena (256-byte aligned pieces), so that a single L2 access-policy window covers the map
     const size_t np = (size_t)m->n_points;
     const size_t arena_bytes = 16 * 256 + np * (8 * 3 + 16 * 2 + 8 * 2 + 8 + 4 * 2 + 2 * 2) + (size_t)m->n_lanes * (4 * 3 + 8 + 4) +
@@ -1296,7 +1302,8 @@ void dp_world_default_params(dp_world_params* p) {
 namespace {
 // the world options are baked into the launches of a cached episode graph: a change drops it
 int drop_episode_graph(dp_ctx* c) {
-    if (c->ep_exec) { cudaGraphExecDestroy(c->ep_exec); c->ep_exec = nullptr; }
+    for (auto& g : c->ep)
+        if (g.exec) { cudaGraphExecDestroy(g.exec); g.exec = nullptr; }
     return DP_OK;
 }
 bool all_finite(std::initializer_list<double> v) {
@@ -1488,98 +1495,182 @@ int dp_world_step_dev(dp_ctx* c, int first, int n, dp_scene_hdr* hdr, dp_agent* 
     return DP_OK;
 }
 namespace {
-// the launches of one closed-loop episode, in order, on st (a capturing stream, or the caller's)
-cudaError_t enqueue_closed_loop(dp_ctx* c, int first, int n, int cycles, dp_scene_hdr* hdr, dp_agent* agents, double* ox, double* oy,
-                                dp_plan_record* rec, dp_scene_hdr* hdr_log, double* olx, double* oly, cudaStream_t st, bool rearm) {
+// the launches of cycles k0 .. k0 + cycles - 1 of a closed-loop episode, in order, on st (a capturing stream, or the caller's):
+// with k0 == 0 the placement step first, with finish the tallies last.  rec / hdr_log / obs_log_* are indexed by the part's own
+// cycle j, every launch gets the episode's cycle k0 + j
+cudaError_t enqueue_closed_loop(dp_ctx* c, int first, int n, int k0, int cycles, int finish, dp_scene_hdr* hdr, dp_agent* agents, double* ox,
+                                double* oy, const dp_plan_record* prev_rec, dp_plan_record* rec, dp_scene_hdr* hdr_log, double* olx, double* oly,
+                                cudaStream_t st, bool rearm) {
     const size_t mo = (size_t)c->max_obs;
     DpWorldBufs b = {n, c->max_obs, hdr, agents, ox, oy, nullptr, c->d_last + (size_t)first * DP_PATH_POINTS};
     cudaError_t e;
     // a replayed graph re-uses its hand-off epochs: the per-scene Decision -> Planning flags start every replay from 0
     if (rearm && (e = cudaMemsetAsync(c->d_done + first, 0, (size_t)n * sizeof(unsigned), st)) != cudaSuccess) return e;
-    c->launches += 1;
-    if ((e = dp_launch_world(c->gmap, c->p, c->world, b, st)) != cudaSuccess) return e;
+    if (k0 == 0) {
+        c->launches += 1;
+        if ((e = dp_launch_world(c->gmap, c->p, c->world, b, st)) != cudaSuccess) return e;
+    }
     // with the V2X road users armed (section 16) every cycle runs on, and the logs record, the view an obstacles launch builds
     const bool obst = c->obst.stats != nullptr;
     dp_scene_hdr* ch = obst ? c->obst.hv : hdr;
     double* cx = obst ? c->obst.vx : ox;
     double* cy = obst ? c->obst.vy : oy;
-    for (int k = 0; k < cycles; ++k) {
+    // the records of the cycle before j (the previous part's last row at j == 0 of a continued episode)
+    auto prev_of = [&](int j) -> const dp_plan_record* { return j > 0 ? rec + (size_t)(j - 1) * n : (k0 > 0 ? prev_rec : nullptr); };
+    for (int j = 0; j < cycles; ++j) {
+        const int k = k0 + j;
         if (obst) {
             c->launches += 1;
-            const dp_plan_record* prev = k > 0 ? rec + (size_t)(k - 1) * n : nullptr;
-            if ((e = dp_launch_world_obstacles(c->gmap, c->v2x, c->obst, n, c->max_obs, hdr, ox, oy, prev, k, false, st)) != cudaSuccess) return e;
+            if ((e = dp_launch_world_obstacles(c->gmap, c->v2x, c->obst, n, c->max_obs, hdr, ox, oy, prev_of(j), k, false, st)) != cudaSuccess) return e;
         }
-        if (hdr_log && (e = cudaMemcpyAsync(hdr_log + (size_t)k * n, ch, (size_t)n * sizeof(dp_scene_hdr), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
-        if (olx && (e = cudaMemcpyAsync(olx + (size_t)k * n * mo, cx, (size_t)n * mo * sizeof(double), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
-        if (oly && (e = cudaMemcpyAsync(oly + (size_t)k * n * mo, cy, (size_t)n * mo * sizeof(double), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
+        if (hdr_log && (e = cudaMemcpyAsync(hdr_log + (size_t)j * n, ch, (size_t)n * sizeof(dp_scene_hdr), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
+        if (olx && (e = cudaMemcpyAsync(olx + (size_t)j * n * mo, cx, (size_t)n * mo * sizeof(double), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
+        if (oly && (e = cudaMemcpyAsync(oly + (size_t)j * n * mo, cy, (size_t)n * mo * sizeof(double), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
         const DpIo io = make_io(c, first, nullptr);
-        if ((e = run_cycle(c, first, n, ch, cx, cy, rec + (size_t)k * n, nullptr, nullptr, nullptr, st, io)) != cudaSuccess) return e;
+        if ((e = run_cycle(c, first, n, ch, cx, cy, rec + (size_t)j * n, nullptr, nullptr, nullptr, st, io)) != cudaSuccess) return e;
         if (c->v2x.spec) {                                  // V2X armed: the flags act on the records before the world step reads them
             c->launches += 1;
-            if ((e = dp_launch_world_v2x(c->gmap, c->p, c->v2x, n, hdr, rec + (size_t)k * n, k, st)) != cudaSuccess) return e;
+            if ((e = dp_launch_world_v2x(c->gmap, c->p, c->v2x, n, hdr, rec + (size_t)j * n, k, st)) != cudaSuccess) return e;
         }
         c->launches += 1;
-        b.rec = rec + (size_t)k * n; b.cycle = k;
+        b.rec = rec + (size_t)j * n; b.cycle = k;
         if ((e = dp_launch_world(c->gmap, c->p, c->world, b, st)) != cudaSuccess) return e;
     }
+    if (!finish) return cudaSuccess;                        // the next part's first launches close the seam
     if (c->v2x.spec) {                                      // the tally: closes the red-crossing check of the last world step
         c->launches += 1;
-        if ((e = dp_launch_world_v2x(c->gmap, c->p, c->v2x, n, hdr, nullptr, cycles, st)) != cudaSuccess) return e;
+        if ((e = dp_launch_world_v2x(c->gmap, c->p, c->v2x, n, hdr, nullptr, k0 + cycles, st)) != cudaSuccess) return e;
     }
     if (obst) {                                             // the tally: the last cycle's bound check, the hits of the final world
         c->launches += 1;
-        const dp_plan_record* prev = cycles > 0 ? rec + (size_t)(cycles - 1) * n : nullptr;
-        if ((e = dp_launch_world_obstacles(c->gmap, c->v2x, c->obst, n, c->max_obs, hdr, ox, oy, prev, cycles, true, st)) != cudaSuccess) return e;
+        if ((e = dp_launch_world_obstacles(c->gmap, c->v2x, c->obst, n, c->max_obs, hdr, ox, oy, prev_of(cycles), k0 + cycles, true, st)) != cudaSuccess)
+            return e;
     }
     return cudaSuccess;
 }
+// capture the part into a graph; with an executable graph of the same shape (the cache key differs only in k0, prev_rec, rec or the
+// log pointers) update it in place, else instantiate a fresh one.  False: no graph on this driver / for these launches
+bool capture_part(dp_ctx* c, dp_ctx::EpGraph& eg, bool update, int first, int n, int k0, int cycles, int finish, dp_scene_hdr* hdr, dp_agent* agents, double* ox,
+                  double* oy, const dp_plan_record* prev_rec, dp_plan_record* rec, dp_scene_hdr* hdr_log, double* olx, double* oly) {
+    if (!c->ep_stream && cudaStreamCreateWithFlags(&c->ep_stream, cudaStreamNonBlocking) != cudaSuccess) return false;
+    dp_launch_prepare(c->lc);                               // function attributes are set outside the capture
+    const long long before = c->launches;
+    cudaGraph_t g = nullptr;
+    cudaError_t e = cudaStreamBeginCapture(c->ep_stream, cudaStreamCaptureModeThreadLocal);
+    if (e == cudaSuccess) {
+        const cudaError_t e1 = enqueue_closed_loop(c, first, n, k0, cycles, finish, hdr, agents, ox, oy, prev_rec, rec, hdr_log, olx, oly,
+                                                   c->ep_stream, true);
+        e = cudaStreamEndCapture(c->ep_stream, &g);
+        if (e1 != cudaSuccess) e = e1;
+    }
+    eg.launches = c->launches - before;
+    c->launches = before;
+    bool updated = false;
+    if (e == cudaSuccess && update && eg.exec) {
+        cudaGraphExecUpdateResultInfo info;
+        updated = cudaGraphExecUpdate(eg.exec, g, &info) == cudaSuccess;
+        if (!updated) cudaGetLastError();                   // refused: a fresh instantiate below
+    }
+    if (e == cudaSuccess && !updated) {
+        if (eg.exec) { cudaGraphExecDestroy(eg.exec); eg.exec = nullptr; }
+        e = cudaGraphInstantiate(&eg.exec, g, 0);
+    }
+    if (g) cudaGraphDestroy(g);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        if (eg.exec) { cudaGraphExecDestroy(eg.exec); eg.exec = nullptr; }
+        return false;
+    }
+    return true;
+}
 }  // namespace
-int dp_run_closed_loop_dev(dp_ctx* c, int first, int n, int cycles, dp_scene_hdr* hdr, dp_agent* agents, double* ox, double* oy,
-                           dp_plan_record* rec, dp_scene_hdr* hdr_log, double* olx, double* oly, void* stream) {
-    if (!c || !hdr || !agents || !ox || !oy || !rec || n < 0 || cycles < 0 || first < 0 || first + n > c->max_scenes)
+int dp_run_closed_loop_part_dev(dp_ctx* c, int first, int n, int k0, int cycles, int finish, dp_scene_hdr* hdr, dp_agent* agents, double* ox,
+                                double* oy, const dp_plan_record* prev_rec, dp_plan_record* rec, dp_scene_hdr* hdr_log, double* olx, double* oly,
+                                void* stream) {
+    if (!c || !hdr || !agents || !ox || !oy || !rec || n < 0 || cycles < 0 || first < 0 || first + n > c->max_scenes || k0 < 0 ||
+        (finish != 0 && finish != 1))
         return fail(DP_ERR_ARG, "dp_run_closed_loop_dev: bad argument");
     if (!c->have_map) return fail(DP_ERR_STATE, "dp_run_closed_loop_dev: map not uploaded");
     if (c->submitted != c->waited) return fail(DP_ERR_STATE, "dp_run_closed_loop_dev: submitted cycles in flight, call dp_cycle_wait first");
     if (c->v2x.spec && n > c->v2x.n) return fail(DP_ERR_ARG, "dp_run_closed_loop_dev: more scenes than the armed V2X specifications");
     if (c->obst.stats && c->tracks_T > 0)
         return fail(DP_ERR_STATE, "dp_run_closed_loop_dev: the V2X road users are armed and predicted tracks are set");
+    if (c->obst.stats && k0 > 0 && !prev_rec)
+        return fail(DP_ERR_ARG, "dp_run_closed_loop_part_dev: the V2X road users are armed and a continued part has no prev_rec");
     CK(cudaSetDevice(c->device));
     c->ep_last_graph = 0;
     if (n == 0) return DP_OK;
+    if (!(c->obst.stats && k0 > 0)) prev_rec = nullptr;     // (not read: out of the cache key)
     // the graph holds the warp-kernel launches of a plain context (no gather armed, no record mirrors, no predicted tracks)
     const bool plain = c->kernel == 0 && c->tracks_T == 0 && !armed_any(c->armed);
     if (c->ep_graph && plain) {
-        const void* key[8] = {hdr, agents, ox, oy, rec, hdr_log, olx, oly};
-        const int dims[3] = {first, n, cycles};
-        if (!c->ep_exec || memcmp(key, c->ep_key, sizeof(key)) != 0 || memcmp(dims, c->ep_dims, sizeof(dims)) != 0) {
-            if (c->ep_exec) { cudaGraphExecDestroy(c->ep_exec); c->ep_exec = nullptr; }
-            if (!c->ep_stream) CK(cudaStreamCreateWithFlags(&c->ep_stream, cudaStreamNonBlocking));
-            dp_launch_prepare(c->lc);                       // function attributes are set outside the capture
-            const long long before = c->launches;
-            cudaGraph_t g = nullptr;
-            cudaError_t e = cudaStreamBeginCapture(c->ep_stream, cudaStreamCaptureModeThreadLocal);
-            if (e == cudaSuccess) {
-                const cudaError_t e1 = enqueue_closed_loop(c, first, n, cycles, hdr, agents, ox, oy, rec, hdr_log, olx, oly, c->ep_stream, true);
-                e = cudaStreamEndCapture(c->ep_stream, &g);
-                if (e1 != cudaSuccess) e = e1;
-            }
-            if (e == cudaSuccess) e = cudaGraphInstantiate(&c->ep_exec, g, 0);
-            if (g) cudaGraphDestroy(g);
-            c->ep_launches = c->launches - before;
-            c->launches = before;
-            if (e != cudaSuccess) {                         // no graph on this driver / for these launches: enqueue them directly from now on
-                cudaGetLastError();
-                c->ep_exec = nullptr; c->ep_graph = 0;
-            } else { memcpy(c->ep_key, key, sizeof(key)); memcpy(c->ep_dims, dims, sizeof(dims)); }
+        const void* key[9] = {hdr, agents, ox, oy, rec, hdr_log, olx, oly, prev_rec};
+        const int dims[5] = {first, n, cycles, finish, k0};
+        // the shape: everything but k0, prev_rec, rec and the logs; a part of the same shape updates the cached graph in place
+        dp_ctx::EpGraph& eg = c->ep[(k0 > 0) * 2 + finish];
+        const bool same_shape = eg.exec && memcmp(key, eg.key, 4 * sizeof(void*)) == 0 && memcmp(dims, eg.dims, 4 * sizeof(int)) == 0;
+        if (!eg.exec || memcmp(key, eg.key, sizeof(key)) != 0 || memcmp(dims, eg.dims, sizeof(dims)) != 0) {
+            if (capture_part(c, eg, same_shape, first, n, k0, cycles, finish, hdr, agents, ox, oy, prev_rec, rec, hdr_log, olx, oly)) {
+                memcpy(eg.key, key, sizeof(key)); memcpy(eg.dims, dims, sizeof(dims));
+            } else c->ep_graph = 0;                         // enqueue the launches directly from now on
         }
-        if (c->ep_exec) {
-            CK(cudaGraphLaunch(c->ep_exec, (cudaStream_t)stream));
-            c->launches += c->ep_launches;
+        if (eg.exec) {
+            CK(cudaGraphLaunch(eg.exec, (cudaStream_t)stream));
+            c->launches += eg.launches;
             c->ep_last_graph = 1;
             return DP_OK;
         }
     }
-    CK(enqueue_closed_loop(c, first, n, cycles, hdr, agents, ox, oy, rec, hdr_log, olx, oly, (cudaStream_t)stream, false));
+    CK(enqueue_closed_loop(c, first, n, k0, cycles, finish, hdr, agents, ox, oy, prev_rec, rec, hdr_log, olx, oly, (cudaStream_t)stream, false));
+    return DP_OK;
+}
+int dp_run_closed_loop_dev(dp_ctx* c, int first, int n, int cycles, dp_scene_hdr* hdr, dp_agent* agents, double* ox, double* oy,
+                           dp_plan_record* rec, dp_scene_hdr* hdr_log, double* olx, double* oly, void* stream) {
+    return dp_run_closed_loop_part_dev(c, first, n, 0, cycles, 1, hdr, agents, ox, oy, nullptr, rec, hdr_log, olx, oly, stream);
+}
+int dp_world_fork_dev(dp_ctx* c, int first, int n, const int32_t* src, int dst, int count, dp_scene_hdr* hdr, dp_agent* agents, double* ox,
+                      double* oy, dp_plan_record* prev_rec, void* stream) {
+    if (!c || !hdr || !agents || !ox || !oy || n < 0 || first < 0 || first + n > c->max_scenes || count < 0 || (count > 0 && !src) || dst < 0 ||
+        dst > n - count)
+        return fail(DP_ERR_ARG, "dp_world_fork_dev: bad argument");
+    if (c->v2x.spec && n > c->v2x.n) return fail(DP_ERR_ARG, "dp_world_fork_dev: more scenes than the armed V2X specifications");
+    if (c->obst.stats && !prev_rec) return fail(DP_ERR_ARG, "dp_world_fork_dev: the V2X road users are armed and prev_rec is NULL");
+    for (int j = 0; j < count; ++j)
+        if (src[j] < 0 || src[j] >= n || (src[j] >= dst && src[j] < dst + count))
+            return fail(DP_ERR_ARG, "dp_world_fork_dev: a source outside [0, n) or inside [dst, dst + count)");
+    if (c->tracks_T > 0) return fail(DP_ERR_STATE, "dp_world_fork_dev: predicted tracks are set (dp_clear_tracks first)");
+    if (c->submitted != c->waited) return fail(DP_ERR_STATE, "dp_world_fork_dev: submitted cycles in flight, call dp_cycle_wait first");
+    if (count == 0) return DP_OK;
+    CK(cudaSetDevice(c->device));
+    const std::unique_ptr<DpForkArgs> ap(new DpForkArgs);  // (16.6 KB: off the stack; every launch copies it into its parameters)
+    DpForkArgs& fa = *ap;
+    fa.n_seg = 0;
+    const size_t mo = (size_t)c->max_obs;
+    auto seg = [&](const void* base, size_t bytes) {
+        unsigned w = 16;
+        while (w > 1 && (((uintptr_t)base | bytes) & (w - 1))) w >>= 1;
+        fa.seg[fa.n_seg++] = DpForkSeg{(unsigned char*)base, (unsigned)bytes, w};
+    };
+    // the caller's world, the context's carry slot and carried path, then every per-world buffer of the armed models
+    seg(hdr, sizeof(dp_scene_hdr)); seg(agents, mo * sizeof(dp_agent)); seg(ox, mo * sizeof(double)); seg(oy, mo * sizeof(double));
+    if (prev_rec) seg(prev_rec, sizeof(dp_plan_record));
+    seg(c->d_carry + first, sizeof(dp_carry)); seg(c->d_last + (size_t)first * DP_PATH_POINTS, DP_PATH_POINTS * sizeof(double2));
+    if (c->world.met) seg(c->world.met, sizeof(dp_episode_metrics));
+    if (c->world.v0) seg(c->world.v0, mo * sizeof(double));
+    if (c->world.lcs) seg(c->world.lcs, mo * sizeof(dp_lane_change_state));
+    if (c->v2x.spec) {
+        seg(c->v2x.spec, sizeof(dp_v2x_event_spec)); seg(c->v2x.stats, sizeof(dp_v2x_episode_stats));
+        if (c->v2x.flags) seg(c->v2x.flags, sizeof(dp_v2x_flags));
+    }
+    if (c->world.ts) seg(c->world.ts, sizeof(dp_v2x_traffic_stats));
+    if (c->obst.stats) seg(c->obst.stats, sizeof(dp_v2x_obstacle_stats));
+    for (int j0 = 0; j0 < count; j0 += DP_FORK_MAX_SRC) {
+        fa.count = std::min(count - j0, DP_FORK_MAX_SRC);
+        fa.dst = dst + j0;
+        memcpy(fa.src, src + j0, (size_t)fa.count * sizeof(int32_t));
+        c->launches += 1;
+        CK(dp_launch_world_fork(fa, (cudaStream_t)stream));
+    }
     return DP_OK;
 }
 int dp_closed_loop_is_graph(dp_ctx* c) { return c ? c->ep_last_graph : 0; }

@@ -63,6 +63,18 @@ struct DpObstOpts {
 // prev: the records of cycle - 1 (nullptr at cycle 0); tally: the row only
 cudaError_t dp_launch_world_obstacles(const DevMap& m, const DpV2xOpts& v, const DpObstOpts& o, int n, int max_obs, const dp_scene_hdr* hdr,
                                       const double* ox, const double* oy, const dp_plan_record* prev, int cycle, bool tally, cudaStream_t st);
+// forking worlds (dp_world_fork.cu, include/dmpp_b200.h section 17): one launch copies world src[j] to world dst + j, j < count, in
+// every segment; a segment is a per-world array at base with `bytes` per world, copied in words of `width` bytes (16, 8, 4 or 1:
+// the largest that divides both base and bytes).  The block travels in the kernel parameters (16.6 KB)
+#define DP_FORK_MAX_SEG 16
+#define DP_FORK_MAX_SRC 4096
+struct DpForkSeg { unsigned char* base; unsigned bytes, width; };
+struct DpForkArgs {
+    DpForkSeg seg[DP_FORK_MAX_SEG];
+    int n_seg, count, dst;
+    int32_t src[DP_FORK_MAX_SRC];
+};
+cudaError_t dp_launch_world_fork(const DpForkArgs& a, cudaStream_t st);
 cudaError_t dp_launch_v2x(const DevMap& m, const dp_params& p, int n, const dp_scene_hdr* hdr, const dp_v2x_data* v2x, const double* wp_lat,
                           const double* wp_lng, int mode, dp_v2x_flags* out, cudaStream_t st);
 cudaError_t dp_launch_v2x_apply(int n, const dp_v2x_flags* flags, dp_plan_record* rec, cudaStream_t st);

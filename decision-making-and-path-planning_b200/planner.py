@@ -29,7 +29,7 @@ SYMBOLS = [
     "dp_metrics_default_params", "dp_world_set_metrics", "dp_agent_model_default_params", "dp_world_set_agent_model",
     "dp_lane_change_default_params", "dp_world_set_lane_change", "dp_world_set_v2x", "dp_v2x_world_dev",
     "dp_v2x_traffic_default_params", "dp_world_set_v2x_traffic", "dp_v2x_obstacle_default_params", "dp_world_set_v2x_obstacles",
-    "dp_v2x_obstacles_dev",
+    "dp_v2x_obstacles_dev", "dp_run_closed_loop_part_dev", "dp_world_fork_dev",
     "dp_gather_create", "dp_gather_attach", "dp_gather_arm", "dp_gather_chain", "dp_gather_arm_deferred", "dp_gather_set_lag", "dp_gather_flush", "dp_gather_disarm", "dp_gather_wait", "dp_gather_buffer", "dp_gather_destroy",
 ]
 
@@ -46,6 +46,9 @@ def load():
         _lib.dp_last_error.restype = C.c_char_p
         _lib.dp_launch_count.restype = C.c_int64
         _lib.dp_launch_count.argtypes = [C.c_void_p]
+        vp, i = C.c_void_p, C.c_int
+        _lib.dp_run_closed_loop_part_dev.argtypes = [vp, i, i, i, i, i] + [vp] * 10
+        _lib.dp_world_fork_dev.argtypes = [vp, i, i, vp, i, i] + [vp] * 6
     return _lib
 
 
@@ -323,6 +326,22 @@ class Planner:
                                             C.c_void_p(d_obs_log_x or 0), C.c_void_p(d_obs_log_y or 0), C.c_void_p(stream)),
             "dp_run_closed_loop_dev")
 
+    def run_closed_loop_part_dev(self, n, k0, cycles, finish, d_hdr, d_agents, d_ox, d_oy, d_rec, d_prev_rec=None, d_hdr_log=None,
+                                 d_obs_log_x=None, d_obs_log_y=None, first=0, stream=0):
+        """cycles k0 .. k0 + cycles - 1 of an episode (include/dmpp_b200.h section 17); finish: the tallies after the last step"""
+        _ck(self.lib.dp_run_closed_loop_part_dev(self.ctx, first, n, k0, cycles, int(finish), d_hdr, d_agents, d_ox, d_oy, d_prev_rec,
+                                                 d_rec, d_hdr_log, d_obs_log_x, d_obs_log_y, stream), "dp_run_closed_loop_part_dev")
+
+    def world_fork_dev(self, n, src, dst, d_hdr, d_agents, d_ox, d_oy, d_prev_rec=None, first=0, stream=0):
+        """world dst + j becomes a copy of world src[j] in every per-world buffer (include/dmpp_b200.h section 17)"""
+        src = np.ascontiguousarray(src, np.int32)
+        _ck(self.lib.dp_world_fork_dev(self.ctx, first, n, src.ctypes.data if src.size else None, dst, src.size, d_hdr, d_agents, d_ox,
+                                       d_oy, d_prev_rec, stream), "dp_world_fork_dev")
+
+    def episode(self, hdr, agents, metrics=None, agent_model=None, lane_change=None, v2x=None, traffic=None, obstacles=None):
+        """an episode to run in parts (Episode): the models are armed as run_closed_loop arms them, until Episode.close()"""
+        return Episode(self, hdr, agents, metrics, agent_model, lane_change, v2x, traffic, obstacles)
+
     def closed_loop_is_graph(self):
         return bool(self.lib.dp_closed_loop_is_graph(self.ctx))
 
@@ -338,100 +357,21 @@ class Planner:
         this call, the rows are returned under "v2x_stats" and the flags of the last launch under "v2x_flags".  traffic: None, or
         V2xTrafficParams (needs agent_model and v2x): the agents obey the V2X events for this call, and their rows are returned
         under "v2x_traffic".  obstacles: None, or V2xObstacleParams (needs v2x): every cycle runs on a view of the world with the V2X
-        road users in it for this call (the logs record the views), and the rows are returned under "v2x_obstacles"."""
-        n, mo = agents.shape
-        assert lane_change is None or agent_model is not None, "lane changes run on the reactive agents"
-        assert traffic is None or (agent_model is not None and v2x is not None), "the agents obey the V2X events on the reactive agents"
-        assert obstacles is None or v2x is not None, "the planner sees the V2X road users of the armed V2X events"
-        assert mo == self.max_obs and hdr.shape == (n,)
-        sizes = {"hdr": n * 128, "agents": n * mo * 32, "ox": n * mo * 8, "oy": n * mo * 8, "rec": cycles * n * 128,
-                 "hdr_log": cycles * n * 128, "obs_log_x": cycles * n * mo * 8, "obs_log_y": cycles * n * mo * 8}
-        if metrics is not None:
-            sizes["metrics"] = n * abi.episode_metrics.itemsize
-        if agent_model is not None:
-            am, v0 = agent_model
-            v0 = np.ascontiguousarray(v0, np.float64)
-            assert v0.shape == (n, mo)
-            sizes["v0"] = n * mo * 8
-        if lane_change is not None:
-            sizes["lane_change_state"] = n * mo * abi.lane_change_state.itemsize
-        if v2x is not None:
-            vp, ev = v2x
-            spec, wx, wy = np.ascontiguousarray(ev.spec), np.ascontiguousarray(ev.wp_x, np.float64), np.ascontiguousarray(ev.wp_y, np.float64)
-            assert spec.dtype == abi.v2x_event_spec and spec.shape == (n,) and wx.shape == wy.shape
-            sizes.update(v2x_spec=n * spec.itemsize, v2x_wp_x=max(wx.nbytes, 8), v2x_wp_y=max(wy.nbytes, 8),
-                         v2x_flags=n * abi.v2x_flags.itemsize, v2x_stats=n * abi.v2x_episode_stats.itemsize)
-        if traffic is not None:
-            sizes["v2x_traffic"] = n * abi.v2x_traffic_stats.itemsize
-        if obstacles is not None:
-            sizes.update(v2x_hdr_view=n * 128, v2x_ox_view=n * mo * 8, v2x_oy_view=n * mo * 8, v2x_obstacles=n * abi.v2x_obstacle_stats.itemsize)
-        d = {}
+        road users in it for this call (the logs record the views), and the rows are returned under "v2x_obstacles".
+        One Episode, one finishing part."""
+        ep = self.episode(hdr, agents, metrics, agent_model, lane_change, v2x, traffic, obstacles)
         try:
-            for k, b in sizes.items():
-                if log or not k.endswith(("_log", "_log_x", "_log_y")):
-                    p = C.c_void_p()
-                    _ck(self.lib.dp_dev_alloc(self.ctx, C.byref(p), C.c_size_t(b)), "dp_dev_alloc")
-                    d[k] = p.value
-            if metrics is not None:
-                self.set_metrics(metrics, d["metrics"])
-            if agent_model is not None:
-                _ck(self.lib.dp_memcpy_h2d(self.ctx, C.c_void_p(d["v0"]), abi.ptr(v0), C.c_size_t(sizes["v0"]), None), "h2d")
-                self.set_agent_model(am, d["v0"])
-            if lane_change is not None:
-                self.set_lane_change(lane_change, d["lane_change_state"])
-            if v2x is not None:
-                for k, a in (("v2x_spec", spec), ("v2x_wp_x", wx), ("v2x_wp_y", wy)):
-                    _ck(self.lib.dp_memcpy_h2d(self.ctx, C.c_void_p(d[k]), abi.ptr(a), C.c_size_t(a.nbytes), None), "h2d")
-                _ck(self.lib.dp_stream_sync(self.ctx, None), "sync")
-                self.set_v2x_world(vp, n, d["v2x_spec"], d["v2x_wp_x"], d["v2x_wp_y"], wx.size, d["v2x_flags"], d["v2x_stats"])
-            if traffic is not None:
-                self.set_v2x_traffic(traffic, d["v2x_traffic"])
-            if obstacles is not None:
-                self.set_v2x_obstacles(obstacles, d["v2x_hdr_view"], d["v2x_ox_view"], d["v2x_oy_view"], d["v2x_obstacles"])
-            h0, a0 = np.ascontiguousarray(hdr), np.ascontiguousarray(agents)
-            for _ in range(repeat):
-                self.reset(0, n)
-                _ck(self.lib.dp_memcpy_h2d(self.ctx, C.c_void_p(d["hdr"]), abi.ptr(h0), C.c_size_t(sizes["hdr"]), None), "h2d")
-                _ck(self.lib.dp_memcpy_h2d(self.ctx, C.c_void_p(d["agents"]), abi.ptr(a0), C.c_size_t(sizes["agents"]), None), "h2d")
-                _ck(self.lib.dp_stream_sync(self.ctx, None), "sync")
-                self.run_closed_loop_dev(n, cycles, d["hdr"], d["agents"], d["ox"], d["oy"], d["rec"], d.get("hdr_log"),
-                                         d.get("obs_log_x"), d.get("obs_log_y"))
-                _ck(self.lib.dp_stream_sync(self.ctx, None), "sync")
-            o = {"hdr": np.zeros(n, abi.scene_hdr), "agents": np.zeros((n, mo), abi.agent), "ox": np.zeros((n, mo)), "oy": np.zeros((n, mo)),
-                 "rec": np.zeros((cycles, n), abi.plan_record)}
-            if log:
-                o.update(hdr_log=np.zeros((cycles, n), abi.scene_hdr), obs_log_x=np.zeros((cycles, n, mo)), obs_log_y=np.zeros((cycles, n, mo)))
-            if metrics is not None:
-                o["metrics"] = np.zeros(n, abi.episode_metrics)
-            if lane_change is not None:
-                o["lane_change_state"] = np.zeros((n, mo), abi.lane_change_state)
-            if v2x is not None:
-                o["v2x_flags"], o["v2x_stats"] = np.zeros(n, abi.v2x_flags), np.zeros(n, abi.v2x_episode_stats)
-            if traffic is not None:
-                o["v2x_traffic"] = np.zeros(n, abi.v2x_traffic_stats)
-            if obstacles is not None:
-                o["v2x_obstacles"] = np.zeros(n, abi.v2x_obstacle_stats)
-            for k in o:
-                _ck(self.lib.dp_memcpy_d2h(self.ctx, abi.ptr(o[k]), C.c_void_p(d[k]), C.c_size_t(sizes[k]), None), "d2h")
-            _ck(self.lib.dp_stream_sync(self.ctx, None), "sync")
-            o["carry"], o["last_path"] = self.download_carry(0, n)
-            o["graph"] = self.closed_loop_is_graph()
+            for r in range(repeat):
+                if r:
+                    ep.restart()
+                o = ep.run(cycles, finish=True, log=log)
+            st = ep.state()
+            graph = st.pop("graph")
+            o = {**{k: st.pop(k) for k in ("hdr", "agents", "ox", "oy")}, **o, **st}
+            o["graph"] = graph
             return o
         finally:
-            if obstacles is not None:
-                self.set_v2x_obstacles(None, None, None, None, None)
-            if traffic is not None:
-                self.set_v2x_traffic(None, None)
-            if v2x is not None:
-                self.set_v2x_world(None, 0, None)
-            if metrics is not None:
-                self.set_metrics(None, None)
-            if lane_change is not None:
-                self.set_lane_change(None, None)
-            if agent_model is not None:
-                self.set_agent_model(None, None)
-            for p in d.values():
-                self.lib.dp_dev_free(self.ctx, C.c_void_p(p))
+            ep.close()
 
     # ---- pipelined form: at most two cycles in flight, buffers page-locked (see include/dmpp_b200.h) ----
     def submit(self, hdr, ox, oy, rec, first=0):
@@ -557,6 +497,172 @@ class Planner:
         a, b = C.c_double(0), C.c_double(0)
         _ck(self.lib.dp_measure_fma_peak(self.ctx, C.byref(a), C.byref(b)), "dp_measure_fma_peak")
         return a.value, b.value
+
+
+class Episode:
+    """a closed-loop episode run in parts (include/dmpp_b200.h section 17) on worlds 0 .. n-1 of a planner: owns the device buffers
+    of the world and of the armed models, which stay armed until close().  run() continues the episode where the last part left
+    it; fork() copies worlds on the device; state() downloads the world and the rows."""
+
+    def __init__(self, planner, hdr, agents, metrics=None, agent_model=None, lane_change=None, v2x=None, traffic=None, obstacles=None):
+        n, mo = agents.shape
+        assert lane_change is None or agent_model is not None, "lane changes run on the reactive agents"
+        assert traffic is None or (agent_model is not None and v2x is not None), "the agents obey the V2X events on the reactive agents"
+        assert obstacles is None or v2x is not None, "the planner sees the V2X road users of the armed V2X events"
+        assert mo == planner.max_obs and hdr.shape == (n,) and n <= planner.max_scenes
+        self.p, self.lib, self.n, self.mo = planner, planner.lib, n, mo
+        self.models = dict(metrics=metrics, agent_model=agent_model, lane_change=lane_change, v2x=v2x, traffic=traffic, obstacles=obstacles)
+        self.h0, self.a0 = np.ascontiguousarray(hdr), np.ascontiguousarray(agents)
+        sizes = {"hdr": n * 128, "agents": n * mo * 32, "ox": n * mo * 8, "oy": n * mo * 8, "prev_rec": n * 128}
+        if metrics is not None:
+            sizes["metrics"] = n * abi.episode_metrics.itemsize
+        if agent_model is not None:
+            am, v0 = agent_model
+            v0 = np.ascontiguousarray(v0, np.float64)
+            assert v0.shape == (n, mo)
+            sizes["v0"] = n * mo * 8
+        if lane_change is not None:
+            sizes["lane_change_state"] = n * mo * abi.lane_change_state.itemsize
+        if v2x is not None:
+            vp, ev = v2x
+            spec, wx, wy = np.ascontiguousarray(ev.spec), np.ascontiguousarray(ev.wp_x, np.float64), np.ascontiguousarray(ev.wp_y, np.float64)
+            assert spec.dtype == abi.v2x_event_spec and spec.shape == (n,) and wx.shape == wy.shape
+            sizes.update(v2x_spec=n * spec.itemsize, v2x_wp_x=max(wx.nbytes, 8), v2x_wp_y=max(wy.nbytes, 8),
+                         v2x_flags=n * abi.v2x_flags.itemsize, v2x_stats=n * abi.v2x_episode_stats.itemsize)
+        if traffic is not None:
+            sizes["v2x_traffic"] = n * abi.v2x_traffic_stats.itemsize
+        if obstacles is not None:
+            sizes.update(v2x_hdr_view=n * 128, v2x_ox_view=n * mo * 8, v2x_oy_view=n * mo * 8, v2x_obstacles=n * abi.v2x_obstacle_stats.itemsize)
+        self.sizes, self.d = sizes, {}
+        self.k, self._cap = 0, {}                   # the next cycle of the episode; allocated part buffers: key -> (bytes, address)
+        try:
+            for k, b in sizes.items():
+                self.d[k] = self._alloc(b)
+            if metrics is not None:
+                planner.set_metrics(metrics, self.d["metrics"])
+            if agent_model is not None:
+                self._h2d("v0", v0)
+                planner.set_agent_model(am, self.d["v0"])
+            if lane_change is not None:
+                planner.set_lane_change(lane_change, self.d["lane_change_state"])
+            if v2x is not None:
+                for k, a in (("v2x_spec", spec), ("v2x_wp_x", wx), ("v2x_wp_y", wy)):
+                    self._h2d(k, a)
+                _ck(self.lib.dp_stream_sync(planner.ctx, None), "sync")
+                planner.set_v2x_world(vp, n, self.d["v2x_spec"], self.d["v2x_wp_x"], self.d["v2x_wp_y"], wx.size, self.d["v2x_flags"],
+                                      self.d["v2x_stats"])
+            if traffic is not None:
+                planner.set_v2x_traffic(traffic, self.d["v2x_traffic"])
+            if obstacles is not None:
+                planner.set_v2x_obstacles(obstacles, self.d["v2x_hdr_view"], self.d["v2x_ox_view"], self.d["v2x_oy_view"], self.d["v2x_obstacles"])
+            self.restart()
+        except BaseException:
+            self.close()
+            raise
+
+    def _alloc(self, b):
+        p = C.c_void_p()
+        _ck(self.lib.dp_dev_alloc(self.p.ctx, C.byref(p), C.c_size_t(b)), "dp_dev_alloc")
+        return p.value
+
+    def _h2d(self, k, a, offset=0):
+        _ck(self.lib.dp_memcpy_h2d(self.p.ctx, C.c_void_p(self.d[k] + offset), abi.ptr(a), C.c_size_t(a.nbytes), None), "h2d")
+
+    def _d2h(self, a, addr, nbytes):
+        _ck(self.lib.dp_memcpy_d2h(self.p.ctx, abi.ptr(a), C.c_void_p(addr), C.c_size_t(nbytes), None), "d2h")
+
+    def _part_buf(self, k, b):
+        """a device buffer of at least b bytes for the parts' records / logs (grown when a longer part needs it)"""
+        have = self._cap.get(k)
+        if have is None or have[0] < b:
+            if have is not None:
+                self.lib.dp_dev_free(self.p.ctx, C.c_void_p(have[1]))
+            self._cap[k] = have = (b, self._alloc(max(b, 8)))
+        return have[1]
+
+    def restart(self):
+        """back to cycle 0 with the initial world (a fresh carry; the placement step of the next part initialises the rows)"""
+        self.p.reset(0, self.n)
+        self._h2d("hdr", self.h0)
+        self._h2d("agents", self.a0)
+        _ck(self.lib.dp_stream_sync(self.p.ctx, None), "sync")
+        self.k = 0
+
+    def run(self, cycles, finish=False, log=True):
+        """cycles k .. k + cycles - 1 of the episode (k = the cycles run so far), then with finish the tallies.  Returns the part's
+        records rec[cycles][n] and, with log, hdr_log / obs_log_x / obs_log_y [cycles][n](max_obs)"""
+        n, mo, d = self.n, self.mo, self.d
+        rec = self._part_buf("rec", cycles * n * 128)
+        logs = {}
+        if log:
+            logs = {"hdr_log": self._part_buf("hdr_log", cycles * n * 128), "obs_log_x": self._part_buf("obs_log_x", cycles * n * mo * 8),
+                    "obs_log_y": self._part_buf("obs_log_y", cycles * n * mo * 8)}
+        self.p.run_closed_loop_part_dev(n, self.k, cycles, finish, d["hdr"], d["agents"], d["ox"], d["oy"], rec, d["prev_rec"],
+                                        logs.get("hdr_log"), logs.get("obs_log_x"), logs.get("obs_log_y"))
+        _ck(self.lib.dp_stream_sync(self.p.ctx, None), "sync")
+        o = {"rec": np.zeros((cycles, n), abi.plan_record)}
+        if log:
+            o.update(hdr_log=np.zeros((cycles, n), abi.scene_hdr), obs_log_x=np.zeros((cycles, n, mo)), obs_log_y=np.zeros((cycles, n, mo)))
+        self._d2h(o["rec"], rec, o["rec"].nbytes)
+        for k in logs:
+            self._d2h(o[k], logs[k], o[k].nbytes)
+        if cycles > 0:                              # the next part's prev_rec (section 16 reads it; fork copies it)
+            self._h2d("prev_rec", o["rec"][-1])
+        _ck(self.lib.dp_stream_sync(self.p.ctx, None), "sync")
+        self.k += cycles
+        o["graph"] = self.p.closed_loop_is_graph()
+        return o
+
+    def fork(self, src, dst):
+        """world dst + j becomes a copy of world src[j] (dp_world_fork_dev): world, carry, carried path, rows, states and inputs"""
+        d = self.d
+        self.p.world_fork_dev(self.n, src, dst, d["hdr"], d["agents"], d["ox"], d["oy"], d["prev_rec"])
+        _ck(self.lib.dp_stream_sync(self.p.ctx, None), "sync")
+
+    def state(self):
+        """run_closed_loop's dictionary without the records and the logs: the world, the rows and states of the armed models, the
+        carry and the carried path, and whether the last part ran as a graph"""
+        n, mo, m = self.n, self.mo, self.models
+        o = {"hdr": np.zeros(n, abi.scene_hdr), "agents": np.zeros((n, mo), abi.agent), "ox": np.zeros((n, mo)), "oy": np.zeros((n, mo))}
+        if m["metrics"] is not None:
+            o["metrics"] = np.zeros(n, abi.episode_metrics)
+        if m["lane_change"] is not None:
+            o["lane_change_state"] = np.zeros((n, mo), abi.lane_change_state)
+        if m["v2x"] is not None:
+            o["v2x_flags"], o["v2x_stats"] = np.zeros(n, abi.v2x_flags), np.zeros(n, abi.v2x_episode_stats)
+        if m["traffic"] is not None:
+            o["v2x_traffic"] = np.zeros(n, abi.v2x_traffic_stats)
+        if m["obstacles"] is not None:
+            o["v2x_obstacles"] = np.zeros(n, abi.v2x_obstacle_stats)
+        for k in o:
+            self._d2h(o[k], self.d[k], self.sizes[k])
+        _ck(self.lib.dp_stream_sync(self.p.ctx, None), "sync")
+        o["carry"], o["last_path"] = self.p.download_carry(0, n)
+        o["graph"] = self.p.closed_loop_is_graph()
+        return o
+
+    def close(self):
+        """disarm the models and free the buffers"""
+        p, m = self.p, self.models
+        if not p.ctx or self.d is None:
+            return
+        try:
+            if m["obstacles"] is not None:
+                p.set_v2x_obstacles(None, None, None, None, None)
+            if m["traffic"] is not None:
+                p.set_v2x_traffic(None, None)
+            if m["v2x"] is not None:
+                p.set_v2x_world(None, 0, None)
+            if m["metrics"] is not None:
+                p.set_metrics(None, None)
+            if m["lane_change"] is not None:
+                p.set_lane_change(None, None)
+            if m["agent_model"] is not None:
+                p.set_agent_model(None, None)
+        finally:
+            for a in list(self.d.values()) + [v[1] for v in self._cap.values()]:
+                self.lib.dp_dev_free(p.ctx, C.c_void_p(a))
+            self.d, self._cap = None, {}
 
 
 class Gather:

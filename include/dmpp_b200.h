@@ -893,6 +893,47 @@ int dp_world_set_v2x_obstacles(dp_ctx* ctx, const dp_v2x_obstacle_params* p, dp_
 int dp_v2x_obstacles_dev(dp_ctx* ctx, int first_scene, int n_scenes, const dp_scene_hdr* hdr, const double* obs_x, const double* obs_y,
                          const dp_plan_record* prev_rec, int cycle, int tally, void* stream);
 
+/* (17) Closed-loop episodes in parts, and forking worlds on the device.  An episode of sections 9-16 may run as consecutive PARTS:
+ * a part runs cycles k0 .. k0 + cycles - 1 of the episode, in the runner's order (obstacles -> logs -> Decision + Planning -> V2X
+ * -> world step), and every launch gets the episode's cycle k0 + j (the V2X and obstacles launches, section 15's t), so a long
+ * episode needs records and logs for one part only, and a run in parts computes byte for byte what one call computes.
+ *   k0 == 0   the part starts with the placement step and the row inits, as dp_run_closed_loop_dev does
+ *   k0 > 0    no placement and no init: the part continues the world that hdr / agents / obs_x / obs_y, the armed models' rows
+ *             and states, and the context's carry slots and carried paths (first ..) hold
+ *   finish    1: the V2X and obstacles tallies follow the last world step, at cycle k0 + cycles, with the part's last record;
+ *             0: they are left out, and the next part's first launches close the seam as the one-call episode would.  Finish
+ *             the last part only.  cycles == 0 with finish == 1 runs the tallies alone
+ *   rec[cycles][n], hdr_log[cycles][n], obs_log_*[cycles][n][max_obs]: indexed by the part's own cycle j (rec may be reused from
+ *             part to part as a ring; it is required, also when cycles is 0)
+ *   prev_rec  the records of cycle k0 - 1 (n of them): read by the part's first obstacles launch, before any cycle of the part
+ *             writes a record, so it may be the last row of the previous part's rec when rec is reused as a ring (that row is
+ *             overwritten only by cycle k0 + cycles - 1 of this part).  Required when k0 > 0 and section 16 is armed, ignored otherwise
+ *   launches  (k0 == 0) + cycles * (3 + V2X + obstacles) + finish * (V2X + obstacles), V2X / obstacles = 1 when armed, 0 otherwise
+ * dp_run_closed_loop_dev is this call with k0 = 0, finish = 1.  The worlds of a call stay in lock step (one k0 for all of them).
+ * The context caches one episode graph per kind of part (k0 == 0 or not, finish 0 or 1), keyed by the buffers, first, n, k0,
+ * cycles, finish and prev_rec; a part that differs from the cached one of its kind only in k0, prev_rec, rec or the log pointers is
+ * re-captured and updates that executable graph in place (cudaGraphExecUpdate, which affects only later launches, so the host may
+ * prepare part k + 1 while part k runs; a refused update instantiates afresh).  The direct launches (gather armed, record mirrors, predicted tracks, the group kernel, DP_EPISODE_GRAPH=0)
+ * run parts the same way.  DP_ERR_ARG as dp_run_closed_loop_dev, and for k0 < 0, finish other than 0 / 1, or a missing prev_rec. */
+int dp_run_closed_loop_part_dev(dp_ctx* ctx, int first_scene, int n_scenes, int k0, int cycles, int finish, dp_scene_hdr* hdr, dp_agent* agents,
+                                double* obs_x, double* obs_y, const dp_plan_record* prev_rec, dp_plan_record* rec, dp_scene_hdr* hdr_log,
+                                double* obs_log_x, double* obs_log_y, void* stream);
+/* World dst + j becomes a byte-for-byte copy of world src[j] (j < count; indices relative to first_scene, as hdr is), so that
+ * copies of a world can be perturbed and continued with dp_run_closed_loop_part_dev (k0 > 0).  Copied: hdr (128 bytes), agents
+ * (32 * max_obs), obs_x / obs_y (8 * max_obs each), prev_rec (128, when not NULL: the records the next part reads as its
+ * prev_rec), the context's carry slot (128) and carried path (3200), and every per-world buffer of the armed models: the metrics
+ * row (192), v0 (8 * max_obs), the lane-change states (24 * max_obs), the V2X specification (160), row (80) and flags (24, when
+ * set), the traffic row (32) and the obstacles row (80) -- about 5 KB per world at max_obs 10 with every model armed.  The armed
+ * read-only inputs (v0, the V2X specifications) are copied too: this call is the only one in the library that writes them, and a
+ * copy without them would be a different world.  Not copied: the section 16 view buffers (every cycle rebuilds them), the logs,
+ * and the per-launch Decision -> Planning hand-off flags.  src is a HOST array; repeated sources are allowed; count == 0 launches
+ * nothing; forks of more than 4096 worlds take one kernel per 4096.  Stream-ordered on `stream`: the caller orders it after the
+ * part that wrote the sources.  Perturbing a copy (v0, dp_agent.v) is the caller's.
+ * DP_ERR_ARG for a source outside [0, n) or inside [dst, dst + count), dst < 0 or dst + count > n, first_scene + n > max_scenes,
+ * n above the armed V2X specifications, or prev_rec NULL while section 16 is armed; DP_ERR_STATE while predicted tracks are set. */
+int dp_world_fork_dev(dp_ctx* ctx, int first_scene, int n_scenes, const int32_t* src, int dst, int count, dp_scene_hdr* hdr, dp_agent* agents,
+                      double* obs_x, double* obs_y, dp_plan_record* prev_rec, void* stream);
+
 /* diagnostic: phase time stamps (globaltimer, ns) of the most recent cycle launch, one row of 32 per CTA (row b = scenes
  * [b*g, (b+1)*g) of the batch; stamp 0 = CTA start, stamp i = end of phase i of csrc/dp_group.cuh).  Only contexts created
  * with DP_TIMELINE=1 in the environment record them; used by tools/group_timeline.py, never by the product path. */

@@ -28,12 +28,20 @@ SM clock read in the same run.
                slots for 10 agents: disarmed, what = 0 (the view is the world: the records must equal the disarmed ones, the delta is
                the obstacles launches alone) and what = 7, for 4096 highway worlds x 25 cycles as ONE graph launch; and
                dp_v2x_obstacles_dev alone (4096 worlds, what = 0 and 7, on the world and records the last episode left).  The effect
-               on seeds 0-511 is the checker's, in tests/test_v2x_obstacles.py."""
+               on seeds 0-511 is the checker's, in tests/test_v2x_obstacles.py.
+  parts        episodes in parts and forked worlds (section 17): 4096 junction worlds x 120 cycles as 1 x 120, 4 x 30 and 12 x 10
+               parts with nothing armed and with every model armed (14 slots for 10 agents), the host not synchronising between parts
+               and the records reused as a ring; the host time per part (capture + graph update or instantiate); the fork kernel
+               (131 072 worlds, max_obs 10, every model armed, 0..65535 -> 65536..) against a cudaMemcpyAsync device-to-device copy
+               of the same byte count, and a 4096-world fork; and the effect of perturbing the agents' v0 in forked copies of the
+               highway worlds (seeds 0-511, metrics + reactive + lane-changing agents): 10 cycles, 7 copies per world with v0 scaled
+               by a seeded uniform factor in [0.9, 1.1] per agent, 15 more cycles."""
 import argparse
 import json
 import os
 import subprocess
 import sys
+import time
 
 import numpy as np
 import torch
@@ -452,9 +460,161 @@ def bench_obstacles():
     return out
 
 
+def parts_ms(a, split, host_ms):
+    """one episode of a.cycles cycles as the parts of `split` (the records a ring of the longest part), the host not synchronising
+    between parts: device time from before the first part to after the last; the host time of every part call into host_ms"""
+    st = torch.cuda.current_stream()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    a.d_h.copy_(a.h0); a.d_a.copy_(a.a0)
+    a.p.reset_dev(0, a.n, stream=st.cuda_stream); torch.cuda.synchronize()
+    ring = a.d_r[:max(split)]
+    e0.record(st)
+    k0, prev = 0, None
+    for i, c in enumerate(split):
+        t = time.perf_counter()
+        a.p.run_closed_loop_part_dev(a.n, k0, c, i == len(split) - 1, a.d_h.data_ptr(), a.d_a.data_ptr(), a.d_x.data_ptr(), a.d_y.data_ptr(),
+                                     ring.data_ptr(), prev, stream=st.cuda_stream)
+        host_ms.append((time.perf_counter() - t) * 1e3)
+        assert a.p.closed_loop_is_graph()
+        k0, prev = k0 + c, ring[c - 1].data_ptr()           # (read by the next part before its cycles overwrite the ring)
+    e1.record(st); torch.cuda.synchronize()
+    return e0.elapsed_time(e1)
+
+
+def fork_bench():
+    """the fork kernel on 131 072 worlds with every model armed against a cudaMemcpyAsync of the same bytes"""
+    N, mo, half = 131072, 10, 65536
+    p = Planner(N, mo); p.upload_map(m)
+    z = lambda b: torch.randint(0, 255, (N * b,), dtype=torch.uint8, device=dev)   # noqa: E731
+    buf = {"hdr": z(128), "agents": z(32 * mo), "ox": z(8 * mo), "oy": z(8 * mo), "prev_rec": z(128), "met": z(192), "v0": z(8 * mo),
+           "lcs": z(24 * mo), "spec": torch.zeros(N * 160, dtype=torch.uint8, device=dev), "vstats": z(80), "vflags": z(24), "ts": z(32),
+           "os": z(80), "hv": z(128), "vx": z(8 * mo), "vy": z(8 * mo)}
+    wx = torch.zeros(1, dtype=torch.float64, device=dev)
+    p.set_metrics(pl.metrics_params(), buf["met"].data_ptr())
+    p.set_agent_model(pl.agent_model_params(), buf["v0"].data_ptr())
+    p.set_lane_change(pl.lane_change_params(), buf["lcs"].data_ptr())
+    p.set_v2x_world(abi.V2xWorldParams(0, 1), N, buf["spec"].data_ptr(), wx.data_ptr(), wx.data_ptr(), 0, buf["vflags"].data_ptr(),
+                    buf["vstats"].data_ptr())
+    p.set_v2x_traffic(pl.v2x_traffic_params(), buf["ts"].data_ptr())
+    p.set_v2x_obstacles(pl.v2x_obstacle_params(), buf["hv"].data_ptr(), buf["vx"].data_ptr(), buf["vy"].data_ptr(), buf["os"].data_ptr())
+    per_world = sum(buf[k].numel() // N for k in buf if k not in ("hv", "vx", "vy")) + 128 + 3200   # + the carry slot and carried path
+    st = torch.cuda.current_stream()
+    src_big = torch.empty(half * per_world, dtype=torch.uint8, device=dev); dst_big = torch.empty_like(src_big)
+    launches = 20
+
+    def fork_us(count):
+        src = np.arange(count, dtype=np.int32)
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record(st)
+        for _ in range(launches):
+            p.world_fork_dev(N, src, half, buf["hdr"].data_ptr(), buf["agents"].data_ptr(), buf["ox"].data_ptr(), buf["oy"].data_ptr(),
+                             buf["prev_rec"].data_ptr(), stream=st.cuda_stream)
+        e1.record(st); torch.cuda.synchronize()
+        return e0.elapsed_time(e1) * 1e3 / launches
+
+    def copy_us():
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record(st)
+        for _ in range(launches):
+            dst_big.copy_(src_big)                           # (contiguous, same dtype and device: cudaMemcpyAsync device to device)
+        e1.record(st); torch.cuda.synchronize()
+        return e0.elapsed_time(e1) * 1e3 / launches
+
+    fork_us(half); copy_us(); fork_us(4096)
+    f, c = [], []
+    for r in range(ROUNDS):
+        for which in ((0, 1) if r % 2 == 0 else (1, 0)):
+            (f if which == 0 else c).extend(fork_us(half) if which == 0 else copy_us() for _ in range(REPS))
+    small = [fork_us(4096) for _ in range(REPS * ROUNDS)]
+    p.set_v2x_obstacles(None, None, None, None, None); p.set_v2x_traffic(None, None); p.set_v2x_world(None, 0, None)
+    p.set_lane_change(None, None); p.set_agent_model(None, None); p.set_metrics(None, None); p.close()
+    moved = 2 * half * per_world                             # read + written
+    return {"worlds": N, "max_obs": mo, "forked": half, "bytes_per_world": per_world, "launches_per_window": launches,
+            "fork_us": summary(f), "memcpy_us": summary(c), "fork_TBps": moved / np.median(f) / 1e6, "memcpy_TBps": moved / np.median(c) / 1e6,
+            "fork_over_memcpy_bandwidth": float(np.median(c) / np.median(f)), "target": 0.8,
+            "target_met": bool(np.median(c) / np.median(f) >= 0.8),
+            "fork_4096_us": summary(small), "fork_4096_note": "20 MB moved: L2-resident after the first launch of the window"}
+
+
+def fork_effect():
+    """highway seeds 0-511 x 8 (n = 4096), metrics + reactive + lane-changing agents: 10 cycles, then worlds 0-511 forked into 7
+    copies each with v0 scaled per agent by a seeded uniform factor in [0.9, 1.1], then 15 cycles; the sources against one
+    25-cycle call"""
+    n0, copies, k1, cycles = 512, 7, 10, 25
+    w = scenes.World(m, np.arange(n0), 10, kind="highway")
+    kw = dict(metrics=pl.metrics_params(), lane_change=pl.lane_change_params())
+    p1 = Planner(n0, 10); p1.upload_map(m)
+    one = p1.run_closed_loop(w.hdr, w.agents, cycles, log=False, agent_model=(pl.agent_model_params(), w.v0), **kw)
+    p1.close()
+    n = n0 * (copies + 1)
+    tile = lambda a: np.ascontiguousarray(np.concatenate([a] * (copies + 1)))   # noqa: E731
+    p = Planner(n, 10); p.upload_map(m)
+    ep = p.episode(tile(w.hdr), tile(w.agents), agent_model=(pl.agent_model_params(), tile(w.v0)), **kw)
+    try:
+        ep.run(k1, log=False)
+        early = ep.state()["metrics"][:n0]
+        src = np.tile(np.arange(n0, dtype=np.int32), copies)
+        ep.fork(src, n0)
+        v0 = np.zeros((n, 10)); ep._d2h(v0, ep.d["v0"], v0.nbytes); p.lib.dp_stream_sync(p.ctx, None)
+        v0[n0:] *= np.random.default_rng(2026).uniform(0.9, 1.1, (n - n0, 10))
+        ep._h2d("v0", v0); p.lib.dp_stream_sync(p.ctx, None)
+        ep.run(cycles - k1, finish=True, log=False)
+        met = ep.state()["metrics"]
+        agents = ep.state()["agents"]
+    finally:
+        ep.close(); p.close()
+    assert met[:n0].tobytes() == one["metrics"].tobytes(), "the unperturbed sources differ from the one-call episode"
+    moved = (agents[n0:].reshape(copies, n0, 10)["u"] != agents[:n0]["u"][None]).any(axis=2)   # the perturbation took effect
+    src_hit = met["collision_steps"][:n0] > 0
+    copy_hit = (met["collision_steps"][n0:] > 0).reshape(copies, n0)
+    late = (early["collision_steps"] == 0)
+    cump = cump_of()
+    h, a = w.hdr, w.agents
+    klass = np.full(n0, "none", object)
+    s = np.nonzero(met["first_collision_step"][:n0] > 0)[0]
+    gl = m.road_lane_base[h["road_num"][s].astype(int) - 1] + h["lane_num"][s].astype(int) - 1
+    se = cump[m.lane_pt_off[gl] + h["id"][s, h["lane_num"][s].astype(int) - 1]]
+    ag = a[s, met["first_collision_agent"][:n0][s]]
+    sk = cump[m.lane_pt_off[ag["lane"]] + ag["i"]] + ag["u"]
+    klass[s] = np.where(ag["lane"] != gl, "other_lane", np.where(sk < se, "behind", "ahead"))
+    table = {}
+    for name in ("behind", "ahead", "other_lane"):
+        sel = late & src_hit & (klass == name)
+        table["collide_after_step_10_first_agent_" + name] = {"worlds": int(sel.sum()), "copies_that_still_collide": float(copy_hit[:, sel].mean()) if sel.any() else None}
+    sel = late & ~src_hit
+    table["no_collision"] = {"worlds": int(sel.sum()), "copies_that_collide": float(copy_hit[:, sel].mean()) if sel.any() else None}
+    return {"worlds": n0, "copies": copies, "fork_after_cycle": k1, "cycles": cycles, "v0_factor": [0.9, 1.1], "seed": 2026,
+            "sources_equal_one_call": True, "copies_whose_agents_end_elsewhere_than_their_source": float(moved.mean()), "worlds_with_collision": int(src_hit.sum()), "worlds_colliding_in_first_10_steps": int((~late).sum()),
+            "table": table}
+
+
+def bench_parts():
+    N, kind, cycles = 4096, "junction", 120
+    out = {"scenes": N, "cycles": cycles, "card": card(), "episode": {}}
+    splits = {"1x120": [120], "4x30": [30] * 4, "12x10": [10] * 12}
+    for arm_name, kw in (("nothing", {}), ("everything", dict(metrics=True, react=True, lanechg=True, v2x=1, traffic=1, obstacles=7, max_obs=14))):
+        a = Arm(kind, N, 10, cycles, **kw)
+        host = {k: [] for k in splits}
+        for k, sp in splits.items():                        # warm every split's graphs
+            parts_ms(a, sp, []); parts_ms(a, sp, [])
+        res = {k: [] for k in splits}
+        for r in range(ROUNDS):
+            for k in (list(splits) if r % 2 == 0 else list(splits)[::-1]):
+                res[k] += [parts_ms(a, splits[k], host[k]) for _ in range(REPS)]
+        a.close()
+        out["episode"][arm_name] = {k: {"ms_per_episode": summary(res[k]), "over_1x120": ratio(res[k], res["1x120"]),
+                                        "host_ms_per_part": summary(host[k])} for k in splits}
+        r430 = ratio(res["4x30"], res["1x120"])
+        out["episode"][arm_name]["target_4x30_over_1x120"] = 1.03
+        out["episode"][arm_name]["target_met"] = bool(r430 <= 1.03)
+    out["fork"] = fork_bench()
+    out["effect_highway_512"] = fork_effect()
+    return out
+
+
 if __name__ == "__main__":
     benches = {"metrics": bench_metrics, "agents": bench_agents, "lane_change": bench_lane_change, "v2x": bench_v2x, "traffic": bench_traffic,
-               "obstacles": bench_obstacles}
+               "obstacles": bench_obstacles, "parts": bench_parts}
     ap = argparse.ArgumentParser(description=__doc__.split("\n")[0])
     ap.add_argument("model", choices=list(benches))
     print(json.dumps(benches[ap.parse_args().model]()))

@@ -111,6 +111,72 @@ class JunctionOracle:
             o["v2x_obstacles"] = ostats
         return o
 
+    @staticmethod
+    def closed_loop_state(hdr, agents, metrics=None, lane_change=None, v2x=None, traffic=None, obstacles=None):
+        """the state run_closed_loop_part carries from part to part, fresh for k0 = 0: copies of hdr / agents, ox / oy, carry and
+        last_path, and the rows and states of the armed models (0xAB-filled, as run_closed_loop hands them over) under
+        run_closed_loop's keys"""
+        n, max_obs = agents.shape
+
+        def junk(dt, shape):
+            return np.frombuffer(np.full(int(np.prod(shape)) * dt.itemsize, 0xAB, np.uint8).tobytes(), dt).reshape(shape).copy()
+
+        st = {"hdr": hdr.copy(), "agents": agents.copy(), "ox": np.zeros((n, max_obs)), "oy": np.zeros((n, max_obs)),
+              "carry": np.zeros(n, abi.carry), "last_path": np.zeros((n, 2, abi.PATH_POINTS))}
+        if metrics is not None:
+            st["metrics"] = junk(abi.episode_metrics, (n,))
+        if lane_change is not None:
+            st["lane_change_state"] = junk(abi.lane_change_state, agents.shape)
+        if v2x is not None:
+            st["v2x_flags"], st["v2x_stats"] = junk(abi.v2x_flags, (n,)), junk(abi.v2x_episode_stats, (n,))
+        if traffic is not None:
+            st["v2x_traffic"] = junk(abi.v2x_traffic_stats, (n,))
+        if obstacles is not None:
+            st["v2x_obstacles"] = junk(abi.v2x_obstacle_stats, (n,))
+        return st
+
+    def run_closed_loop_part(self, state, k0, cycles, finish=False, prev_rec=None, wp=None, paths=False, threads=1, metrics=None,
+                             agent_model=None, lane_change=None, v2x=None, traffic=None, obstacles=None):
+        """cycles k0 .. k0 + cycles - 1 of an episode (jo_run_closed_loop_part), on the state of closed_loop_state (k0 = 0) or of the
+        previous part, in place; prev_rec[n] the records of cycle k0 - 1 (needed with obstacles when k0 > 0); finish: the tallies.
+        The models as run_closed_loop takes them, their rows in the state.  Returns the part's rec, hdr_log, obs_log_x / obs_log_y
+        (and path_xy) [cycles][n], ub_scene and status"""
+        assert lane_change is None or agent_model is not None
+        assert traffic is None or (agent_model is not None and v2x is not None)
+        assert obstacles is None or v2x is not None
+        st = state
+        n, max_obs = st["agents"].shape
+        am, v0 = agent_model if agent_model is not None else (None, None)
+        if v0 is not None:
+            v0 = np.ascontiguousarray(v0, np.float64)
+            assert v0.shape == (n, max_obs)
+        ref = lambda p: None if p is None else C.byref(p)
+        get = lambda k, armed: abi.ptr(st[k]) if armed is not None else None
+        models = (ref(metrics), get("metrics", metrics), ref(am), abi.ptr(v0), ref(lane_change), get("lane_change_state", lane_change))
+        if v2x is not None:
+            vp, ev = v2x
+            spec, wx, wy = self._v2x_inputs(ev)
+            assert spec.shape == (n,)
+            models += (C.byref(vp), abi.ptr(spec), abi.ptr(wx), abi.ptr(wy), C.c_int(wx.size), abi.ptr(st["v2x_flags"]), abi.ptr(st["v2x_stats"]))
+        else:
+            models += (None,) * 4 + (C.c_int(0), None, None)
+        models += (ref(traffic), get("v2x_traffic", traffic), ref(obstacles), get("v2x_obstacles", obstacles))
+        prev_rec = None if prev_rec is None else np.ascontiguousarray(prev_rec)
+        assert prev_rec is None or prev_rec.shape == (n,)
+        o = {"rec": np.zeros((cycles, n), abi.plan_record), "hdr_log": np.zeros((cycles, n), abi.scene_hdr),
+             "obs_log_x": np.zeros((cycles, n, max_obs)), "obs_log_y": np.zeros((cycles, n, max_obs)),
+             "path_xy": np.zeros((cycles, n, 2, abi.PATH_POINTS)) if paths else None, "ub_scene": np.zeros(n, np.int32)}
+        f = self.lib.jo_run_closed_loop_part
+        f.restype = C.c_longlong
+        rc = f(C.byref(self.params), C.byref(wp or self.world_params()), C.c_int(n), C.c_int(k0), C.c_int(cycles), C.c_int(int(finish)),
+               C.c_int(max_obs), abi.ptr(st["hdr"]), abi.ptr(st["agents"]), abi.ptr(st["ox"]), abi.ptr(st["oy"]), abi.ptr(prev_rec),
+               abi.ptr(o["rec"]), abi.ptr(o["hdr_log"]), abi.ptr(o["obs_log_x"]), abi.ptr(o["obs_log_y"]), abi.ptr(o["path_xy"]),
+               abi.ptr(st["carry"]), abi.ptr(st["last_path"]), C.c_int(threads), abi.ptr(o["ub_scene"]), *models)
+        if rc < 0:
+            raise RuntimeError("jo_run_closed_loop_part failed: %d" % rc)
+        o["status"] = rc
+        return o
+
     def v2x_obstacles_view(self, op, ev, hdr, ox, oy, k, stats, prev=None, tally=False, view=None):
         """one obstacles launch of cycle k for every world (jo_v2x_obstacles_view): stats in place; returns the view (hdr, ox, oy),
         built into `view` when given (slots beyond the view's n_obs keep what they held), fresh zero arrays otherwise"""

@@ -1,7 +1,7 @@
 // tools/junction_oracle/junction_api.cpp -- TEST INFRASTRUCTURE. C API of libjunction_oracle.so: the restated cycle of oracle/
 // (planner_oracle.cpp, compiled in unchanged) with the junction world step of world_junction.cpp between its cycles; the
 // same arrays as oracle_world_step / oracle_run_closed_loop of oracle/oracle_api.cpp; in jo_run_closed_loop, the models each
-// world step may carry: the episode metrics of episode_metrics.cpp (alone: jo_metrics_step), the reactive agents of
+// world step may carry (in parts: jo_run_closed_loop_part): the episode metrics of episode_metrics.cpp (alone: jo_metrics_step), the reactive agents of
 // agent_model.cpp (alone: jo_react_step) and their lane changes of lane_change.cpp (alone: jo_lane_change_step); and the V2X launch
 // of v2x_world.cpp between a cycle and its world step (alone: jo_v2x_cycle, its data builder: jo_v2x_data); and the agents that
 // obey the V2X events of v2x_traffic.cpp (alone: jo_traffic_step, its candidates: jo_traffic_leader / jo_traffic_side); and the view of
@@ -57,25 +57,29 @@ int jo_world_step(const dp_params* p, const dp_world_params* wp, int n, int max_
     return 0;
 }
 
-// the closed loop: the junction world step between the cycles of oracle/, the same arrays as oracle_run_closed_loop.  Each model is
-// armed by a non-null pair, or off with both NULL: mp / met[n] the episode metrics of include/dmpp_b200.h section 11, accumulated
-// after every world step; am / v0[n][max_obs] the reactive agents of section 12, before every world step; lp / lcs[n][max_obs]
-// (with am) their lane changes of section 13, states initialised by the placement step and holding the final states; vp / spec[n]
-// (wp_x / wp_y[n_wp], flags[n] nullable, stats[n]) the V2X events of section 14 between every cycle and its world step; tp / ts[n]
-// (with am and vp) the agents that obey them, section 15; op / os[n] (with vp) the V2X road users the planner sees, section 16: every
-// cycle runs on the view its obstacles launch builds, and hdr_log / obs_log_* record the views
-long long jo_run_closed_loop(const dp_params* p, const dp_world_params* wp, int n, int cycles, int max_obs, dp_scene_hdr* hdr,
-                             dp_agent* agents, double* ox, double* oy, dp_plan_record* rec, dp_scene_hdr* hdr_log, double* obs_log_x,
-                             double* obs_log_y, double* path_xy, dp_carry* carry_out, double* last_path_out, int threads,
-                             int32_t* ub_scene, const dp_metrics_params* mp, dp_episode_metrics* met, const dp_agent_model_params* am,
-                             const double* v0, const dp_lane_change_params* lp, dp_lane_change_state* lcs, const dp_v2x_world_params* vp,
-                             const dp_v2x_event_spec* spec, const double* wp_x, const double* wp_y, int n_wp, dp_v2x_flags* flags,
-                             dp_v2x_episode_stats* stats, const dp_v2x_traffic_params* tp, dp_v2x_traffic_stats* ts,
-                             const dp_v2x_obstacle_params* op, dp_v2x_obstacle_stats* os) {
+// a closed loop in parts (include/dmpp_b200.h section 17): cycles k0 .. k0 + cycles - 1 of the episode, rec / hdr_log / obs_log_* /
+// path_xy indexed by the part's cycle j.  k0 == 0: a fresh state (reset_state), the placement step and the row inits; k0 > 0: the
+// world hdr / agents / ox / oy, the rows and states, and carry[n] / last_path[n][2][200] (in and out) continue where the previous
+// part left them, and prev_rec[n] holds the records of cycle k0 - 1 (required with os).  finish: the V2X and obstacles tallies at
+// cycle k0 + cycles.  Each model is armed by a non-null pair, or off with both NULL: mp / met[n] the episode metrics of section 11,
+// accumulated after every world step; am / v0[n][max_obs] the reactive agents of section 12, before every world step; lp /
+// lcs[n][max_obs] (with am) their lane changes of section 13, states initialised by the placement step; vp / spec[n] (wp_x / wp_y[n_wp],
+// flags[n] nullable, stats[n]) the V2X events of section 14 between every cycle and its world step; tp / ts[n] (with am and vp) the
+// agents that obey them, section 15; op / os[n] (with vp) the V2X road users the planner sees, section 16: every cycle runs on the view
+// its obstacles launch builds, and hdr_log / obs_log_* record the views (slots beyond a view's n_obs hold zeros from the part's start)
+long long jo_run_closed_loop_part(const dp_params* p, const dp_world_params* wp, int n, int k0, int cycles, int finish, int max_obs,
+                                  dp_scene_hdr* hdr, dp_agent* agents, double* ox, double* oy, const dp_plan_record* prev_rec, dp_plan_record* rec,
+                                  dp_scene_hdr* hdr_log, double* obs_log_x, double* obs_log_y, double* path_xy, dp_carry* carry,
+                                  double* last_path, int threads, int32_t* ub_scene, const dp_metrics_params* mp, dp_episode_metrics* met,
+                                  const dp_agent_model_params* am, const double* v0, const dp_lane_change_params* lp, dp_lane_change_state* lcs,
+                                  const dp_v2x_world_params* vp, const dp_v2x_event_spec* spec, const double* wp_x, const double* wp_y,
+                                  int n_wp, dp_v2x_flags* flags, dp_v2x_episode_stats* stats, const dp_v2x_traffic_params* tp,
+                                  dp_v2x_traffic_stats* ts, const dp_v2x_obstacle_params* op, dp_v2x_obstacle_stats* os) {
     if (!g_have_map) return -1;
     if ((!mp) != (!met) || (!am) != (!v0) || (!lp) != (!lcs) || (lcs && !v0) || (!vp) != (!spec) || (spec && !stats)) return -1;
     if ((!tp) != (!ts) || (ts && (!v0 || !spec))) return -1;
     if ((!op) != (!os) || (os && !spec)) return -1;
+    if (k0 < 0 || cycles < 0 || (finish != 0 && finish != 1) || (k0 > 0 && (!carry || !last_path || (os && !prev_rec)))) return -1;
     if (threads < 1) threads = 1;
     std::vector<double> wla, wlo;
     if (spec) wp_gps(*p, wp_x, wp_y, n_wp, wla, wlo);
@@ -85,22 +89,33 @@ long long jo_run_closed_loop(const dp_params* p, const dp_world_params* wp, int 
         for (int s = s0; s < s1; ++s) {
             const long long lub0 = lub;
             oracle::SceneState st;
-            oracle::reset_state(st);
             dp_agent* ag = agents + (size_t)s * max_obs;
             double* sx = ox + (size_t)s * max_obs; double* sy = oy + (size_t)s * max_obs;
-            junction::world_step(g_map, *p, *wp, hdr[s], ag, sx, sy, nullptr, nullptr, nullptr);
-            if (met) metrics::init(met[s]);
-            if (lcs) lanechg::init(ag, std::min((int)hdr[s].n_obs, max_obs), lcs + (size_t)s * max_obs);
-            if (ts) traffic::init(ts[s]);
+            if (k0 == 0) {
+                oracle::reset_state(st);
+                junction::world_step(g_map, *p, *wp, hdr[s], ag, sx, sy, nullptr, nullptr, nullptr);
+                if (met) metrics::init(met[s]);
+                if (lcs) lanechg::init(ag, std::min((int)hdr[s].n_obs, max_obs), lcs + (size_t)s * max_obs);
+                if (ts) traffic::init(ts[s]);
+            } else {
+                st.c = carry[s];
+                std::memcpy(st.last_x, last_path + (size_t)s * 400, sizeof(st.last_x));
+                std::memcpy(st.last_y, last_path + (size_t)s * 400 + 200, sizeof(st.last_y));
+            }
             std::vector<int> kinds((size_t)max_obs);
             std::vector<dp_agent> a1((size_t)max_obs);
             // the cycle's inputs: the world, or with os the view of it (slots beyond the view's n_obs keep what they held)
             dp_scene_hdr hv{};
             std::vector<double> vx((size_t)max_obs), vy((size_t)max_obs);
-            for (int c = 0; c < cycles; ++c) {
-                const size_t e = (size_t)c * n + s;
-                if (os) v2xobs::launch(g_map, *op, max_obs, spec[s], wp_x, wp_y, hdr[s], sx, sy, c > 0 ? rec + e - n : nullptr, c, false, &hv,
-                                       vx.data(), vy.data(), os[s]);
+            // the records of the cycle before j (prev_rec at j == 0 of a continued part)
+            auto prev_of = [&](int j) -> const dp_plan_record* {
+                return j > 0 ? rec + (size_t)(j - 1) * n + s : (k0 > 0 ? prev_rec + s : nullptr);
+            };
+            for (int j = 0; j < cycles; ++j) {
+                const int c = k0 + j;
+                const size_t e = (size_t)j * n + s;
+                if (os) v2xobs::launch(g_map, *op, max_obs, spec[s], wp_x, wp_y, hdr[s], sx, sy, prev_of(j), c, false, &hv, vx.data(), vy.data(),
+                                       os[s]);
                 const dp_scene_hdr& ch = os ? hv : hdr[s];
                 const double* cx = os ? vx.data() : sx;
                 const double* cy = os ? vy.data() : sy;
@@ -125,14 +140,16 @@ long long jo_run_closed_loop(const dp_params* p, const dp_world_params* wp, int 
                 if (ts && metrics::header_valid(g_map.m, h0)) traffic_update(*p, *am, tw, ts[s], a1.data(), ag, sx, sy, na, kinds.data());
                 if (met) metrics::update(g_map, *wp, *mp, met[s], h0, hdr[s], ag, sx, sy, std::min((int)h0.n_obs, max_obs), rec[e]);
             }
-            if (spec) v2x::cycle(g_map, *p, *vp, spec[s], wla.data(), wlo.data(), hdr[s], cycles, nullptr, stats[s], flags ? flags + s : nullptr);
-            if (os) v2xobs::launch(g_map, *op, max_obs, spec[s], wp_x, wp_y, hdr[s], sx, sy, cycles > 0 ? rec + (size_t)(cycles - 1) * n + s : nullptr,
-                                   cycles, true, nullptr, nullptr, nullptr, os[s]);
+            if (finish) {
+                if (spec) v2x::cycle(g_map, *p, *vp, spec[s], wla.data(), wlo.data(), hdr[s], k0 + cycles, nullptr, stats[s], flags ? flags + s : nullptr);
+                if (os) v2xobs::launch(g_map, *op, max_obs, spec[s], wp_x, wp_y, hdr[s], sx, sy, prev_of(cycles), k0 + cycles, true, nullptr, nullptr,
+                                       nullptr, os[s]);
+            }
             if (ub_scene) ub_scene[s] = (int32_t)(lub - lub0);
-            if (carry_out) carry_out[s] = st.c;
-            if (last_path_out) {
-                std::memcpy(last_path_out + (size_t)s * 400, st.last_x, sizeof(st.last_x));
-                std::memcpy(last_path_out + (size_t)s * 400 + 200, st.last_y, sizeof(st.last_y));
+            if (carry) carry[s] = st.c;
+            if (last_path) {
+                std::memcpy(last_path + (size_t)s * 400, st.last_x, sizeof(st.last_x));
+                std::memcpy(last_path + (size_t)s * 400 + 200, st.last_y, sizeof(st.last_y));
             }
         }
         ub += lub;
@@ -144,6 +161,21 @@ long long jo_run_closed_loop(const dp_params* p, const dp_world_params* wp, int 
         for (auto& t : th) t.join();
     }
     return ub.load();
+}
+
+// the closed loop: the junction world step between the cycles of oracle/, the same arrays as oracle_run_closed_loop, and the models
+// of jo_run_closed_loop_part: the whole episode as one part (k0 = 0, finish = 1) from a fresh state
+long long jo_run_closed_loop(const dp_params* p, const dp_world_params* wp, int n, int cycles, int max_obs, dp_scene_hdr* hdr,
+                             dp_agent* agents, double* ox, double* oy, dp_plan_record* rec, dp_scene_hdr* hdr_log, double* obs_log_x,
+                             double* obs_log_y, double* path_xy, dp_carry* carry_out, double* last_path_out, int threads,
+                             int32_t* ub_scene, const dp_metrics_params* mp, dp_episode_metrics* met, const dp_agent_model_params* am,
+                             const double* v0, const dp_lane_change_params* lp, dp_lane_change_state* lcs, const dp_v2x_world_params* vp,
+                             const dp_v2x_event_spec* spec, const double* wp_x, const double* wp_y, int n_wp, dp_v2x_flags* flags,
+                             dp_v2x_episode_stats* stats, const dp_v2x_traffic_params* tp, dp_v2x_traffic_stats* ts,
+                             const dp_v2x_obstacle_params* op, dp_v2x_obstacle_stats* os) {
+    return jo_run_closed_loop_part(p, wp, n, 0, cycles, 1, max_obs, hdr, agents, ox, oy, nullptr, rec, hdr_log, obs_log_x, obs_log_y, path_xy,
+                                   carry_out, last_path_out, threads, ub_scene, mp, met, am, v0, lp, lcs, vp, spec, wp_x, wp_y, n_wp, flags,
+                                   stats, tp, ts, op, os);
 }
 
 // the react phase alone, for every scene (agents[n][max_obs], v0[n][max_obs], k < min(n_obs, max_obs)), as the armed kernel runs
