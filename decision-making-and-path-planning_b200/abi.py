@@ -217,6 +217,17 @@ v2x_obstacle_stats = np.dtype(
 assert v2x_obstacle_stats.itemsize == 80
 
 
+class SplitParams(C.Structure):
+    _fields_ = [("group", C.c_int32), ("pad", C.c_int32), ("beta", C.c_double), ("c_max", C.c_double), ("amp_v", C.c_double),
+                ("amp_v0", C.c_double), ("seed", C.c_uint64)]
+
+
+split_row = np.dtype([("v_prev", "<f8"), ("lw", "<f8"), ("root", "<i4"), ("pad", "<i4")])
+assert split_row.itemsize == 24
+split_group = np.dtype([("norm", "<f8"), ("levels", "<i4"), ("copies", "<i4"), ("roots_alive", "<i4"), ("pad", "<i4")])
+assert split_group.itemsize == 24
+
+
 class MapDesc(C.Structure):
     _fields_ = [
         ("n_roads", C.c_int32), ("road_lane_base", C.c_void_p),

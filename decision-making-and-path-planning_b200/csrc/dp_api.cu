@@ -70,6 +70,10 @@ struct dp_ctx {
     int v2x_cycle = 0;                                      // the cycle of the last dp_v2x_world_dev call: section 15's t of a
                                                             // hand-stepped world step
     DpObstOpts obst;                                        // dp_world_set_v2x_obstacles: the views every cycle runs on
+    // dp_world_set_split: armed by rows != nullptr; map[split_n] the sources of the last split (context-owned)
+    dp_split_params split = {};
+    dp_split_row* split_rows = nullptr; dp_split_group* split_groups = nullptr;
+    int32_t* split_map = nullptr; int split_n = 0;
     cudaStream_t ep_stream = nullptr;
     // one cached graph per kind of part, (k0 > 0) * 2 + finish: the parts of a long episode update theirs in place, and a
     // one-call episode (k0 = 0, finish = 1) keeps its own
@@ -329,7 +333,7 @@ int dp_destroy(dp_ctx* c) {
     for (void* p : c->map_allocs) cudaFree(p);
     for (auto& g : c->ep) if (g.exec) cudaGraphExecDestroy(g.exec);
     if (c->ep_stream) cudaStreamDestroy(c->ep_stream);
-    cudaFree(c->d_timeline); cudaFree(c->d_trk);
+    cudaFree(c->d_timeline); cudaFree(c->d_trk); cudaFree(c->split_map);
     cudaFree(c->d_carry); cudaFree(c->d_last); cudaFree(c->d_done); cudaFree(c->d_inflag); cudaFree(c->d_tally); cudaFree(c->d_tally_g);
     if (c->h_done) cudaFreeHost(c->h_done);
     for (int s = 0; s < 2; ++s) {
@@ -1628,6 +1632,36 @@ int dp_run_closed_loop_dev(dp_ctx* c, int first, int n, int cycles, dp_scene_hdr
                            dp_plan_record* rec, dp_scene_hdr* hdr_log, double* olx, double* oly, void* stream) {
     return dp_run_closed_loop_part_dev(c, first, n, 0, cycles, 1, hdr, agents, ox, oy, nullptr, rec, hdr_log, olx, oly, stream);
 }
+namespace {
+// the per-world buffers a fork or a split copies: the caller's world, the context's carry slot and carried path, then every
+// per-world buffer of the armed models; returns the number of segments
+int fork_segments(const dp_ctx* c, int first, dp_scene_hdr* hdr, dp_agent* agents, double* ox, double* oy, dp_plan_record* prev_rec,
+                  DpForkSeg* out) {
+    int n_seg = 0;
+    bool full = false;
+    const size_t mo = (size_t)c->max_obs;
+    auto seg = [&](const void* base, size_t bytes) {
+        if (n_seg == DP_FORK_MAX_SEG) { full = true; return; }
+        unsigned w = 16;
+        while (w > 1 && (((uintptr_t)base | bytes) & (w - 1))) w >>= 1;
+        out[n_seg++] = DpForkSeg{(unsigned char*)base, (unsigned)bytes, w};
+    };
+    seg(hdr, sizeof(dp_scene_hdr)); seg(agents, mo * sizeof(dp_agent)); seg(ox, mo * sizeof(double)); seg(oy, mo * sizeof(double));
+    if (prev_rec) seg(prev_rec, sizeof(dp_plan_record));
+    seg(c->d_carry + first, sizeof(dp_carry)); seg(c->d_last + (size_t)first * DP_PATH_POINTS, DP_PATH_POINTS * sizeof(double2));
+    if (c->world.met) seg(c->world.met, sizeof(dp_episode_metrics));
+    if (c->world.v0) seg(c->world.v0, mo * sizeof(double));
+    if (c->world.lcs) seg(c->world.lcs, mo * sizeof(dp_lane_change_state));
+    if (c->v2x.spec) {
+        seg(c->v2x.spec, sizeof(dp_v2x_event_spec)); seg(c->v2x.stats, sizeof(dp_v2x_episode_stats));
+        if (c->v2x.flags) seg(c->v2x.flags, sizeof(dp_v2x_flags));
+    }
+    if (c->world.ts) seg(c->world.ts, sizeof(dp_v2x_traffic_stats));
+    if (c->obst.stats) seg(c->obst.stats, sizeof(dp_v2x_obstacle_stats));
+    if (c->split_rows) seg(c->split_rows, sizeof(dp_split_row));    // (16 segments with every model armed: DP_FORK_MAX_SEG)
+    return full ? -1 : n_seg;
+}
+}  // namespace
 int dp_world_fork_dev(dp_ctx* c, int first, int n, const int32_t* src, int dst, int count, dp_scene_hdr* hdr, dp_agent* agents, double* ox,
                       double* oy, dp_plan_record* prev_rec, void* stream) {
     if (!c || !hdr || !agents || !ox || !oy || n < 0 || first < 0 || first + n > c->max_scenes || count < 0 || (count > 0 && !src) || dst < 0 ||
@@ -1644,26 +1678,8 @@ int dp_world_fork_dev(dp_ctx* c, int first, int n, const int32_t* src, int dst, 
     CK(cudaSetDevice(c->device));
     const std::unique_ptr<DpForkArgs> ap(new DpForkArgs);  // (16.6 KB: off the stack; every launch copies it into its parameters)
     DpForkArgs& fa = *ap;
-    fa.n_seg = 0;
-    const size_t mo = (size_t)c->max_obs;
-    auto seg = [&](const void* base, size_t bytes) {
-        unsigned w = 16;
-        while (w > 1 && (((uintptr_t)base | bytes) & (w - 1))) w >>= 1;
-        fa.seg[fa.n_seg++] = DpForkSeg{(unsigned char*)base, (unsigned)bytes, w};
-    };
-    // the caller's world, the context's carry slot and carried path, then every per-world buffer of the armed models
-    seg(hdr, sizeof(dp_scene_hdr)); seg(agents, mo * sizeof(dp_agent)); seg(ox, mo * sizeof(double)); seg(oy, mo * sizeof(double));
-    if (prev_rec) seg(prev_rec, sizeof(dp_plan_record));
-    seg(c->d_carry + first, sizeof(dp_carry)); seg(c->d_last + (size_t)first * DP_PATH_POINTS, DP_PATH_POINTS * sizeof(double2));
-    if (c->world.met) seg(c->world.met, sizeof(dp_episode_metrics));
-    if (c->world.v0) seg(c->world.v0, mo * sizeof(double));
-    if (c->world.lcs) seg(c->world.lcs, mo * sizeof(dp_lane_change_state));
-    if (c->v2x.spec) {
-        seg(c->v2x.spec, sizeof(dp_v2x_event_spec)); seg(c->v2x.stats, sizeof(dp_v2x_episode_stats));
-        if (c->v2x.flags) seg(c->v2x.flags, sizeof(dp_v2x_flags));
-    }
-    if (c->world.ts) seg(c->world.ts, sizeof(dp_v2x_traffic_stats));
-    if (c->obst.stats) seg(c->obst.stats, sizeof(dp_v2x_obstacle_stats));
+    fa.n_seg = fork_segments(c, first, hdr, agents, ox, oy, prev_rec, fa.seg);
+    if (fa.n_seg < 0) return fail(DP_ERR_STATE, "dp_world_fork_dev: more per-world buffers armed than DP_FORK_MAX_SEG");
     for (int j0 = 0; j0 < count; j0 += DP_FORK_MAX_SRC) {
         fa.count = std::min(count - j0, DP_FORK_MAX_SRC);
         fa.dst = dst + j0;
@@ -1671,6 +1687,70 @@ int dp_world_fork_dev(dp_ctx* c, int first, int n, const int32_t* src, int dst, 
         c->launches += 1;
         CK(dp_launch_world_fork(fa, (cudaStream_t)stream));
     }
+    return DP_OK;
+}
+void dp_split_default_params(dp_split_params* p) {
+    if (!p) return;
+    memset(p, 0, sizeof(*p));
+    p->group = 256; p->beta = 0.5; p->c_max = 10.0; p->amp_v = 0.1;
+}
+int dp_world_set_split(dp_ctx* c, const dp_split_params* p, int n, dp_split_row* rows, dp_split_group* groups) {
+    if (!c || (rows && (!p || !groups))) return fail(DP_ERR_ARG, "dp_world_set_split: bad argument");
+    if (!rows) {
+        cudaSetDevice(c->device);
+        cudaFree(c->split_map);
+        c->split_map = nullptr; c->split_rows = nullptr; c->split_groups = nullptr; c->split_n = 0;
+        return DP_OK;
+    }
+    if (p->group < 1 || p->group > 1024 || n < 0 || n % p->group != 0)
+        return fail(DP_ERR_ARG, "dp_world_set_split: group outside 1 .. 1024, or n not a multiple of it");
+    if (!all_finite({p->beta, p->c_max, p->amp_v, p->amp_v0})) return fail(DP_ERR_ARG, "dp_world_set_split: parameters must be finite");
+    if (!(p->beta >= 0) || !(p->c_max > 0) || !(p->beta * p->c_max <= 50) || !(p->amp_v >= 0 && p->amp_v < 1) || !(p->amp_v0 >= 0 && p->amp_v0 < 1))
+        return fail(DP_ERR_ARG, "dp_world_set_split: beta >= 0, c_max > 0, beta * c_max <= 50 and amplitudes in [0, 1)");
+    CK(cudaSetDevice(c->device));
+    if (n > c->split_n || !c->split_map) {
+        cudaFree(c->split_map);
+        c->split_map = nullptr; c->split_rows = nullptr; c->split_n = 0;
+        cudaError_t e = cudaMalloc(&c->split_map, (size_t)(n > 0 ? n : 1) * sizeof(int32_t));
+        if (e != cudaSuccess) { c->split_map = nullptr; return fail(DP_ERR_NOMEM, "dp_world_set_split: cudaMalloc", e); }
+    }
+    CK(cudaMemset(c->split_map, 0xff, (size_t)(n > 0 ? n : 1) * sizeof(int32_t)));
+    c->split = *p; c->split_rows = rows; c->split_groups = groups; c->split_n = n;
+    return DP_OK;
+}
+int dp_world_split_dev(dp_ctx* c, int first, int n, int level, dp_scene_hdr* hdr, dp_agent* agents, double* ox, double* oy,
+                       dp_plan_record* prev_rec, void* stream) {
+    if (!c || !hdr || !agents || !ox || !oy || n < 0 || first < 0 || first + n > c->max_scenes || level < 0)
+        return fail(DP_ERR_ARG, "dp_world_split_dev: bad argument");
+    if (!c->split_rows) return fail(DP_ERR_STATE, "dp_world_split_dev: the model is not armed (dp_world_set_split)");
+    if (!c->world.met) return fail(DP_ERR_STATE, "dp_world_split_dev: the metrics are not armed (dp_world_set_metrics): they are the score");
+    if (c->tracks_T > 0) return fail(DP_ERR_STATE, "dp_world_split_dev: predicted tracks are set (dp_clear_tracks first)");
+    if (n % c->split.group != 0 || n > c->split_n)
+        return fail(DP_ERR_ARG, "dp_world_split_dev: n is not a multiple of the group or exceeds the armed rows");
+    if (c->v2x.spec && n > c->v2x.n) return fail(DP_ERR_ARG, "dp_world_split_dev: more scenes than the armed V2X specifications");
+    if (c->obst.stats && !prev_rec) return fail(DP_ERR_ARG, "dp_world_split_dev: the V2X road users are armed and prev_rec is NULL");
+    if (c->submitted != c->waited) return fail(DP_ERR_STATE, "dp_world_split_dev: submitted cycles in flight, call dp_cycle_wait first");
+    if (n == 0) return DP_OK;
+    CK(cudaSetDevice(c->device));
+    const cudaStream_t st = (cudaStream_t)stream;
+    // select -> copy -> perturb: three launches, so that every copy has read its source before any world is perturbed
+    DpForkTable t;
+    t.n_seg = fork_segments(c, first, hdr, agents, ox, oy, prev_rec, t.seg);
+    if (t.n_seg < 0) return fail(DP_ERR_STATE, "dp_world_split_dev: more per-world buffers armed than DP_FORK_MAX_SEG");
+    c->launches += 3;
+    CK(dp_launch_world_split_select(c->split, n, level, c->world.met, c->split_rows, c->split_groups, c->split_map, st));
+    CK(dp_launch_world_fork_map(t, n, c->split_map, st));
+    CK(dp_launch_world_perturb(c->split, n, level, c->max_obs, hdr, agents, const_cast<double*>(c->world.v0), st));
+    return DP_OK;
+}
+int dp_world_split_map(dp_ctx* c, int n, int32_t* host_map, void* stream) {
+    if (!c || n < 0 || (n > 0 && !host_map)) return fail(DP_ERR_ARG, "dp_world_split_map: bad argument");
+    if (!c->split_rows) return fail(DP_ERR_STATE, "dp_world_split_map: the model is not armed (dp_world_set_split)");
+    if (n > c->split_n) return fail(DP_ERR_ARG, "dp_world_split_map: n exceeds the armed rows");
+    CK(cudaSetDevice(c->device));
+    if (n == 0) return DP_OK;
+    CK(cudaMemcpyAsync(host_map, c->split_map, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, (cudaStream_t)stream));
+    CK(cudaStreamSynchronize((cudaStream_t)stream));
     return DP_OK;
 }
 int dp_closed_loop_is_graph(dp_ctx* c) { return c ? c->ep_last_graph : 0; }

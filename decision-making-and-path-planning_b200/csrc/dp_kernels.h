@@ -75,6 +75,18 @@ struct DpForkArgs {
     int32_t src[DP_FORK_MAX_SRC];
 };
 cudaError_t dp_launch_world_fork(const DpForkArgs& a, cudaStream_t st);
+// the copy of a split (section 18): world i becomes a copy of world map[i] (device array, -1: no copy) in every segment of t
+struct DpForkTable {
+    DpForkSeg seg[DP_FORK_MAX_SEG];
+    int n_seg;
+};
+cudaError_t dp_launch_world_fork_map(const DpForkTable& t, int n, const int32_t* map, cudaStream_t st);
+// splitting worlds (dp_world_split.cu, include/dmpp_b200.h section 18): the select launch of the n / p.group populations (rows,
+// groups and map written) and the perturb launch (v0 nullptr: the reactive agents are disarmed)
+cudaError_t dp_launch_world_split_select(const dp_split_params& p, int n, int level, const dp_episode_metrics* met, dp_split_row* rows,
+                                         dp_split_group* groups, int32_t* map, cudaStream_t st);
+cudaError_t dp_launch_world_perturb(const dp_split_params& p, int n, int level, int max_obs, const dp_scene_hdr* hdr, dp_agent* agents,
+                                    double* v0, cudaStream_t st);
 cudaError_t dp_launch_v2x(const DevMap& m, const dp_params& p, int n, const dp_scene_hdr* hdr, const dp_v2x_data* v2x, const double* wp_lat,
                           const double* wp_lng, int mode, dp_v2x_flags* out, cudaStream_t st);
 cudaError_t dp_launch_v2x_apply(int n, const dp_v2x_flags* flags, dp_plan_record* rec, cudaStream_t st);

@@ -29,12 +29,10 @@ __device__ __forceinline__ void fork_copy(unsigned char* base, unsigned bytes, i
     }
 }
 
-__global__ void __launch_bounds__(FORK_WPB * 32) dp_world_fork_kernel(const __grid_constant__ DpForkArgs a) {
-    const int lane = threadIdx.x & 31, j = blockIdx.x * FORK_WPB + (threadIdx.x >> 5);
-    if (j >= a.count) return;
-    const int s = a.src[j], d = a.dst + j;
-    for (int k = 0; k < a.n_seg; ++k) {
-        const DpForkSeg& g = a.seg[k];
+// world d becomes a copy of world s in every segment of the table (one warp)
+__device__ __forceinline__ void fork_world(const DpForkSeg* seg, int n_seg, int s, int d, int lane) {
+    for (int k = 0; k < n_seg; ++k) {
+        const DpForkSeg& g = seg[k];
         switch (g.width) {
             case 16: fork_copy<uint4>(g.base, g.bytes, s, d, lane); break;
             case 8: fork_copy<unsigned long long>(g.base, g.bytes, s, d, lane); break;
@@ -43,10 +41,32 @@ __global__ void __launch_bounds__(FORK_WPB * 32) dp_world_fork_kernel(const __gr
         }
     }
 }
+
+__global__ void __launch_bounds__(FORK_WPB * 32) dp_world_fork_kernel(const __grid_constant__ DpForkArgs a) {
+    const int lane = threadIdx.x & 31, j = blockIdx.x * FORK_WPB + (threadIdx.x >> 5);
+    if (j >= a.count) return;
+    fork_world(a.seg, a.n_seg, a.src[j], a.dst + j, lane);
+}
+
+// the copy of a split (include/dmpp_b200.h section 18): world i becomes a copy of world map[i] where map[i] >= 0.  The map lives in
+// device memory (the select launch wrote it), so one launch covers any number of worlds
+__global__ void __launch_bounds__(FORK_WPB * 32) dp_world_fork_map_kernel(const __grid_constant__ DpForkTable t, int n, const int32_t* __restrict__ map) {
+    const int lane = threadIdx.x & 31, i = blockIdx.x * FORK_WPB + (threadIdx.x >> 5);
+    if (i >= n) return;
+    const int s = map[i];
+    if (s < 0) return;
+    fork_world(t.seg, t.n_seg, s, i, lane);
+}
 }  // namespace
 
 cudaError_t dp_launch_world_fork(const DpForkArgs& a, cudaStream_t st) {
     if (a.count <= 0) return cudaSuccess;
     dp_world_fork_kernel<<<(a.count + FORK_WPB - 1) / FORK_WPB, FORK_WPB * 32, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t dp_launch_world_fork_map(const DpForkTable& t, int n, const int32_t* map, cudaStream_t st) {
+    if (n <= 0) return cudaSuccess;
+    dp_world_fork_map_kernel<<<(n + FORK_WPB - 1) / FORK_WPB, FORK_WPB * 32, 0, st>>>(t, n, map);
     return cudaGetLastError();
 }

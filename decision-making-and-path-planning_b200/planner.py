@@ -29,7 +29,8 @@ SYMBOLS = [
     "dp_metrics_default_params", "dp_world_set_metrics", "dp_agent_model_default_params", "dp_world_set_agent_model",
     "dp_lane_change_default_params", "dp_world_set_lane_change", "dp_world_set_v2x", "dp_v2x_world_dev",
     "dp_v2x_traffic_default_params", "dp_world_set_v2x_traffic", "dp_v2x_obstacle_default_params", "dp_world_set_v2x_obstacles",
-    "dp_v2x_obstacles_dev", "dp_run_closed_loop_part_dev", "dp_world_fork_dev",
+    "dp_v2x_obstacles_dev", "dp_run_closed_loop_part_dev", "dp_world_fork_dev", "dp_split_default_params", "dp_world_set_split",
+    "dp_world_split_dev", "dp_world_split_map",
     "dp_gather_create", "dp_gather_attach", "dp_gather_arm", "dp_gather_chain", "dp_gather_arm_deferred", "dp_gather_set_lag", "dp_gather_flush", "dp_gather_disarm", "dp_gather_wait", "dp_gather_buffer", "dp_gather_destroy",
 ]
 
@@ -49,6 +50,9 @@ def load():
         vp, i = C.c_void_p, C.c_int
         _lib.dp_run_closed_loop_part_dev.argtypes = [vp, i, i, i, i, i] + [vp] * 10
         _lib.dp_world_fork_dev.argtypes = [vp, i, i, vp, i, i] + [vp] * 6
+        _lib.dp_world_set_split.argtypes = [vp, vp, i, vp, vp]
+        _lib.dp_world_split_dev.argtypes = [vp, i, i, i] + [vp] * 6
+        _lib.dp_world_split_map.argtypes = [vp, i, vp, vp]
     return _lib
 
 
@@ -98,6 +102,24 @@ def v2x_obstacle_params(**kw):
     for k, v in kw.items():
         setattr(p, k, v)
     return p
+
+
+def split_params(**kw):
+    """dp_split_default_params (no GPU needed), then the keyword fields"""
+    p = abi.SplitParams()
+    load().dp_split_default_params(C.byref(p))
+    for k, v in kw.items():
+        setattr(p, k, v)
+    return p
+
+
+def split_estimate(state):
+    """the collision probability of every population (include/dmpp_b200.h section 18) from Episode.state() after the last part:
+    p_g = norm_g * (1 / M) * sum_j [first_collision_step_j >= 0] / lw_j"""
+    rows, groups = state["split_rows"], state["split_groups"]
+    M = len(rows) // len(groups)
+    hit = (state["metrics"]["first_collision_step"] >= 0).astype(np.float64)
+    return groups["norm"] * (hit / rows["lw"]).reshape(-1, M).mean(axis=1)
 
 
 def default_params():
@@ -338,9 +360,24 @@ class Planner:
         _ck(self.lib.dp_world_fork_dev(self.ctx, first, n, src.ctypes.data if src.size else None, dst, src.size, d_hdr, d_agents, d_ox,
                                        d_oy, d_prev_rec, stream), "dp_world_fork_dev")
 
-    def episode(self, hdr, agents, metrics=None, agent_model=None, lane_change=None, v2x=None, traffic=None, obstacles=None):
-        """an episode to run in parts (Episode): the models are armed as run_closed_loop arms them, until Episode.close()"""
-        return Episode(self, hdr, agents, metrics, agent_model, lane_change, v2x, traffic, obstacles)
+    def set_split(self, params, n, d_rows, d_groups):
+        """arm splitting (include/dmpp_b200.h section 18) with rows[n] / groups[n / group] on the device; d_rows None disarms"""
+        _ck(self.lib.dp_world_set_split(self.ctx, C.byref(params) if params is not None else None, n, d_rows, d_groups), "dp_world_set_split")
+
+    def world_split_dev(self, n, level, d_hdr, d_agents, d_ox, d_oy, d_prev_rec=None, first=0, stream=0):
+        """one split of worlds 0 .. n-1: select -> copy -> perturb (three launches)"""
+        _ck(self.lib.dp_world_split_dev(self.ctx, first, n, level, d_hdr, d_agents, d_ox, d_oy, d_prev_rec, stream), "dp_world_split_dev")
+
+    def split_map(self, n, stream=0):
+        """the sources of the last split (copied on the split's stream and synchronised), -1 for the worlds that were not copied"""
+        m = np.zeros(n, np.int32)
+        _ck(self.lib.dp_world_split_map(self.ctx, n, m.ctypes.data, stream), "dp_world_split_map")
+        return m
+
+    def episode(self, hdr, agents, metrics=None, agent_model=None, lane_change=None, v2x=None, traffic=None, obstacles=None, split=None):
+        """an episode to run in parts (Episode): the models are armed as run_closed_loop arms them, until Episode.close(); split:
+        SplitParams (needs metrics) arms splitting between the parts (Episode.split)"""
+        return Episode(self, hdr, agents, metrics, agent_model, lane_change, v2x, traffic, obstacles, split)
 
     def closed_loop_is_graph(self):
         return bool(self.lib.dp_closed_loop_is_graph(self.ctx))
@@ -504,14 +541,17 @@ class Episode:
     of the world and of the armed models, which stay armed until close().  run() continues the episode where the last part left
     it; fork() copies worlds on the device; state() downloads the world and the rows."""
 
-    def __init__(self, planner, hdr, agents, metrics=None, agent_model=None, lane_change=None, v2x=None, traffic=None, obstacles=None):
+    def __init__(self, planner, hdr, agents, metrics=None, agent_model=None, lane_change=None, v2x=None, traffic=None, obstacles=None,
+                 split=None):
         n, mo = agents.shape
+        assert split is None or (metrics is not None and n % split.group == 0), "the split scores the metrics rows of whole populations"
         assert lane_change is None or agent_model is not None, "lane changes run on the reactive agents"
         assert traffic is None or (agent_model is not None and v2x is not None), "the agents obey the V2X events on the reactive agents"
         assert obstacles is None or v2x is not None, "the planner sees the V2X road users of the armed V2X events"
         assert mo == planner.max_obs and hdr.shape == (n,) and n <= planner.max_scenes
         self.p, self.lib, self.n, self.mo = planner, planner.lib, n, mo
-        self.models = dict(metrics=metrics, agent_model=agent_model, lane_change=lane_change, v2x=v2x, traffic=traffic, obstacles=obstacles)
+        self.models = dict(metrics=metrics, agent_model=agent_model, lane_change=lane_change, v2x=v2x, traffic=traffic, obstacles=obstacles,
+                           split=split)
         self.h0, self.a0 = np.ascontiguousarray(hdr), np.ascontiguousarray(agents)
         sizes = {"hdr": n * 128, "agents": n * mo * 32, "ox": n * mo * 8, "oy": n * mo * 8, "prev_rec": n * 128}
         if metrics is not None:
@@ -533,6 +573,8 @@ class Episode:
             sizes["v2x_traffic"] = n * abi.v2x_traffic_stats.itemsize
         if obstacles is not None:
             sizes.update(v2x_hdr_view=n * 128, v2x_ox_view=n * mo * 8, v2x_oy_view=n * mo * 8, v2x_obstacles=n * abi.v2x_obstacle_stats.itemsize)
+        if split is not None:
+            sizes.update(split_rows=n * abi.split_row.itemsize, split_groups=n // split.group * abi.split_group.itemsize)
         self.sizes, self.d = sizes, {}
         self.k, self._cap = 0, {}                   # the next cycle of the episode; allocated part buffers: key -> (bytes, address)
         try:
@@ -555,6 +597,8 @@ class Episode:
                 planner.set_v2x_traffic(traffic, self.d["v2x_traffic"])
             if obstacles is not None:
                 planner.set_v2x_obstacles(obstacles, self.d["v2x_hdr_view"], self.d["v2x_ox_view"], self.d["v2x_oy_view"], self.d["v2x_obstacles"])
+            if split is not None:
+                planner.set_split(split, n, self.d["split_rows"], self.d["split_groups"])
             self.restart()
         except BaseException:
             self.close()
@@ -619,6 +663,12 @@ class Episode:
         self.p.world_fork_dev(self.n, src, dst, d["hdr"], d["agents"], d["ox"], d["oy"], d["prev_rec"])
         _ck(self.lib.dp_stream_sync(self.p.ctx, None), "sync")
 
+    def split(self, level):
+        """split the populations between two parts (dp_world_split_dev): level = the index of this split in the episode, from 0"""
+        d = self.d
+        self.p.world_split_dev(self.n, level, d["hdr"], d["agents"], d["ox"], d["oy"], d["prev_rec"])
+        _ck(self.lib.dp_stream_sync(self.p.ctx, None), "sync")
+
     def state(self):
         """run_closed_loop's dictionary without the records and the logs: the world, the rows and states of the armed models, the
         carry and the carried path, and whether the last part ran as a graph"""
@@ -634,6 +684,8 @@ class Episode:
             o["v2x_traffic"] = np.zeros(n, abi.v2x_traffic_stats)
         if m["obstacles"] is not None:
             o["v2x_obstacles"] = np.zeros(n, abi.v2x_obstacle_stats)
+        if m["split"] is not None:
+            o["split_rows"], o["split_groups"] = np.zeros(n, abi.split_row), np.zeros(n // m["split"].group, abi.split_group)
         for k in o:
             self._d2h(o[k], self.d[k], self.sizes[k])
         _ck(self.lib.dp_stream_sync(self.p.ctx, None), "sync")
@@ -647,6 +699,8 @@ class Episode:
         if not p.ctx or self.d is None:
             return
         try:
+            if m["split"] is not None:
+                p.set_split(None, 0, None, None)
             if m["obstacles"] is not None:
                 p.set_v2x_obstacles(None, None, None, None, None)
             if m["traffic"] is not None:

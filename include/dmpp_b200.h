@@ -930,9 +930,68 @@ int dp_run_closed_loop_part_dev(dp_ctx* ctx, int first_scene, int n_scenes, int 
  * nothing; forks of more than 4096 worlds take one kernel per 4096.  Stream-ordered on `stream`: the caller orders it after the
  * part that wrote the sources.  Perturbing a copy (v0, dp_agent.v) is the caller's.
  * DP_ERR_ARG for a source outside [0, n) or inside [dst, dst + count), dst < 0 or dst + count > n, first_scene + n > max_scenes,
- * n above the armed V2X specifications, or prev_rec NULL while section 16 is armed; DP_ERR_STATE while predicted tracks are set. */
+ * n above the armed V2X specifications, or prev_rec NULL while section 16 is armed; DP_ERR_STATE while predicted tracks are set,
+ * or when the armed per-world buffers exceed the copy's segment table (DP_FORK_MAX_SEG = 16). */
 int dp_world_fork_dev(dp_ctx* ctx, int first_scene, int n_scenes, const int32_t* src, int dst, int count, dp_scene_hdr* hdr, dp_agent* agents,
                       double* obs_x, double* obs_y, dp_plan_record* prev_rec, void* stream);
+
+/* (18) Splitting worlds between parts (opt-in): the genealogical particle method (Del Moral & Garnier 2005) that estimates the
+ * probability of a rare ego collision.  Between two parts of section 17, each POPULATION of M worlds is tilted towards the worlds
+ * closest to a collision, resampled with weights (the chosen worlds are forked over the dropped ones, on the device) and every world
+ * gets fresh speed noise.  The score is the metrics row of section 11, which must be armed.  The rules are frozen in
+ * tools/junction_oracle/world_split.h.  With the model disarmed (the default) nothing changes anywhere.
+ *
+ * IEEE binary64, operations in the order written, no contraction.  World i = g * M + j (relative to first_scene) is world j of
+ * population g; a call splits n / M populations at `level` (the index of the split within the episode, 0 for the first).
+ *   keys      mix = the SplitMix64 finaliser (z ^= z >> 30; z *= 0xbf58476d1ce4e5b9; z ^= z >> 27; z *= 0x94d049bb133111eb;
+ *             z ^= z >> 31), key(a, b) = mix(mix(mix(mix(seed) ^ level) ^ a) ^ b), u01(h) = (h >> 11) * 2^-53;
+ *             population g: a = 2^63 | g, b = 0; world i, agent k, field f: a = i, b = 2k + f
+ *   spec_exp  k = rint(x * (1 / ln 2)), r = fma(-k, ln2_hi, x), r = fma(-k, ln2_lo, r), the degree-13 Taylor polynomial of e^r in
+ *             Horner form with fma, times 2^k; spec_exp(0) == 1 exactly, within 2 ulp of exp on [-50, 50]
+ *   init      level 0 first sets every row to v_prev = -c_max, lw = 1, root = j and every population row to norm = 1,
+ *             levels = copies = 0, roots_alive = M
+ *   score     c = metrics.min_clearance, V = -(c < c_max ? c : c_max) (never decreases along an episode; 0 with an agent in the box)
+ *   potential w_j = spec_exp(beta * (V_j - v_prev_j))
+ *   resample  C_j = C_{j-1} + w_j (C_{-1} = 0, j in order), W = C_{M-1}, u = u01(key(2^63 | g, 0)),
+ *             A_j = min(M, max(0, ceil((M * C_j) / W - u))) for j < M - 1, A_{M-1} = M, A_{-1} = 0; N_j = A_j - A_{j-1}
+ *             (sum N_j = M, E[N_j] = M w_j / W)
+ *   lineage   every world: lw *= w, v_prev = V; the population: norm *= W / M, levels += 1 (before the copy: copies inherit it)
+ *   assign    a world with N_j >= 1 keeps its slot; the N_j - 1 extra copies of j (j in increasing order) go to the worlds with
+ *             N = 0 (in increasing index), paired in order: map[dst] = src, -1 elsewhere; copies += sum (N_j - 1)+, roots_alive =
+ *             the distinct roots after the copy
+ *   copy      each destination becomes a byte copy of its source in every buffer dp_world_fork_dev copies, its split row included
+ *   perturb   after the copy, every world i, agents k < min(hdr.n_obs, max_obs): f = 1.0 + amp * (2.0 * u01(key(i, 2k + field)) - 1.0);
+ *             dp_agent.v *= f (field 0, amp_v); v0 *= f (field 1, amp_v0) while the reactive agents of section 12 are armed
+ * With beta = 0 every w = 1 and N = 1: no copies, norm = lw = 1, and the call only perturbs (the Monte-Carlo baseline); with beta = 0
+ * and both amplitudes 0 it changes nothing but the split rows.  Estimator of P(ego collision within the episode), population g:
+ *   p_g = norm_g * (1 / M) * sum_j [first_collision_step_j >= 0] / lw_j */
+typedef struct dp_split_params {
+    int32_t group;                   /* M: worlds per population, 1 .. 1024 */
+    int32_t pad;                     /* zero */
+    double beta;                     /* tilt per metre of clearance, >= 0, beta * c_max <= 50; 0 = plain Monte Carlo (default 0.5) */
+    double c_max;                    /* clearance cap, metres, > 0; default 10 */
+    double amp_v;                    /* agent speed noise, [0, 1); default 0.1 */
+    double amp_v0;                   /* desired-speed noise with the reactive agents armed, [0, 1); default 0 */
+    uint64_t seed;                   /* default 0 */
+} dp_split_params;                   /* 48 bytes */
+typedef struct dp_split_row { double v_prev, lw; int32_t root, pad; } dp_split_row;                      /* per world, 24 bytes */
+typedef struct dp_split_group { double norm; int32_t levels, copies, roots_alive, pad; } dp_split_group; /* per population, 24 bytes */
+void dp_split_default_params(dp_split_params* p);
+/* rows[n] (indexed like hdr), groups[n / M] (population g of a call): device arrays; rows == NULL disarms (everything else may then
+ * be NULL).  Arming allocates the context's map[n].  While armed, dp_world_fork_dev copies the split rows too.  DP_ERR_ARG for M
+ * outside 1 .. 1024, n < 0 or not a multiple of M, non-finite parameters, beta < 0, c_max <= 0, beta * c_max > 50, amplitudes
+ * outside [0, 1), or groups NULL. */
+int dp_world_set_split(dp_ctx* ctx, const dp_split_params* p, int n, dp_split_row* rows, dp_split_group* groups);
+/* one split of worlds 0 .. n-1 (relative to first_scene) at `level`, three launches on `stream` (select -> copy -> perturb), ordered
+ * after the part that wrote the worlds; hdr / agents / obs_x / obs_y / prev_rec as dp_world_fork_dev takes them.  DP_ERR_STATE when
+ * the model or the metrics are disarmed, predicted tracks are set, or the armed models' per-world buffers would exceed the copy's
+ * segment table (DP_FORK_MAX_SEG = 16: every model of sections 11-18 armed fills it); DP_ERR_ARG for n not a multiple of M, n above the armed rows,
+ * level < 0, first_scene + n > max_scenes, n above the armed V2X specifications, or prev_rec NULL while section 16 is armed. */
+int dp_world_split_dev(dp_ctx* ctx, int first_scene, int n_scenes, int level, dp_scene_hdr* hdr, dp_agent* agents, double* obs_x,
+                       double* obs_y, dp_plan_record* prev_rec, void* stream);
+/* the map of the last split (host_map[n], n <= the armed rows): the source of every destination world, -1 elsewhere.  Copied on
+ * `stream` (pass the split's stream, so that the copy follows its select launch) and synchronised with it before returning */
+int dp_world_split_map(dp_ctx* ctx, int n, int32_t* host_map, void* stream);
 
 /* diagnostic: phase time stamps (globaltimer, ns) of the most recent cycle launch, one row of 32 per CTA (row b = scenes
  * [b*g, (b+1)*g) of the batch; stamp 0 = CTA start, stamp i = end of phase i of csrc/dp_group.cuh).  Only contexts created

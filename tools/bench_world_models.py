@@ -612,9 +612,157 @@ def bench_parts():
     return out
 
 
+def split_worlds(kind, n, seeds=None, everything=True):
+    """an Episode of n worlds with every model armed (metrics only with everything False) and splitting armed"""
+    seeds = np.arange(n) if seeds is None else seeds
+    w = scenes.World(m, seeds, 10, kind=kind, max_obs=14)
+    kw = dict(metrics=pl.metrics_params(), agent_model=(pl.agent_model_params(), w.v0), lane_change=pl.lane_change_params())
+    if everything:
+        kw.update(v2x=(abi.V2xWorldParams(0, 1), scenes.V2xEvents(w, seeds)), traffic=pl.v2x_traffic_params(), obstacles=pl.v2x_obstacle_params())
+    return w, kw
+
+
+def split_cost(kind, n, M):
+    """dp_world_split_dev alone after 10 cycles, every model armed.  Every split of the ladder and every timed split is a level-0
+    split (the rows start afresh) on the metrics rows of cycle 10, restored before each call: a copy overwrites the metrics row of
+    its destination, so without the restore later calls would resample ever fewer distinct worlds.  (beta, c_max) is the rung of
+    the ladder whose copied fraction is closest to one half; the copied fraction of every timed call is recorded"""
+    p = Planner(n, 14); p.upload_map(m)
+    wp = p.world_params(); wp.pre_junction_pts = scenes.World.PRE_JUNCTION_PTS[kind]; p.set_world_params(wp)
+    w, kw = split_worlds(kind, n)
+    ep = p.episode(w.hdr, w.agents, split=pl.split_params(group=M), **kw)
+    st = torch.cuda.current_stream()
+    d = ep.d
+    try:
+        ep.run(10, log=False)
+        met0 = ep.state()["metrics"]
+
+        def restore():
+            ep._h2d("metrics", met0); p.lib.dp_stream_sync(p.ctx, None)
+
+        frac = {}
+        for c_max in (10.0, 50.0):
+            for beta in (0.1, 0.25, 0.5, 1.0, 2.0, 5.0):
+                if beta * c_max > 50:
+                    continue
+                restore()
+                p.set_split(pl.split_params(group=M, beta=beta, c_max=c_max), n, d["split_rows"], d["split_groups"])
+                ep.split(0)
+                frac["beta=%g,c_max=%g" % (beta, c_max)] = (beta, c_max, float((p.split_map(n) >= 0).mean()))
+        rung = min(frac, key=lambda k: abs(frac[k][2] - 0.5))
+        beta, c_max, _ = frac[rung]
+        p.set_split(pl.split_params(group=M, beta=beta, c_max=c_max), n, d["split_rows"], d["split_groups"])
+
+        def one_split():
+            """device time of one split: the stream is held by a spin so that the three launches queue up behind the first event"""
+            restore()
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            torch.cuda._sleep(2_000_000)
+            e0.record(st)
+            p.world_split_dev(n, 0, d["hdr"], d["agents"], d["ox"], d["oy"], d["prev_rec"], stream=st.cuda_stream)
+            e1.record(st); torch.cuda.synchronize()
+            copied.append(float((p.split_map(n) >= 0).mean()))
+            return e0.elapsed_time(e1) * 1e3
+        copied = []
+        one_split(); one_split()
+        copied = []
+        xs = [one_split() for _ in range(REPS * ROUNDS)]
+    finally:
+        ep.close(); p.close()
+    return {"kind": kind, "worlds": n, "group": M, "every_model_armed": True, "level": 0, "beta": beta, "c_max": c_max,
+            "copied_fraction_by_rung": {k: v[2] for k, v in frac.items()},
+            "copied_fraction_of_timed_splits": summary(copied), "split_us": summary(xs)}
+
+
+def split_overhead():
+    """4096 junction worlds x 120 cycles as 12 x 10 parts, a split at each of the 11 seams (beta = 0, no noise) against none"""
+    N, kind, cycles, every = 4096, "junction", 120, 10
+    p = Planner(N, 14); p.upload_map(m)
+    wp = p.world_params(); wp.pre_junction_pts = scenes.World.PRE_JUNCTION_PTS[kind]; p.set_world_params(wp)
+    w, kw = split_worlds(kind, N)
+    ep = p.episode(w.hdr, w.agents, split=pl.split_params(group=256, beta=0.0, amp_v=0.0), **kw)
+    st = torch.cuda.current_stream()
+    d = ep.d
+    ring = torch.empty(every * N * 128, dtype=torch.uint8, device=dev)
+
+    def episode_ms(splits):
+        ep.restart()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record(st)
+        prev = None
+        for k0 in range(0, cycles, every):
+            p.run_closed_loop_part_dev(N, k0, every, k0 + every == cycles, d["hdr"], d["agents"], d["ox"], d["oy"], ring.data_ptr(), prev,
+                                       stream=st.cuda_stream)
+            prev = ring.data_ptr() + (every - 1) * N * 128  # (the ring's last row: read by the next part before its cycles overwrite it)
+            if splits and k0 + every < cycles:
+                p.world_split_dev(N, k0 // every, d["hdr"], d["agents"], d["ox"], d["oy"], prev, stream=st.cuda_stream)
+        e1.record(st); torch.cuda.synchronize()
+        return e0.elapsed_time(e1)
+    try:
+        arms = {"no_split": False, "split": True}
+        finals = {}
+        for k, v in arms.items():
+            episode_ms(v); episode_ms(v)
+            finals[k] = {x: y for x, y in ep.state().items() if x not in ("graph", "split_rows", "split_groups", "ox", "oy", "lane_change_state")}
+        res = {k: [] for k in arms}
+        for r in range(ROUNDS):
+            for k in (list(arms) if r % 2 == 0 else list(arms)[::-1]):
+                res[k] += [episode_ms(arms[k]) for _ in range(REPS)]
+    finally:
+        ep.close(); p.close()
+    same = all(finals["split"][k].tobytes() == finals["no_split"][k].tobytes() for k in finals["split"])
+    r = ratio(res["split"], res["no_split"])
+    return {"worlds": N, "cycles": cycles, "parts": "12x10", "splits": 11, "every_model_armed": True,
+            "ms_per_episode": {k: summary(v) for k, v in res.items()}, "split_over_no_split": r, "target": 1.03,
+            "target_met": bool(r <= 1.03), "final_states_identical": same}
+
+
+def split_effect(max_sources=32):
+    """junction sources among seeds 0-511 that do not collide in 120 cycles (metrics, reactive agents, lane changes); per source 16
+    populations of 256 copies, amp_v = 0.1, a split every 10 cycles, beta = 0 against beta = 0.3 at the same budget"""
+    kind, cycles, every, P, M, beta = "junction", 120, 10, 16, 256, 0.3
+    p = Planner(P * M, 14); p.upload_map(m)
+    wp = p.world_params(); wp.pre_junction_pts = scenes.World.PRE_JUNCTION_PTS[kind]; p.set_world_params(wp)
+    w, kw = split_worlds(kind, 512, everything=False)
+    one = p.run_closed_loop(w.hdr, w.agents, cycles, log=False, **kw)
+    quiet = np.nonzero(one["metrics"]["first_collision_step"] < 0)[0]
+    rows = []
+    try:
+        for s in quiet[:max_sources]:
+            wc, kwc = split_worlds(kind, P * M, seeds=np.full(P * M, s), everything=False)
+            row = {"seed": int(s)}
+            for name, b in (("beta0", 0.0), ("beta%g" % beta, beta)):
+                ep = p.episode(wc.hdr, wc.agents, split=pl.split_params(group=M, beta=b, amp_v=0.1, seed=int(s)), **kwc)
+                try:
+                    for k0 in range(0, cycles, every):
+                        ep.run(every, finish=k0 + every == cycles, log=False)
+                        if k0 + every < cycles:
+                            ep.split(k0 // every)
+                    stt = ep.state()
+                finally:
+                    ep.close()
+                g = pl.split_estimate(stt)
+                row[name] = {"p": float(g.mean()), "se": float(g.std(ddof=1) / np.sqrt(P)),
+                             "raw_collision_fraction": float((stt["metrics"]["first_collision_step"] >= 0).mean()),
+                             "roots_alive_mean": float(stt["split_groups"]["roots_alive"].mean())}
+            rows.append(row)
+    finally:
+        p.close()
+    bname = "beta%g" % beta
+    return {"sources_checked": 512, "non_colliding_sources": int(quiet.size), "sources_run": len(rows), "populations": P, "group": M,
+            "amp_v": 0.1, "split_every": every, "cycles": cycles, "beta": beta,
+            "sources_with_p_gt_0": {"beta0": sum(r["beta0"]["p"] > 0 for r in rows), bname: sum(r[bname]["p"] > 0 for r in rows)},
+            "per_source": rows}
+
+
+def bench_split():
+    return {"card": card(), "split_4096_junction": split_cost("junction", 4096, 256), "split_131072_highway": split_cost("highway", 131072, 256),
+            "targets_us": {"4096": 20, "131072": 400}, "episode_overhead": split_overhead(), "effect": split_effect()}
+
+
 if __name__ == "__main__":
     benches = {"metrics": bench_metrics, "agents": bench_agents, "lane_change": bench_lane_change, "v2x": bench_v2x, "traffic": bench_traffic,
-               "obstacles": bench_obstacles, "parts": bench_parts}
+               "obstacles": bench_obstacles, "parts": bench_parts, "split": bench_split}
     ap = argparse.ArgumentParser(description=__doc__.split("\n")[0])
     ap.add_argument("model", choices=list(benches))
     print(json.dumps(benches[ap.parse_args().model]()))

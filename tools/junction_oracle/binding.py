@@ -177,6 +177,31 @@ class JunctionOracle:
         o["status"] = rc
         return o
 
+    def split_select(self, sp, level, met, rows, groups):
+        """the select launch of a split (jo_world_split_select) for the populations of met[n]: rows[n] / groups[n / M] in place;
+        returns map[n] (the source of every destination, -1 elsewhere)"""
+        n = len(met)
+        out = np.zeros(n, np.int32)
+        assert self.lib.jo_world_split_select(C.byref(sp), C.c_int(n), C.c_int(level), abi.ptr(met), abi.ptr(rows), abi.ptr(groups),
+                                              abi.ptr(out)) == 0
+        return out
+
+    def perturb(self, sp, level, hdr, agents, v0=None):
+        """the perturb launch of a split (jo_world_perturb): agents[n][max_obs] and v0 (when given) in place"""
+        n, max_obs = agents.shape
+        assert v0 is None or (v0.shape == agents.shape and v0.dtype == np.float64 and v0.flags["C_CONTIGUOUS"])
+        assert self.lib.jo_world_perturb(C.byref(sp), C.c_int(n), C.c_int(level), C.c_int(max_obs), abi.ptr(hdr), abi.ptr(agents),
+                                         abi.ptr(v0)) == 0
+
+    def spec_exp(self, x):
+        x = np.ascontiguousarray(x, np.float64)
+        y = np.zeros_like(x)
+        assert self.lib.jo_spec_exp(C.c_int(x.size), abi.ptr(x), abi.ptr(y)) == 0
+        return y
+
+    def split_sizeof(self, which):
+        return self.lib.jo_split_sizeof(C.c_int(which))
+
     def v2x_obstacles_view(self, op, ev, hdr, ox, oy, k, stats, prev=None, tally=False, view=None):
         """one obstacles launch of cycle k for every world (jo_v2x_obstacles_view): stats in place; returns the view (hdr, ox, oy),
         built into `view` when given (slots beyond the view's n_obs keep what they held), fresh zero arrays otherwise"""

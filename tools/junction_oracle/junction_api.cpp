@@ -18,6 +18,7 @@
 #include "v2x_traffic.h"
 #include "v2x_world.h"
 #include "world_junction.h"
+#include "world_split.h"
 #include "../../oracle/cshare_spec.h"
 
 namespace {
@@ -340,5 +341,37 @@ int jo_v2x_obstacles_view(const dp_v2x_obstacle_params* op, int max_obs, int n, 
 int jo_v2x_obstacles_sizeof(int which) { return which ? (int)sizeof(dp_v2x_obstacle_stats) : (int)sizeof(dp_v2x_obstacle_params); }
 
 int jo_traffic_sizeof(int which) { return which ? (int)sizeof(dp_v2x_traffic_stats) : (int)sizeof(dp_v2x_traffic_params); }
+
+// the select launch of a split (include/dmpp_b200.h section 18) for the n / M populations of worlds 0 .. n-1: met[n], rows[n] and
+// groups[n / M] in place, map[n] the source of every destination (relative to world 0), -1 elsewhere
+int jo_world_split_select(const dp_split_params* p, int n, int level, const dp_episode_metrics* met, dp_split_row* rows,
+                          dp_split_group* groups, int32_t* map) {
+    const int M = p->group;
+    if (M < 1 || M > 1024 || n < 0 || n % M != 0 || level < 0) return -1;
+    for (int g = 0; g < n / M; ++g) {
+        const size_t o = (size_t)g * M;
+        split::select(*p, M, g, level, met + o, rows + o, groups[g], map + o);
+        for (int j = 0; j < M; ++j)
+            if (map[o + j] >= 0) map[o + j] += (int32_t)o;
+    }
+    return 0;
+}
+
+// the perturb launch of a split: every world i < n, agents[n][max_obs] and (nullable) v0[n][max_obs] in place
+int jo_world_perturb(const dp_split_params* p, int n, int level, int max_obs, const dp_scene_hdr* hdr, dp_agent* agents, double* v0) {
+    for (int i = 0; i < n; ++i)
+        split::perturb(*p, level, i, hdr[i].n_obs, max_obs, agents + (size_t)i * max_obs, v0 ? v0 + (size_t)i * max_obs : nullptr);
+    return 0;
+}
+
+// y[i] = spec_exp(x[i])
+int jo_spec_exp(int n, const double* x, double* y) {
+    for (int i = 0; i < n; ++i) y[i] = split::spec_exp(x[i]);
+    return 0;
+}
+
+int jo_split_sizeof(int which) {
+    return which == 0 ? (int)sizeof(dp_split_params) : which == 1 ? (int)sizeof(dp_split_row) : (int)sizeof(dp_split_group);
+}
 
 }  // extern "C"
